@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- DDPM samples/sec of the 1000-step reverse-diffusion loop on the CIFAR-shape U-Net (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is ONE reverse-diffusion step of the hot path over one batch: the whole U-Net evaluation (every launch of
@@ -24,6 +24,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 CFG2 = dict(dim=128, dim_mults=[1, 2, 2, 2], channels=3, groups=8)
@@ -258,7 +259,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-library-bar", action="store_true")
     ap.add_argument("--dump-ops", default="", help="write the per-launch table of one step (name, ms, TFLOP/s, GB/s) to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the state the timed loop returns after its last step to DIR/final.npy (float32; all ranks' samples "
+                         "when --gpus > 1; every n-th sample if it would exceed 64 MB).  Inputs are seeded, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -284,31 +290,36 @@ def main():
     coef, times = sampler._loop_tables(ts, dev)
     shape = [B, 3, IMAGE, IMAGE]
     lib = L.lib()
+    plan = unet.plan(IMAGE, B, dev, time_rows=int(times.shape[0]))    # the plan run_native_loop uses
 
-    # time a K-step prefix of the T-step schedule (same kernels, same shapes, same graph as the full run)
+    # time K steps of the T-step schedule (same kernels, same shapes, same graph as the full run); K > T runs in chunks of at most T
+    # steps, each continuing from the previous chunk's state, so K is the number of timed steps whatever its value
     def timed(n_steps):
         torch.cuda.synchronize(dev)
         if ws > 1:
             dist.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        res = R.run_native_loop(unet, kind=L.LOOP_DDPM, shape=shape, device=dev, times=times, coef=coef, seed=1234, use_graph=True,
-                                n_steps=n_steps)
+        res, done, launches = None, 0, 0
+        while done < n_steps:
+            k = min(n_steps - done, T)
+            res = R.run_native_loop(unet, kind=L.LOOP_DDPM, shape=shape, device=dev, times=times, coef=coef, seed=1234, use_graph=True,
+                                    x_init=None if res is None else res.final, n_steps=k)
+            launches += plan.last_loop_launches
+            done += k
         e1.record()
         torch.cuda.synchronize(dev)
-        return e0.elapsed_time(e1), res
+        return e0.elapsed_time(e1), res, launches
 
     clk = ClockSampler(local)                # started before the warm-up: nvidia-smi takes a while to deliver its first sample
     clk.start()
-    _, res_w = timed(args.warmup)            # builds the plan, uploads weights, captures the graph, warms clocks
+    _, res_w, _ = timed(args.warmup)         # uploads weights, captures the graph, warms clocks
     if ws > 1:
         D.all_gather_samples(res_w.final, total=B * ws)   # warm-up: creates the NCCL communicator outside the timed region
         torch.cuda.synchronize(dev)
-    plan = unet.plan(IMAGE, B, dev)
     clk.mark_begin()
-    ms_total, res = timed(args.steps)
+    ms_total, res, loop_launches = timed(args.steps)      # loop_launches: kernels launched inside the timed region (per step x K)
     clocks = clk.stop()
-    loop_launches = getattr(plan, "last_loop_launches", 0)      # kernels launched inside the timed region (launches per step x K)
     # the single collective of the job: all-gather of the final samples (timed once, amortised over T steps)
     ag_ms = 0.0
     gather_check = None
@@ -329,6 +340,11 @@ def main():
         dist.all_reduce(okt, op=dist.ReduceOp.MIN)
         gather_check = bool(okt.item())
         assert gather_check, "all-gather content check failed"
+    if args.dump_outputs and rank == 0:
+        final = (full if ws > 1 else res.final).float().cpu().numpy()
+        stride = -(-final.nbytes // (64 << 20))          # keep every stride-th sample: at most 64 MB
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "final.npy"), np.ascontiguousarray(final[::stride]))
     ms_step = ms_total / args.steps + ag_ms / T
     if ws > 1:
         tmax = torch.tensor([ms_step], device=dev)
