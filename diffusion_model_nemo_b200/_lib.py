@@ -39,6 +39,25 @@ class LoopDesc(C.Structure):
     ]
 
 
+SDE_VP, SDE_VE = 0, 1
+ODE_RUNNING, ODE_DONE, ODE_TOO_SMALL_STEP, ODE_LIMIT = 0, 1, -1, -2
+
+
+class OdeResult(C.Structure):
+    _fields_ = [("status", C.c_int32), ("nfev", C.c_int32), ("n_accepted", C.c_int32), ("n_rejected", C.c_int32),
+                ("t_final", C.c_double)]
+
+
+class OdeDesc(C.Structure):
+    _fields_ = [
+        ("sde_kind", C.c_int32), ("N", C.c_int32), ("beta_0", C.c_double), ("beta_1", C.c_double), ("sigma_min", C.c_double),
+        ("sigma_max", C.c_double), ("t0", C.c_double), ("t1", C.c_double), ("rtol", C.c_double), ("atol", C.c_double),
+        ("max_nfe", C.c_int32), ("batch", C.c_int32), ("use_graph", C.c_int32), ("reserved", C.c_int32),
+        ("classes_dev", C.c_void_p), ("state_dev", C.c_void_p), ("state_elems", C.c_int64), ("work_dev", C.c_void_p),
+        ("work_bytes", C.c_size_t), ("result_dev", C.c_void_p),
+    ]
+
+
 class ConvArgs(C.Structure):
     _fields_ = [
         ("mode", C.c_int32), ("ksize", C.c_int32), ("batch", C.c_int32), ("cin", C.c_int32), ("cout", C.c_int32),
@@ -96,6 +115,8 @@ SYMBOLS = {
     "dmn_axpby": (_I, [_P, _P, _F, _F, _P, _L, _P]),
     "dmn_sample_loop": (_I, [_P, C.POINTER(LoopDesc), _P]),
     "dmn_loop_launches_per_step": (_I, [_P, C.POINTER(LoopDesc)]),
+    "dmn_ode_sample": (_I, [_P, C.POINTER(OdeDesc), _P]),
+    "dmn_ode_work_bytes": (C.c_size_t, [_P, _I]),
     "dmn_conv_forward": (_I, [C.POINTER(ConvArgs), _P]),
     "dmn_conv_scratch_bytes": (C.c_size_t, [C.POINTER(ConvArgs)]),
     "dmn_linear_attention_core": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, C.c_size_t, _P]),

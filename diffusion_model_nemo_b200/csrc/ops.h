@@ -7,6 +7,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/dmn_b200.h"
+
 namespace dmn {
 
 typedef long long stat_t;   // fixed-point GroupNorm statistics (common.cuh)
@@ -174,5 +176,43 @@ int class_embed_add(void* x, const float* cls_w, const int64_t* classes, int pad
 int nchw_to_nhwc(const float* in, void* out, int B, int C, int HW, int act, cudaStream_t s);
 int nhwc_to_nchw(const void* in, float* out, int B, int C, int HW, int act, cudaStream_t s);
 int stats_to_mean_rstd(const stat_t* stats, float* out, int n, float inv_count, cudaStream_t s);
+
+// ---- probability-flow ODE, device-side RK45 (ode.cu) ----
+// solver constants of one solve (baked into the cached graph)
+struct OdeParams {
+  int sde_kind = 0, N = 0, max_nfe = 0;
+  double beta_0 = 0, beta_1 = 0, sigma_min = 0, sigma_max = 0;
+  double t0 = 0, t1 = 0, rtol = 0, atol = 0;
+};
+// solver record in device memory; the controller owns it between attempts
+struct OdeRec {
+  double t, t_new, h, h_abs, min_step;
+  double h0, d1;                         // select_initial_step carry
+  int cur;                               // y[cur] = y, y[cur ^ 1] = y_new
+  int k0, k6;                            // physical K slots of the FSAL pair (swapped on accept)
+  int rejected;                          // a rejection happened in the current step (growth capped at 1)
+  int status, nfev, n_acc, n_rej;
+  float labels[6], fx[6], sc[6], g2[6];  // per stage of an attempt: U-Net time label, f(x,t) = fx * x, score scale, g(t)^2
+};
+// views into the caller's work buffer
+struct OdeWork {
+  long n = 0;                            // batch * C * H * W
+  OdeRec* rec = nullptr;
+  int32_t* rows = nullptr;               // {0..5}: time-table row of each stage (row_dev of the U-Net forwards)
+  double* y = nullptr;                   // [2][n]
+  float* K = nullptr;                    // [7][n]
+  float* x32 = nullptr;                  // [n] U-Net input
+  float* mo = nullptr;                   // [n] U-Net output
+  double* partials = nullptr;            // [ode_grid(n)][2]
+  dmn_ode_result* result = nullptr;
+};
+size_t ode_work_layout(long n, char* base, OdeWork* w);    // bytes; fills w when given
+int ode_grid(long n);
+int launch_ode_init(const OdeWork& w, const OdeParams& P, cudaStream_t st);
+int launch_ode_init_elem(const OdeWork& w, const OdeParams& P, const float* state, int mode, cudaStream_t st);
+int launch_ode_init_step(const OdeWork& w, const OdeParams& P, int mode, cudaGraphConditionalHandle hnd, int use_cond, cudaStream_t st);
+int launch_ode_stage(const OdeWork& w, const OdeParams& P, int s, cudaStream_t st);
+int launch_ode_control(const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd, int use_cond, cudaStream_t st);
+int launch_ode_finish(const OdeWork& w, float* state, cudaStream_t st);
 
 }  // namespace dmn

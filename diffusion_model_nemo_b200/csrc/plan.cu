@@ -16,6 +16,8 @@
 //   conv 1x1 (to_out)             : + bias (+ statistics of GroupNorm(1) | + residual for the bottleneck Attention)
 //   gn_finalize                   : GroupNorm(1) + residual
 //   concat                        : never materialised (two-source operand load)
+#include <cfloat>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <map>
@@ -169,10 +171,20 @@ struct dmn_plan {
     dmn_loop_desc key;
   };
   std::vector<GraphEntry> graphs;
-  ~dmn_plan() {
+  struct OdeGraphEntry {
+    cudaGraphExec_t exec = nullptr;
+    dmn_ode_desc key;
+  };
+  std::vector<OdeGraphEntry> ode_graphs;
+  void drop_graphs() {
     for (auto& g : graphs)
       if (g.exec) cudaGraphExecDestroy(g.exec);
+    graphs.clear();
+    for (auto& g : ode_graphs)
+      if (g.exec) cudaGraphExecDestroy(g.exec);
+    ode_graphs.clear();
   }
+  ~dmn_plan() { drop_graphs(); }
 };
 
 namespace dmn {
@@ -841,9 +853,7 @@ int dmn_plan_bind(dmn_plan* p, void* weights_dev, size_t weights_bytes, void* wo
   DMN_REQUIRE(((uintptr_t)weights_dev % 256) == 0 && ((uintptr_t)workspace_dev % 256) == 0, "device buffers must be 256-byte aligned");
   p->wbase = (char*)weights_dev;
   p->wsbase = (char*)workspace_dev;
-  for (auto& g : p->graphs)
-    if (g.exec) cudaGraphExecDestroy(g.exec);
-  p->graphs.clear();
+  p->drop_graphs();
   return 0;
 }
 
@@ -1345,6 +1355,174 @@ int dmn_loop_launches_per_step(const dmn_plan* p, const dmn_loop_desc* d) {
   } else n = per_fwd + 1 + (d->cfg_on ? 2 : 0);
   if (d->traj_dev && d->traj_every > 0) n += 1;
   return n + 1;   // + advance_counter
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------------
+// probability-flow ODE driver (kernels: ode.cu)
+// ---------------------------------------------------------------------------------------------------------
+// One RK45 attempt: the input of stage 1, the 6 stage rows of the time table, then per stage the U-Net and the stage kernel,
+// then the controller (accept / reject, next step, WHILE condition).
+static int enqueue_ode_attempt(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd,
+                               int use_cond, cudaStream_t st) {
+  int rc;
+  if ((rc = launch_ode_stage(w, P, 0, st))) return rc;
+  if ((rc = dmn_time_table(p, w.rec->labels, 0, 6, st))) return rc;
+  for (int s = 1; s <= 6; ++s) {
+    if ((rc = run_forward(p, w.x32, w.rows + (s - 1), d->classes_dev, w.mo, d->batch, st))) return rc;
+    if ((rc = launch_ode_stage(w, P, s, st))) return rc;
+  }
+  return launch_ode_control(w, P, hnd, use_cond, st);
+}
+
+// init phase: y0, f0 = f(t0, y0), select_initial_step (one more evaluation), first attempt's stage rows
+static int enqueue_ode_init(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd,
+                            int use_cond, cudaStream_t st) {
+  int rc;
+  if ((rc = launch_ode_init(w, P, st))) return rc;
+  if ((rc = launch_ode_init_elem(w, P, d->state_dev, 0, st))) return rc;
+  for (int k = 0; k < 2; ++k) {
+    if ((rc = dmn_time_table(p, w.rec->labels, 0, 6, st))) return rc;
+    if ((rc = run_forward(p, w.x32, w.rows, d->classes_dev, w.mo, d->batch, st))) return rc;
+    if ((rc = launch_ode_init_elem(w, P, nullptr, k == 0 ? 1 : 3, st))) return rc;
+    if ((rc = launch_ode_init_step(w, P, k, hnd, use_cond && k == 1, st))) return rc;
+    if (k == 0 && (rc = launch_ode_init_elem(w, P, nullptr, 2, st))) return rc;
+  }
+  return 0;
+}
+
+// the graph bakes in every pointer and scalar of the descriptor
+static bool same_ode_key(const dmn_ode_desc& a, const dmn_ode_desc& b) {
+  return a.sde_kind == b.sde_kind && a.N == b.N && a.beta_0 == b.beta_0 && a.beta_1 == b.beta_1 && a.sigma_min == b.sigma_min &&
+         a.sigma_max == b.sigma_max && a.t0 == b.t0 && a.t1 == b.t1 && a.rtol == b.rtol && a.atol == b.atol && a.max_nfe == b.max_nfe &&
+         a.batch == b.batch && a.classes_dev == b.classes_dev && a.state_dev == b.state_dev && a.work_dev == b.work_dev &&
+         a.result_dev == b.result_dev;
+}
+
+static int build_ode_graph(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w, const OdeParams& P, cudaGraphExec_t* out) {
+  cudaStream_t cs, bs;
+  DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+  if (cudaStreamCreateWithFlags(&bs, cudaStreamNonBlocking) != cudaSuccess) {
+    cudaStreamDestroy(cs);
+    return fail(DMN_ECUDA, "ode graph: stream create");
+  }
+  int rc = 0;
+  const char* where = "begin capture";
+  cudaGraph_t graph = nullptr;
+  cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
+  bool capturing = e == cudaSuccess;
+  cudaGraphConditionalHandle hnd = 0;
+  if (capturing) {
+    cudaStreamCaptureStatus cst;
+    const cudaGraphNode_t* deps = nullptr;
+    size_t ndeps = 0;
+    where = "capture info";
+    e = cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps);
+    if (e == cudaSuccess) { where = "conditional handle"; e = cudaGraphConditionalHandleCreate(&hnd, graph, 0, cudaGraphCondAssignDefault); }
+    if (e == cudaSuccess) rc = enqueue_ode_init(p, d, w, P, hnd, 1, cs);
+    cudaGraph_t body = nullptr;
+    if (e == cudaSuccess && !rc) {
+      where = "while node";
+      e = cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps);
+      cudaGraphNodeParams np = {};
+      np.type = cudaGraphNodeTypeConditional;
+      np.conditional.handle = hnd;
+      np.conditional.type = cudaGraphCondTypeWhile;
+      np.conditional.size = 1;
+      cudaGraphNode_t node = nullptr;
+      if (e == cudaSuccess) e = cudaGraphAddNode(&node, graph, deps, ndeps, &np);
+      if (e == cudaSuccess) e = cudaStreamUpdateCaptureDependencies(cs, &node, 1, cudaStreamSetCaptureDependencies);
+      body = np.conditional.phGraph_out ? np.conditional.phGraph_out[0] : nullptr;
+      if (e == cudaSuccess) { where = "body capture"; e = cudaStreamBeginCaptureToGraph(bs, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal); }
+      if (e == cudaSuccess) {
+        rc = enqueue_ode_attempt(p, d, w, P, hnd, 1, bs);
+        cudaGraph_t bg = nullptr;
+        const cudaError_t e2 = cudaStreamEndCapture(bs, &bg);
+        if (!rc && e2 != cudaSuccess) { where = "body end capture"; e = e2; }
+      }
+    }
+    if (e == cudaSuccess && !rc) rc = launch_ode_finish(w, d->state_dev, cs);
+    cudaGraph_t g2 = nullptr;
+    const cudaError_t e3 = cudaStreamEndCapture(cs, &g2);
+    graph = g2;
+    if (e == cudaSuccess && !rc && e3 != cudaSuccess) { where = "end capture"; e = e3; }
+  }
+  cudaStreamDestroy(bs);
+  cudaStreamDestroy(cs);
+  if (!rc && e == cudaSuccess) { where = "instantiate"; e = cudaGraphInstantiate(out, graph, 0); }
+  if (graph) cudaGraphDestroy(graph);
+  cudaGetLastError();
+  if (rc) return rc;
+  if (e != cudaSuccess) return fail(DMN_ECUDA, std::string("ode graph (") + where + "): " + cudaGetErrorString(e));
+  return 0;
+}
+
+extern "C" {
+
+size_t dmn_ode_work_bytes(const dmn_plan* p, int batch) {
+  if (!p || batch < 1) return 0;
+  const dmn_unet_cfg& c = p->cfg;
+  return ode_work_layout((long)batch * c.channels * c.image_size * c.image_size, nullptr, nullptr);
+}
+
+int dmn_ode_sample(dmn_plan* p, const dmn_ode_desc* d, void* stream) {
+  if (!p) return fail(DMN_EINVAL, "null plan");
+  if (!d) return fail(DMN_EINVAL, "null descriptor");
+  const dmn_unet_cfg& c = p->cfg;
+  DMN_REQUIRE(d->sde_kind == DMN_SDE_VP || d->sde_kind == DMN_SDE_VE, "unknown SDE kind");
+  if (d->sde_kind == DMN_SDE_VP) DMN_REQUIRE(d->N >= 1 && std::isfinite(d->beta_0) && std::isfinite(d->beta_1), "VP-SDE needs N >= 1 and finite betas");
+  else DMN_REQUIRE(d->sigma_min > 0 && d->sigma_max > 0 && std::isfinite(d->sigma_min) && std::isfinite(d->sigma_max), "VE-SDE needs positive sigmas");
+  DMN_REQUIRE(std::isfinite(d->t0) && std::isfinite(d->t1) && d->t0 != d->t1, "t0 and t1 must be finite and different");
+  DMN_REQUIRE(std::isfinite(d->rtol) && d->rtol > 0 && std::isfinite(d->atol) && d->atol >= 0, "tolerances: rtol > 0, atol >= 0, finite");
+  DMN_REQUIRE(d->max_nfe >= 2, "max_nfe must be >= 2 (the initial step selection evaluates twice)");
+  DMN_REQUIRE(d->batch >= 1 && d->batch <= c.max_batch, "batch exceeds the plan's max_batch");
+  DMN_REQUIRE(d->state_dev && d->work_dev && d->result_dev, "null device pointer in ODE descriptor");
+  DMN_REQUIRE(((uintptr_t)d->work_dev % 256) == 0, "work buffer must be 256-byte aligned");
+  const long n = (long)d->batch * c.channels * c.image_size * c.image_size;
+  DMN_REQUIRE(d->state_elems == n, "state_dev does not hold batch * channels * image_size^2 floats for this plan");
+  DMN_REQUIRE(d->work_bytes >= dmn_ode_work_bytes(p, d->batch), "work buffer smaller than dmn_ode_work_bytes()");
+  DMN_REQUIRE(c.out_dim == c.channels && !c.film, "the ODE drift needs a U-Net with out_dim == channels (no FiLM)");
+  DMN_REQUIRE(c.max_time_rows >= 6, "the plan's time table needs >= 6 rows (one per stage of an attempt)");
+  int rc = check_ready(p);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  OdeParams P;
+  P.sde_kind = d->sde_kind; P.N = d->N; P.max_nfe = d->max_nfe;
+  P.beta_0 = d->beta_0; P.beta_1 = d->beta_1; P.sigma_min = d->sigma_min; P.sigma_max = d->sigma_max;
+  P.t0 = d->t0; P.t1 = d->t1; P.atol = d->atol;
+  P.rtol = d->rtol < 100 * DBL_EPSILON ? 100 * DBL_EPSILON : d->rtol;     // scipy validate_tol
+  OdeWork w;
+  ode_work_layout(n, (char*)d->work_dev, &w);
+  w.result = d->result_dev;
+  if (!d->use_graph) {
+    if ((rc = enqueue_ode_init(p, d, w, P, 0, 0, st))) return rc;
+    dmn_ode_result r;
+    for (long it = 0;; ++it) {
+      DMN_CUDA_CHECK(cudaMemcpyAsync(&r, d->result_dev, sizeof(r), cudaMemcpyDeviceToHost, st));
+      DMN_CUDA_CHECK(cudaStreamSynchronize(st));
+      if (r.status != DMN_ODE_RUNNING) break;
+      if (it > (long)d->max_nfe) return fail(DMN_ESTATE, "ODE controller did not stop within max_nfe");
+      if ((rc = enqueue_ode_attempt(p, d, w, P, 0, 0, st))) return rc;
+    }
+    return launch_ode_finish(w, d->state_dev, st);
+  }
+  cudaGraphExec_t exec = nullptr;
+  for (auto& g : p->ode_graphs)
+    if (same_ode_key(g.key, *d)) exec = g.exec;
+  if (!exec) {
+    if ((rc = build_ode_graph(p, d, w, P, &exec))) return rc;
+    if (p->ode_graphs.size() >= 4) {
+      cudaGraphExecDestroy(p->ode_graphs.front().exec);
+      p->ode_graphs.erase(p->ode_graphs.begin());
+    }
+    dmn_plan::OdeGraphEntry ge;
+    ge.exec = exec;
+    ge.key = *d;
+    p->ode_graphs.push_back(ge);
+  }
+  DMN_CUDA_CHECK(cudaGraphLaunch(exec, st));
+  return 0;
 }
 
 }  // extern "C"

@@ -14,7 +14,7 @@ _API = {
     "generalized_gaussian_diffusion": ("GeneralizedGaussianDiffusion",),
     "wavegrad_diffusion": ("WaveGradDiffusion",),
     "sde": (
-        "SDE", "VPSDE", "VESDE", "PredictorCorrectorSampler", "resolve_score_function",
+        "SDE", "VPSDE", "VESDE", "PredictorCorrectorSampler", "ProbabilityFlowSampler", "resolve_score_function",
         "Predictor", "NonePredictor", "EulerMaruyamaPredictor", "AncestralSamplingPredictor", "ReverseDiffusionPredictor",
         "register_predictor", "get_predictor",
         "Corrector", "NoneCorrector", "LangevinCorrector", "AnnealedLangevinDynamics", "register_corrector", "get_corrector",

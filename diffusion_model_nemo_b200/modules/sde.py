@@ -6,8 +6,13 @@ Every built-in predictor / corrector update is affine in (x, model output, z) on
 host folds the SDE algebra (discretisation, score wrapper `-model/std`, step sizes) into per-step coefficient rows
 computed with the reference's torch CPU ops, and the device runs ONE fused kernel per update
 (dmn_affine_noise_step / dmn_langevin_step).  With this package's Unet the whole N-step loop is a CUDA graph.
+
+ProbabilityFlowSampler (modules/sde_samplers/probability_flow_sampler.py) solves the probability-flow ODE with scipy's RK45
+rules on the device (dmn_ode_sample): the step control runs in device code, so the adaptive solve is one CUDA graph.
 """
 import abc
+import ctypes as C
+import warnings
 from typing import List, Optional
 
 import numpy as np
@@ -181,8 +186,10 @@ def _alpha(sde, t):
     return torch.ones_like(t)
 
 
-def predictor_rows(name: Optional[str], sde, sf: ScoreFunction, t: torch.Tensor):
-    """x_mean = a*x + b*model_out ; x = x_mean + g*z   -> columns (a, b, g) for the time vector t (CPU fp32)."""
+def predictor_rows(name: Optional[str], sde, sf: ScoreFunction, t: torch.Tensor, probability_flow: bool = False):
+    """x_mean = a*x + b*model_out ; x = x_mean + g*z   -> columns (a, b, g) for the time vector t (CPU fp32).
+    probability_flow=True is the reference's RSDE with the halved score term and no diffusion (sde_lib.py:91-105): g = 0, but the
+    update still takes its z, so the draw order is unchanged."""
     scale = sf.scale(t)
     if name in (None, "none", "null"):
         return [torch.ones_like(t), torch.zeros_like(t), torch.zeros_like(t)]
@@ -196,6 +203,8 @@ def predictor_rows(name: Optional[str], sde, sf: ScoreFunction, t: torch.Tensor)
             adj = torch.where(ts == 0, torch.zeros_like(t), sde.discrete_sigmas[ts - 1])
             G = torch.sqrt(sig ** 2 - adj ** 2)
             a = torch.ones_like(t)
+        if probability_flow:
+            return [a, G ** 2 * scale * 0.5, torch.zeros_like(t)]
         return [a, G ** 2 * scale, G]
     if name == "euler_maruyama":            # euler_maruyama_predictor.py:11-17 + sde_lib.py:91-98
         dt = -1.0 / sde.N
@@ -207,6 +216,8 @@ def predictor_rows(name: Optional[str], sde, sf: ScoreFunction, t: torch.Tensor)
             sigma = sde.sigma_min * (sde.sigma_max / sde.sigma_min) ** t
             diff = sigma * torch.sqrt(torch.tensor(2 * (np.log(sde.sigma_max) - np.log(sde.sigma_min))))
             a = torch.ones_like(t)
+        if probability_flow:
+            return [a, -(diff ** 2) * scale * 0.5 * dt, torch.zeros_like(t)]
         return [a, -(diff ** 2) * scale * dt, diff * np.sqrt(-dt)]
     raise NotImplementedError(f"predictor `{name}` has no native update (built: reverse_diffusion, euler_maruyama, none)")
 
@@ -279,14 +290,12 @@ class Predictor(abc.ABC):
 
     def __init__(self, sde, score_fn, probability_flow=False):
         super().__init__()
-        if probability_flow:
-            raise NotImplementedError("probability_flow=True is outside the built sampling path")
-        self.sde, self.score_fn = sde, score_fn
+        self.sde, self.score_fn, self.probability_flow = sde, score_fn, probability_flow
 
     def update_fn(self, x, t, noise=None):
         """(x, x_mean) after one predictor step; one model call + one fused kernel."""
         tc = _uniform(t)
-        rows = predictor_rows(self.native_name, self.sde, self.score_fn, tc)
+        rows = predictor_rows(self.native_name, self.sde, self.score_fn, tc, self.probability_flow)
         return _affine_update(x.float(), self.score_fn.raw(x, t), rows, noise)
 
     @classmethod
@@ -426,8 +435,6 @@ class PredictorCorrectorSampler(torch.nn.Module):
     def forward(self, model, shape: List[int], device, return_nfe: bool = True, use_tqdm: bool = True, noise=None):
         if self.sde is None:
             raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling forward()")
-        if self.probability_flow:
-            raise NotImplementedError("probability_flow=True is outside the built sampling path")
         R.require_cuda(device)
         sde = self.sde
         ts = self.timesteps()
@@ -436,10 +443,10 @@ class PredictorCorrectorSampler(torch.nn.Module):
         n_corr = self.n_steps if _NATIVE_CORRECTORS.get(self.corrector) else 0
         init_scale = float(sde.sigma_max) if isinstance(sde, VESDE) else 1.0
         if unet is not None and self._native_ok():
-            key = (str(device), self.predictor, self.corrector, float(self.snr), sde.N, self.eps)
+            key = (str(device), self.predictor, self.corrector, float(self.snr), sde.N, self.eps, bool(self.probability_flow))
             hit = self._cache.get(key)
             if hit is None:
-                coef = R.coef_rows(predictor_rows(_NATIVE_PREDICTORS[self.predictor], sde, sf, ts), device)
+                coef = R.coef_rows(predictor_rows(_NATIVE_PREDICTORS[self.predictor], sde, sf, ts, bool(self.probability_flow)), device)
                 kind, coef2 = 0, None
                 if n_corr:
                     kind, rows = corrector_rows(_NATIVE_CORRECTORS[self.corrector], sde, sf, ts, self.snr)
@@ -474,6 +481,124 @@ class PredictorCorrectorSampler(torch.nn.Module):
             imgs = R.to_image_list((x_mean if self.denoise else x).float().contiguous(), None)
         nfe = sde.N * (self.n_steps + 1)
         return (imgs, nfe) if return_nfe else imgs
+
+    def sample(self, model, shape: List[int], device=None, return_nfe: bool = False, noise=None):
+        if device is None:
+            device = next(model.parameters()).device
+        return self.forward(model=model, shape=shape, device=device, return_nfe=return_nfe, noise=noise)
+
+
+# ------------------------------------------------------------------------------------------------------
+# the probability-flow ODE sampler (reference modules/sde_samplers/probability_flow_sampler.py, score_sde get_ode_sampler)
+# ------------------------------------------------------------------------------------------------------
+
+
+class ProbabilityFlowSampler(torch.nn.Module):
+    """Deterministic sampler of a score-SDE model: integrates the probability-flow ODE dx/dt = f(x,t) - 0.5 g(t)^2 score(x,t) from
+    sde.T down to eps with scipy's adaptive RK45 rules (solve_ivp(..., method='RK45')), entirely on the GPU: every model
+    evaluation, the error norm, the accept / reject decision and the step-size update run in device code, and with
+    `use_cuda_graph` (default) the whole solve is one CUDA graph replay.  Needs this package's Unet (or a
+    functools.partial of it with `classes`); any other model callable raises NotImplementedError (there is no host solver).
+
+    Differences to the reference: eps=None uses sde.sampling_epsilon (the reference fails inside solve_ivp); a solve that would
+    need more than `max_nfe` model evaluations stops and raises RuntimeError; `last_stats` holds the solver counters of the last
+    call.  Step sizes are chosen per process: under torchrun every rank solves its own batch with its own steps."""
+
+    def __init__(self, denoise: bool = False, rtol: float = 1e-5, atol: float = 1e-5, method: str = "RK45", eps: float = None,
+                 max_nfe: int = 100_000):
+        super().__init__()
+        if method != "RK45":
+            raise NotImplementedError(f"method={method!r}: only the RK45 solver is built")
+        for name, v in (("rtol", rtol), ("atol", atol)):
+            if isinstance(v, bool) or not isinstance(v, (int, float, np.floating, np.integer)):
+                raise ValueError(f"{name} must be a scalar number (per-component tolerances are not supported), got {type(v).__name__}")
+            if not np.isfinite(v) or v < 0 or (name == "rtol" and v == 0):
+                raise ValueError(f"{name} must be finite and {'> 0' if name == 'rtol' else '>= 0'}, got {v}")
+        if isinstance(max_nfe, bool) or not isinstance(max_nfe, (int, np.integer)) or max_nfe < 2:
+            raise ValueError(f"max_nfe must be an integer >= 2, got {max_nfe!r}")
+        self.denoise, self.rtol, self.atol, self.method, self.eps = denoise, float(rtol), float(atol), method, eps
+        self.max_nfe = int(max_nfe)
+        self.sde: Optional[SDE] = None
+        self.use_cuda_graph = True
+        self.last_stats: Optional[dict] = None
+
+    def update_sde(self, sde: SDE):
+        self.sde = sde
+
+    def forward(self, model, shape: List[int], device, return_nfe: bool = True, use_tqdm: bool = True, noise=None):
+        if self.sde is None:
+            raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling forward()")
+        sde = self.sde
+        if not isinstance(sde, (VPSDE, VESDE)):
+            raise NotImplementedError(f"SDE class {sde.__class__.__name__} not yet supported.")
+        R.require_cuda(device)
+        device = torch.device(device)
+        unet, classes = R.resolve_model(model)
+        if unet is None:
+            raise NotImplementedError("ProbabilityFlowSampler runs this package's Unet natively; other model callables have no "
+                                      "host solver path")
+        b, c, h, w = (int(v) for v in shape)
+        if c != unet.channels or h != w:
+            raise ValueError(f"shape {list(shape)} does not fit the U-Net ({unet.channels} channels, square images)")
+        if unet.out_dim != unet.channels:
+            raise ValueError("the probability-flow drift needs a U-Net whose output has as many channels as its input")
+        eps = sde.sampling_epsilon if self.eps is None else float(self.eps)
+        init_scale = float(sde.sigma_max) if isinstance(sde, VESDE) else 1.0
+        x = noise[0] * init_scale if noise is not None else sde.prior_sampling(shape)
+        if tuple(x.shape) != (b, c, h, w):
+            raise ValueError(f"x_T has shape {tuple(x.shape)}; expected {(b, c, h, w)}")
+        lib = L.lib()
+        plan = unet.plan(h, b, device, time_rows=6)
+        with torch.cuda.device(device):
+            st = L.stream_ptr(device)
+            # buffers live with the plan so the addresses baked into the cached graph stay valid
+            bufs = plan.__dict__.setdefault("_ode_bufs", {})
+            if b not in bufs:
+                nbytes = int(lib.dmn_ode_work_bytes(plan.h, b))
+                bufs[b] = {"state": torch.empty((b, c, h, w), dtype=torch.float32, device=device),
+                           "work": torch.empty(nbytes + 256, dtype=torch.uint8, device=device),
+                           "result": torch.zeros(3, dtype=torch.float64, device=device)}
+            buf = bufs[b]
+            state, work, result = buf["state"], buf["work"], buf["result"]
+            state.copy_(x.to(device, torch.float32))
+            if classes is not None:
+                classes = classes.to(device, torch.int64).reshape(-1)
+                cb = buf.get("classes")
+                if cb is None or cb.shape != classes.shape:
+                    cb = buf["classes"] = torch.empty_like(classes)
+                cb.copy_(classes)
+                classes = cb
+            wp = (work.data_ptr() + 255) // 256 * 256
+            d = L.OdeDesc()
+            if isinstance(sde, VPSDE):
+                d.sde_kind, d.N, d.beta_0, d.beta_1 = L.SDE_VP, int(sde.N), float(sde.beta_0), float(sde.beta_1)
+            else:
+                d.sde_kind, d.N, d.sigma_min, d.sigma_max = L.SDE_VE, int(sde.N), float(sde.sigma_min), float(sde.sigma_max)
+            d.t0, d.t1, d.rtol, d.atol = float(sde.T), eps, self.rtol, self.atol
+            d.max_nfe, d.batch, d.use_graph = self.max_nfe, b, int(bool(self.use_cuda_graph))
+            d.classes_dev = classes.data_ptr() if classes is not None else None
+            d.state_dev, d.state_elems = state.data_ptr(), state.numel()
+            d.work_dev, d.work_bytes = wp, work.numel() - (wp - work.data_ptr())
+            d.result_dev = result.data_ptr()
+            L.check(lib.dmn_ode_sample(plan.h, C.byref(d), st), "dmn_ode_sample")
+            plan.time_rows_key = None            # the solve rewrote rows 0..5 of the time table
+            raw = result.cpu().numpy().tobytes()
+            x = state.clone()
+        res = L.OdeResult.from_buffer_copy(raw)
+        self.last_stats = {"status": int(res.status), "nfev": int(res.nfev), "n_accepted": int(res.n_accepted),
+                           "n_rejected": int(res.n_rejected), "t_final": float(res.t_final)}
+        if res.status == L.ODE_LIMIT:
+            raise RuntimeError(f"probability-flow ODE: stopped at {res.nfev} model evaluations (max_nfe={self.max_nfe}) at "
+                               f"t={res.t_final:.6g}, before reaching eps={eps:g}")
+        if res.status == L.ODE_TOO_SMALL_STEP:
+            warnings.warn(f"probability-flow ODE: required step size became too small at t={res.t_final:.6g} (scipy status -1); "
+                          "returning the last accepted state, as solve_ivp does")
+        if self.denoise:      # one reverse-diffusion predictor step at eps, probability_flow=False, keeping x_mean
+            vec_eps = torch.ones(b, device=device) * eps
+            pred = ReverseDiffusionPredictor(sde, ScoreFunction(model, sde), probability_flow=False)
+            _, x = pred.update_fn(x, vec_eps)
+        imgs = R.to_image_list(x.float().contiguous(), None)
+        return (imgs, int(res.nfev)) if return_nfe else imgs
 
     def sample(self, model, shape: List[int], device=None, return_nfe: bool = False, noise=None):
         if device is None:

@@ -240,6 +240,57 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream);
 int dmn_loop_launches_per_step(const dmn_plan* p, const dmn_loop_desc* d);
 
 /* ------------------------------------------------------------------------------------------------------
+ * Probability-flow ODE sampler.  Replaces ProbabilityFlowSampler.forward (sde_samplers/probability_flow_sampler.py:46-100,
+ * score_sde's get_ode_sampler): solve_ivp(ode_func, (t0, t1), x_T, rtol, atol, method='RK45') where ode_func is the drift of
+ * the reverse SDE with probability_flow=True, f(x,t) - 0.5 g(t)^2 score(x,t), over this plan's U-Net (score wrapper of
+ * score_function_loss.py:47-91: VP labels t*(N-1) and score = -model/std(t); VE labels sigma(t) and score = model).
+ * Every model evaluation, the error norm, the accept / reject decision and the step-size update run on the device with
+ * scipy.integrate.RK45's rules (Dormand-Prince 5(4), FSAL, select_initial_step, SAFETY 0.9, factors 0.2..10, exponent -1/5).
+ * use_graph = 1: one cached CUDA graph per (plan, descriptor): init phase, then a WHILE conditional node over attempts; the
+ * call enqueues and returns.  use_graph = 0: the same kernels with a host read of the status after every attempt (syncs).
+ * The solve stops at t1 (DMN_ODE_DONE), at a step below scipy's min_step (DMN_ODE_TOO_SMALL_STEP: the last accepted state is
+ * returned, as solve_ivp does) or before an attempt that would exceed max_nfe evaluations (DMN_ODE_LIMIT).
+ * The plan needs max_time_rows >= 6 (the 6 stage rows of an attempt), out_dim == channels and no FiLM.
+ * ---------------------------------------------------------------------------------------------------- */
+#define DMN_SDE_VP 0
+#define DMN_SDE_VE 1
+
+#define DMN_ODE_RUNNING         0
+#define DMN_ODE_DONE            1
+#define DMN_ODE_TOO_SMALL_STEP -1
+#define DMN_ODE_LIMIT          -2
+
+typedef struct dmn_ode_result {
+  int32_t status;          /* DMN_ODE_* */
+  int32_t nfev;            /* model evaluations (solution.nfev) */
+  int32_t n_accepted;
+  int32_t n_rejected;
+  double  t_final;         /* time of the returned state */
+} dmn_ode_result;
+
+typedef struct dmn_ode_desc {
+  int32_t sde_kind;        /* DMN_SDE_VP / DMN_SDE_VE */
+  int32_t N;               /* VP: label = t * (N - 1) */
+  double  beta_0, beta_1;  /* VP */
+  double  sigma_min, sigma_max;   /* VE */
+  double  t0, t1;          /* integration interval (sde.T -> eps); t0 != t1 */
+  double  rtol, atol;      /* scalar tolerances: rtol > 0 (raised to 100 * DBL_EPSILON like scipy), atol >= 0 */
+  int32_t max_nfe;         /* evaluation budget, >= 2 */
+  int32_t batch;
+  int32_t use_graph;
+  int32_t reserved;
+  const int64_t* classes_dev;     /* optional class labels [batch] */
+  float*   state_dev;      /* in: x_T (fp32 NCHW); out: the final state (fp32) */
+  int64_t  state_elems;    /* floats behind state_dev: batch * channels * image_size^2 */
+  void*    work_dev;       /* caller-owned, 256-byte aligned, >= dmn_ode_work_bytes(plan, batch) */
+  size_t   work_bytes;
+  dmn_ode_result* result_dev;     /* device record, valid once the stream has run the solve */
+} dmn_ode_desc;
+
+int    dmn_ode_sample(dmn_plan* p, const dmn_ode_desc* d, void* stream);
+size_t dmn_ode_work_bytes(const dmn_plan* p, int batch);
+
+/* ------------------------------------------------------------------------------------------------------
  * Layer-level entry points (unit tests and INTEGRATION.md's per-module swap).  Activations are fp32 NCHW at
  * this boundary; the call converts to the plan-independent engine layout (NHWC) internally, so they are for
  * validation, not speed.  `engine`/`act` as in the plan.
