@@ -155,17 +155,18 @@ __global__ void __launch_bounds__(256) affine_noise_kernel(const float* __restri
   }
 }
 
-// Langevin: per-sample sums of squares of g = scale*model_out and z  -> ssq[b][2]
+// Langevin: per-sample sums of squares of g = scale*model_out and z  -> ssq[b][2].  One block per sample adds its partials in a
+// fixed order and writes ssq[b] itself (no float atomics), so the step size -- and the whole loop -- is bit-reproducible.
 __global__ void __launch_bounds__(256) langevin_sumsq_kernel(const float* __restrict__ mo, const float* __restrict__ z,
                                                              float* __restrict__ ssq, long chw4, const float* __restrict__ coef,
                                                              const int32_t* step_dev, int step, int draw, dmn_rng rng_v, const dmn_rng* rng_dev) {
   const dmn_rng rng = pick_rng(rng_v, rng_dev);
   __shared__ float red[2][8];
-  const int b = blockIdx.y;
+  const int b = blockIdx.x;
   const float scale = coef_row(coef, step_dev, step)[0];
   const uint32_t sw = step_word(step_dev, step, draw);
   float sg = 0.f, sz = 0.f;
-  for (long r = (long)blockIdx.x * blockDim.x + threadIdx.x; r < chw4; r += (long)gridDim.x * blockDim.x) {
+  for (long r = threadIdx.x; r < chw4; r += blockDim.x) {
     const long i = (long)b * chw4 + r;
     float4 g = reinterpret_cast<const float4*>(mo)[i];
     g.x *= scale; g.y *= scale; g.z *= scale; g.w *= scale;
@@ -181,8 +182,8 @@ __global__ void __launch_bounds__(256) langevin_sumsq_kernel(const float* __rest
   if (threadIdx.x == 0) {
     float a = 0.f, c = 0.f;
     for (int i = 0; i < 8; ++i) { a += red[0][i]; c += red[1][i]; }
-    atomicAdd(ssq + 2 * b, a);
-    atomicAdd(ssq + 2 * b + 1, c);
+    ssq[2 * b] = a;
+    ssq[2 * b + 1] = c;
   }
 }
 // batch means of the per-sample norms  -> means[0] = mean ||g_b||, means[1] = mean ||z_b||
@@ -508,11 +509,7 @@ int launch_langevin(const float* x, const float* mo, const float* z, float* out,
   DMN_REQUIRE(chw % 4 == 0, "langevin: C*H*W must be a multiple of 4");
   float* ssq = scratch;                 // [batch][2]
   float* means = scratch + 2 * batch;   // [2]
-  DMN_CUDA_CHECK(cudaMemsetAsync(ssq, 0, sizeof(float) * 2 * batch, st));
-  count_launch();
-  int bps = (int)((chw / 4 + 255) / 256);
-  if (bps > 8) bps = 8;
-  langevin_sumsq_kernel<<<dim3(bps, batch), 256, 0, st>>>(mo, z, ssq, chw / 4, coef, step_dev, step, draw, rng, rng_dev);
+  langevin_sumsq_kernel<<<batch, 256, 0, st>>>(mo, z, ssq, chw / 4, coef, step_dev, step, draw, rng, rng_dev);
   count_launch();
   DMN_LAUNCH_CHECK("langevin_sumsq");
   langevin_means_kernel<<<1, 32, 0, st>>>(ssq, means, batch);

@@ -157,7 +157,8 @@ int dmn_ddim_step(const float* x, const float* eps, const float* z_dev, float* x
 int dmn_affine_noise_step(const float* x, const float* model_out, const float* z_dev, float* x_out, float* x_mean_out,
                           int64_t n, const float* coef_dev, const int32_t* step_dev, int step, dmn_rng rng, void* stream);
 /* LangevinCorrector.update_fn (langevin_corrector.py:15-35), two kernels:
- *   norms: per-sample ||g_b||, ||z_b|| -> batch means (scratch_dev: 2 floats, zeroed by the call)
+ *   norms: per-sample ||g_b||, ||z_b|| -> batch means (scratch_dev: 2*batch + 2 floats; one block per sample, fixed summation
+ *          order, so the result is bit-reproducible)
  *   apply: step = (snr*mean||z|| / mean||g||)^2 * 2*alpha ; x_mean = x + step*g ; x = x_mean + sqrt(2 step) z
  * where g = score_scale * model_out (VP: -1/std(t), VE: 1).  coef row: {score_scale, alpha}.
  * z_dev == NULL draws z in-kernel (the same Philox counters in both kernels). */

@@ -66,6 +66,14 @@ def test_config4_score_sde_pc_32x32(kind):
     pc.seed = 3
     out = pc.sample(u, [2, 3, 32, 32], device=DEV)[-1]
     assert out.shape == (2, 3, 32, 32) and torch.isfinite(out).all()
+    # seeded mode at the benchmark batch: the Langevin step size depends on batch-mean norms, which are summed in a fixed order,
+    # so two graph runs and a plain-launch run give the same bits
+    shape = [256, 3, 32, 32]
+    a = pc.sample(u, shape, device=DEV)[-1]
+    b = pc.sample(u, shape, device=DEV)[-1]
+    pc.use_cuda_graph = False
+    c = pc.sample(u, shape, device=DEV)[-1]
+    assert torch.isfinite(a).all() and torch.equal(a, b) and torch.equal(a, c)
 
 
 def test_config2_full_batch_properties():
