@@ -11,7 +11,7 @@ LIB_PATH = os.environ.get("DMN_LIB_PATH") or os.path.join(_HERE, "libdmn_b200.so
 
 ACT_F32, ACT_BF16 = 0, 1
 CONV_SIMT, CONV_TCGEN05 = 0, 1
-LOOP_DDPM, LOOP_LEARNED, LOOP_DDIM, LOOP_PC, LOOP_BPD = 0, 1, 2, 3, 4
+LOOP_DDPM, LOOP_LEARNED, LOOP_DDIM, LOOP_PC, LOOP_BPD, LOOP_DPMPP = 0, 1, 2, 3, 4, 5
 COEF_STRIDE = 8
 
 
@@ -106,6 +106,7 @@ SYMBOLS = {
     "dmn_ddpm_step": (_I, [_P, _P, _P, _P, _L, _P, _P, _I, Rng, _P]),
     "dmn_learned_step": (_I, [_P, _P, _P, _P, _I, _L, _P, _P, _I, Rng, _P]),
     "dmn_ddim_step": (_I, [_P, _P, _P, _P, _L, _P, _P, _I, Rng, _P]),
+    "dmn_dpmpp_step": (_I, [_P, _P, _P, _P, _I, _L, _L, _P, _P, _I, _P]),
     "dmn_affine_noise_step": (_I, [_P, _P, _P, _P, _P, _L, _P, _P, _I, Rng, _P]),
     "dmn_langevin_step": (_I, [_P, _P, _P, _P, _P, _I, _L, _F, _P, _P, _I, _P, Rng, _P]),
     "dmn_bpd_qsample": (_I, [_P, _P, _P, _L, _P, _P, _I, Rng, _P]),

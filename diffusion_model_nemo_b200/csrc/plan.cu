@@ -54,6 +54,8 @@ int launch_learned(const float* x, const float* mo, const float* z, float* out, 
                    const int32_t* step_dev, int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
 int launch_ddim(const float* x, const float* eps, const float* z, float* out, long n, const float* coef, const int32_t* step_dev,
                 int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
+int launch_dpmpp(const float* x, const float* mo, float* hist, float* out, int batch, long chw, long mo_chw, const float* coef,
+                 const int32_t* step_dev, int step, cudaStream_t st);
 bool fused_tail_supported(const FinalProjP& p, int act);
 int launch_final_proj_ddpm(const FinalProjP& p, const float* x, const float* z, float* out, const float* coef, const int32_t* step_dev,
                            int step, dmn_rng rng, const dmn_rng* rng_dev, int32_t* advance, cudaStream_t st);
@@ -1175,6 +1177,13 @@ int dmn_plan_profile_forward_graph(dmn_plan* p, const float* x_dev, const int32_
 // ---------------------------------------------------------------------------------------------------------
 // loop driver
 // ---------------------------------------------------------------------------------------------------------
+// DMN_LOOP_DPMPP's history ring: 3*n floats behind the scratch every other kind uses (layout documented in dmn_loop_desc)
+static size_t dpmpp_ring_offset(const dmn_loop_desc* d, long n, long n_out) {
+  const long base = d->cfg_on ? 3 * n_out + 3 * n + 2 * d->batch + 36 : n_out + n + 2 * d->batch + 16;
+  return (size_t)((base + 3) & ~3L);
+}
+static float* dpmpp_ring(const dmn_loop_desc* d, long n, long n_out) { return d->scratch_dev + dpmpp_ring_offset(d, n, n_out); }
+
 // One loop step.  `ctr` = device step counter (graph mode) or nullptr with host step `s` (injected-noise mode);
 // `z0` = this step's injected noise block (draws x n floats) or nullptr for in-kernel Philox with device rng state.
 static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, int32_t* ctr_dev, bool use_ctr, int s, const float* z0,
@@ -1241,8 +1250,11 @@ static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, int32_t* ctr_dev, b
       rc = launch_ddpm(d->state_dev, mo, z0, d->state_dev, n, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
     else if (d->kind == DMN_LOOP_LEARNED)
       rc = launch_learned(d->state_dev, mo, z0, d->state_dev, d->batch, chw, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
-    else
+    else if (d->kind == DMN_LOOP_DDIM)
       rc = launch_ddim(d->state_dev, mo, z0, d->state_dev, n, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
+    else
+      rc = launch_dpmpp(d->state_dev, mo, dpmpp_ring(d, n, n_out), d->state_dev, d->batch, chw, n_out / d->batch, d->coef_dev, step_dev,
+                        s, st);
     if (rc) return rc;
   }
   if (d->traj_dev && d->traj_every > 0)
@@ -1266,7 +1278,7 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
   if (rc) return rc;
   if (!d) return fail(DMN_EINVAL, "null descriptor");
   const dmn_unet_cfg& c = p->cfg;
-  DMN_REQUIRE(d->kind >= DMN_LOOP_DDPM && d->kind <= DMN_LOOP_BPD, "unknown loop kind");
+  DMN_REQUIRE(d->kind >= DMN_LOOP_DDPM && d->kind <= DMN_LOOP_DPMPP, "unknown loop kind");
   DMN_REQUIRE(d->kind != DMN_LOOP_BPD || (d->aux_dev && d->coef2_dev && !d->cfg_on && !d->traj_dev),
               "BPD loop needs the terms buffer (aux_dev) and the second coefficient table; no guidance / trajectory");
   DMN_REQUIRE(d->batch >= 1 && d->batch <= c.max_batch, "batch exceeds the plan's max_batch");
@@ -1276,6 +1288,8 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
   DMN_REQUIRE(d->n_corr >= 0 && d->n_corr <= 6, "n_corr out of range (0..6)");
   if (d->kind == DMN_LOOP_LEARNED) DMN_REQUIRE(c.out_dim == 2 * c.channels, "learned-variance loop needs a U-Net with 2*channels outputs");
   else if (d->kind == DMN_LOOP_BPD) DMN_REQUIRE(c.out_dim == c.channels || c.out_dim == 2 * c.channels, "BPD: out_dim must be C or 2C");
+  else if (d->kind == DMN_LOOP_DPMPP)
+    DMN_REQUIRE(c.out_dim == c.channels || c.out_dim == 2 * c.channels, "DPM-Solver++: out_dim must be C or 2C");
   else DMN_REQUIRE(c.out_dim == c.channels, "U-Net out_dim must equal channels for this sampler");
   const long chw = (long)c.channels * c.image_size * c.image_size;
   const long n = (long)d->batch * chw;
@@ -1283,12 +1297,15 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
   DMN_REQUIRE(d->scratch_bytes >= (size_t)(n_out + n + 2 * d->batch + 16) * sizeof(float), "loop scratch too small");
   DMN_REQUIRE(d->state_elems == 0 || d->state_elems == n, "state_dev does not hold batch * channels * image_size^2 floats for this plan");
   if (d->cfg_on) {
-    DMN_REQUIRE(d->kind != DMN_LOOP_PC, "classifier-free guidance is built for the DDPM / learned / DDIM loops");
+    DMN_REQUIRE(d->kind != DMN_LOOP_PC, "classifier-free guidance is built for the DDPM / learned / DDIM / DPM-Solver++ loops");
     DMN_REQUIRE(c.num_classes >= 0 && d->classes_dev, "classifier-free guidance needs a class-conditional U-Net and 2*batch labels");
     DMN_REQUIRE(2 * d->batch <= c.max_batch, "classifier-free guidance doubles the batch: plan max_batch too small");
     DMN_REQUIRE(d->scratch_bytes >= (size_t)(3 * n_out + 3 * n + 2 * d->batch + 36) * sizeof(float), "loop scratch too small for guidance");
     DMN_REQUIRE(n % 4 == 0 && n_out % 4 == 0, "guidance kernels need 16-byte multiples");
   }
+  if (d->kind == DMN_LOOP_DPMPP)
+    DMN_REQUIRE(d->scratch_bytes >= (dpmpp_ring_offset(d, n, n_out) + 3 * (size_t)n) * sizeof(float),
+                "loop scratch too small for the DPM-Solver++ history ring");
   cudaStream_t st = (cudaStream_t)stream;
   int32_t* ctr = (int32_t*)(p->wsbase + p->counters.off);
   float* xmean = d->scratch_dev + n_out;
@@ -1296,7 +1313,7 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
 
   if (d->noise_dev) {
     // parity mode: injected noise => per-step pointers differ, plain launches with the host step index
-    const int draws = (d->kind == DMN_LOOP_PC) ? d->n_corr + 1 : 1;
+    const int draws = (d->kind == DMN_LOOP_PC) ? d->n_corr + 1 : (d->kind == DMN_LOOP_DPMPP ? 0 : 1);
     for (int s = 0; s < d->n_steps; ++s)
       if ((rc = enqueue_step(p, d, ctr, false, s, d->noise_dev + (long)s * draws * n, st))) return rc;
   } else if (!d->use_graph) {
@@ -1352,7 +1369,7 @@ int dmn_loop_launches_per_step(const dmn_plan* p, const dmn_loop_desc* d) {
   else if (d->kind == DMN_LOOP_DDPM && !d->cfg_on && tail_fusable(p)) {
     // fused tail: the update (and, without trajectory capture, the counter) ride on the last launch of the forward program
     return (d->traj_dev && d->traj_every > 0) ? per_fwd + 2 : per_fwd;
-  } else n = per_fwd + 1 + (d->cfg_on ? 2 : 0);
+  } else n = per_fwd + 1 + (d->cfg_on ? 2 : 0);   // one update kernel: DDPM (unfused), learned, DDIM, DPM-Solver++
   if (d->traj_dev && d->traj_every > 0) n += 1;
   return n + 1;   // + advance_counter
 }

@@ -135,6 +135,41 @@ __global__ void __launch_bounds__(256) ddim_step_kernel(const float* __restrict_
   }
 }
 
+// DPM-Solver++ multistep (Lu et al. 2022): the update is affine in (x, m_i, m_{i-1}, m_{i-2}), m = clamped data prediction.
+// row: {c_x, c_0, c_1, c_2, k_x, k_m, slot, pred_x0}.  hist is a 3-slot ring [3][n]: slot = i mod 3 receives m_i, (slot+2)%3 holds
+// m_{i-1} and (slot+1)%3 holds m_{i-2}.  A slot whose coefficient is 0 is never read (the ring starts as uninitialised scratch).
+// The model output has `mo_chw4` float4 per sample (C or 2C channels); only the first chw4 of them are used.
+__global__ void __launch_bounds__(256) dpmpp_step_kernel(const float* x, const float* __restrict__ mo, float* __restrict__ hist,
+                                                         float* out, long chw4, long mo_chw4, long n4, const float* __restrict__ coef,
+                                                         const int32_t* step_dev, int step) {
+  const float* c = coef_row(coef, step_dev, step);
+  const float cx = c[0], c0 = c[1], c1 = c[2], c2 = c[3], kx = c[4], km = c[5];
+  const int slot = (int)c[6];
+  const bool pred_x0 = c[7] != 0.f;
+  float4* h_cur = reinterpret_cast<float4*>(hist) + (long)slot * n4;
+  const float4* h_m1 = reinterpret_cast<const float4*>(hist) + (long)((slot + 2) % 3) * n4;
+  const float4* h_m2 = reinterpret_cast<const float4*>(hist) + (long)((slot + 1) % 3) * n4;
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
+    const long mi = mo_chw4 == chw4 ? i : (i / chw4) * mo_chw4 + i % chw4;
+    const float4 xv = reinterpret_cast<const float4*>(x)[i];
+    const float4 ev = reinterpret_cast<const float4*>(mo)[mi];
+    float4 m, o;
+#define DMN_DPM_M(f) m.f = clamp1(pred_x0 ? ev.f : (kx * xv.f - km * ev.f)); o.f = cx * xv.f + c0 * m.f;
+    DMN_DPM_M(x) DMN_DPM_M(y) DMN_DPM_M(z) DMN_DPM_M(w)
+#undef DMN_DPM_M
+    if (c1 != 0.f) {
+      const float4 h = h_m1[i];
+      o.x += c1 * h.x; o.y += c1 * h.y; o.z += c1 * h.z; o.w += c1 * h.w;
+    }
+    if (c2 != 0.f) {
+      const float4 h = h_m2[i];
+      o.x += c2 * h.x; o.y += c2 * h.y; o.z += c2 * h.z; o.w += c2 * h.w;
+    }
+    h_cur[i] = m;
+    reinterpret_cast<float4*>(out)[i] = o;
+  }
+}
+
 __global__ void __launch_bounds__(256) affine_noise_kernel(const float* __restrict__ x, const float* __restrict__ mo,
                                                            const float* __restrict__ z, float* __restrict__ out,
                                                            float* __restrict__ mean_out, long n4, const float* __restrict__ coef,
@@ -593,6 +628,17 @@ int launch_ddim(const float* x, const float* eps, const float* z, float* out, lo
   DMN_LAUNCH_CHECK("ddim_step");
   return 0;
 }
+int launch_dpmpp(const float* x, const float* mo, float* hist, float* out, int batch, long chw, long mo_chw, const float* coef,
+                 const int32_t* step_dev, int step, cudaStream_t st) {
+  DMN_REQUIRE(batch > 0 && chw > 0 && chw % 4 == 0 && mo_chw >= chw && mo_chw % 4 == 0,
+              "dpmpp_step: C*H*W must be a positive multiple of 4 and the model output at least C*H*W per sample");
+  DMN_REQUIRE(x && mo && hist && out && coef, "dpmpp_step: null pointer");
+  const long n4 = (long)batch * chw / 4;
+  dpmpp_step_kernel<<<grid_for(n4), 256, 0, st>>>(x, mo, hist, out, chw / 4, mo_chw / 4, n4, coef, step_dev, step);
+  count_launch();
+  DMN_LAUNCH_CHECK("dpmpp_step");
+  return 0;
+}
 
 }  // namespace dmn
 
@@ -613,6 +659,11 @@ int dmn_learned_step(const float* x, const float* model_out, const float* z_dev,
 int dmn_ddim_step(const float* x, const float* eps, const float* z_dev, float* x_out, int64_t n, const float* coef_dev,
                   const int32_t* step_dev, int step, dmn_rng rng, void* stream) {
   return launch_ddim(x, eps, z_dev, x_out, n, coef_dev, step_dev, step, rng, nullptr, (cudaStream_t)stream);
+}
+
+int dmn_dpmpp_step(const float* x, const float* model_out, float* hist, float* x_out, int batch, int64_t chw, int64_t mo_chw,
+                   const float* coef_dev, const int32_t* step_dev, int step, void* stream) {
+  return launch_dpmpp(x, model_out, hist, x_out, batch, chw, mo_chw, coef_dev, step_dev, step, (cudaStream_t)stream);
 }
 
 int dmn_affine_noise_step(const float* x, const float* model_out, const float* z_dev, float* x_out, float* x_mean_out, int64_t n,

@@ -12,6 +12,7 @@ _API = {
     "gaussian_diffusion": ("GaussianDiffusion",),
     "learned_gaussian_diffusion": ("LearnedGaussianDiffusion",),
     "generalized_gaussian_diffusion": ("GeneralizedGaussianDiffusion",),
+    "dpm_solver_diffusion": ("DPMSolverDiffusion",),
     "wavegrad_diffusion": ("WaveGradDiffusion",),
     "sde": (
         "SDE", "VPSDE", "VESDE", "PredictorCorrectorSampler", "ProbabilityFlowSampler", "resolve_score_function",

@@ -74,8 +74,8 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
                     seed: Optional[int] = None, traj_every: int = 0, use_graph: bool = True,
                     init_scale: float = 1.0, n_steps: Optional[int] = None, cfg_scale: Optional[float] = None) -> LoopResult:
     """Run n_steps of (U-Net + update) natively.  noise: [1 + n_steps*draws, B, C, H, W] injected N(0,1) tensors in
-    the reference's draw order (element 0 = x_T), or None for in-kernel Philox.  cfg_scale: classifier-free guidance weight
-    (None = off; 0.0 is a valid weight and gives the unconditional prediction)."""
+    the reference's draw order (element 0 = x_T), or None for in-kernel Philox; LOOP_DPMPP draws nothing and uses only noise[0].
+    cfg_scale: classifier-free guidance weight (None = off; 0.0 is a valid weight and gives the unconditional prediction)."""
     lib = L.lib()
     device = torch.device(device)
     require_cuda(device)
@@ -93,10 +93,10 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
         if unet.num_classes is None or classes is None:
             raise ValueError("classifier-free guidance needs a class-conditional Unet and `classes` labels")
         if kind == L.LOOP_PC:
-            raise NotImplementedError("classifier-free guidance is built for the DDPM / learned-variance / DDIM loops")
+            raise NotImplementedError("classifier-free guidance is built for the DDPM / learned-variance / DDIM / DPM-Solver++ loops")
     plan = unet.plan(h, 2 * b if guided else b, device, time_rows=int(times.shape[0]))
     n = b * c * h * w
-    draws = (n_corr + 1) if kind == L.LOOP_PC else 1
+    draws = (n_corr + 1) if kind == L.LOOP_PC else (0 if kind == L.LOOP_DPMPP else 1)
     with torch.cuda.device(device):
         st = L.stream_ptr(device)
         tkey = (times.data_ptr(), int(times.shape[0]), tuple(times[:: max(1, int(times.shape[0]) // 7)].tolist()))
@@ -112,7 +112,9 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
         if bkey not in bufs:
             bufs[bkey] = {
                 "state": torch.empty((b, c, h, w), dtype=torch.float32, device=device),
-                "scratch": torch.empty((3 if guided else 1) * (n_out + n) + 2 * b + 64, dtype=torch.float32, device=device),
+                # + the DPM-Solver++ history ring (3 states) behind the common layout
+                "scratch": torch.empty((3 if guided else 1) * (n_out + n) + 2 * b + 64 + (3 * n if kind == L.LOOP_DPMPP else 0),
+                                       dtype=torch.float32, device=device),
                 "aux": (torch.empty((b, c, h, w), dtype=torch.float32, device=device) if (kind == L.LOOP_PC and denoise) else
                         torch.zeros((b, n_steps), dtype=torch.float32, device=device) if kind == L.LOOP_BPD else None),
                 "traj": torch.empty((n_traj, b, c, h, w), dtype=torch.float32, device=device) if n_traj > 0 else None,
@@ -129,7 +131,7 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
             L.check(lib.dmn_randn(L.ptr(state), n, rng, -1, st), "dmn_randn")
             if init_scale != 1.0:
                 state.mul_(init_scale)
-        if noise is not None:
+        if noise is not None and draws:
             need = n_steps * draws + (0 if x_init is not None else 1)
             assert noise.shape[0] >= need, f"need {need} injected noise tensors, got {noise.shape[0]}"
             nz = noise[(0 if x_init is not None else 1):]

@@ -8,6 +8,13 @@ from . import _runtime as R
 from .gaussian_diffusion import GaussianDiffusion, _default
 
 
+def strided_pairs(timesteps: int, steps: int):
+    """[(t, t_next)] in visiting order (reference :110-112,119): stride = timesteps // steps, the last t_next is -1."""
+    stride = timesteps // steps
+    seq = list(range(0, timesteps, stride))
+    return list(zip(reversed(seq), reversed([-1] + seq[:-1])))
+
+
 class GeneralizedGaussianDiffusion(GaussianDiffusion):
     _loop_kind = L.LOOP_DDIM
 
@@ -29,9 +36,7 @@ class GeneralizedGaussianDiffusion(GaussianDiffusion):
 
     def timestep_pairs(self):
         """[(t, t_next)] in visiting order (reference :110-112,119): stride = T // ddim_timesteps."""
-        stride = self.timesteps // self.ddim_timesteps
-        seq = list(range(0, self.timesteps, stride))
-        return list(zip(reversed(seq), reversed([-1] + seq[:-1])))
+        return strided_pairs(self.timesteps, self.ddim_timesteps)
 
     def _pair_rows(self, t: torch.Tensor, t_next: torch.Tensor):
         at = self.alphas_extended_cumprod[t + 1]

@@ -151,6 +151,16 @@ int dmn_learned_step(const float* x, const float* model_out, const float* z_dev,
  * coef row: {sqrt(1-a_t), 1/sqrt(a_t)... see modules/generalized_gaussian_diffusion.py in the package} */
 int dmn_ddim_step(const float* x, const float* eps, const float* z_dev, float* x_out, int64_t n,
                   const float* coef_dev, const int32_t* step_dev, int step, dmn_rng rng, void* stream);
+/* DPM-Solver++ multistep update, orders 1-3 (Lu et al. 2022, "DPM-Solver++", Algorithm 2 and its third-order extension; not in
+ * the reference: modules/dpm_solver_diffusion.py in the package builds the rows).  Deterministic: draws no noise.
+ *   m  = clamp(pred_x0 ? model_out : k_x * x - k_m * model_out, -1, 1)      (data prediction; first C channels of each sample)
+ *   x' = c_x * x + c_0 * m + c_1 * hist[(slot+2)%3] + c_2 * hist[(slot+1)%3] ;  hist[slot] = m
+ * coef row: {c_x, c_0, c_1, c_2, k_x, k_m, slot, pred_x0 ? 1 : 0}.  hist_dev is a ring of 3 slots [3][batch*chw] fp32 holding the
+ * previous steps' m (slot = step mod 3); a slot whose coefficient is 0 is not read, so the ring needs no initialisation.
+ * model_out is [batch, mo_chw] with mo_chw = C*H*W or 2*C*H*W (learned variance: the variance channels are ignored).
+ * x_out may alias x. */
+int dmn_dpmpp_step(const float* x, const float* model_out, float* hist_dev, float* x_out, int batch, int64_t chw, int64_t mo_chw,
+                   const float* coef_dev, const int32_t* step_dev, int step, void* stream);
 /* ReverseDiffusionPredictor / EulerMaruyamaPredictor with the score wrapper folded in
  * (reverse_diffusion_predictor.py:11-16, euler_maruyama_predictor.py:11-17, sde_lib.py:91-105,
  *  score_function_loss.py:47-91):  x_mean = a*x + b*model_out ; x = x_mean + g*z.  coef row: {a, b, g} */
@@ -201,6 +211,9 @@ int dmn_axpby(const float* x, const float* y, float a, float b, float* out, int6
                                  (AbstractDiffusionModel.calculate_bits_per_dimension, models/abstract_diffusion_model.py:137-197).
                                  state_dev = x_0 (read only), aux_dev = terms [batch][n_steps] (column = coef2 row[1]),
                                  coef_dev / coef2_dev rows as documented at dmn_bpd_term; noise_dev injects the q_sample draws */
+#define DMN_LOOP_DPMPP    5   /* DPM-Solver++ multistep: per step U-Net (or the guidance path) -> dmn_dpmpp_step; rows as documented
+                                 there, one per (t_i, t_{i+1}) pair.  out_dim = C or 2C.  Draws nothing: noise_dev, if given, only
+                                 selects plain launches with the host step index.  The history ring lives in scratch_dev (below). */
 
 typedef struct dmn_loop_desc {
   int32_t kind;            /* DMN_LOOP_* */
@@ -218,7 +231,10 @@ typedef struct dmn_loop_desc {
   dmn_rng        rng;            /* throughput mode */
   float*         state_dev;      /* in: x_T (fp32 NCHW); out: final state in [-1,1] space */
   float*         aux_dev;        /* PC: x_mean of the last step when denoise */
-  float*         scratch_dev;    /* >= 2*out_dim*S*S*batch floats + 64 bytes: model output, x_mean, counters */
+  float*         scratch_dev;    /* >= 2*out_dim*S*S*batch floats + 64 bytes: model output, x_mean, counters.
+                                    DMN_LOOP_DPMPP appends its history ring of 3*C*S*S*batch floats at float offset
+                                    R = round_up(base, 4), base = out_dim*S*S*batch + C*S*S*batch + 2*batch + 16 (guidance:
+                                    3*out_dim*S*S*batch + 3*C*S*S*batch + 2*batch + 36), so it needs R + 3*C*S*S*batch floats */
   size_t         scratch_bytes;
   float*         traj_dev;       /* optional [n_traj][batch*C*H*W] trajectory capture, every traj_every steps */
   int32_t        traj_every;
@@ -227,7 +243,8 @@ typedef struct dmn_loop_desc {
                                     evaluates the U-Net on the doubled batch [x ; x] with classes_dev[0..batch) = labels and
                                     classes_dev[batch..2*batch) = num_classes (the null / padding row, unet.py:118-120) and uses
                                     eps = eps_u + cfg_scale * (eps_c - eps_u).  Needs max_batch >= 2*batch and scratch for
-                                    3*out_dim*S*S*batch + 3*C*S*S*batch + 2*batch + 16 floats.  DDPM / learned / DDIM loops only.
+                                    3*out_dim*S*S*batch + 3*C*S*S*batch + 2*batch + 16 floats.  DDPM / learned / DDIM /
+                                    DPM-Solver++ loops only.
                                     With a learned-variance U-Net only the eps half is guided; the variance channels are the
                                     conditional branch's. */
   int32_t        cfg_on;         /* 1 = classifier-free guidance with weight cfg_scale, 0 = off */
