@@ -39,6 +39,10 @@ class LoopDesc(C.Structure):
     ]
 
 
+class InpaintDesc(C.Structure):
+    _fields_ = [("known_dev", C.c_void_p), ("mask_dev", C.c_void_p), ("prep_coef_dev", C.c_void_p)]
+
+
 SDE_VP, SDE_VE = 0, 1
 ODE_RUNNING, ODE_DONE, ODE_TOO_SMALL_STEP, ODE_LIMIT = 0, 1, -1, -2
 
@@ -116,6 +120,8 @@ SYMBOLS = {
     "dmn_axpby": (_I, [_P, _P, _F, _F, _P, _L, _P]),
     "dmn_sample_loop": (_I, [_P, C.POINTER(LoopDesc), _P]),
     "dmn_loop_launches_per_step": (_I, [_P, C.POINTER(LoopDesc)]),
+    "dmn_inpaint_prepare": (_I, [_P, _P, _P, _P, _L, _P, _P, _I, Rng, _P]),
+    "dmn_sample_loop_inpaint": (_I, [_P, C.POINTER(LoopDesc), C.POINTER(InpaintDesc), _P]),
     "dmn_ode_sample": (_I, [_P, C.POINTER(OdeDesc), _P]),
     "dmn_ode_work_bytes": (C.c_size_t, [_P, _I]),
     "dmn_conv_forward": (_I, [C.POINTER(ConvArgs), _P]),

@@ -56,6 +56,8 @@ int launch_ddim(const float* x, const float* eps, const float* z, float* out, lo
                 int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
 int launch_dpmpp(const float* x, const float* mo, float* hist, float* out, int batch, long chw, long mo_chw, const float* coef,
                  const int32_t* step_dev, int step, cudaStream_t st);
+int launch_inpaint_prepare(const float* x, const float* known, const float* mask, float* out, long n, const float* coef,
+                           const int32_t* step_dev, int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
 bool fused_tail_supported(const FinalProjP& p, int act);
 int launch_final_proj_ddpm(const FinalProjP& p, const float* x, const float* z, float* out, const float* coef, const int32_t* step_dev,
                            int step, dmn_rng rng, const dmn_rng* rng_dev, int32_t* advance, cudaStream_t st);
@@ -171,6 +173,7 @@ struct dmn_plan {
   struct GraphEntry {
     cudaGraphExec_t exec = nullptr;
     dmn_loop_desc key;
+    dmn_inpaint_desc ip{};   // all null for a plain sampling loop
   };
   std::vector<GraphEntry> graphs;
   struct OdeGraphEntry {
@@ -1186,8 +1189,9 @@ static float* dpmpp_ring(const dmn_loop_desc* d, long n, long n_out) { return d-
 
 // One loop step.  `ctr` = device step counter (graph mode) or nullptr with host step `s` (injected-noise mode);
 // `z0` = this step's injected noise block (draws x n floats) or nullptr for in-kernel Philox with device rng state.
-static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, int32_t* ctr_dev, bool use_ctr, int s, const float* z0,
-                        cudaStream_t st) {
+// `ip` (inpainting, never with injected noise): dmn_inpaint_prepare runs first, so everything after it sees the merged state.
+static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc* ip, int32_t* ctr_dev, bool use_ctr, int s,
+                        const float* z0, cudaStream_t st) {
   const dmn_unet_cfg& c = p->cfg;
   const long chw = (long)c.channels * c.image_size * c.image_size;
   const long n = (long)d->batch * chw;
@@ -1198,6 +1202,9 @@ static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, int32_t* ctr_dev, b
   const int32_t* step_dev = use_ctr ? ctr_dev : nullptr;
   const dmn_rng* rng_dev = z0 ? nullptr : reinterpret_cast<const dmn_rng*>(ctr_dev + 4);
   int rc;
+  if (ip && (rc = launch_inpaint_prepare(d->state_dev, ip->known_dev, ip->mask_dev, d->state_dev, n, ip->prep_coef_dev, step_dev, s,
+                                         d->rng, rng_dev, st)))
+    return rc;
   if (d->kind == DMN_LOOP_BPD) {
     // bits-per-dimension term of one timestep: x_t ~ q(x_t | x_0), U-Net on x_t, fused KL / decoder-NLL reduction into terms[b][t]
     float* xt = xmean;
@@ -1263,17 +1270,17 @@ static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, int32_t* ctr_dev, b
 }
 
 // the graph bakes in every pointer and scalar below; the RNG seed is NOT baked (it lives in device memory)
-static bool same_graph_key(const dmn_loop_desc& a, const dmn_loop_desc& b) {
+static bool same_graph_key(const dmn_loop_desc& a, const dmn_inpaint_desc& ia, const dmn_loop_desc& b, const dmn_inpaint_desc& ib) {
   const bool traj = a.traj_dev || b.traj_dev;   // only the trajectory kernel bakes n_steps in
   return a.kind == b.kind && (!traj || a.n_steps == b.n_steps) && a.batch == b.batch && a.n_corr == b.n_corr && a.snr == b.snr &&
          a.corr_kind == b.corr_kind && a.coef_dev == b.coef_dev && a.coef2_dev == b.coef2_dev && a.classes_dev == b.classes_dev &&
          a.state_dev == b.state_dev && a.scratch_dev == b.scratch_dev && a.traj_dev == b.traj_dev && a.traj_every == b.traj_every &&
-         a.cfg_scale == b.cfg_scale && a.cfg_on == b.cfg_on && (a.kind != DMN_LOOP_BPD || (a.aux_dev == b.aux_dev && a.n_steps == b.n_steps));
+         a.cfg_scale == b.cfg_scale && a.cfg_on == b.cfg_on && (a.kind != DMN_LOOP_BPD || (a.aux_dev == b.aux_dev && a.n_steps == b.n_steps)) &&
+         ia.known_dev == ib.known_dev && ia.mask_dev == ib.mask_dev && ia.prep_coef_dev == ib.prep_coef_dev;
 }
 
-extern "C" {
-
-int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
+// the loop driver of dmn_sample_loop (ip = nullptr) and dmn_sample_loop_inpaint
+static int run_loop(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc* ip, void* stream) {
   int rc = check_ready(p);
   if (rc) return rc;
   if (!d) return fail(DMN_EINVAL, "null descriptor");
@@ -1315,14 +1322,15 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
     // parity mode: injected noise => per-step pointers differ, plain launches with the host step index
     const int draws = (d->kind == DMN_LOOP_PC) ? d->n_corr + 1 : (d->kind == DMN_LOOP_DPMPP ? 0 : 1);
     for (int s = 0; s < d->n_steps; ++s)
-      if ((rc = enqueue_step(p, d, ctr, false, s, d->noise_dev + (long)s * draws * n, st))) return rc;
+      if ((rc = enqueue_step(p, d, ip, ctr, false, s, d->noise_dev + (long)s * draws * n, st))) return rc;
   } else if (!d->use_graph) {
     for (int s = 0; s < d->n_steps; ++s)
-      if ((rc = enqueue_step(p, d, ctr, true, 0, nullptr, st))) return rc;
+      if ((rc = enqueue_step(p, d, ip, ctr, true, 0, nullptr, st))) return rc;
   } else {
+    const dmn_inpaint_desc ip_key = ip ? *ip : dmn_inpaint_desc{};
     cudaGraphExec_t exec = nullptr;
     for (auto& g : p->graphs)
-      if (same_graph_key(g.key, *d)) exec = g.exec;
+      if (same_graph_key(g.key, g.ip, *d, ip_key)) exec = g.exec;
     if (!exec) {
       cudaStream_t cs;
       DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
@@ -1332,7 +1340,7 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
         cudaStreamDestroy(cs);
         return fail(DMN_ECUDA, std::string("begin capture: ") + cudaGetErrorString(e));
       }
-      rc = enqueue_step(p, d, ctr, true, 0, nullptr, cs);
+      rc = enqueue_step(p, d, ip, ctr, true, 0, nullptr, cs);
       e = cudaStreamEndCapture(cs, &graph);
       cudaStreamDestroy(cs);
       if (rc) {
@@ -1350,14 +1358,33 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) {
       dmn_plan::GraphEntry ge;
       ge.exec = exec;
       ge.key = *d;
+      ge.ip = ip_key;
       p->graphs.push_back(ge);
     }
     for (int s = 0; s < d->n_steps; ++s) DMN_CUDA_CHECK(cudaGraphLaunch(exec, st));
-    count_launch((int)((long)d->n_steps * dmn_loop_launches_per_step(p, d)));
+    count_launch((int)((long)d->n_steps * (dmn_loop_launches_per_step(p, d) + (ip ? 1 : 0))));
   }
   if (d->kind == DMN_LOOP_PC && d->aux_dev)
     DMN_CUDA_CHECK(cudaMemcpyAsync(d->aux_dev, xmean, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return 0;
+}
+
+extern "C" {
+
+int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) { return run_loop(p, d, nullptr, stream); }
+
+int dmn_sample_loop_inpaint(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc* ip, void* stream) {
+  if (!d || !ip) return fail(DMN_EINVAL, "null descriptor");
+  DMN_REQUIRE(d->kind == DMN_LOOP_DDPM || d->kind == DMN_LOOP_LEARNED || d->kind == DMN_LOOP_DDIM,
+              "inpainting is built for the DDPM / learned-variance / DDIM loops");
+  DMN_REQUIRE(!d->noise_dev, "inpainting has no injected-noise mode: noise_dev must be NULL");
+  DMN_REQUIRE(ip->known_dev && ip->mask_dev && ip->prep_coef_dev, "null device pointer in inpaint descriptor");
+  int rc = run_loop(p, d, ip, stream);
+  if (rc) return rc;
+  // final composite: row n_steps = {1, 0, 1, 0} puts the known pixels back exactly and draws nothing
+  const long n = (long)d->batch * p->cfg.channels * p->cfg.image_size * p->cfg.image_size;
+  return launch_inpaint_prepare(d->state_dev, ip->known_dev, ip->mask_dev, d->state_dev, n, ip->prep_coef_dev, nullptr, d->n_steps,
+                                d->rng, nullptr, (cudaStream_t)stream);
 }
 
 int dmn_loop_launches_per_step(const dmn_plan* p, const dmn_loop_desc* d) {

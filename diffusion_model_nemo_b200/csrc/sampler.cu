@@ -170,6 +170,40 @@ __global__ void __launch_bounds__(256) dpmpp_step_kernel(const float* x, const f
   }
 }
 
+// RePaint inpainting (Lugmayr et al. 2022), run before the model at every event: the forward jump into this event and the merge of
+// the noised known image.  row: {a_j, g_j, a_0, s_0}.
+//   y = a_j x + g_j z2 ;  k = a_0 known + s_0 z1 ;  x' = m k + (1 - m) y
+// z1 / z2 are draws 1 / 2 of the step word; each is drawn only when its coefficient is nonzero (uniform over the grid), so a row
+// {1, 0, 1, 0} draws nothing and returns `known` exactly where m = 1 and x exactly where m = 0.
+__global__ void __launch_bounds__(256) inpaint_prepare_kernel(const float* x, const float* __restrict__ known,
+                                                              const float* __restrict__ mask, float* out, long n4,
+                                                              const float* __restrict__ coef, const int32_t* step_dev, int step,
+                                                              dmn_rng rng_v, const dmn_rng* rng_dev) {
+  const dmn_rng rng = pick_rng(rng_v, rng_dev);
+  const float* c = coef_row(coef, step_dev, step);
+  const float aj = c[0], gj = c[1], a0 = c[2], s0 = c[3];
+  const bool need_z1 = s0 != 0.f, need_z2 = gj != 0.f;
+  const uint32_t sw1 = step_word(step_dev, step, 1), sw2 = step_word(step_dev, step, 2);
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
+    const float4 xv = reinterpret_cast<const float4*>(x)[i];
+    const float4 kv = reinterpret_cast<const float4*>(known)[i];
+    const float4 mv = reinterpret_cast<const float4*>(mask)[i];
+    float4 z1 = make_float4(0.f, 0.f, 0.f, 0.f), z2 = z1;
+    if (need_z1) z1 = Philox::normal4(rng.seed, rng.stream_id, sw1, (uint64_t)i);
+    if (need_z2) z2 = Philox::normal4(rng.seed, rng.stream_id, sw2, (uint64_t)i);
+    float4 o;
+#define DMN_INP(f)                                                     \
+  {                                                                    \
+    const float y = aj * xv.f + gj * z2.f;                             \
+    const float k = a0 * kv.f + s0 * z1.f;                             \
+    o.f = mv.f * k + (1.0f - mv.f) * y;                                \
+  }
+    DMN_INP(x) DMN_INP(y) DMN_INP(z) DMN_INP(w)
+#undef DMN_INP
+    reinterpret_cast<float4*>(out)[i] = o;
+  }
+}
+
 __global__ void __launch_bounds__(256) affine_noise_kernel(const float* __restrict__ x, const float* __restrict__ mo,
                                                            const float* __restrict__ z, float* __restrict__ out,
                                                            float* __restrict__ mean_out, long n4, const float* __restrict__ coef,
@@ -639,6 +673,15 @@ int launch_dpmpp(const float* x, const float* mo, float* hist, float* out, int b
   DMN_LAUNCH_CHECK("dpmpp_step");
   return 0;
 }
+int launch_inpaint_prepare(const float* x, const float* known, const float* mask, float* out, long n, const float* coef,
+                           const int32_t* step_dev, int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st) {
+  DMN_REQUIRE(n % 4 == 0 && n > 0, "inpaint_prepare: element count must be a positive multiple of 4");
+  DMN_REQUIRE(x && known && mask && out && coef, "inpaint_prepare: null pointer");
+  inpaint_prepare_kernel<<<grid_for(n / 4), 256, 0, st>>>(x, known, mask, out, n / 4, coef, step_dev, step, rng, rng_dev);
+  count_launch();
+  DMN_LAUNCH_CHECK("inpaint_prepare");
+  return 0;
+}
 
 }  // namespace dmn
 
@@ -664,6 +707,11 @@ int dmn_ddim_step(const float* x, const float* eps, const float* z_dev, float* x
 int dmn_dpmpp_step(const float* x, const float* model_out, float* hist, float* x_out, int batch, int64_t chw, int64_t mo_chw,
                    const float* coef_dev, const int32_t* step_dev, int step, void* stream) {
   return launch_dpmpp(x, model_out, hist, x_out, batch, chw, mo_chw, coef_dev, step_dev, step, (cudaStream_t)stream);
+}
+
+int dmn_inpaint_prepare(const float* x, const float* known, const float* mask, float* x_out, int64_t n, const float* coef_dev,
+                        const int32_t* step_dev, int step, dmn_rng rng, void* stream) {
+  return launch_inpaint_prepare(x, known, mask, x_out, n, coef_dev, step_dev, step, rng, nullptr, (cudaStream_t)stream);
 }
 
 int dmn_affine_noise_step(const float* x, const float* model_out, const float* z_dev, float* x_out, float* x_mean_out, int64_t n,

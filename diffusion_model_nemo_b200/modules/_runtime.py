@@ -72,10 +72,13 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
                     noise: Optional[torch.Tensor] = None, classes: Optional[torch.Tensor] = None,
                     n_corr: int = 0, corr_kind: int = 0, snr: float = 0.0, denoise: bool = False,
                     seed: Optional[int] = None, traj_every: int = 0, use_graph: bool = True,
-                    init_scale: float = 1.0, n_steps: Optional[int] = None, cfg_scale: Optional[float] = None) -> LoopResult:
+                    init_scale: float = 1.0, n_steps: Optional[int] = None, cfg_scale: Optional[float] = None,
+                    inpaint: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None) -> LoopResult:
     """Run n_steps of (U-Net + update) natively.  noise: [1 + n_steps*draws, B, C, H, W] injected N(0,1) tensors in
     the reference's draw order (element 0 = x_T), or None for in-kernel Philox; LOOP_DPMPP draws nothing and uses only noise[0].
-    cfg_scale: classifier-free guidance weight (None = off; 0.0 is a valid weight and gives the unconditional prediction)."""
+    cfg_scale: classifier-free guidance weight (None = off; 0.0 is a valid weight and gives the unconditional prediction).
+    inpaint: (known [B, C, H, W], mask broadcasting to it, prep_coef [n_steps + 1][8] device rows) runs the loop through
+    dmn_sample_loop_inpaint (in-kernel noise only)."""
     lib = L.lib()
     device = torch.device(device)
     require_cuda(device)
@@ -164,8 +167,23 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
         d.cfg_scale = float(cfg_scale) if guided else 0.0
         d.cfg_on = 1 if guided else 0
         d.state_elems = state.numel()
-        L.check(lib.dmn_sample_loop(plan.h, C.byref(d), st), "dmn_sample_loop")
-        plan.last_loop_launches = lib.dmn_loop_launches_per_step(plan.h, C.byref(d)) * n_steps
+        if inpaint is None:
+            L.check(lib.dmn_sample_loop(plan.h, C.byref(d), st), "dmn_sample_loop")
+            plan.last_loop_launches = lib.dmn_loop_launches_per_step(plan.h, C.byref(d)) * n_steps
+        else:
+            assert noise_dev is None, "inpainting draws its noise in-kernel"
+            known, mask, prep_coef = inpaint
+            # persistent expanded fp32 copies: the cached CUDA graph bakes the pointers in
+            for name, src in (("known", known), ("mask", mask)):
+                if name not in bufs[bkey]:
+                    bufs[bkey][name] = torch.empty_like(state)
+                bufs[bkey][name].copy_(src)
+            kb, mb = bufs[bkey]["known"], bufs[bkey]["mask"]
+            ip = L.InpaintDesc()
+            ip.known_dev, ip.mask_dev, ip.prep_coef_dev = kb.data_ptr(), mb.data_ptr(), prep_coef.data_ptr()
+            L.check(lib.dmn_sample_loop_inpaint(plan.h, C.byref(d), C.byref(ip), st), "dmn_sample_loop_inpaint")
+            # + one prepare kernel per event and the final composite
+            plan.last_loop_launches = (lib.dmn_loop_launches_per_step(plan.h, C.byref(d)) + 1) * n_steps + 1
         # keep every buffer alive until the stream has consumed it
         torch.cuda.current_stream(device).synchronize()
     return LoopResult(state.clone(), None if aux is None else aux.clone(), traj)

@@ -114,6 +114,10 @@ class DPMSolverDiffusion(GaussianDiffusion):
     def interpolate(self, model, x1, x2, t: Optional[int] = None, lambd: float = 0.5, noise=None):
         raise NotImplementedError("DPMSolverDiffusion has no interpolate(); decode a given latent with p_sample_loop(img=...)")
 
+    def inpaint(self, model, x_known, mask, device=None, noise=None, jump_length: int = 1, jump_n_sample: int = 1):
+        raise NotImplementedError("DPMSolverDiffusion has no inpaint(): its history ring would mix data predictions across merged "
+                                  "states; use GaussianDiffusion, LearnedGaussianDiffusion or GeneralizedGaussianDiffusion")
+
     @torch.no_grad()
     def p_sample_loop(self, model, shape, device=None, use_tqdm=True, noise=None, img=None):
         """Solve from x_T (img, else noise[0], else a Philox draw with self.seed -- the draw DDIM makes for that seed) to the data

@@ -4,8 +4,10 @@ Hot path (`sample`, `p_sample_loop`, `p_sample`, `interpolate`) runs natively: w
 `Unet` the whole T-step loop is a replayed CUDA graph (U-Net + one fused update kernel per step, no host sync, no
 per-step D2H); for any other callable the model is called per step and only the update is the fused kernel.
 Helper methods used by training / BPD code (`q_sample`, `q_posterior`, ...) keep the reference's torch semantics.
+`inpaint` (RePaint, an extension) runs the same loop with one merge kernel in front of every model evaluation.
 """
-from typing import Optional
+import math
+from typing import List, Optional, Tuple
 
 import torch
 
@@ -16,6 +18,36 @@ from .diffusion_process import AbstractDiffusionProcess, SCHEDULE_FNS, gaussian_
 
 def _default(val, d):
     return val if val is not None else (d() if callable(d) else d)
+
+
+def repaint_schedule(k: int, jump_length: int = 1, jump_n_sample: int = 1) -> List[int]:
+    """RePaint's get_schedule_jump (Lugmayr et al. 2022) with only jump_length / jump_n_sample: the state indices 0..k-1 of the
+    sampler's grid in the order they are visited, ending with -1 (the output).  j = r = 1 is the plain visit order."""
+    jumps = {p: jump_n_sample - 1 for p in range(0, k - jump_length, jump_length)}
+    t, ts = k, []
+    while t >= 1:
+        t -= 1
+        ts.append(t)
+        if jumps.get(t, 0) > 0:
+            jumps[t] -= 1
+            for _ in range(jump_length):
+                t += 1
+                ts.append(t)
+    ts.append(-1)
+    return ts
+
+
+def inpaint_events(ts: List[int]) -> List[Tuple[int, Optional[int]]]:
+    """[(i, a)] per reverse event: one per decreasing pair (i, i - 1) of the schedule, with a = the index the forward jump into it
+    starts from (a run of increasing pairs a -> i), or None when the event follows another event."""
+    events, src = [], None
+    for u, v in zip(ts[:-1], ts[1:]):
+        if v < u:
+            events.append((u, src))
+            src = None
+        elif src is None:
+            src = u
+    return events
 
 
 class GaussianDiffusion(AbstractDiffusionProcess):
@@ -226,6 +258,115 @@ class GaussianDiffusion(AbstractDiffusionProcess):
                                      L.stream_ptr(device)), "dmn_bpd_term(prior)")
             torch.cuda.current_stream(device).synchronize()
         return {"total_bpd": terms.sum(dim=1) + prior, "terms_bpd": terms, "prior_bpd": prior}
+
+    # ---- RePaint inpainting (extension) -------------------------------------------------------------------------------------------
+    def _inpaint_tables(self, jump_length: int, jump_n_sample: int, device):
+        """-> (update rows [E][8], time labels [E], prepare rows [E + 1][8], labels list) for the E events of the schedule.  The update
+        row and label of an event at grid index i are the sampler's own visit-order row for that index; prepare rows as documented at
+        dmn_inpaint_prepare in include/dmn_b200.h, expanded in fp64 from the fp32 alphas_cumprod table and rounded to fp32 once."""
+        ts = self._visit_order()
+        coef, times = self._loop_tables(ts, device)
+        key = ("inpaint", str(device), coef.data_ptr(), jump_length, jump_n_sample)
+        hit = self._coef_cache.get(key)
+        if hit is None:
+            k = len(ts)
+            events = inpaint_events(repaint_schedule(k, jump_length, jump_n_sample))
+            rows = [k - 1 - i for i, _ in events]               # grid index i is visit-order row k - 1 - i
+            ac = self.alphas_cumprod.double()
+
+            def abar(i):
+                return float(ac[int(ts[k - 1 - i])])
+
+            prep = []
+            for i, a in events:
+                ab = abar(i)
+                ratio = 1.0 if a is None else ab / abar(a)
+                prep.append([math.sqrt(ratio), math.sqrt(1.0 - ratio), math.sqrt(ab), math.sqrt(1.0 - ab)])
+            prep.append([1.0, 0.0, 1.0, 0.0])                      # final composite: the known pixels exactly, no draw
+            prep = torch.tensor(prep, dtype=torch.float64).to(torch.float32)
+            idx = torch.tensor(rows, dtype=torch.long, device=coef.device)
+            hit = (coef[idx].contiguous(), times[idx].contiguous(), R.coef_rows([prep[:, c] for c in range(4)], device),
+                   [int(ts[r]) for r in rows], coef, times)      # the base tables stay alive: their address is in the key
+            self._coef_cache[key] = hit
+        return hit[:4]
+
+    def _check_inpaint_args(self, x_known, mask, jump_length, jump_n_sample):
+        if not (isinstance(jump_length, int) and isinstance(jump_n_sample, int) and jump_length >= 1 and jump_n_sample >= 1):
+            raise ValueError(f"jump_length and jump_n_sample must be integers >= 1, got {jump_length!r}, {jump_n_sample!r}")
+        k = len(self._visit_order())
+        if jump_n_sample > 1 and jump_length >= k:
+            raise ValueError(f"jump_length={jump_length} must be smaller than the sampler's {k} grid points when jump_n_sample > 1")
+        if not (torch.is_tensor(x_known) and x_known.dim() == 4):
+            raise ValueError(f"x_known must be a [B, C, H, W] tensor, got {getattr(x_known, 'shape', type(x_known))}")
+        if not torch.is_tensor(mask):
+            raise ValueError("mask must be a tensor that broadcasts to x_known's shape")
+        try:
+            ok = torch.broadcast_shapes(mask.shape, x_known.shape) == x_known.shape
+        except RuntimeError:
+            ok = False
+        if not ok:
+            raise ValueError(f"mask of shape {tuple(mask.shape)} does not broadcast to x_known's shape {tuple(x_known.shape)}")
+        if not bool(((mask >= 0) & (mask <= 1)).all()):
+            raise ValueError("mask values must lie in [0, 1] (1 = keep the known pixel)")
+
+    @torch.no_grad()
+    def inpaint(self, model, x_known, mask, device=None, noise=None, jump_length: int = 1, jump_n_sample: int = 1):
+        """RePaint inpainting (Lugmayr et al. 2022) with the trained model unchanged: keep the pixels of `x_known` ([B, C, H, W] in the
+        model's data space [-1, 1]) where `mask` (broadcasts to x_known, values in [0, 1], 1 = keep) is 1 and generate the rest.
+
+        The sampler visits its own grid in RePaint's jump schedule (`repaint_schedule`).  Every reverse event merges
+        mask * q_sample(x_known, t) + (1 - mask) * x before the model at label t, then applies the sampler's own update.
+        `jump_n_sample` > 1 resamples: every `jump_length` grid points the state is noised forward by `jump_length` points and
+        denoised again, so that the generated region agrees with the known one.  A forward jump is one draw,
+        x_b = sqrt(abar_b / abar_a) x_a + sqrt(1 - abar_b / abar_a) z, which has the distribution of RePaint's `jump_length` single-step
+        undos.  After the last event the known pixels are put back exactly.
+
+        x_T is the draw `sample()` makes for `self.seed`, or `noise[0]` (further elements are ignored).  `trajectory_every` counts
+        events.  Returns the reference's list of CPU images in [0, 1], the last being the final sample."""
+        device = R.default_device(model, device)
+        R.require_cuda(device)
+        self._check_inpaint_args(x_known, mask, jump_length, jump_n_sample)
+        shape = list(x_known.shape)
+        if noise is not None and tuple(noise.shape[1:]) != tuple(shape):
+            raise ValueError(f"noise has shape {tuple(noise.shape)}; expected [n, {', '.join(map(str, shape))}]")
+        coef, times, prep, labels = self._inpaint_tables(jump_length, jump_n_sample, device)
+        unet, classes = R.resolve_model(model)
+        if unet is not None:
+            res = R.run_native_loop(unet, kind=self._loop_kind, shape=shape, device=device, times=times, coef=coef,
+                                    x_init=None if noise is None else noise[0], classes=classes, seed=self.seed,
+                                    traj_every=self.trajectory_every, use_graph=self.use_cuda_graph,
+                                    cfg_scale=float(self.guidance_scale) if (self.guidance_scale is not None and classes is not None) else None,
+                                    inpaint=(x_known, mask, prep))
+            return R.to_image_list(res.final, res.traj)
+        # foreign model: call it per event; the same kernels, rows and step words as the graph
+        if self.guidance_scale is not None:
+            raise NotImplementedError("guidance_scale needs this package's class-conditional Unet (doubled-batch native loop)")
+        b = shape[0]
+        seed = self.seed if self.seed is not None else R.draw_seed()
+        lib = L.lib()
+        with torch.cuda.device(device):
+            st = L.stream_ptr(device)
+            known = x_known.to(device, torch.float32).contiguous()
+            m = torch.empty_like(known)
+            m.copy_(mask)
+            x = torch.empty(tuple(shape), dtype=torch.float32, device=device)
+            rng = L.Rng(seed, R.rank_stream_id())
+            if noise is not None:
+                x.copy_(noise[0])
+            else:
+                L.check(lib.dmn_randn(L.ptr(x), x.numel(), rng, -1, st), "dmn_randn")
+            keep = []
+            for e, ti in enumerate(labels):
+                L.check(lib.dmn_inpaint_prepare(L.ptr(x), L.ptr(known), L.ptr(m), L.ptr(x), x.numel(), L.ptr(prep), None, e, rng, st),
+                        "dmn_inpaint_prepare")
+                mo = model(x, self._model_arg(ti, b, device)).float().contiguous()
+                self._launch_step(lib, x, mo, None, x, coef, e, rng, st)
+                if self.trajectory_every and (e + 1) % self.trajectory_every == 0:
+                    keep.append(x.clone())
+            L.check(lib.dmn_inpaint_prepare(L.ptr(x), L.ptr(known), L.ptr(m), L.ptr(x), x.numel(), L.ptr(prep), None, len(labels), rng,
+                                            st), "dmn_inpaint_prepare(final)")
+            traj = torch.stack(keep) if keep else None
+        return R.to_image_list(x, traj)
 
     @torch.no_grad()
     def sample(self, model, shape, device=None, noise=None):

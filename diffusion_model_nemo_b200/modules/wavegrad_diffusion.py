@@ -117,3 +117,7 @@ class WaveGradDiffusion(GaussianDiffusion):
             raise NotImplementedError("WaveGradDiffusion drives a (x, noise_level) denoiser; the native Unet takes timesteps. "
                                       "Pass this package's WaveGradUNet (native loop) or any other (x, noise_level) callable")
         return super().p_sample_loop(model, shape, device=device, use_tqdm=use_tqdm, noise=noise, img=img, start=start)
+
+    def inpaint(self, model, x_known, mask, device=None, noise=None, jump_length: int = 1, jump_n_sample: int = 1):
+        raise NotImplementedError("WaveGradDiffusion has no inpaint(): use GaussianDiffusion, LearnedGaussianDiffusion or "
+                                  "GeneralizedGaussianDiffusion")

@@ -257,6 +257,28 @@ int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream);
 /* kernels launched per loop step for the given descriptor (bench.py's gpu_launches). */
 int dmn_loop_launches_per_step(const dmn_plan* p, const dmn_loop_desc* d);
 
+/* RePaint inpainting (Lugmayr et al. 2022, "RePaint: Inpainting using Denoising Diffusion Probabilistic Models"; not in the
+ * reference: modules/gaussian_diffusion.py in the package builds the rows).  One elementwise step before the model of every event:
+ *   y  = a_j * x + g_j * z2             (forward jump into this event; a_j = 1, g_j = 0 when there is none)
+ *   k  = a_0 * known + s_0 * z1         (q_sample of the known image at this event's time: a_0 = sqrt(abar_t), s_0 = sqrt(1 - abar_t))
+ *   x' = mask * k + (1 - mask) * y
+ * coef row: {a_j, g_j, a_0, s_0}.  z1 / z2 are Philox draws 1 / 2 of step word (step + 1) * 8 + draw, keyed by element index; a draw
+ * whose coefficient is 0 is not made.  known, mask: [n] fp32 (mask in [0, 1], 1 = keep).  x_out may alias x.  16 B per element. */
+int dmn_inpaint_prepare(const float* x, const float* known, const float* mask, float* x_out, int64_t n, const float* coef_dev,
+                        const int32_t* step_dev, int step, dmn_rng rng, void* stream);
+
+typedef struct dmn_inpaint_desc {
+  const float* known_dev;        /* [batch*C*H*W] fp32 known image in [-1, 1] */
+  const float* mask_dev;         /* [batch*C*H*W] fp32 mask in [0, 1], 1 = keep */
+  const float* prep_coef_dev;    /* [n_steps + 1][DMN_COEF_STRIDE] dmn_inpaint_prepare rows; row n_steps = the final composite */
+} dmn_inpaint_desc;
+
+/* dmn_sample_loop with dmn_inpaint_prepare in front of every step ("event": one model evaluation and the sampler's own update, rows
+ * coef_dev[e] and time table row e), then the final composite (prepare with row n_steps, host step n_steps) after the last event.
+ * Graph mode replays one captured event; the graph cache key adds the three pointers.  DMN_LOOP_DDPM / LEARNED / DDIM only (others:
+ * DMN_EINVAL); noise_dev must be NULL (there is no injected-noise mode).  Kernels per event: dmn_loop_launches_per_step + 1. */
+int dmn_sample_loop_inpaint(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc* ip, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * Probability-flow ODE sampler.  Replaces ProbabilityFlowSampler.forward (sde_samplers/probability_flow_sampler.py:46-100,
  * score_sde's get_ode_sampler): solve_ivp(ode_func, (t0, t1), x_T, rtol, atol, method='RK45') where ode_func is the drift of
