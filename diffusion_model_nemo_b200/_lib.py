@@ -126,6 +126,7 @@ SYMBOLS = {
     "dmn_ode_work_bytes": (C.c_size_t, [_P, _I]),
     "dmn_conv_forward": (_I, [C.POINTER(ConvArgs), _P]),
     "dmn_conv_scratch_bytes": (C.c_size_t, [C.POINTER(ConvArgs)]),
+    "dmn_conv_forward_cat": (_I, [C.POINTER(ConvArgs), _P, C.c_int32, _P]),
     "dmn_linear_attention_core": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, C.c_size_t, _P]),
     "dmn_attention_core": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, C.c_size_t, _P]),
     "dmn_selftest_umma_gemm": (_I, [_P, _P, _P, _I, _I, _I, _P]),

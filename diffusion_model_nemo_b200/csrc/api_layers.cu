@@ -59,6 +59,7 @@ __global__ void group_stats_kernel(const T* x, stat_t* stats, int HW, int C, int
 
 namespace dmn {
 int conv_tcgen05_read_trace(long long* out, int n);
+int conv_tcgen05_read_log(int32_t* out, int cap);
 int fa_read_trace(long long* out, int n);
 }
 
@@ -66,15 +67,22 @@ extern "C" {
 
 /* debug only (not part of the documented ABI): timeline of one CTA of the last tcgen05 conv launched with DMN_TC_TRACE=1 */
 int dmn_debug_conv_trace(long long* out, int n) { return conv_tcgen05_read_trace(out, n); }
+/* debug only: one record of 64 int32 per tcgen05 conv launch since the previous call (see conv_tcgen05.cu,
+ * conv_tcgen05_read_log); copies at most `cap` records, clears the log and returns how many there were.  Recording starts with the
+ * first call. */
+int dmn_debug_conv_log(int32_t* out, int cap) { return conv_tcgen05_read_log(out, cap); }
 /* debug only: phase timeline of CTA 0 of the last fused attention launch with DMN_FA_TRACE=1 (clock64 at: image start, phase A done,
  * context built, phase B done, phase C done; slots 0..4 first image, 8..12 last image of the CTA) */
 int dmn_debug_fa_trace(long long* out, int n) { return fa_read_trace(out, n); }
 
 size_t dmn_conv_scratch_bytes(const dmn_conv_args* a) { return a ? conv_layout(a).total : 0; }
 
-int dmn_conv_forward(const dmn_conv_args* a, void* stream) {
+// x2 / cin2: second source of a channel concatenation (cin2 = 0: none)
+static int conv_forward(const dmn_conv_args* a, const float* x2, int cin2, void* stream) {
   if (!a) return fail(DMN_EINVAL, "null args");
   DMN_REQUIRE(a->x && a->w && a->y && a->scratch_dev, "null tensor");
+  DMN_REQUIRE(cin2 >= 0 && cin2 < a->cin && (cin2 == 0 || x2), "concat source");
+  DMN_REQUIRE(cin2 == 0 || a->gn_groups == 0, "the concat form takes a plain operand (gn_groups = 0)");
   DMN_REQUIRE(a->mode >= 0 && a->mode <= 2, "mode");
   DMN_REQUIRE(a->act == DMN_ACT_F32 || a->act == DMN_ACT_BF16, "act");
   DMN_REQUIRE(a->engine == DMN_CONV_SIMT || a->act == DMN_ACT_BF16, "tcgen05 engine needs bf16 activations");
@@ -87,10 +95,15 @@ int dmn_conv_forward(const dmn_conv_args* a, void* stream) {
   const int wout = a->mode == CONV_DOWN ? a->win / 2 : (a->mode == CONV_UP ? a->win * 2 : a->win);
   const int k = a->mode == CONV_SAME ? a->ksize : 4;
   int rc;
-  if ((rc = nchw_to_nhwc(a->x, base + L.x, a->batch, a->cin, a->hin * a->win, a->act, st))) return rc;
+  // both sources NHWC back to back in the x region
+  const int cin1 = a->cin - cin2;
+  const size_t x2_off = L.x + (size_t)a->batch * a->hin * a->win * cin1 * (a->act == DMN_ACT_F32 ? 4 : 2);
+  if ((rc = nchw_to_nhwc(a->x, base + L.x, a->batch, cin1, a->hin * a->win, a->act, st))) return rc;
+  if (cin2 && (rc = nchw_to_nhwc(x2, base + x2_off, a->batch, cin2, a->hin * a->win, a->act, st))) return rc;
 
   ConvP c;
-  c.src1 = base + L.x; c.C1 = a->cin; c.C2 = 0;
+  c.src1 = base + L.x; c.C1 = cin1; c.C2 = cin2;
+  c.src2 = cin2 ? base + x2_off : nullptr;
   c.B = a->batch; c.Hin = a->hin; c.Win = a->win; c.Hout = hout; c.Wout = wout; c.Cout = a->cout;
   c.mode = a->mode; c.ksize = a->ksize;
   c.bias = a->bias;
@@ -138,6 +151,12 @@ int dmn_conv_forward(const dmn_conv_args* a, void* stream) {
       return rc;
   }
   return 0;
+}
+
+int dmn_conv_forward(const dmn_conv_args* a, void* stream) { return conv_forward(a, nullptr, 0, stream); }
+int dmn_conv_forward_cat(const dmn_conv_args* a, const float* x2, int32_t cin2, void* stream) {
+  if (cin2 <= 0) return fail(DMN_EINVAL, "dmn_conv_forward_cat: cin2 must be positive");
+  return conv_forward(a, x2, cin2, stream);
 }
 
 static int attn_common(bool linear, const float* qkv, float* out, int batch, int heads, int dh, int n, int act, void* scratch,

@@ -50,8 +50,11 @@
 // Garbage rows: flat positions that fall on a pad column/row are computed and discarded (1 - HW/S of the MMA
 // work for 3x3: 6 % at 32x32, 11 % at 16x16, 21 % at 8x8, 36 % at 4x4).
 #include <cuda.h>     // CUtensorMap (type and enums only; the encoder is fetched through cudaGetDriverEntryPoint)
+#include <array>
+#include <atomic>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <type_traits>
 #include <vector>
 
@@ -2050,10 +2053,37 @@ static cudaError_t ensure_smem_attr(const void* fn) {
   if (e == cudaSuccess) done.emplace_back(dev, fn);
   return e;
 }
+// launch log (dmn_debug_conv_log): one record of kLogInts int32 per launch, written on the host when the launch is enqueued (a replayed
+// graph records nothing).  Tests read it to show which instantiation and tiling regime a convolution ran.  Off until first read.
+//   [0, 1] kernel function pointer (low, high 32 bits), [2] geo, [3] ksize, [4] C1, [5] C2, [6] Cout, [7] H (input), [8] B, [9] pro,
+//   [10] pgroups, [11] ogroups, [12] swap, [13] atma, [14] mt, [15] n_big_tiles, [16] total_tiles, [17] grid, [18] threads,
+//   [19] n_tiles_n, [20] big_rows, [21] total_flat, [22] n_pass, [23] reserved; [24, 64) kernel name (cudaFuncGetName), NUL-terminated
+constexpr int kLogInts = 64, kLogNameAt = 24, kLogMax = 1 << 16;
+static std::mutex g_log_mu;
+static std::vector<std::array<int32_t, kLogInts>> g_log;
+static std::atomic<bool> g_log_on{false};
+static void log_launch(const void* fn, int grid, int threads, const Params& p) {
+  if (!g_log_on.load(std::memory_order_relaxed)) return;
+  std::array<int32_t, kLogInts> r{};
+  const uint64_t f = (uint64_t)(uintptr_t)fn;
+  const int32_t v[kLogNameAt] = {(int32_t)(uint32_t)f, (int32_t)(uint32_t)(f >> 32), p.geo, p.ksize, p.c.C1, p.c.C2, p.c.Cout, p.H, p.c.B,
+                                 p.c.pro, p.c.pgroups, p.c.ogroups, p.swap, p.atma, p.mt, p.n_big_tiles, p.total_tiles, grid, threads,
+                                 p.n_tiles_n, p.big_rows, (int32_t)p.total_flat, p.n_pass, 0};
+  std::memcpy(r.data(), v, sizeof(v));
+  const char* name = nullptr;
+  if (cudaFuncGetName(&name, fn) == cudaSuccess && name)
+    std::strncpy(reinterpret_cast<char*>(r.data() + kLogNameAt), name, (kLogInts - kLogNameAt) * 4 - 1);
+  else
+    cudaGetLastError();
+  std::lock_guard<std::mutex> g(g_log_mu);
+  if (g_log.size() < (size_t)kLogMax) g_log.push_back(r);
+}
+
 template <typename K>
 static cudaError_t launch_kernel(K kern, int grid, int threads, const Params& p, cudaStream_t st, bool cooperative = false) {
   const cudaError_t e = ensure_smem_attr((const void*)kern);
   if (e != cudaSuccess) return e;
+  log_launch((const void*)kern, grid, threads, p);
   if (cooperative) {      // grid-wide barrier inside the kernel: the runtime guarantees (or refuses) co-residency of the whole grid
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
@@ -2136,10 +2166,10 @@ static int launch(Params p, cudaStream_t st) {
         DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<G2, 128, false, false, true, 3, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
         DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<G2, 128, false, false, false, 3, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
       }
-      if (extra) DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<G2, 128, false, false, true, 3, 16>, dim3(grid), dim3(kThreads16), smem_bytes(p), st, p));
-      else DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<G2, 128, false, false, false, 3, 16>, dim3(grid), dim3(kThreads16), smem_bytes(p), st, p));
-    } else if (extra) DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<G2, 128, false, false, true, 3>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
-    else DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<G2, 128, false, false, false, 3>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
+      if (extra) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, true, 3, 16>, grid, kThreads16, p, st));
+      else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 3, 16>, grid, kThreads16, p, st));
+    } else if (extra) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, true, 3>, grid, kThreads, p, st));
+    else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 3>, grid, kThreads, p, st));
     count_launch();
     DMN_LAUNCH_CHECK("conv_tcgen05");
     return 0;
@@ -2246,12 +2276,12 @@ static int launch(Params p, cudaStream_t st) {
     return 0;
   }
   if (GEO == GEO_SAME && (p.c.pro & PRO_LRELU)) {
-    if (p.NT == 128) DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<GEO_SAME, 128, true>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
-    else if (p.NT == 64) DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<GEO_SAME, 64, true>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
-    else DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<GEO_SAME, 32, true>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
-  } else if (p.NT == 128) DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<GEO, 128>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
-  else if (p.NT == 64) DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<GEO, 64>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
-  else DMN_CUDA_CHECK(launch_pdl(conv_tcgen05_kernel<GEO, 32>, dim3(grid), dim3(kThreads), smem_bytes(p), st, p));
+    if (p.NT == 128) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, true>, grid, kThreads, p, st));
+    else if (p.NT == 64) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 64, true>, grid, kThreads, p, st));
+    else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 32, true>, grid, kThreads, p, st));
+  } else if (p.NT == 128) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO, 128>, grid, kThreads, p, st));
+  else if (p.NT == 64) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO, 64>, grid, kThreads, p, st));
+  else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO, 32>, grid, kThreads, p, st));
   count_launch();
   DMN_LAUNCH_CHECK("conv_tcgen05");
   return 0;
@@ -2363,6 +2393,15 @@ int conv_tcgen05_read_trace(long long* out, int n) {
   DMN_CUDA_CHECK(cudaDeviceSynchronize());
   DMN_CUDA_CHECK(cudaMemcpyFromSymbol(out, tc::g_trace, (size_t)n * sizeof(long long)));
   return 0;
+}
+
+int conv_tcgen05_read_log(int32_t* out, int cap) {
+  std::lock_guard<std::mutex> g(tc::g_log_mu);
+  tc::g_log_on.store(true);
+  const int n = (int)tc::g_log.size();
+  for (int i = 0; i < n && i < cap && out; ++i) std::memcpy(out + (size_t)i * tc::kLogInts, tc::g_log[i].data(), sizeof(int32_t) * tc::kLogInts);
+  tc::g_log.clear();
+  return n;
 }
 
 int conv_tcgen05(const ConvP& c, cudaStream_t st) {

@@ -353,6 +353,11 @@ typedef struct dmn_conv_args {
 } dmn_conv_args;
 int dmn_conv_forward(const dmn_conv_args* a, void* stream);
 size_t dmn_conv_scratch_bytes(const dmn_conv_args* a);
+/* The same convolution over the channel concatenation cat(x, x2) [ResnetBlock of the up path, unet.py cat((x, h.pop()), dim=1)]:
+ * a->cin = C1 + C2 is the total, a->x holds the first C1 = cin - cin2 channels ([batch][C1][hin][win]), x2 the other cin2
+ * ([batch][cin2][hin][win]), a->w is the concat weight [cout][cin][k][k].  Plain operand only: a->gn_groups must be 0 (DMN_EINVAL
+ * otherwise).  Scratch as for dmn_conv_forward (dmn_conv_scratch_bytes(a)). */
+int dmn_conv_forward_cat(const dmn_conv_args* a, const float* x2, int32_t cin2, void* stream);
 
 /* LinearAttention core (mha.py:44-58, between to_qkv and to_out) / Attention core (mha.py:16-29).
  * qkv fp32 NCHW [batch, 3*heads*dim_head, H, W] -> out fp32 NCHW [batch, heads*dim_head, H, W]. */

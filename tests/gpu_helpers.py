@@ -7,11 +7,14 @@ from diffusion_model_nemo_b200 import _lib as L
 
 
 def conv_forward(x, w, bias=None, *, mode=0, ksize=3, gn=None, silu=False, temb=None, out_groups=0, act=L.ACT_F32,
-                 engine=L.CONV_SIMT):
-    """x fp32 NCHW cuda; w torch-layout weights; gn = (groups, gamma, beta) prologue.  Returns (y NCHW fp32, stats|None)."""
+                 engine=L.CONV_SIMT, x2=None):
+    """x fp32 NCHW cuda; w torch-layout weights; gn = (groups, gamma, beta) prologue; x2: second source of a channel concatenation
+    cat(x, x2) (dmn_conv_forward_cat; w is then the concat weight).  Returns (y NCHW fp32, stats|None)."""
     lib = L.lib()
     dev = x.device
     b, cin, h, wd = x.shape
+    cin2 = 0 if x2 is None else x2.shape[1]
+    cin += cin2
     cout = w.shape[1] if mode == 2 else w.shape[0]
     ho = h // 2 if mode == 1 else (h * 2 if mode == 2 else h)
     a = L.ConvArgs()
@@ -42,9 +45,39 @@ def conv_forward(x, w, bias=None, *, mode=0, ksize=3, gn=None, silu=False, temb=
     a.scratch_dev = (scratch.data_ptr() + 255) // 256 * 256
     a.scratch_bytes = scratch.numel() - 256
     with torch.cuda.device(dev):
-        L.check(lib.dmn_conv_forward(C.byref(a), L.stream_ptr(dev)), "dmn_conv_forward")
+        if x2 is None:
+            L.check(lib.dmn_conv_forward(C.byref(a), L.stream_ptr(dev)), "dmn_conv_forward")
+        else:
+            keep.append(x2.float().contiguous())
+            L.check(lib.dmn_conv_forward_cat(C.byref(a), L.ptr(keep[-1]), cin2, L.stream_ptr(dev)), "dmn_conv_forward_cat")
     torch.cuda.synchronize(dev)
     return y, stats
+
+
+LOG_INTS = 64
+
+
+def conv_log(cap=4096):
+    """Records of the tcgen05 conv launches since the previous call (dmn_debug_conv_log, a debug symbol outside the header; the
+    first call starts the recording).  Each: dict of the launch parameters, the kernel's name and its tiling regime."""
+    lib = L.lib()
+    fn = lib.dmn_debug_conv_log
+    fn.restype, fn.argtypes = C.c_int, [C.c_void_p, C.c_int]
+    buf = (C.c_int32 * (LOG_INTS * cap))()
+    n = fn(buf, cap)
+    assert n <= cap, "launch log overflow"
+    keys = ("fn_lo", "fn_hi", "geo", "ksize", "C1", "C2", "Cout", "H", "B", "pro", "pgroups", "ogroups", "swap", "atma", "mt",
+            "n_big_tiles", "total_tiles", "grid", "threads", "n_tiles_n", "big_rows", "total_flat", "n_pass")
+    out = []
+    for i in range(n):
+        r = buf[i * LOG_INTS:(i + 1) * LOG_INTS]
+        d = dict(zip(keys, r))
+        raw = b"".join(int(v & 0xffffffff).to_bytes(4, "little") for v in r[24:])
+        d["name"] = raw.split(b"\0")[0].decode() or f"fn@{(d['fn_hi'] & 0xffffffff) << 32 | (d['fn_lo'] & 0xffffffff):x}"
+        d["mixed"] = 0 < d["n_big_tiles"] < d["total_tiles"]
+        d["multi"] = d["total_tiles"] > d["grid"]
+        out.append(d)
+    return out
 
 
 def attention_core(qkv, linear, act=L.ACT_F32, heads=4, dh=32):
