@@ -24,8 +24,8 @@ def needs_rebuild() -> bool:
 
 
 def build_variant(path: str, extra_flags) -> str:
-    """Build a differently-configured copy of the library (e.g. -DDMN_TC_TRACE_BUILD=1 for tools/trace_conv.py, the DMN_EXP_*
-    experiment switches) at `path`; select it with DMN_LIB_PATH.  Objects go to a scratch directory, the in-tree build is untouched."""
+    """Build a differently-configured copy of the library (e.g. -DDMN_TC_TRACE_BUILD=1 for tools/trace_conv.py) at `path`;
+    select it with DMN_LIB_PATH.  Objects go to a scratch directory, the in-tree build is untouched."""
     import tempfile
 
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
@@ -92,7 +92,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
 
 if __name__ == "__main__":
-    if "--variant" in sys.argv:       # python -m diffusion_model_nemo_b200._build --variant tools/libdmn_x.so -DDMN_EXP_NO_LEAN=1 ...
+    if "--variant" in sys.argv:       # python -m diffusion_model_nemo_b200._build --variant tools/libdmn_x.so -DDMN_TC_TRACE_BUILD=1 ...
         i = sys.argv.index("--variant")
         print(build_variant(sys.argv[i + 1], sys.argv[i + 2:]))
     else:

@@ -41,11 +41,10 @@
 // loop of tile i+1 and the per-CTA setup is paid once per launch.
 //
 // The kernel is a template over <geometry, N tile, FiLM prologue, lean issue, rare epilogue terms, prologue mode, epilogue warps,
-// swapped operand roles, producer warps, fused block tail, TMA operand feed>:
+// swapped operand roles, TMA operand feed>:
 // the engine is sensitive to the amount of code around its inner loops, so every launch picks the smallest instantiation that
-// covers it (launch<>() below).  Compile-time switches DMN_EXP_* keep the measured alternatives buildable
-// (python -m diffusion_model_nemo_b200._build --variant <lib.so> -DDMN_EXP_...=1; select with DMN_LIB_PATH); profiles/README.md
-// records what each of them measured.
+// covers it (launch<>() below).  profiles/README.md and DESIGN.md record the alternatives that were measured and rejected (more
+// producer warps, CTA-pair weight multicast, the block tail behind a grid barrier, ...); their code was removed, git history has it.
 //
 // Garbage rows: flat positions that fall on a pad column/row are computed and discarded (1 - HW/S of the MMA
 // work for 3x3: 6 % at 32x32, 11 % at 16x16, 21 % at 8x8, 36 % at 4x4).
@@ -61,25 +60,6 @@
 #include "common.cuh"
 #include "ops.h"
 #include "tc_ptx.cuh"
-
-#ifndef DMN_EXP_PRO_DEPTH
-#define DMN_EXP_PRO_DEPTH 2
-#endif
-#ifndef DMN_EXP_PRO_ABUF
-#define DMN_EXP_PRO_ABUF 5
-#endif
-#ifndef DMN_EXP_SMEM_KB
-#define DMN_EXP_SMEM_KB 226
-#endif
-#ifndef DMN_EXP_ONE_ABUF
-#define DMN_EXP_ONE_ABUF 5
-#endif
-#ifndef DMN_EXP_PLAIN_ABUF
-#define DMN_EXP_PLAIN_ABUF 3        // operand ring of the plain (no prologue) swapped-role instantiations ...
-#endif
-#ifndef DMN_EXP_PLAIN_DEPTH
-#define DMN_EXP_PLAIN_DEPTH 1       // ... and the passes of cp.async copies a producer thread keeps in flight
-#endif
 
 namespace dmn {
 namespace tc {
@@ -97,12 +77,19 @@ constexpr int kCk = 32;                // channels per pass (4 k-chunks of 8)
 constexpr int kStagesMax = 8;          // weight-ring depth (chosen per launch to fit shared memory); one stage = G taps
 constexpr int kABuf = 3;               // operand (A) buffers: the producers run up to kABuf passes ahead of the MMA issuer
 constexpr int kABufMax = 6;            // barrier-array spacing / host sizing; the 1x1 instantiations use kABufOne buffers
-constexpr int kABufPro = DMN_EXP_PRO_ABUF;   // GroupNorm-prologue instantiations (PRO = 1): ncu shows 13 % of producer time waiting for the copies
-                                       // of the pass issued one iteration earlier; a deeper ring hides it at the price of shared memory
-constexpr int kABufOne = DMN_EXP_ONE_ABUF, kDepthOne = kABufOne - 2;   // 1x1 convs: MMA work per pass is tiny, the producers are
+constexpr int kABufPro = 5, kDepthPro = 2;   // GroupNorm-prologue instantiations (PRO = 1): ncu shows 13 % of producer time waiting for the
+                                       // copies of the pass issued one iteration earlier; a deeper ring hides it at the price of shared memory
+constexpr int kABufOne = 5, kDepthOne = kABufOne - 2;   // 1x1 convs: MMA work per pass is tiny, the producers are
                                        // bound by the global-load latency of the passes they keep in flight
+constexpr int kABufPlain = 3, kDepthPlain = 1;   // plain (no prologue) swapped-role instantiations: operand ring and passes in flight
 constexpr int kDepth = 1;              // passes a producer thread keeps in flight (cp.async groups) before it finishes the oldest;
                                        // kABuf >= kDepth + 2, else finishing pass c would wait for the MMAs of pass c-1
+constexpr int kGS = 3;                 // items of a thread transformed side by side in one basic block (TMA prologue tiles)
+// lean (unrolled) issue path: with fewer passes per tile the tile is epilogue-bound and the faster main loop only adds contention
+// (level-0 convs 0.078 -> 0.084 ms); the GroupNorm-prologue 3x3 on the TMA feed measured the same threshold (level-0: 0.0843 ms
+// looped, 0.0877 ms unrolled)
+constexpr int kLeanMinPass = 8;
+constexpr size_t kSmemLimit = (size_t)226 * 1024;   // dynamic shared memory per CTA (a CTA may opt in to 227 KB)
 constexpr int kMaxItems = 7;           // 16-byte operand items per producer thread per pass (P <= 448)
 constexpr int kNimgMax = 20;           // images a 256-position window may touch
 constexpr int kGroupsMax = 32;         // GroupNorm groups of the prologue
@@ -115,8 +102,6 @@ struct Params {
   int ksize, ntap, NT, n_pass, tiles_per_phase, n_tiles_n, m_tiles, total_tiles;
   int abuf;                // operand buffers of the instantiation that will be launched (kABuf, or kABufOne for the 1x1 form)
   int n_big_tiles, big_rows, halo_hi;   // tiles [0, n_big_tiles) have 256 rows, the rest 128 rows starting at flat position big_rows
-  int cl;                  // CTAs per cluster (1 | 2): the CTAs of a cluster work on neighbouring pixel tiles of the SAME N tile in lock step
-                           // and share every weight stage (each loads 1 / cl of it and multicasts it to all)
   long total_flat;
   uint32_t lbo_a, sbo_a, lbo_b, sbo_b;   // bytes
   uint32_t tmem_cols;
@@ -126,7 +111,6 @@ struct Params {
   int delta[64];           // [4 phases][16 taps] tap offsets in flat positions (constant bank => uniform registers in the issuer)
   uint32_t magic_S, magic_W;   // ceil(2^26 / S), ceil(2^24 / Wv): exact small-number division in vdecode_rel
   unsigned long long magic64_S;   // ceil(2^64 / S): f / S == umul64hi(f, magic64_S) for every 32-bit f (the per-tile decodes of the TMA path)
-  int pg_shift;                // log2(pgroups) (TMA prologue instantiations: pgroups is a power of two)
   float inv_cnt_in;
   long long* trace;        // debug timeline (null in production)
   int trace_cta;
@@ -153,71 +137,8 @@ __device__ long long g_trace[1024];
 #define DMN_TC_TRACE_PRODUCER 0     // 1: also account the producers' wait clocks (slots 14 / 15); costs registers in the hot role
 #endif
 constexpr bool kTraceProducer = DMN_TC_TRACE_PRODUCER != 0;
-#ifndef DMN_EXP_LEAN_MIN_PASS_TMA_PRO
-#define DMN_EXP_LEAN_MIN_PASS_TMA_PRO 8
-#endif
-#ifndef DMN_EXP_TMA_REGTABLES
-#define DMN_EXP_TMA_REGTABLES 0
-#endif
-#ifndef DMN_EXP_PRO_GROUP
-#define DMN_EXP_PRO_GROUP 3        // items of a thread transformed side by side in one basic block (TMA tiles)
-#endif
-constexpr int kGS = DMN_EXP_PRO_GROUP;
-#ifndef DMN_EXP_SERIAL_PRO
-#define DMN_EXP_SERIAL_PRO 0       // 1: the item-by-item prologue transform of the TMA tiles (A/B)
-#endif
-#ifndef DMN_EXP_ZFILL_PLAIN
-#define DMN_EXP_ZFILL_PLAIN 0
-#endif
-#ifndef DMN_EXP_ZFILL
-#define DMN_EXP_ZFILL 1
-#endif
 #ifndef DMN_EXP_MMATRACE
 #define DMN_EXP_MMATRACE 0          // 1: account the MMA issuer's wait clocks (slots 12 / 13); measured -1.3 % on the whole step
-#endif
-// contention experiments (tools/trace_conv.py with a variant build; results are garbage, only the timeline is meaningful)
-#ifndef DMN_EXP_NO_FENCE
-#define DMN_EXP_NO_FENCE 0          // MMA issuer: no tcgen05.fence::after_thread_sync after the operand / weight barrier waits
-#endif
-#ifndef DMN_EXP_NO_LEAN
-#define DMN_EXP_NO_LEAN 0           // 1: the generic (looped) MMA issue path for every geometry
-#endif
-#ifndef DMN_EXP_LEAN_MIN_PASS
-#define DMN_EXP_LEAN_MIN_PASS 8
-#endif
-#ifndef DMN_EXP_ACC_RELAXED
-#define DMN_EXP_ACC_RELAXED 0       // 1: the MMA issuer backs off while it waits for the epilogue to drain an accumulator set
-#endif
-#ifndef DMN_EXP_BRANCHY_PRO
-#define DMN_EXP_BRANCHY_PRO 1       // 0: the in-window item slots of the prologue transform without per-item branches (interleaved chains);
-                                    // measured SLOWER on every conv of the step, including those without a prologue (+0.002..0.004 ms each):
-                                    // the three extra unrolled copies grow the kernel, and the engine is sensitive to code size
-#endif
-#ifndef DMN_EXP_NO_ONETAP
-#define DMN_EXP_NO_ONETAP 0
-#endif
-#ifndef DMN_EXP_PRO_COST
-#define DMN_EXP_PRO_COST 0          // timing probes of the prologue transform (results are wrong): 1 = no tanh, 2 = LDS + STS only (no math),
-                                    // 3 = nothing at all (copies, fence and barrier arrival only)
-#endif
-#ifndef DMN_EXP_EW16_LEAN
-#define DMN_EXP_EW16_LEAN 1
-#endif
-#ifndef DMN_EXP_EW16
-#define DMN_EXP_EW16 1              // 0: never use the 16-epilogue-warp instantiations
-#endif
-#ifndef DMN_EXP_FENCE_MODE
-#define DMN_EXP_FENCE_MODE 0        // 0: every producer thread fences (generic -> async proxy) before it arrives on the operand barrier;
-                                    // 1: no fence at all (timing probe only, NOT correct); 2: the MMA warp fences after it has acquired the barrier
-#endif
-#ifndef DMN_EXP_NO_EPI
-#define DMN_EXP_NO_EPI 0            // epilogue: TMEM reads only (no staging, no global stores, no statistics)
-#endif
-#ifndef DMN_EXP_NO_LOAD
-#define DMN_EXP_NO_LOAD 0           // producers: no operand copies
-#endif
-#ifndef DMN_EXP_NO_WEIGHTS
-#define DMN_EXP_NO_WEIGHTS 0        // weight loader: barrier arrivals without the bulk copies
 #endif
 #ifndef DMN_TC_TRACE_BUILD
 #define DMN_TC_TRACE_BUILD 0        // 1: compile the role timeline in (tools/trace_conv.py builds such a library); costs 1.5 % of the step
@@ -251,15 +172,12 @@ __device__ __forceinline__ VPos vdecode(int f, const Params& p) {
 struct TileGeom {
   int m0, mt, n_tile;
 };
-// Cluster-aware order: tile = cl * q + r (r = rank in the cluster); the cl tiles of one q share the N tile q % n_tiles_n and are
-// neighbouring M tiles, so the CTAs of a cluster consume identical weight stages in the same order.  cl = 1 is the plain order.
 __device__ __forceinline__ TileGeom tile_geom(int tile, const Params& p) {
   TileGeom g;
   const bool big = tile < p.n_big_tiles;
   const int k = big ? tile : tile - p.n_big_tiles;
-  const int q = p.cl == 2 ? (k >> 1) : k, r = p.cl == 2 ? (k & 1) : 0;
-  const int m = (q / p.n_tiles_n) * p.cl + r;
-  g.n_tile = q % p.n_tiles_n;
+  const int m = k / p.n_tiles_n;
+  g.n_tile = k % p.n_tiles_n;
   g.mt = big ? 2 : 1;
   g.m0 = big ? m * 256 : p.big_rows + m * 128;
   return g;
@@ -362,12 +280,6 @@ __device__ __forceinline__ void stats_flush(const float* val, int key, bool vali
   }
 }
 
-// release of a weight stage: with a cluster every CTA's loader writes into every CTA's stage, so the release is multicast
-__device__ __forceinline__ void commit_stage(uint32_t bar, uint32_t cmask) {
-  if (cmask > 1u) umma_commit_mc(bar, (uint16_t)cmask);
-  else umma_commit(bar);
-}
-
 // One weight stage (G taps x two k16 steps x 1|2 accumulators) of the MMA issuer.  Descriptor words are computed OUTSIDE the
 // elected branch so that they are warp-uniform values (uniform registers); `didx` indexes the tap-offset table in the constant bank.
 template <int G, bool TWO>
@@ -422,7 +334,7 @@ template <int NTAP, int GG, bool TWO>
 __device__ __forceinline__ void issue_pass(bool leader, uint32_t d0, uint32_t d1, uint32_t au_lo, const int (&dl)[NTAP], uint32_t b_lo0,
                                            uint32_t b_stage_units, uint32_t b_tap_units, uint32_t hi_a, uint32_t hi_b, uint32_t a_k16,
                                            uint32_t b_k16, uint32_t idesc, uint32_t acc_first, uint64_t* full_b, uint64_t* empty_b, int nst,
-                                           int& st, uint32_t& ph, uint32_t a_half, uint32_t cmask = 1u) {
+                                           int& st, uint32_t& ph, uint32_t a_half) {
 #pragma unroll
   for (int s = 0; s < NTAP / GG; ++s) {
     mbar_wait(smem_u32(&full_b[st]), ph);
@@ -432,7 +344,7 @@ __device__ __forceinline__ void issue_pass(bool leader, uint32_t d0, uint32_t d1
     for (int g = 0; g < GG; ++g)
       issue_tap<TWO>(leader, d0, d1, au_lo + (uint32_t)dl[s * GG + g], b_lo + (uint32_t)g * b_tap_units, hi_a, hi_b, a_k16, b_k16, idesc,
                      (s | g) ? 1u : acc_first, a_half);
-    if (leader) commit_stage(smem_u32(&empty_b[st]), cmask);     // frees the weight stage once these MMAs retire
+    if (leader) umma_commit(smem_u32(&empty_b[st]));     // frees the weight stage once these MMAs retire
     __syncwarp();
     if (++st == nst) { st = 0; ph ^= 1; }
   }
@@ -452,8 +364,7 @@ __device__ __forceinline__ void issue_tap_swap(bool leader, uint32_t d, uint32_t
 template <int NTAP, int GG>
 __device__ __forceinline__ void issue_pass_swap(bool leader, uint32_t d, uint32_t au_lo, const int (&dl)[NTAP], uint32_t b_lo0, uint32_t b_stage_units,
                                                 uint32_t b_tap_units, uint32_t hi_a, uint32_t hi_b, uint32_t a_k16, uint32_t b_k16, uint32_t idesc,
-                                                uint32_t acc_first, uint64_t* full_b, uint64_t* empty_b, int nst, int& st, uint32_t& ph,
-                                                uint32_t cmask) {
+                                                uint32_t acc_first, uint64_t* full_b, uint64_t* empty_b, int nst, int& st, uint32_t& ph) {
 #pragma unroll
   for (int s = 0; s < NTAP / GG; ++s) {
     mbar_wait(smem_u32(&full_b[st]), ph);
@@ -463,7 +374,7 @@ __device__ __forceinline__ void issue_pass_swap(bool leader, uint32_t d, uint32_
     for (int g = 0; g < GG; ++g)
       issue_tap_swap(leader, d, au_lo + (uint32_t)dl[s * GG + g], b_lo + (uint32_t)g * b_tap_units, hi_a, hi_b, a_k16, b_k16, idesc,
                      (s | g) ? 1u : acc_first);
-    if (leader) commit_stage(smem_u32(&empty_b[st]), cmask);
+    if (leader) umma_commit(smem_u32(&empty_b[st]));
     __syncwarp();
     if (++st == nst) { st = 0; ph ^= 1; }
   }
@@ -491,24 +402,15 @@ __device__ __forceinline__ void issue_pass_swap(bool leader, uint32_t d, uint32_
 //     slows the operand producers and the epilogue staging down), and the single issuing thread has half as many instructions to feed.
 //     The epilogue becomes channel-per-lane: bias and GroupNorm statistics are per-thread scalars / serial sums, the bf16 output is
 //     transposed through a small per-warp staging tile (2 x 2 register transposes with one shuffle per pixel pair).
-// PW: operand-producer warps, 8 or 16.  The GroupNorm-prologue producers are latency bound (cp.async -> LDS -> transform -> STS chains with
-//     two warps per scheduler): 16 warps halve the items per thread and double the chains in flight.
-// TAIL: the ResnetBlock tail fused behind a grid-wide barrier (cooperative launch: every CTA of the persistent grid is resident): once all
-//     tiles of the launch are stored and their GroupNorm statistics complete, each CTA walks its own tiles again (they are still in L2)
-//     and writes SiLU(GroupNorm(out)) + residual -- the pass that used to be a separate gn_finalize launch reading the raw output from HBM.
-template <int GEO, int NT, bool FILM = false, bool LEAN = false, bool EXTRA = true, int PRO = 2, int EW = kEpiWarps, bool SWAP = false, int PW = 8,
-          bool TAIL = false, bool ATMA = false>
-__global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(const __grid_constant__ Params p) {
-  static_assert(!ATMA || (NT == 128 && !FILM && !EXTRA && !TAIL && (PRO == 0 || PRO == 1 || PRO == 3) && GEO != GEO_INIT),
+template <int GEO, int NT, bool FILM = false, bool LEAN = false, bool EXTRA = true, int PRO = 2, int EW = kEpiWarps, bool SWAP = false,
+          bool ATMA = false>
+__global__ void __launch_bounds__((kProdWarps + EW + 2) * 32, 1) conv_tcgen05_kernel(const __grid_constant__ Params p) {
+  static_assert(!ATMA || (NT == 128 && !FILM && !EXTRA && (PRO == 0 || PRO == 1 || PRO == 3) && GEO != GEO_INIT),
                 "TMA operand path: the hot 128-column instantiations");
-  static_assert(!TAIL || (GEO == GEO_SAME && NT == 128 && PRO == 1 && !EXTRA && !SWAP), "fused block tail: the GroupNorm-prologue 3x3 instantiations");
   static_assert(!SWAP || (NT == 128 && !EXTRA && !FILM && GEO != GEO_INIT), "swapped operand roles: hot 128-channel instantiations only");
-  static_assert(PW == 8 || ((PW == 16 || PW == 12) && EW == 8 && PRO == 1), "12 / 16 producer warps: the GroupNorm-prologue instantiations");
-  constexpr int kProdWarps = PW, kProdThreads = PW * 32;       // (shadow the 8-warp defaults of the namespace)
-  constexpr int kMaxItems = PW == 16 ? 4 : (PW == 12 ? 5 : 7);
   constexpr int kLoaderW = kProdWarps + EW, kMmaW = kLoaderW + 1, kEpiT = EW * 32;
-  constexpr int AB = (PRO == 3 && GEO == GEO_SAME) ? kABufOne : ((PRO == 1 && GEO == GEO_SAME) ? kABufPro : ((PRO == 0 && SWAP) ? DMN_EXP_PLAIN_ABUF : kABuf));
-  constexpr int DEPTH = (PRO == 3 && GEO == GEO_SAME) ? kDepthOne : ((PRO == 1 && GEO == GEO_SAME) ? DMN_EXP_PRO_DEPTH : ((PRO == 0 && SWAP) ? DMN_EXP_PLAIN_DEPTH : kDepth));
+  constexpr int AB = (PRO == 3 && GEO == GEO_SAME) ? kABufOne : ((PRO == 1 && GEO == GEO_SAME) ? kABufPro : ((PRO == 0 && SWAP) ? kABufPlain : kABuf));
+  constexpr int DEPTH = (PRO == 3 && GEO == GEO_SAME) ? kDepthOne : ((PRO == 1 && GEO == GEO_SAME) ? kDepthPro : ((PRO == 0 && SWAP) ? kDepthPlain : kDepth));
   static_assert(AB <= kABufMax && DEPTH >= 1 && DEPTH <= 3 && AB >= DEPTH + 2, "operand ring geometry");
   static_assert(EW == 8 || (EW == 16 && NT == 128 && (PRO == 0 || PRO == 3)), "16 epilogue warps: 128-column tiles without prologue");
   static_assert(!(LEAN && PRO == 3), "the lean issue path is for 9- and 4-tap convolutions");
@@ -545,7 +447,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
 
   // ---- one-time setup ----
   if (warp == kLoaderW) {          // one lane per barrier
-    if (lane < nst) { mbar_init(smem_u32(&full_b[lane]), 1); mbar_init(smem_u32(&empty_b[lane]), (uint32_t)p.cl); }
+    if (lane < nst) { mbar_init(smem_u32(&full_b[lane]), 1); mbar_init(smem_u32(&empty_b[lane]), 1); }
     if (lane >= 16 && lane < 16 + AB) {
       mbar_init(smem_u32(&full_a[lane - 16]), (ATMA && PRO != 1) ? 1 : kProdWarps);     // one arrival per producer WARP (see finish())
       mbar_init(smem_u32(&empty_a[lane - 16]), 1);
@@ -558,7 +460,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
   if (warp == kMmaW) tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   tc_fence_before();
   __syncthreads();
-  if (p.cl > 1) cluster_sync_all();      // the peer's barriers are initialised before any multicast copy / commit can reach them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   pdl_trigger();        // the next kernel may start its prologue; it waits for this grid's completion before reading our output
@@ -566,7 +467,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
   if (warp < kProdWarps) {
     // =============================== operand producers ===============================
     if (EW == 16) asm volatile("setmaxnreg.dec.sync.aligned.u32 40;");
-    if (PW == 16 && !SWAP) asm volatile("setmaxnreg.dec.sync.aligned.u32 64;");     // 512 x 8 registers handed to the 8 epilogue warps
     // Each thread owns up to kMaxItems 16-byte items (pixel, k-chunk) of every pass.  A pass is ISSUED as cp.async (LDGSTS)
     // copies straight into the operand buffer (padding is stored as zeros), and FINISHED kDepth passes later: wait for the
     // thread's own copies, apply the fused prologue in place (GroupNorm-apply, SiLU, time-embedding add), make the writes
@@ -680,7 +580,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
           }
           *reinterpret_cast<uint4*>(sA + ibuf * a_bytes + (uint32_t)kc * p.lbo_a + pixel * 16) = pack8(f);
         }
-        if (DMN_EXP_FENCE_MODE == 0) fence_proxy_async();
+        fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_u32(&full_a[ibuf]));
         if (++ibuf == AB) { ibuf = 0; iph ^= 1; }
@@ -689,10 +589,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
       }
       int goff[kMaxItems];      // SAME/UP: img*HW + pix (or -1 = padding); DOWN: packed (img, u, v) (or -1); -2 = outside the window
       int imgl[kMaxItems];
-      float2* s_gn_cur = s_gn;
-      stat_t nx_s0 = 0, nx_s1 = 0;       // ATMA: this thread's statistics entry of the next tile's table (loaded early, used late)
-      bool nx_have = false, nx_tile = false;
-      const int nfull = Pt / (kProdThreads / 4);      // item slots that are inside the window for EVERY thread (uniform)
       if constexpr (kOneTap) {
 #pragma unroll
         for (int j = 0; j < kMaxItems; ++j) {
@@ -700,51 +596,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
           imgl[j] = 0;
           goff[j] = (pixel < Pt && m0 + pixel < (int)p.total_flat) ? m0 + pixel : -2;
         }
-      } else if constexpr (ATMA && DMN_EXP_TMA_REGTABLES) {
-        // TMA operands: per item the producers only need "is it a real pixel" (padding stays zero) and its image -- decoded in
-        // registers with multiply-shift divisions, no shared tables.  The (mean, rstd) table is double buffered in the unused half of
-        // each image's 32-slot row (pgroups <= 16): this thread's entry of the NEXT tile's table is loaded here and turned into
-        // (mean, rstd) after this tile's passes, so neither its L2 latency nor a second barrier sits in front of the first pass
-        const int fs = m0 - p.halo_lo, fl = fs > 0 ? fs : 0;
-        const int il0 = (int)__umul64hi((unsigned long long)(unsigned)fl, p.magic64_S), rl0 = fl - il0 * p.S;      // == img_lo
-#pragma unroll
-        for (int j = 0; j < kMaxItems; ++j) {
-          const int pixel = px0 + (kProdThreads / 4) * j;
-          goff[j] = -2;
-          imgl[j] = 0;
-          if (pixel < Pt) {
-            goff[j] = -1;
-            if (fs + pixel >= 0) {
-              const VPos v = vdecode_rel(il0, rl0, fs + pixel - fl, p);
-              if (v.img >= 0 && v.row >= p.pad && v.col >= p.pad) { goff[j] = 0; imgl[j] = v.img - il0; }
-            }
-          }
-        }
-        s_gn_cur = s_gn + (pit & 1) * 16;
-        const int t_il = tid >> p.pg_shift, t_g = tid & (p.c.pgroups - 1);
-        const bool t_ent = tid < kNimgMax * p.c.pgroups;
-        if (pit == 0) {                                   // first tile of this CTA: its own table, synchronously
-          if (t_ent) {
-            float mean = 0.f, rstd = 0.f;
-            if (il0 + t_il < p.c.B) gn_mean_rstd(p.c.pstats + ((long)(il0 + t_il) * p.c.pgroups + t_g) * 2, p.inv_cnt_in, kGnEps, mean, rstd);
-            s_gn_cur[t_il * kGroupsMax + t_g] = make_float2(mean, rstd);
-          }
-          bar_sync_named(2, kProdThreads);
-        }
-        nx_have = false;
-        nx_tile = tile + (int)gridDim.x < p.total_tiles;
-        if (nx_tile && t_ent) {
-          int f2 = tile_geom(tile + (int)gridDim.x, p).m0 - p.halo_lo;
-          if (f2 < 0) f2 = 0;
-          const int img = (int)__umul64hi((unsigned long long)(unsigned)f2, p.magic64_S) + t_il;
-          if (img < p.c.B) {
-            const stat_t* sp = p.c.pstats + ((long)img * p.c.pgroups + t_g) * 2;
-            nx_s0 = __ldcg(sp);
-            nx_s1 = __ldcg(sp + 1);
-            nx_have = true;
-          }
-        }
-        if (tid == 0) TRACE(pit, 1);
       } else {
       // ---- per-tile tables: operand source per window pixel, GroupNorm (mean, rstd) per touched image ----
       if (DMN_TC_TRACE_BUILD && p.trace && tid == 0 && pit == 2 && blockIdx.x == (unsigned)p.trace_cta) p.trace[900] = clock64();
@@ -824,16 +675,14 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
             beh2[e] = pack2(0.5f * be[2 * e], 0.5f * be[2 * e + 1]);
             te2[e] = pack2(te[2 * e], te[2 * e + 1]);
           }
-          // one item = one independent chain (LDS -> FFMA2 -> MUFU -> FFMA2 -> STS).  The first `nfull` item slots of a thread are
-          // always inside the window, so they are transformed WITHOUT a per-item branch (one basic block: the scheduler interleaves
-          // their chains; only the store is predicated, padding stays zero AFTER the transform); the tail slots keep the branch so
-          // that slots outside the window cost nothing
-          auto do_item = [&](int j, bool check) {
-            if (DMN_EXP_PRO_COST == 3) return;
-            if (check && goff[j] < 0) return;
+          // one item = one independent chain (LDS -> FFMA2 -> MUFU -> FFMA2 -> STS), behind a per-item branch so that padding and slots
+          // outside the window cost nothing.  (Transforming the slots that are always inside the window without the branch, as one
+          // basic block, measured SLOWER on every conv of the step, including those without a prologue (+0.002..0.004 ms each): the
+          // extra unrolled copies grow the kernel, and the engine is sensitive to code size.)
+          auto do_item = [&](int j) {
+            if (goff[j] < 0) return;
             uint4* slot = reinterpret_cast<uint4*>(base + (px0 + (kProdThreads / 4) * j) * (ATMA ? 64 : 16));
-            if (DMN_EXP_PRO_COST == 2) { uint4 t = *slot; t.x ^= 0x00010001u; *slot = t; return; }
-            const float2 mr = FILM ? make_float2(0.f, 1.f) : s_gn_cur[imgl[j] * kGroupsMax + g];
+            const float2 mr = FILM ? make_float2(0.f, 1.f) : s_gn[imgl[j] * kGroupsMax + g];
             if ((p.c.pro & PRO_TEMB) && !temb_shared) {
               const float* tp = temb_base + (long)(img_lo + imgl[j]) * p.c.temb_bstride + cb;
               const float4 t0 = *reinterpret_cast<const float4*>(tp), t1 = *reinterpret_cast<const float4*>(tp + 4);
@@ -855,9 +704,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
                 unsigned long long x2 = fma2(pack2(v[2 * e], v[2 * e + 1]), sc2, sh2);
                 x2 = fma2(x2, gah2[e], beh2[e]);                       // hx
                 unsigned long long y2;
-                if (DMN_EXP_PRO_COST == 1) {
-                  y2 = fma2(x2, x2, x2);
-                } else if (p.c.pro & PRO_SILU) {
+                if (p.c.pro & PRO_SILU) {
                   float h0, h1, t0, t1;
                   unpack2(x2, h0, h1);
                   asm("tanh.approx.f32 %0, %1;" : "=f"(t0) : "f"(h0));
@@ -870,12 +717,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
                 unpack2(y2, v[2 * e], v[2 * e + 1]);
               }
             }
-            if (goff[j] >= 0) *slot = pack8(v);
-          };
-          auto run = [&](auto nf_tag) {
-            constexpr int NF = decltype(nf_tag)::value;
-#pragma unroll
-            for (int j = 0; j < kMaxItems; ++j) do_item(j, j >= NF);
+            *slot = pack8(v);
           };
           // TMA tiles: groups of three items as ONE basic block -- all loads first (an item slot outside the window reads the thread's
           // first slot instead), then the three arithmetic chains side by side, then stores predicated in the instruction itself
@@ -893,7 +735,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
               const int j = J0 + i;
               const int px = goff[j] >= -1 ? px0 + (kProdThreads / 4) * j : px0;
               raw[i] = lds128(base_u + (uint32_t)px * 64u);
-              mr[i] = s_gn_cur[imgl[j] * kGroupsMax + g];
+              mr[i] = s_gn[imgl[j] * kGroupsMax + g];
             }
 #pragma unroll
             for (int i = 0; i < N; ++i) {
@@ -930,7 +772,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
             }
           };
           if (fst) p.trace[912] = clock64();
-          if (ATMA && !FILM && DMN_EXP_PRO_COST == 0 && !DMN_EXP_SERIAL_PRO && !((p.c.pro & PRO_TEMB) && !temb_shared)) {
+          if (ATMA && !FILM && !((p.c.pro & PRO_TEMB) && !temb_shared)) {
             const int n_it = (Pt + kProdThreads / 4 - 1) / (kProdThreads / 4);     // item slots that reach into the window (uniform)
             auto all_groups = [&](auto silu_tag) {
               do_group(std::integral_constant<int, 0>(), silu_tag);
@@ -940,19 +782,15 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
             };
             if (p.c.pro & PRO_SILU) all_groups(std::true_type());
             else all_groups(std::false_type());
-          } else
-          switch (DMN_EXP_BRANCHY_PRO ? 0 : nfull) {
-            // the window sizes of the U-Net's 3x3 convs: 256-row tiles at 32x32 (5 full slots), at 16x16 / 8x8 (4), 128-row tiles (2)
-            case 7: case 6: case 5: run(std::integral_constant<int, 5>()); break;
-            case 4: run(std::integral_constant<int, 4>()); break;
-            case 3: case 2: run(std::integral_constant<int, 2>()); break;
-            default: run(std::integral_constant<int, 0>()); break;
+          } else {
+#pragma unroll
+            for (int j = 0; j < kMaxItems; ++j) do_item(j);
           }
         }
         // every writer fences its own stores towards the async proxy, then ONE lane per warp arrives: 256 / 512 arrivals on one
         // mbarrier serialise (measured: a pass that only loads and stores its items took 1.6k clk with per-thread arrivals)
         if (fst) p.trace[913] = clock64();
-        if (DMN_EXP_FENCE_MODE == 0) fence_proxy_async();
+        fence_proxy_async();
         if (fst) p.trace[914] = clock64();
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_u32(&full_a[fbuf]));
@@ -991,7 +829,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
         const uint32_t dst0 = sA_u + ibuf * a_bytes + (uint32_t)kc * p.lbo_a + (uint32_t)px0 * 16u;
         // measured: the predicated zero-fill form wins when the fused prologue follows (-0.003 ms on the level-0 GroupNorm convs)
         // and loses for plain copies (+0.004 ms), so plain operands keep the branchy issue
-        if (GEO == GEO_DOWN || !DMN_EXP_ZFILL || (!has_pro && !DMN_EXP_ZFILL_PLAIN)) {
+        if (GEO == GEO_DOWN || !has_pro) {
 #pragma unroll
           for (int j = 0; j < kMaxItems; ++j) {
             if (goff[j] < -1) continue;                  // outside the window
@@ -1017,7 +855,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
           for (int j = 0; j < kMaxItems; ++j) {
             const bool ok = goff[j] >= 0;
             const uint8_t* sp = sbase + (size_t)((uint32_t)(ok ? goff[j] : 0) * row_bytes);
-            cp_async16_zfill_pred(dst0 + (uint32_t)((kProdThreads / 4) * j) * 16u, sp, ok ? 16u : 0u, !DMN_EXP_NO_LOAD && goff[j] >= -1);
+            cp_async16_zfill_pred(dst0 + (uint32_t)((kProdThreads / 4) * j) * 16u, sp, ok ? 16u : 0u, goff[j] >= -1);
           }
         }
         cp_async_commit();
@@ -1050,19 +888,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
         if constexpr (!ATMA) cp_async_wait<0>();
         finish(p.n_pass - 1);
       }
-      if constexpr (ATMA && DMN_EXP_TMA_REGTABLES) {
-        if (nx_tile) {                   // (uniform) the next tile's table, in the other half of the rows
-          if (tid < kNimgMax * p.c.pgroups) {
-            float mean = 0.f, rstd = 0.f;
-            if (nx_have) {
-              const stat_t st2[2] = {nx_s0, nx_s1};
-              gn_mean_rstd(st2, p.inv_cnt_in, kGnEps, mean, rstd);
-            }
-            s_gn[((pit + 1) & 1) * 16 + (tid >> p.pg_shift) * kGroupsMax + (tid & (p.c.pgroups - 1))] = make_float2(mean, rstd);
-          }
-          bar_sync_named(2, kProdThreads);      // table complete; everybody is done reading this tile's
-        }
-      }
       if (tid == 0) TRACE(pit, 2);
     }
     }   // !(ATMA && PRO != 1)
@@ -1071,7 +896,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
     // register pool of the CTA: the 8 producer warps release 8 x 32 x (72 - 40) = 8192 registers, exactly what 16 epilogue warps need to
     // grow from 72 to 88 (setmaxnreg only moves registers inside the CTA's launch allocation; asking for 96 here deadlocks)
     if (EW == 16) asm volatile("setmaxnreg.inc.sync.aligned.u32 88;");
-    if (PW == 16 && !SWAP) asm volatile("setmaxnreg.inc.sync.aligned.u32 88;");
     // Warps are independent: no shared tables and no block barriers.  Each thread decodes its own accumulator rows
     // (flat position -> output pixel / image), reads 32-column chunks from TMEM, adds bias (+ class embedding, + residual),
     // stores bf16 and accumulates the GroupNorm statistics of its rows; a warp then reduces 8 partials at a time with a
@@ -1409,10 +1233,9 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
             unpack2(v2[q * 4 + 1], a0, a1); o.y = pack_bf16x2(a0, a1);
             unpack2(v2[q * 4 + 2], a0, a1); o.z = pack_bf16x2(a0, a1);
             unpack2(v2[q * 4 + 3], a0, a1); o.w = pack_bf16x2(a0, a1);
-            if (!DMN_EXP_NO_EPI) sts128(my_wr + (uint32_t)(((pc * 2 + q) ^ my_swz) << 4), o);
-            else if (o.x == 0x12345678u && o.w == 0x9abcdef0u) sts128(my_wr, o);     // keep the values alive
+            sts128(my_wr + (uint32_t)(((pc * 2 + q) ^ my_swz) << 4), o);
           }
-          if (do_stats && !DMN_EXP_NO_EPI) {
+          if (do_stats) {
             // (sum, sum of squares) of this row's 16 columns: two independent packed chains each
             unsigned long long s0 = 0ull, q0 = 0ull, s1 = 0ull, q1 = 0ull;
             if (valid) {
@@ -1447,7 +1270,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
         // the warp's 32 x NCOL block is staged: coalesced 16-byte stores, LPR consecutive lanes cover one output row.  Batches
         // of 4 store instructions: all row lookups (SHFL) and staging reads (LDS) first, then the predicated stores
         __syncwarp();
-        if (DMN_EXP_NO_EPI) continue;
 #pragma unroll
         for (int i0 = 0; i0 < 32; i0 += 4 * RPI) {
           int ropix[4];
@@ -1475,23 +1297,14 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
     int st = 0;
     uint32_t ph = 1;
     const int per_tile = p.n_pass * p.stages_per_pass;
-    // cluster: this CTA copies its 1 / cl share of every stage and multicasts it to all CTAs of the cluster; a stage may be refilled
-    // once EVERY CTA of the cluster has released it (empty_b counts cl arrivals: the MMA issuers commit with a multicast arrive)
-    const uint32_t share = b_bytes / (uint32_t)p.cl, my_off = share * cluster_ctarank();
-    const uint16_t cmask = (uint16_t)((1u << p.cl) - 1u);
     for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
       const int n_tile = tile_geom(tile, p).n_tile;
       const uint8_t* wsrc = (const uint8_t*)p.c.w + (size_t)n_tile * per_tile * b_bytes;
       for (int s = 0; s < per_tile; ++s) {
         mbar_wait_relaxed(smem_u32(&empty_b[st]), ph);
         if (leader) {
-          if (DMN_EXP_NO_WEIGHTS) {
-            mbar_arrive(smem_u32(&full_b[st]));
-          } else {
-            mbar_arrive_expect_tx(smem_u32(&full_b[st]), b_bytes);
-            if (p.cl > 1) bulk_g2s_mc(smem_u32(sB + st * b_bytes) + my_off, wsrc + (size_t)s * b_bytes + my_off, share, smem_u32(&full_b[st]), cmask);
-            else bulk_g2s(smem_u32(sB + st * b_bytes), wsrc + (size_t)s * b_bytes, b_bytes, smem_u32(&full_b[st]));
-          }
+          mbar_arrive_expect_tx(smem_u32(&full_b[st]), b_bytes);
+          bulk_g2s(smem_u32(sB + st * b_bytes), wsrc + (size_t)s * b_bytes, b_bytes, smem_u32(&full_b[st]));
         }
         __syncwarp();
         if (++st == nst) { st = 0; ph ^= 1; }
@@ -1506,7 +1319,6 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
     const bool leader = elect_one();
     const uint32_t idesc = make_idesc(128, NT);
     const uint32_t idesc_s2 = make_idesc(128, 256), idesc_s1 = make_idesc(128, 128);     // SWAP: N = pixels of the tile
-    const uint32_t cmask = (1u << p.cl) - 1u;
     // ATMA: the operand tile is [P rows][64 B] SWIZZLE_64B (layout type 4 in descriptor bits 61-63, SBO = 512 B between 8-row groups,
     // LBO unused); a k16 step is 32 B inside the row, a tap offset of d rows is d * 64 B.  The swizzle is a function of the absolute
     // shared-memory address (buffers are 1 KB aligned), so the shifted views need no base-offset field (tools/micro/im2col_umma_test.cu)
@@ -1533,8 +1345,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
       const bool two = tg.mt == 2;
       const int phase = (GEO == GEO_UP) ? n_tile / p.tiles_per_phase : 0;
       const int as = it & 1;
-      if (DMN_EXP_ACC_RELAXED) mbar_wait_relaxed(smem_u32(&acc_empty[as]), ((it >> 1) & 1) ^ 1);
-      else mbar_wait(smem_u32(&acc_empty[as]), ((it >> 1) & 1) ^ 1);      // epilogue has drained this accumulator set
+      mbar_wait(smem_u32(&acc_empty[as]), ((it >> 1) & 1) ^ 1);      // epilogue has drained this accumulator set
       tc_fence_after();
       if (leader) TRACE(it, 4);
       const uint32_t d0 = tmem_base + (uint32_t)(as * 2 * NT), d1 = d0 + (uint32_t)NT;
@@ -1544,20 +1355,19 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
         long long w0 = tracing ? clock64() : 0;
         mbar_wait(smem_u32(&full_a[cbuf]), cph);
         if (tracing) wait_a += clock64() - w0;
-        if (DMN_EXP_FENCE_MODE == 2) fence_proxy_async();     // consumer-side generic -> async proxy fence (see DMN_EXP_FENCE_MODE)
-        if (!DMN_EXP_NO_FENCE) tc_fence_after();
+        tc_fence_after();
         if (c == 0 && leader) TRACE(it, 5);
         const uint32_t au = a_units0 + (uint32_t)cbuf * a_buf_units;
         if constexpr (SWAP && (lean9 || lean4)) {
           const uint32_t au_lo = au | lbo_a_f, acc0 = c ? 1u : 0u;
           const uint32_t ids = two ? idesc_s2 : idesc_s1;
           if constexpr (lean9) {
-            issue_pass_swap<9, 3>(leader, d0, au_lo, dl9, b_lo0, b_stage_units, b_tap_units, hi_a, hi_b, a_k16, b_k16, ids, acc0, full_b, empty_b, nst, st, ph, cmask);
+            issue_pass_swap<9, 3>(leader, d0, au_lo, dl9, b_lo0, b_stage_units, b_tap_units, hi_a, hi_b, a_k16, b_k16, ids, acc0, full_b, empty_b, nst, st, ph);
           } else {
             int dl4[4];
 #pragma unroll
             for (int t = 0; t < 4; ++t) dl4[t] = p.delta[phase * 16 + t];
-            issue_pass_swap<4, 2>(leader, d0, au_lo, dl4, b_lo0, b_stage_units, b_tap_units, hi_a, hi_b, a_k16, b_k16, ids, acc0, full_b, empty_b, nst, st, ph, cmask);
+            issue_pass_swap<4, 2>(leader, d0, au_lo, dl4, b_lo0, b_stage_units, b_tap_units, hi_a, hi_b, a_k16, b_k16, ids, acc0, full_b, empty_b, nst, st, ph);
           }
         } else if constexpr (lean9 || lean4) {
           const uint32_t au_lo = au | lbo_a_f, acc0 = c ? 1u : 0u;
@@ -1577,7 +1387,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
           w0 = tracing ? clock64() : 0;
           mbar_wait(smem_u32(&full_b[st]), ph);
           if (tracing) wait_b += clock64() - w0;
-          if (!DMN_EXP_NO_FENCE) tc_fence_after();
+          tc_fence_after();
           const uint32_t bs = b_units0 + (uint32_t)st * b_stage_units;
           const uint32_t acc0 = c ? 1u : 0u;
           if constexpr (SWAP) {
@@ -1614,7 +1424,7 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
             else if (G == 2) issue_stage<2, false>(p, leader, d0, d1, au, bs, phase * 16 + t0, t0, acc0, idesc, hi_a, hi_b, lbo_a_f, lbo_b_f, a_k16, b_k16, b_tap_units, a_half);
             else issue_stage<1, false>(p, leader, d0, d1, au, bs, phase * 16 + t0, t0, acc0, idesc, hi_a, hi_b, lbo_a_f, lbo_b_f, a_k16, b_k16, b_tap_units, a_half);
           }
-          if (leader) commit_stage(smem_u32(&empty_b[st]), cmask);     // frees the weight stage once these MMAs retire
+          if (leader) umma_commit(smem_u32(&empty_b[st]));     // frees the weight stage once these MMAs retire
           __syncwarp();
           if (++st == nst) { st = 0; ph ^= 1; }
         }
@@ -1631,137 +1441,8 @@ __global__ void __launch_bounds__((PW + EW + 2) * 32, 1) conv_tcgen05_kernel(con
     }
   }
 
-  if constexpr (TAIL) {
-    if (p.c.fin_out) {
-      // ---- grid barrier: every tile of the launch is stored, every statistics atomic has landed ----
-      __threadfence();
-      __syncthreads();
-      if (tid == 0) {
-        atomicAdd(p.c.fin_sync, 1u);
-        const long long t0 = clock64();
-        unsigned int seen;
-        do {
-          __nanosleep(64);
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(p.c.fin_sync) : "memory");
-          if (clock64() - t0 > 4000000000LL) __trap();
-        } while (seen < gridDim.x);
-      }
-      __syncthreads();
-      // ---- finalise this CTA's tiles: y = SiLU(GroupNorm(raw)) + res, 16-byte items, coalesced rows ----
-      constexpr int kAll = (PW + EW + 2) * 32;
-      float2* t_gn = reinterpret_cast<float2*>(smem);                          // [kNimgMax][8] (mean, rstd) of (image, group of this N tile)
-      float* t_gb = reinterpret_cast<float*>(t_gn + kNimgMax * 8);             // [2][128] gamma | beta of this N tile
-      unsigned long long* t_st = reinterpret_cast<unsigned long long*>(t_gb + 256);   // [kNimgMax][8][2] statistics of y (fixed point)
-      const int sh = p.cpg_out_shift, gpt = NT >> sh;                          // groups per N tile (<= 8)
-      const float inv_cnt_out = 1.f / (float)(p.HW * p.cpg_out);
-      const bf16* raw = (const bf16*)p.c.out;
-      const bf16* res = (const bf16*)p.c.fin_res;
-      bf16* fout = (bf16*)p.c.fin_out;
-      const int fog = p.c.fin_ostats ? p.c.fin_ogroups : 0;
-      const int fcpg = fog ? p.c.Cout / fog : 1;                               // channels per statistics group of y (>= 16)
-      const int chunk = tid & 15, row0 = tid >> 4;                             // this thread's 8 channels of the N tile; first row
-      for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-        const TileGeom tg = tile_geom(tile, p);
-        const int m0 = tg.m0, rows = tg.mt * 128, n0 = tg.n_tile * NT;
-        const int img0 = m0 / p.S, rem0 = m0 - img0 * p.S;
-        for (int i = tid; i < kNimgMax * gpt; i += kAll) {
-          const int il = i / gpt, g = i - il * gpt, img = img0 + il;
-          float mean = 0.f, rstd = 0.f;
-          if (img < p.c.B) gn_mean_rstd(p.c.ostats + ((long)img * p.c.ogroups + (n0 >> sh) + g) * 2, inv_cnt_out, kGnEps, mean, rstd);
-          t_gn[il * 8 + g] = make_float2(mean, rstd);
-        }
-        for (int i = tid; i < NT; i += kAll) {
-          t_gb[i] = p.c.fin_gamma[n0 + i];
-          t_gb[128 + i] = p.c.fin_beta[n0 + i];
-        }
-        if (fog)
-          for (int i = tid; i < kNimgMax * 16; i += kAll) t_st[i] = 0ull;
-        __syncthreads();
-        float ga[8], be[8];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) { ga[e] = t_gb[chunk * 8 + e]; be[e] = t_gb[128 + chunk * 8 + e]; }
-        const int gl = (chunk * 8) >> sh;                                      // group of this thread's channels within the N tile
-        constexpr int RS = kAll / 16, U = 4;                                   // row stride between a thread's rows; rows in flight
-        for (int rb = row0; rb < rows; rb += U * RS) {
-          long off[U];
-          int iml[U];
-          uint4 rv[U], sv[U];
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            const int r = rb + u * RS;
-            off[u] = -1;
-            iml[u] = 0;
-            if (r < rows) {
-              const VPos v = vdecode_rel(img0, rem0, r, p);
-              if (v.img >= 0 && v.row >= p.pad && v.col >= p.pad) {
-                off[u] = ((long)v.img * p.HW + (v.row - p.pad) * p.W + (v.col - p.pad)) * p.c.Cout + n0 + chunk * 8;
-                iml[u] = v.img - img0;
-              }
-            }
-          }
-#pragma unroll
-          for (int u = 0; u < U; ++u)
-            if (off[u] >= 0) {
-              asm volatile("ld.global.cg.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(rv[u].x), "=r"(rv[u].y), "=r"(rv[u].z), "=r"(rv[u].w) : "l"(raw + off[u]));
-              asm volatile("ld.global.cg.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(sv[u].x), "=r"(sv[u].y), "=r"(sv[u].z), "=r"(sv[u].w) : "l"(res + off[u]));
-            }
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            const bool valid = off[u] >= 0;
-            float y[8];
-            float s8 = 0.f, q8 = 0.f;
-            if (valid) {
-              float xr[8], xs[8];
-              unpack8(rv[u], xr);
-              unpack8(sv[u], xs);
-              const float2 mr = t_gn[iml[u] * 8 + gl];
-#pragma unroll
-              for (int e = 0; e < 8; ++e) {
-                const float sc = mr.y * ga[e];
-                y[e] = silu_fast(fmaf(xr[e], sc, be[e] - mr.x * sc)) + xs[e];
-                s8 += y[e];
-                q8 = fmaf(y[e], y[e], q8);
-              }
-              *reinterpret_cast<uint4*>(fout + off[u]) = pack8(y);
-            }
-            if (fog) {
-              // lanes 0-15 / 16-31 of a warp hold one pixel row each: reduce over the lanes that share a statistics group of y, then one
-              // fixed-point shared-memory atomic per (row, group): order independent => deterministic
-              const int span = fcpg >= 128 ? 16 : (fcpg >> 3);                 // lanes (8-channel chunks) per group inside the N tile
-#pragma unroll
-              for (int o = 8; o > 0; o >>= 1)
-                if (o < span) { s8 += __shfl_xor_sync(0xffffffffu, s8, o); q8 += __shfl_xor_sync(0xffffffffu, q8, o); }
-              if (valid && (chunk & (span - 1)) == 0) {
-                const int og = (n0 + chunk * 8) / fcpg;                        // statistics group of y (global index)
-                const int slot = (iml[u] * 8 + (og & 7)) * 2;
-                atomicAdd(&t_st[slot], (unsigned long long)__float2ll_rn(s8 * kStatScaleSum));
-                atomicAdd(&t_st[slot + 1], (unsigned long long)__float2ll_rn(q8 * kStatScaleSq));
-              }
-            }
-          }
-        }
-        __syncthreads();
-        if (fog) {
-          // flush the tile's partial statistics: slot (image, og & 7) -> global (image, og); with fog == 1 only slot 0 of an image is used
-          const int og_base = fog == 1 ? 0 : (n0 / fcpg);
-          const int nog = fog == 1 ? 1 : NT / fcpg;
-          for (int i = tid; i < kNimgMax * nog; i += kAll) {
-            const int il = i / nog, k = i - il * nog, img = img0 + il;
-            const int og = og_base + k;
-            const unsigned long long a = t_st[(il * 8 + (og & 7)) * 2], b2 = t_st[(il * 8 + (og & 7)) * 2 + 1];
-            if (img < p.c.B && (a | b2)) {
-              atomicAdd(reinterpret_cast<unsigned long long*>(p.c.fin_ostats) + ((long)img * fog + og) * 2, a);
-              atomicAdd(reinterpret_cast<unsigned long long*>(p.c.fin_ostats) + ((long)img * fog + og) * 2 + 1, b2);
-            }
-          }
-          __syncthreads();
-        }
-      }
-    }
-  }
   tc_fence_before();
   __syncthreads();
-  if (p.cl > 1) cluster_sync_all();      // nobody leaves while a peer may still multicast into its shared memory
   if (warp == kMmaW) {
     tc_fence_after();
     tmem_dealloc(tmem_base, p.tmem_cols);
@@ -1776,7 +1457,6 @@ static size_t smem_fixed_bytes(const Params& p) {
          2 * (size_t)p.c.Cout * 4 + (p.c.fold_s1 ? (size_t)p.c.B * 8 : 0) + 32;
 }
 static size_t smem_bytes(const Params& p) { return smem_fixed_bytes(p) + (size_t)p.nstage * p.stage_bytes; }
-constexpr size_t kSmemLimit = (size_t)DMN_EXP_SMEM_KB * 1024;     // a CTA may opt in to 227 KB
 // taps per weight stage: a whole filter row for 3x3, a tap pair for the 2x2 forms; bulk copies of 16-24 KB stream well
 static bool pick_stages(Params& p) {
   const size_t fixed = smem_fixed_bytes(p);
@@ -1807,15 +1487,6 @@ static int swap_mode() {
     return !e ? 2 : (e[0] == '1' ? 1 : (e[0] == '0' ? 0 : 2));
   }();
   return m;
-}
-static bool cluster_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("DMN_CONV_CLUSTER");
-    return e && e[0] == '1';                // EXPERIMENT, default off: CTA pairs share the weight stream through multicast bulk copies.
-                                            // Measured neutral (+-1 % per conv: the weight stream from L2 is not what bounds the engine, the
-                                            // shared-memory port is) and one unit test (3x3 128->128 @16x16, batch 2) does not pass with it.
-  }();
-  return on;
 }
 
 // ---- TMA operand path ----
@@ -1911,28 +1582,20 @@ static bool fill_params(const ConvP& c, int geo, Params& p) {
     p.mcta = 128 * p.mt;
   }
   p.halo_hi = halo_hi;
-  // clusters of two CTAs sharing the weight stream (multicast): the swapped-role hot instantiations with enough tiles for every SM
-  p.cl = 1;
-  if (swap_mode() == 1 && cluster_enabled() && geo != GEO_INIT && p.NT == 128 && !(c.pro & PRO_LRELU) && !c.res && !c.fold_s1 &&
-      (geo != GEO_SAME || p.ntap == 9) && (num_sms() % 2) == 0)
-    p.cl = 2;
   {
     // mixed tiling: whole rounds of 256-row tiles, the remainder in 128-row tiles (the last round then costs half)
     const long nsm = num_sms();
     const long m2 = (p.total_flat + 255) / 256, t2 = m2 * p.n_tiles_n;
-    const long clm = p.cl;       // M-tile counts are multiples of the cluster size (a tile past the end of the flat range computes nothing)
     if (p.mt == 2) {
       long big_m = m2;
       if (t2 % nsm != 0) big_m = (t2 / nsm) * nsm / p.n_tiles_n;       // m-tiles inside the whole rounds
-      big_m = big_m / clm * clm;
       long rem = p.total_flat - big_m * 256;
       long small_m = rem > 0 ? (rem + 127) / 128 : 0;
-      small_m = (small_m + clm - 1) / clm * clm;
       // a 128-row tile costs ~0.6 of a 256-row tile (it streams the same weights): mix only when the estimate is lower
       const double cost_uniform = (double)((t2 + nsm - 1) / nsm);
       const double cost_mixed = (double)(t2 / nsm) + 0.6 * (double)((small_m * p.n_tiles_n + nsm - 1) / nsm);
       if (cost_mixed >= cost_uniform - 0.05) {
-        big_m = (m2 + clm - 1) / clm * clm;
+        big_m = m2;
         rem = 0;
         small_m = 0;
       }
@@ -1942,16 +1605,13 @@ static bool fill_params(const ConvP& c, int geo, Params& p) {
     } else {
       p.n_big_tiles = 0;
       p.big_rows = 0;
-      p.total_tiles = (int)(((p.total_flat + 127) / 128 + clm - 1) / clm * clm) * p.n_tiles_n;
+      p.total_tiles = (int)((p.total_flat + 127) / 128) * p.n_tiles_n;
     }
     p.m_tiles = p.total_tiles / p.n_tiles_n;
   }
   p.P = p.mcta + p.halo_lo + halo_hi;
   p.PA = p.P;
-  {
-    static const bool align_taps = [] { const char* e = getenv("DMN_EXP_ALIGN_TAPS"); return e && e[0] == '1'; }();
-    while (p.PA % 8 != (align_taps ? 0 : 2)) ++p.PA;
-  }
+  while (p.PA % 8 != 2) ++p.PA;
   if (geo != GEO_INIT && (4 * p.P + kProdThreads - 1) / kProdThreads > kMaxItems) return false;
   if (kMcta / p.S + 3 > kNimgMax || p.S < 16) return false;
   p.lbo_a = (uint32_t)p.PA * 16u;
@@ -1993,33 +1653,24 @@ static bool fill_params(const ConvP& c, int geo, Params& p) {
   p.magic_S = (uint32_t)(((1ull << 26) + p.S - 1) / p.S);
   p.magic_W = (uint32_t)(((1ull << 24) + p.Wv - 1) / p.Wv);
   p.magic64_S = ~0ull / (unsigned long long)p.S + 1ull;
-  p.pg_shift = 0;
-  while (c.pgroups > 0 && (1 << p.pg_shift) < c.pgroups) ++p.pg_shift;
   for (int ph = 0; ph < 4; ++ph)
     for (int t = 0; t < 16; ++t) p.delta[ph * 16 + t] = t < p.ntap ? tap_delta(p, geo, t, ph) : 0;
-  {
-    // timing experiment only (results are wrong): every tap offset rounded so that the shifted operand view starts on an 8-row
-    // (128-byte) boundary -- measures what the unaligned start addresses of the shifted views cost the tensor core's operand fetch
-    static const bool align_taps = [] { const char* e = getenv("DMN_EXP_ALIGN_TAPS"); return e && e[0] == '1'; }();
-    if (align_taps)
-      for (int i = 0; i < 64; ++i) p.delta[i] = (p.halo_lo + p.delta[i]) / 8 * 8 - p.halo_lo;
-  }
-  p.abuf = (geo == GEO_SAME && p.NT == 128 && p.ntap == 1 && c.pro == PRO_NONE && !DMN_EXP_NO_ONETAP) ? kABufOne : kABuf;
+  p.abuf = (geo == GEO_SAME && p.NT == 128 && p.ntap == 1 && c.pro == PRO_NONE) ? kABufOne : kABuf;
   // plain swapped-role instantiations (launch<>: hot path without prologue)
   {
-    const bool eligible = geo != GEO_INIT && p.NT == 128 && !(c.pro & PRO_LRELU) && !c.res && !c.fold_s1 && !c.fin_out && (geo != GEO_SAME || p.ntap == 9);
+    const bool eligible = geo != GEO_INIT && p.NT == 128 && !(c.pro & PRO_LRELU) && !c.res && !c.fold_s1 && (geo != GEO_SAME || p.ntap == 9);
     // the rule depends on the per-image geometry only, never on the batch: the two forms sum the GroupNorm statistics in different
     // fp32 orders, so a sample must meet the same form whatever batch it is part of (batch-slice invariance)
     const bool rule = atma_enabled() && p.S >= 64 && (p.n_pass >= 8 || (geo == GEO_SAME && c.pro == PRO_NONE));
     p.swap = eligible && (swap_mode() == 1 || (swap_mode() == 2 && rule));
   }
-  if (p.swap && c.pro == PRO_NONE) p.abuf = DMN_EXP_PLAIN_ABUF;
+  if (p.swap && c.pro == PRO_NONE) p.abuf = kABufPlain;
   // the GroupNorm-prologue instantiation (PRO = 1) is launched for 128-column tiles without residual / fold / FiLM (launch<>)
   if (geo == GEO_SAME && p.NT == 128 && c.pro != PRO_NONE && !(c.pro & PRO_LRELU) && !c.res && !c.fold_s1) p.abuf = kABufPro;
   // TMA operand path: the hot instantiations (launch<>: 128-column tiles, 3x3 / k4s2 / transposed k4s2, no FiLM / residual / fold terms)
-  const bool hot = geo != GEO_INIT && p.NT == 128 && !(c.pro & PRO_LRELU) && !c.res && !c.fold_s1 && !c.fin_out &&
+  const bool hot = geo != GEO_INIT && p.NT == 128 && !(c.pro & PRO_LRELU) && !c.res && !c.fold_s1 &&
                    ((geo == GEO_SAME && (p.ntap == 9 || (p.ntap == 1 && c.pro == PRO_NONE))) || geo == GEO_DOWN || geo == GEO_UP);
-  // (prologue form: power-of-two group count <= 16 and one table entry per producer thread -- the double-buffered (mean, rstd) table)
+  // (prologue form: power-of-two group count <= 16, at most one (mean, rstd) table entry per producer thread)
   const bool pro_ok = c.pro == PRO_NONE || ((c.pro & PRO_GN) && kNimgMax * c.pgroups <= kProdThreads && c.pgroups <= 16 && (c.pgroups & (c.pgroups - 1)) == 0);
   if (hot && pro_ok && atma_enabled() && p.P <= 1024 && p.halo_lo < p.S) {
     Params q = p;
@@ -2079,40 +1730,29 @@ static void log_launch(const void* fn, int grid, int threads, const Params& p) {
   if (g_log.size() < (size_t)kLogMax) g_log.push_back(r);
 }
 
-template <typename K>
-static cudaError_t launch_kernel(K kern, int grid, int threads, const Params& p, cudaStream_t st, bool cooperative = false) {
+typedef void (*ConvKernel)(Params);
+
+static cudaError_t launch_kernel(ConvKernel kern, int grid, int threads, const Params& p, cudaStream_t st) {
   const cudaError_t e = ensure_smem_attr((const void*)kern);
   if (e != cudaSuccess) return e;
   log_launch((const void*)kern, grid, threads, p);
-  if (cooperative) {      // grid-wide barrier inside the kernel: the runtime guarantees (or refuses) co-residency of the whole grid
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = smem_bytes(p);
-    cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeCooperative;
-    at[0].val.cooperative = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kern, p);
+  return launch_pdl(kern, dim3(grid), dim3(threads), smem_bytes(p), st, p);
+}
+
+// The hot instantiations: 128-column tiles without FiLM, residual or fold terms, on the operand feed ATMA with operand roles SWAP.
+// Sets `ew16` when it picks a 16-epilogue-warp form.
+template <int GEO, bool SWAP, bool ATMA>
+static ConvKernel hot_kernel(bool pro, bool lean, bool lean_shape, bool& ew16) {
+  if constexpr (GEO == GEO_SAME) {
+    if (pro) return lean ? conv_tcgen05_kernel<GEO, 128, false, true, false, 1, 8, SWAP, ATMA> : conv_tcgen05_kernel<GEO, 128, false, false, false, 1, 8, SWAP, ATMA>;
+    if (lean) return conv_tcgen05_kernel<GEO, 128, false, true, false, 0, 8, SWAP, ATMA>;
+    // epilogue-bound plain 3x3 tiles (fewer than kLeanMinPass passes): 16 epilogue warps; ncu then shows the epilogue waiting for the
+    // accumulators 24 % of the time, so these tiles take the lean issue path as well
+    ew16 = true;
+    return lean_shape ? conv_tcgen05_kernel<GEO, 128, false, true, false, 0, 16, SWAP, ATMA> : conv_tcgen05_kernel<GEO, 128, false, false, false, 0, 16, SWAP, ATMA>;
+  } else {
+    return lean ? conv_tcgen05_kernel<GEO, 128, false, true, false, 0, 8, SWAP, ATMA> : conv_tcgen05_kernel<GEO, 128, false, false, false, 0, 8, SWAP, ATMA>;
   }
-  if (p.cl <= 1) return launch_pdl(kern, dim3(grid), dim3(threads), smem_bytes(p), st, p);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid / p.cl * p.cl);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem_bytes(p);
-  cfg.stream = st;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = (unsigned)p.cl;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
-  return cudaLaunchKernelEx(&cfg, kern, p);
 }
 
 template <int GEO>
@@ -2128,160 +1768,34 @@ static int launch(Params p, cudaStream_t st) {
     p.trace = (long long*)sym;
     p.trace_cta = 3;
   }
-  static DeviceOnce attr_set;
-  if (attr_set.first()) {
-    DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<GEO, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<GEO, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<GEO, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    if (GEO == GEO_SAME) {
-      DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<GEO_SAME, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-      DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<GEO_SAME, 64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-      DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<GEO_SAME, 128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    }
-  }
   const int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
-  // measured rule for the lean issue path: with fewer than DMN_EXP_LEAN_MIN_PASS passes per tile the tile is epilogue-bound and the
-  // faster main loop only adds contention (level-0 convs 0.078 -> 0.084 ms), so those keep the looped path
-  const bool lean_ok = !DMN_EXP_NO_LEAN && p.NT == 128 && !(p.c.pro & PRO_LRELU) && p.n_pass >= DMN_EXP_LEAN_MIN_PASS &&
-                       ((GEO == GEO_SAME && p.ntap == 9 && p.G == 3) || ((GEO == GEO_DOWN || GEO == GEO_UP) && p.ntap == 4 && p.G == 2));
+  const bool film = (p.c.pro & PRO_LRELU) != 0;
   const bool extra = p.c.res != nullptr || p.c.fold_s1 != nullptr;
-  if (GEO == GEO_SAME && p.NT == 128 && p.ntap == 1 && p.c.pro == PRO_NONE && !DMN_EXP_NO_ONETAP) {
-    // 1x1 convolutions (to_qkv with the folded GroupNorm, to_out, res_conv): table-free producers
-    constexpr int G2 = GEO_SAME;
-    static DeviceOnce one_attr;
-    if (one_attr.first()) {
-      DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<G2, 128, false, false, true, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-      DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<G2, 128, false, false, false, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
+  ConvKernel kern = nullptr;
+  bool ew16 = false;
+  if (GEO == GEO_SAME && p.NT == 128 && p.ntap == 1 && p.c.pro == PRO_NONE) {
+    // 1x1 convolutions (to_qkv with the folded GroupNorm, to_out, res_conv): table-free producers, 16 epilogue warps
+    ew16 = true;
+    if (p.atma) kern = conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 3, 16, false, true>;
+    else if (extra) kern = conv_tcgen05_kernel<GEO_SAME, 128, false, false, true, 3, 16>;
+    else kern = conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 3, 16>;
+  } else if (GEO != GEO_INIT && p.NT == 128 && !film && !extra) {
+    if constexpr (GEO != GEO_INIT) {
+      const bool pro = GEO == GEO_SAME && p.c.pro != PRO_NONE;
+      // lean (unrolled) issue path: 9 taps in stages of 3, or 4 in stages of 2, with at least kLeanMinPass passes.  The 2x2 forms on
+      // the TMA feed with plain roles take it whatever the pass count (transposed 16x16 -> 32x32 conv 0.0392 -> 0.0299 ms)
+      const bool lean_shape = (GEO == GEO_SAME && p.ntap == 9 && p.G == 3) || (GEO != GEO_SAME && p.ntap == 4 && p.G == 2);
+      const bool lean = lean_shape && (p.n_pass >= kLeanMinPass || (GEO != GEO_SAME && p.atma && !p.swap));
+      const auto pick = p.swap ? (p.atma ? hot_kernel<GEO, true, true> : hot_kernel<GEO, true, false>)
+                               : (p.atma ? hot_kernel<GEO, false, true> : hot_kernel<GEO, false, false>);
+      kern = pick(pro, lean, lean_shape, ew16);
     }
-    if (p.atma && !extra) {
-      if (DMN_EXP_EW16) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 3, 16, false, 8, false, true>, grid, kThreads16, p, st));
-      else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 3, 8, false, 8, false, true>, grid, kThreads, p, st));
-      count_launch();
-      DMN_LAUNCH_CHECK("conv_tcgen05");
-      return 0;
-    }
-    if (DMN_EXP_EW16) {
-      static DeviceOnce a16;
-      if (a16.first()) {
-        DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<G2, 128, false, false, true, 3, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-        DMN_CUDA_CHECK(cudaFuncSetAttribute(conv_tcgen05_kernel<G2, 128, false, false, false, 3, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-      }
-      if (extra) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, true, 3, 16>, grid, kThreads16, p, st));
-      else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 3, 16>, grid, kThreads16, p, st));
-    } else if (extra) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, true, 3>, grid, kThreads, p, st));
-    else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 3>, grid, kThreads, p, st));
-    count_launch();
-    DMN_LAUNCH_CHECK("conv_tcgen05");
-    return 0;
+  } else if (GEO == GEO_SAME && film) {
+    kern = p.NT == 128 ? conv_tcgen05_kernel<GEO_SAME, 128, true> : (p.NT == 64 ? conv_tcgen05_kernel<GEO_SAME, 64, true> : conv_tcgen05_kernel<GEO_SAME, 32, true>);
+  } else {
+    kern = p.NT == 128 ? conv_tcgen05_kernel<GEO, 128> : (p.NT == 64 ? conv_tcgen05_kernel<GEO, 64> : conv_tcgen05_kernel<GEO, 32>);
   }
-  if (GEO != GEO_INIT && p.NT == 128 && !(p.c.pro & PRO_LRELU) && !extra) {
-    // the hot instantiations: no residual / fold terms in the epilogue, lean or looped issue
-    constexpr int G2 = GEO == GEO_INIT ? GEO_SAME : GEO;
-    const bool swap_on = p.swap != 0;
-    const bool pro = G2 == GEO_SAME && p.c.pro != PRO_NONE;
-    if (G2 == GEO_SAME && p.c.fin_out) {
-      // ResnetBlock.block2 with the block tail fused behind a grid barrier (cooperative launch)
-      if (!pro || p.ntap != 9) return fail(-2, "conv_tcgen05: the fused block tail needs the GroupNorm-prologue 3x3 instantiation");
-      if (lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, false, 8, true>, grid, kThreads, p, st, true));
-      else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, false, 8, true>, grid, kThreads, p, st, true));
-      count_launch();
-      DMN_LAUNCH_CHECK("conv_tcgen05");
-      return 0;
-    }
-    if (swap_on && (G2 != GEO_SAME || p.ntap == 9)) {
-      static const bool pw16 = [] { const char* e = getenv("DMN_CONV_PW16"); return e && e[0] == '1'; }();
-      if (p.atma) {
-        static const bool pro_lean_s = [] { const char* e = getenv("DMN_CONV_PRO_LEAN"); return e && e[0] == '1'; }();
-        if (pro && !pw16 && pro_lean_s && p.ntap == 9 && p.G == 3) {
-          DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, true, 8, false, true>, grid, kThreads, p, st));
-          count_launch();
-          DMN_LAUNCH_CHECK("conv_tcgen05");
-          return 0;
-        }
-        if (pro && pw16 && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, true, 16, false, true>, grid, kThreads16, p, st));
-        else if (pro && pw16) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, true, 16, false, true>, grid, kThreads16, p, st));
-        else if (pro && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, true, 8, false, true>, grid, kThreads, p, st));
-        else if (pro) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, true, 8, false, true>, grid, kThreads, p, st));
-        else if (lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, true, false, 0, 8, true, 8, false, true>, grid, kThreads, p, st));
-        else if (DMN_EXP_EW16 && G2 == GEO_SAME) {
-          if (DMN_EXP_EW16_LEAN && p.ntap == 9 && p.G == 3)
-            DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 0, 16, true, 8, false, true>, grid, kThreads16, p, st));
-          else
-            DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 0, 16, true, 8, false, true>, grid, kThreads16, p, st));
-        } else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 0, 8, true, 8, false, true>, grid, kThreads, p, st));
-        count_launch();
-        DMN_LAUNCH_CHECK("conv_tcgen05");
-        return 0;
-      }
-      if (pro && pw16 && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, true, 16>, grid, kThreads16, p, st));
-      else if (pro && pw16) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, true, 16>, grid, kThreads16, p, st));
-      else if (pro && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, true>, grid, kThreads, p, st));
-      else if (pro) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, true>, grid, kThreads, p, st));
-      else if (lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, true, false, 0, 8, true>, grid, kThreads, p, st));
-      else if (DMN_EXP_EW16 && G2 == GEO_SAME) {
-        if (DMN_EXP_EW16_LEAN && p.ntap == 9 && p.G == 3)
-          DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 0, 16, true>, grid, kThreads16, p, st));
-        else
-          DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 0, 16, true>, grid, kThreads16, p, st));
-      } else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 0, 8, true>, grid, kThreads, p, st));
-      count_launch();
-      DMN_LAUNCH_CHECK("conv_tcgen05");
-      return 0;
-    }
-    if (p.atma) {
-      // TMA operand path (fill_params).  The 2x2 forms take the unrolled issue loop whatever the pass count (transposed 16x16 -> 32x32 conv
-      // 0.0392 -> 0.0299 ms); the GroupNorm-prologue 3x3 keeps the round-1 rule (level-0: 0.0843 ms looped, 0.0877 ms unrolled)
-      const bool lean4 = !DMN_EXP_NO_LEAN && (GEO == GEO_DOWN || GEO == GEO_UP) && p.ntap == 4 && p.G == 2;
-      const bool lean_ok = lean4 || (!DMN_EXP_NO_LEAN && GEO == GEO_SAME && p.n_pass >= (pro ? DMN_EXP_LEAN_MIN_PASS_TMA_PRO : DMN_EXP_LEAN_MIN_PASS) && p.ntap == 9 && p.G == 3);
-      static const bool pw16a = [] { const char* e = getenv("DMN_CONV_PW16"); return e && e[0] == '1'; }();     // (64 registers per producer spill the grouped transform)
-      // EXPERIMENT (DMN_CONV_PW=12): 12 producer warps (704 threads leave 88 registers per thread, enough for the grouped transform);
-      // DMN_CONV_PRO_LEAN=1: the unrolled issue loop for the prologue convs at any pass count
-      static const bool pw12 = [] { const char* e = getenv("DMN_CONV_PW"); return e && !strcmp(e, "12"); }();
-      static const bool pro_lean = [] { const char* e = getenv("DMN_CONV_PRO_LEAN"); return e && e[0] == '1'; }();
-      const bool lean_pro = lean_ok || (pro_lean && pro && p.ntap == 9 && p.G == 3);
-      if (pro && pw12 && lean_pro) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, false, 12, false, true>, grid, (12 + 8 + 2) * 32, p, st));
-      else if (pro && pw12) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, false, 12, false, true>, grid, (12 + 8 + 2) * 32, p, st));
-      else if (pro && pro_lean && lean_pro && !pw16a) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, false, 8, false, true>, grid, kThreads, p, st));
-      else if (pro && pw16a && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, false, 16, false, true>, grid, kThreads16, p, st));
-      else if (pro && pw16a) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, false, 16, false, true>, grid, kThreads16, p, st));
-      else if (pro && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, false, 8, false, true>, grid, kThreads, p, st));
-      else if (pro) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, false, 8, false, true>, grid, kThreads, p, st));
-      else if (lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, true, false, 0, 8, false, 8, false, true>, grid, kThreads, p, st));
-      else if (DMN_EXP_EW16 && G2 == GEO_SAME) {
-        if (DMN_EXP_EW16_LEAN && p.ntap == 9 && p.G == 3)
-          DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 0, 16, false, 8, false, true>, grid, kThreads16, p, st));
-        else
-          DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 0, 16, false, 8, false, true>, grid, kThreads16, p, st));
-      } else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 0, 8, false, 8, false, true>, grid, kThreads, p, st));
-      count_launch();
-      DMN_LAUNCH_CHECK("conv_tcgen05");
-      return 0;
-    }
-    static const bool pw16n = [] { const char* e = getenv("DMN_CONV_PW16"); return e && e[0] == '1'; }();
-    if (pro && pw16n && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1, 8, false, 16>, grid, kThreads16, p, st));
-    else if (pro && pw16n) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1, 8, false, 16>, grid, kThreads16, p, st));
-    else if (pro && lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 1>, grid, kThreads, p, st));
-    else if (pro) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 1>, grid, kThreads, p, st));
-    else if (lean_ok) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, true, false, 0>, grid, kThreads, p, st));
-    else if (DMN_EXP_EW16 && G2 == GEO_SAME) {
-      // epilogue-bound plain 3x3 tiles (fewer than 8 passes): 16 epilogue warps; ncu then shows the epilogue waiting for the
-      // accumulators 24 % of the time, so these tiles take the lean issue path as well (DMN_EXP_EW16_LEAN)
-      if (DMN_EXP_EW16_LEAN && p.ntap == 9 && p.G == 3)
-        DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, true, false, 0, 16>, grid, kThreads16, p, st));
-      else
-        DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, false, false, false, 0, 16>, grid, kThreads16, p, st));
-    } else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<G2, 128, false, false, false, 0>, grid, kThreads, p, st));
-    count_launch();
-    DMN_LAUNCH_CHECK("conv_tcgen05");
-    return 0;
-  }
-  if (GEO == GEO_SAME && (p.c.pro & PRO_LRELU)) {
-    if (p.NT == 128) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 128, true>, grid, kThreads, p, st));
-    else if (p.NT == 64) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 64, true>, grid, kThreads, p, st));
-    else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO_SAME, 32, true>, grid, kThreads, p, st));
-  } else if (p.NT == 128) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO, 128>, grid, kThreads, p, st));
-  else if (p.NT == 64) DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO, 64>, grid, kThreads, p, st));
-  else DMN_CUDA_CHECK(launch_kernel(conv_tcgen05_kernel<GEO, 32>, grid, kThreads, p, st));
+  DMN_CUDA_CHECK(launch_kernel(kern, grid, ew16 ? kThreads16 : kThreads, p, st));
   count_launch();
   DMN_LAUNCH_CHECK("conv_tcgen05");
   return 0;
@@ -2292,23 +1806,6 @@ static int launch(Params p, cudaStream_t st) {
 bool conv_tcgen05_supported(const ConvP& c) {
   tc::Params p;
   return tc::fill_params(c, tc::geo_of(c), p);
-}
-// can this convolution carry the fused block tail (ConvP::fin_*)?  fin_ogroups = statistics groups of the tail's output (0 = none)
-bool conv_tcgen05_tail_supported(const ConvP& c) {
-  tc::Params p;
-  if (c.mode != CONV_SAME || c.ksize != 3 || !tc::fill_params(c, tc::GEO_SAME, p)) return false;
-  if (p.NT != 128 || !(c.pro & PRO_GN) || (c.pro & PRO_LRELU) || c.res || c.fold_s1 || c.ogroups <= 0 || p.cpg_out < 16) return false;
-  if (c.fin_ogroups < 0 || (c.fin_ogroups > 0 && c.Cout % c.fin_ogroups)) return false;
-  if (c.fin_ogroups > 0) {
-    const int fcpg = c.Cout / c.fin_ogroups;
-    if (fcpg < 16 || (fcpg < 128 && (fcpg & (fcpg - 1))) || (fcpg >= 128 && fcpg % 128)) return false;
-    if (fcpg >= 128 && c.fin_ogroups != 1) return false;      // a group wider than the N tile: only the single-group (GroupNorm(1)) form
-  }
-  // EXPERIMENT, default off (DMN_FUSED_FINALIZE=1): parity-green, but measured SLOWER than the separate gn_finalize launch -- level-0
-  // block2 conv + tail 0.168 ms against 0.101 + 0.044 ms: the pass over the CTA's own tiles runs at ~12 B/clk/SM behind the grid barrier
-  // (576 threads per SM, tiles no longer L2-resident after 8 rounds), the stand-alone kernel streams at 4.5 TB/s with 3 x 256 threads per SM
-  static const bool on = [] { const char* e = getenv("DMN_FUSED_FINALIZE"); return e && e[0] == '1'; }();
-  return on;
 }
 bool init_conv_tcgen05_supported(int Cin, int S, int Cout, int B) {
   ConvP c;
@@ -2408,14 +1905,6 @@ int conv_tcgen05(const ConvP& c, cudaStream_t st) {
   tc::Params p;
   const int geo = tc::geo_of(c);
   if (!tc::fill_params(c, geo, p)) return fail(-2, "conv_tcgen05: unsupported convolution shape");
-  static const bool swap = [] {
-    const char* e = getenv("DMN_UMMA_SWAP_LBO_SBO");
-    return e && e[0] == '1';
-  }();
-  if (swap) {   // negative control for the descriptor encoding (tests only)
-    std::swap(p.lbo_a, p.sbo_a);
-    std::swap(p.lbo_b, p.sbo_b);
-  }
   if (geo == tc::GEO_SAME) return tc::launch<tc::GEO_SAME>(p, st);
   if (geo == tc::GEO_DOWN) return tc::launch<tc::GEO_DOWN>(p, st);
   return tc::launch<tc::GEO_UP>(p, st);

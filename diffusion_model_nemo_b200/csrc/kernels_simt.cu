@@ -293,15 +293,8 @@ template <> struct VecIO<bf16, 8> {
 };
 
 // raw conv output and residual are dead (raw) or cold (residual) after this kernel while the result is read by the very next kernel:
-// streaming loads (evict-first) keep the 126 MB L2 for the output.  DMN_EXP_FIN_STREAM=0 restores plain loads.
-#ifndef DMN_EXP_FIN_STREAM
-#define DMN_EXP_FIN_STREAM 1
-#endif
-#if DMN_EXP_FIN_STREAM
+// streaming loads (evict-first) keep the 126 MB L2 for the output
 #define DMN_FIN_LD(ptr) __ldcs(ptr)
-#else
-#define DMN_FIN_LD(ptr) (*(ptr))
-#endif
 template <typename T, int V>
 __global__ void __launch_bounds__(256, 3) gn_finalize_kernel(const FinalizeP p) {
   pdl_trigger();

@@ -47,18 +47,7 @@ struct ConvP {
   const void* res = nullptr;       // optional residual added to the output (same layout as out)
   stat_t* ostats = nullptr;        // [B][ogroups][2] accumulated with integer atomics (must be zeroed beforehand)
   int ogroups = 0;
-  // fused block tail (tcgen05 engine, 3x3 with the GroupNorm prologue = ResnetBlock.block2): after a grid-wide barrier the persistent
-  // CTAs finalise their own tiles in place of a separate gn_finalize launch:
-  //   fin_out = SiLU(GroupNorm_ogroups(out; fin_gamma, fin_beta)) + fin_res      (+ statistics of fin_out into fin_ostats)
-  void* fin_out = nullptr;
-  const void* fin_res = nullptr;
-  const float* fin_gamma = nullptr;
-  const float* fin_beta = nullptr;
-  stat_t* fin_ostats = nullptr;    // [B][fin_ogroups][2] or null
-  int fin_ogroups = 0;
-  unsigned int* fin_sync = nullptr;   // grid barrier counter (zeroed beforehand)
 };
-bool conv_tcgen05_tail_supported(const ConvP& p);
 
 int conv_simt(const ConvP& p, int act, cudaStream_t s);
 int conv_tcgen05(const ConvP& p, cudaStream_t s);              // bf16 activations only

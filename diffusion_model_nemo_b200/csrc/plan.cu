@@ -125,10 +125,6 @@ struct Op {
   int ogroups = 0;
   int temb_col = -1;
   bool tc = false;                  // tcgen05 engine for this conv
-  // fused block tail (ConvP::fin_*): the finalize of the ResnetBlock rides on block2's conv
-  bool fin = false;
-  Buf fin_out, fin_res, fin_ostats, fin_sync;
-  int fin_gamma = -1, fin_beta = -1, fin_ogroups = 0;
   // to_qkv with the PreNorm GroupNorm(1) folded into weights + epilogue affine (ops.h: ConvP::fold_s1)
   bool fold = false;
   int fold_gamma = -1, fold_beta = -1;
@@ -307,7 +303,6 @@ struct Builder {
     int c1 = conv(p + ".block1.proj", CONV_SAME, 3, s1, C1, s2, C2, Cout, H, h1, true, G);
     int g1w = add_param(p + ".block1.norm.weight", {Cout}, PK_RAW);
     int g1b = add_param(p + ".block1.norm.bias", {Cout}, PK_RAW);
-    // the residual branch first: the fused tail of block2 reads it
     Buf res = s1;
     if (Cin != Cout) {
       conv(p + ".res_conv", CONV_SAME, 1, s1, C1, s2, C2, Cout, H, rbuf, true, 0);
@@ -319,25 +314,6 @@ struct Builder {
                   temb_col);
     int g2w = add_param(p + ".block2.norm.weight", {Cout}, PK_RAW);
     int g2b = add_param(p + ".block2.norm.bias", {Cout}, PK_RAW);
-    if (P.ops[c2].tc) {
-      // tensor-core engine: SiLU(GroupNorm(h2)) + residual is the tail of block2's conv launch (grid barrier + in-place pass over
-      // the CTA's own tiles) instead of a separate HBM pass
-      ConvP q;
-      q.mode = CONV_SAME; q.ksize = 3; q.C1 = Cout; q.Cout = Cout; q.B = P.cfg.max_batch; q.Hin = q.Win = q.Hout = q.Wout = H;
-      q.pro = pro; q.pgroups = G; q.ogroups = G; q.fin_ogroups = ostats_groups;
-      if (conv_tcgen05_tail_supported(q)) {
-        Op& o = P.ops[c2];
-        o.fin = true;
-        o.fin_out = out; o.fin_res = res; o.fin_gamma = g2w; o.fin_beta = g2b; o.fin_ogroups = ostats_groups;
-        if (ostats_groups > 0) {
-          o.fin_ostats = stats(ostats_groups);
-          if (ostats_out) *ostats_out = o.fin_ostats;
-        }
-        o.fin_sync.off = P.stats_off + P.stats_bytes;      // one counter in the (per-forward zeroed) statistics arena
-        P.stats_bytes += 256;
-        return;
-      }
-    }
     Op f;
     f.kind = OP_FINALIZE;
     f.name = p + ".finalize";
@@ -741,11 +717,6 @@ static int run_forward(dmn_plan* P, const float* x_dev, const int32_t* row_dev, 
         }
         q.out = B(o.out); q.res = B(o.res);
         q.ostats = (stat_t*)B(o.ostats); q.ogroups = o.ogroups;
-        if (o.fin) {
-          q.fin_out = B(o.fin_out); q.fin_res = B(o.fin_res); q.fin_gamma = W(o.fin_gamma); q.fin_beta = W(o.fin_beta);
-          q.fin_ostats = (stat_t*)B(o.fin_ostats); q.fin_ogroups = o.fin_ogroups;
-          q.fin_sync = (unsigned int*)B(o.fin_sync);
-        }
         rc = o.tc ? conv_tcgen05(q, st) : conv_simt(q, P->act, st);
         break;
       }
@@ -1077,7 +1048,6 @@ int dmn_plan_op_info(const dmn_plan* p, int i, char* name_out, int name_cap, int
       const double mpix = o.mode == CONV_UP ? (double)o.Hin * o.Hin : (double)o.Hout * o.Hout;   // MACs counted on the strided side
       fl = 2.0 * mpix * taps * cin * o.Cout;
       by = esz * ((double)o.Hin * o.Hin * cin + (double)o.Hout * o.Hout * o.Cout * (o.res.valid() ? 2.0 : 1.0)) + 2.0 * taps * cin * o.Cout / c.max_batch;
-      if (o.fin) by += esz * (double)o.Hout * o.Hout * o.Cout * 2.0;      // fused tail: + residual read, + final output written
       break;
     }
     case OP_FINALIZE: by = esz * (double)o.HW * o.C * 3.0; break;

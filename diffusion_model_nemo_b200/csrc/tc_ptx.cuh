@@ -52,26 +52,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                "r"(bytes), "r"(bar)
                : "memory");
 }
-// multicast forms (thread-block cluster): the copy lands at the same shared-memory offset in every CTA of `mask` and signals the
-// mbarrier at the same offset there; with a 1-CTA cluster and mask 1 they degenerate to the plain forms
-__device__ __forceinline__ void bulk_g2s_mc(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, uint16_t mask) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(dst),
-               "l"(src), "r"(bytes), "r"(bar), "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -83,11 +63,7 @@ __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t cols) {
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
 }
-#ifndef DMN_EXP_NO_MMA
-#define DMN_EXP_NO_MMA 0     // timing probe (results are wrong): the issuer runs every handshake but no tcgen05.mma is issued
-#endif
 __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  if (DMN_EXP_NO_MMA) return;
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"

@@ -13,7 +13,7 @@ that end in a partial 128-row tile.  Per case (tests/conv_ref.py):
   * GroupNorm output statistics against their derived bound, where the production conv has them;
   * the launch log (dmn_debug_conv_log) shows the tiling regime the case claims: (mt, mixed 256 / 128-row tiling, tiles > CTAs).
 
-The reference runs on the GPU in float64.  Production defaults: no DMN_CONV_* / DMN_EXP_* switch is set.
+The reference runs on the GPU in float64.  Production defaults: no DMN_CONV_* switch is set.
 """
 import math
 
