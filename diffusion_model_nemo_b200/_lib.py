@@ -119,6 +119,7 @@ SYMBOLS = {
     "dmn_randn": (_I, [_P, _L, Rng, _I, _P]),
     "dmn_axpby": (_I, [_P, _P, _F, _F, _P, _L, _P]),
     "dmn_sample_loop": (_I, [_P, C.POINTER(LoopDesc), _P]),
+    "dmn_loop_scratch_bytes": (C.c_size_t, [_P, C.POINTER(LoopDesc)]),
     "dmn_loop_launches_per_step": (_I, [_P, C.POINTER(LoopDesc)]),
     "dmn_inpaint_prepare": (_I, [_P, _P, _P, _P, _L, _P, _P, _I, Rng, _P]),
     "dmn_sample_loop_inpaint": (_I, [_P, C.POINTER(LoopDesc), C.POINTER(InpaintDesc), _P]),

@@ -783,6 +783,30 @@ static int check_ready(const dmn_plan* p) {
   return 0;
 }
 
+// Captures enqueue(stream) on a private non-blocking stream (thread-local capture) and instantiates the graph into *out.
+// An error enqueue returns is passed through; a failing CUDA call of the capture itself becomes DMN_ECUDA naming `what`.
+template <class Enqueue>
+static int capture_graph(const char* what, Enqueue&& enqueue, cudaGraphExec_t* out) {
+  cudaStream_t cs;
+  DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+  int rc = 0;
+  const char* where = "begin capture";
+  cudaGraph_t graph = nullptr;
+  cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
+  if (e == cudaSuccess) {
+    rc = enqueue(cs);
+    const cudaError_t e2 = cudaStreamEndCapture(cs, &graph);
+    if (!rc && e2 != cudaSuccess) { where = "end capture"; e = e2; }
+  }
+  cudaStreamDestroy(cs);
+  if (!rc && e == cudaSuccess) { where = "instantiate"; e = cudaGraphInstantiate(out, graph, 0); }
+  if (graph) cudaGraphDestroy(graph);
+  cudaGetLastError();
+  if (rc) return rc;
+  if (e != cudaSuccess) return fail(DMN_ECUDA, std::string(what) + " (" + where + "): " + cudaGetErrorString(e));
+  return 0;
+}
+
 }  // namespace dmn
 
 extern "C" {
@@ -1108,22 +1132,15 @@ int dmn_plan_profile_forward_graph(dmn_plan* p, const float* x_dev, const int32_
   // Measurement aid only: the one other place (besides the GEMM self-test) where the library allocates device memory itself.
   unsigned long long* stamps = nullptr;
   DMN_CUDA_CHECK(cudaMalloc(&stamps, (n + 2) * sizeof(unsigned long long)));
-  cudaStream_t cs;
-  DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-  cudaGraph_t graph = nullptr;
   cudaGraphExec_t exec = nullptr;
-  const char* where = "begin capture";
-  cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-  if (e == cudaSuccess) {
-    rc = run_forward(p, x_dev, row_dev, classes_dev, out_dev, batch, cs, nullptr, nullptr, stamps);
-    where = "end capture";
-    e = cudaStreamEndCapture(cs, &graph);
-  }
-  if (!rc && e == cudaSuccess) { where = "instantiate"; e = cudaGraphInstantiate(&exec, graph, 0); }
+  rc = capture_graph("profile_forward_graph", [&](cudaStream_t cs) {
+    return run_forward(p, x_dev, row_dev, classes_dev, out_dev, batch, cs, nullptr, nullptr, stamps);
+  }, &exec);
   std::vector<unsigned long long> host(n + 2);
-  if (!rc && e == cudaSuccess) {
+  const char* where = "launch";
+  cudaError_t e = cudaSuccess;
+  if (!rc) {
     cudaStream_t st = (cudaStream_t)stream;
-    where = "launch";
     e = cudaGraphLaunch(exec, st);
     if (e == cudaSuccess) e = cudaGraphLaunch(exec, st);
     if (e == cudaSuccess) { where = "synchronize"; e = cudaStreamSynchronize(st); }
@@ -1137,8 +1154,6 @@ int dmn_plan_profile_forward_graph(dmn_plan* p, const float* x_dev, const int32_
     }
   }
   if (exec) cudaGraphExecDestroy(exec);
-  if (graph) cudaGraphDestroy(graph);
-  cudaStreamDestroy(cs);
   cudaFree(stamps);
   if (!rc && e != cudaSuccess) rc = fail(DMN_ECUDA, std::string("profile_forward_graph (") + where + "): " + cudaGetErrorString(e));
   cudaGetLastError();
@@ -1150,65 +1165,87 @@ int dmn_plan_profile_forward_graph(dmn_plan* p, const float* x_dev, const int32_
 // ---------------------------------------------------------------------------------------------------------
 // loop driver
 // ---------------------------------------------------------------------------------------------------------
-// DMN_LOOP_DPMPP's history ring: 3*n floats behind the scratch every other kind uses (layout documented in dmn_loop_desc)
-static size_t dpmpp_ring_offset(const dmn_loop_desc* d, long n, long n_out) {
-  const long base = d->cfg_on ? 3 * n_out + 3 * n + 2 * d->batch + 36 : n_out + n + 2 * d->batch + 16;
-  return (size_t)((base + 3) & ~3L);
+// Slack of the loop scratch, in floats: the sizes the loop has always required, from which every offset below derives.
+//  kLoopSlack: the tail behind x_mean is 2*batch + kLoopSlack floats; the Langevin norms use 2*batch + 2 of them.
+//  kLoopGuidedSlack: with guidance the layout ends 2*batch + kLoopGuidedSlack floats behind its 3*(n_out + n) buffers: the tail
+//    rounded up to 4 floats, so x2 and mo2 stay 16-byte aligned for the float4 guidance kernels, then 18 or 20 spare floats.
+static constexpr long kLoopSlack = 16, kLoopGuidedSlack = 36;
+
+// views into dmn_loop_desc.scratch_dev; the buffers a descriptor does not use are nullptr
+struct LoopWork {
+  long chw = 0, n = 0, n_out = 0;        // C*S*S; batch * chw (the state); batch * out_dim*S*S (the model output)
+  float* mo = nullptr;                   // [n_out] model output (guidance: the mixed eps)
+  float* xmean = nullptr;                // [n] PC: x_mean; BPD: x_t
+  float* lscr = nullptr;                 // [2*batch + 2] Langevin norms
+  float* x2 = nullptr;                   // guidance: [2n] the doubled batch [x ; x]
+  float* mo2 = nullptr;                  // guidance: [2*n_out] its model output
+  float* ring = nullptr;                 // DPM-Solver++: [3n] history ring, float4-aligned
+};
+
+// floats of scratch the descriptor needs (reads kind, batch and cfg_on); fills w with views into base when given
+static size_t loop_work_layout(const dmn_unet_cfg& c, const dmn_loop_desc& d, float* base, LoopWork* w) {
+  const auto round4 = [](long v) { return (v + 3) & ~3L; };
+  const long chw = (long)c.channels * c.image_size * c.image_size;
+  const long n = d.batch * chw;
+  const long n_out = (long)d.batch * c.out_dim * c.image_size * c.image_size;
+  const long common = d.cfg_on ? 3 * n_out + 3 * n + 2 * d.batch + kLoopGuidedSlack : n_out + n + 2 * d.batch + kLoopSlack;
+  const long o_x2 = n_out + n + round4(2 * d.batch + kLoopSlack), o_ring = round4(common);
+  const bool dpmpp = d.kind == DMN_LOOP_DPMPP;
+  if (w) {
+    w->chw = chw; w->n = n; w->n_out = n_out;
+    w->mo = base;
+    w->xmean = base + n_out;
+    w->lscr = base + n_out + n;
+    w->x2 = d.cfg_on ? base + o_x2 : nullptr;
+    w->mo2 = d.cfg_on ? base + o_x2 + 2 * n : nullptr;
+    w->ring = dpmpp ? base + o_ring : nullptr;
+  }
+  return (size_t)(dpmpp ? o_ring + 3 * n : common);
 }
-static float* dpmpp_ring(const dmn_loop_desc* d, long n, long n_out) { return d->scratch_dev + dpmpp_ring_offset(d, n, n_out); }
 
 // One loop step.  `ctr` = device step counter (graph mode) or nullptr with host step `s` (injected-noise mode);
 // `z0` = this step's injected noise block (draws x n floats) or nullptr for in-kernel Philox with device rng state.
 // `ip` (inpainting, never with injected noise): dmn_inpaint_prepare runs first, so everything after it sees the merged state.
-static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc* ip, int32_t* ctr_dev, bool use_ctr, int s,
-                        const float* z0, cudaStream_t st) {
-  const dmn_unet_cfg& c = p->cfg;
-  const long chw = (long)c.channels * c.image_size * c.image_size;
-  const long n = (long)d->batch * chw;
-  const long n_out = (long)d->batch * c.out_dim * c.image_size * c.image_size;
-  float* mo = d->scratch_dev;              // model output
-  float* xmean = d->scratch_dev + n_out;   // PC: x_mean
-  float* lscr = xmean + n;                 // Langevin scratch: 2*batch + 2 floats
+static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, const LoopWork& w, const dmn_inpaint_desc* ip, int32_t* ctr_dev,
+                        bool use_ctr, int s, const float* z0, cudaStream_t st) {
   const int32_t* step_dev = use_ctr ? ctr_dev : nullptr;
   const dmn_rng* rng_dev = z0 ? nullptr : reinterpret_cast<const dmn_rng*>(ctr_dev + 4);
   int rc;
-  if (ip && (rc = launch_inpaint_prepare(d->state_dev, ip->known_dev, ip->mask_dev, d->state_dev, n, ip->prep_coef_dev, step_dev, s,
+  if (ip && (rc = launch_inpaint_prepare(d->state_dev, ip->known_dev, ip->mask_dev, d->state_dev, w.n, ip->prep_coef_dev, step_dev, s,
                                          d->rng, rng_dev, st)))
     return rc;
   if (d->kind == DMN_LOOP_BPD) {
     // bits-per-dimension term of one timestep: x_t ~ q(x_t | x_0), U-Net on x_t, fused KL / decoder-NLL reduction into terms[b][t]
-    float* xt = xmean;
-    if ((rc = launch_bpd_qsample(d->state_dev, z0, xt, n, d->coef_dev, step_dev, s, d->rng, rng_dev, st))) return rc;
-    if ((rc = run_forward(p, xt, ctr_dev, d->classes_dev, mo, d->batch, st))) return rc;
-    if ((rc = launch_bpd_term(d->state_dev, xt, mo, d->aux_dev, d->batch, chw, c.out_dim == 2 * c.channels ? 1 : 0, d->n_steps, 0,
-                              d->coef_dev, d->coef2_dev, step_dev, s, st)))
+    float* xt = w.xmean;
+    if ((rc = launch_bpd_qsample(d->state_dev, z0, xt, w.n, d->coef_dev, step_dev, s, d->rng, rng_dev, st))) return rc;
+    if ((rc = run_forward(p, xt, ctr_dev, d->classes_dev, w.mo, d->batch, st))) return rc;
+    if ((rc = launch_bpd_term(d->state_dev, xt, w.mo, d->aux_dev, d->batch, w.chw, p->cfg.out_dim == 2 * p->cfg.channels ? 1 : 0,
+                              d->n_steps, 0, d->coef_dev, d->coef2_dev, step_dev, s, st)))
       return rc;
     return launch_advance_counter(ctr_dev, st);
   }
   if (d->kind == DMN_LOOP_PC) {
     for (int k = 0; k < d->n_corr; ++k) {
-      if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, mo, d->batch, st))) return rc;
-      const float* zk = z0 ? z0 + (long)k * n : nullptr;
+      if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, w.mo, d->batch, st))) return rc;
+      const float* zk = z0 ? z0 + (long)k * w.n : nullptr;
       if (d->corr_kind == 1)
-        rc = launch_affine_noise(d->state_dev, mo, zk, d->state_dev, xmean, n, d->coef2_dev, step_dev, s, k, d->rng, rng_dev, st);
+        rc = launch_affine_noise(d->state_dev, w.mo, zk, d->state_dev, w.xmean, w.n, d->coef2_dev, step_dev, s, k, d->rng, rng_dev, st);
       else
-        rc = launch_langevin(d->state_dev, mo, zk, d->state_dev, xmean, d->batch, chw, d->snr, d->coef2_dev, step_dev, s, k, lscr,
-                             d->rng, rng_dev, st);
+        rc = launch_langevin(d->state_dev, w.mo, zk, d->state_dev, w.xmean, d->batch, w.chw, d->snr, d->coef2_dev, step_dev, s, k,
+                             w.lscr, d->rng, rng_dev, st);
       if (rc) return rc;
     }
-    if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, mo, d->batch, st))) return rc;
-    const float* zp = z0 ? z0 + (long)d->n_corr * n : nullptr;
-    if ((rc = launch_affine_noise(d->state_dev, mo, zp, d->state_dev, xmean, n, d->coef_dev, step_dev, s, 7, d->rng, rng_dev, st)))
+    if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, w.mo, d->batch, st))) return rc;
+    const float* zp = z0 ? z0 + (long)d->n_corr * w.n : nullptr;
+    if ((rc = launch_affine_noise(d->state_dev, w.mo, zp, d->state_dev, w.xmean, w.n, d->coef_dev, step_dev, s, 7, d->rng, rng_dev, st)))
       return rc;
   } else {
     if (d->cfg_on) {
       // classifier-free guidance: one U-Net evaluation on the doubled batch [x ; x] (labels ; null class), then the mix
-      float* x2 = lscr + ((2 * d->batch + 16 + 3) & ~3);
-      float* mo2 = x2 + 2 * n;
-      if ((rc = launch_cfg_dup(d->state_dev, x2, n, st))) return rc;
-      if ((rc = run_forward(p, x2, ctr_dev, d->classes_dev, mo2, 2 * d->batch, st))) return rc;
+      if ((rc = launch_cfg_dup(d->state_dev, w.x2, w.n, st))) return rc;
+      if ((rc = run_forward(p, w.x2, ctr_dev, d->classes_dev, w.mo2, 2 * d->batch, st))) return rc;
       // a learned-variance U-Net returns [eps | v] per sample: only eps is guided, v is the conditional branch's
-      if ((rc = launch_cfg_combine(mo2, mo, n_out, n_out / d->batch, chw, d->cfg_scale, st))) return rc;
+      if ((rc = launch_cfg_combine(w.mo2, w.mo, w.n_out, w.n_out / d->batch, w.chw, d->cfg_scale, st))) return rc;
     } else if (d->kind == DMN_LOOP_DDPM && tail_fusable(p)) {
       // final_conv tail + posterior update (+ step counter unless a trajectory copy still has to see this step's index) in one launch
       TailFuse tf;
@@ -1216,26 +1253,25 @@ static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_d
       tf.rng = d->rng; tf.rng_dev = rng_dev;
       const bool traj = d->traj_dev && d->traj_every > 0;
       tf.advance = traj ? nullptr : ctr_dev;
-      if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, mo, d->batch, st, nullptr, &tf))) return rc;
+      if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, w.mo, d->batch, st, nullptr, &tf))) return rc;
       if (!traj) return 0;
-      if ((rc = launch_traj(d->state_dev, d->traj_dev, n, ctr_dev, d->traj_every, d->n_steps, st))) return rc;
+      if ((rc = launch_traj(d->state_dev, d->traj_dev, w.n, ctr_dev, d->traj_every, d->n_steps, st))) return rc;
       return launch_advance_counter(ctr_dev, st);
-    } else if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, mo, d->batch, st))) {
+    } else if ((rc = run_forward(p, d->state_dev, ctr_dev, d->classes_dev, w.mo, d->batch, st))) {
       return rc;
     }
     if (d->kind == DMN_LOOP_DDPM)
-      rc = launch_ddpm(d->state_dev, mo, z0, d->state_dev, n, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
+      rc = launch_ddpm(d->state_dev, w.mo, z0, d->state_dev, w.n, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
     else if (d->kind == DMN_LOOP_LEARNED)
-      rc = launch_learned(d->state_dev, mo, z0, d->state_dev, d->batch, chw, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
+      rc = launch_learned(d->state_dev, w.mo, z0, d->state_dev, d->batch, w.chw, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
     else if (d->kind == DMN_LOOP_DDIM)
-      rc = launch_ddim(d->state_dev, mo, z0, d->state_dev, n, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
+      rc = launch_ddim(d->state_dev, w.mo, z0, d->state_dev, w.n, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
     else
-      rc = launch_dpmpp(d->state_dev, mo, dpmpp_ring(d, n, n_out), d->state_dev, d->batch, chw, n_out / d->batch, d->coef_dev, step_dev,
-                        s, st);
+      rc = launch_dpmpp(d->state_dev, w.mo, w.ring, d->state_dev, d->batch, w.chw, w.n_out / d->batch, d->coef_dev, step_dev, s, st);
     if (rc) return rc;
   }
   if (d->traj_dev && d->traj_every > 0)
-    if ((rc = launch_traj(d->state_dev, d->traj_dev, n, ctr_dev, d->traj_every, d->n_steps, st))) return rc;
+    if ((rc = launch_traj(d->state_dev, d->traj_dev, w.n, ctr_dev, d->traj_every, d->n_steps, st))) return rc;
   return launch_advance_counter(ctr_dev, st);
 }
 
@@ -1268,59 +1304,37 @@ static int run_loop(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc*
   else if (d->kind == DMN_LOOP_DPMPP)
     DMN_REQUIRE(c.out_dim == c.channels || c.out_dim == 2 * c.channels, "DPM-Solver++: out_dim must be C or 2C");
   else DMN_REQUIRE(c.out_dim == c.channels, "U-Net out_dim must equal channels for this sampler");
-  const long chw = (long)c.channels * c.image_size * c.image_size;
-  const long n = (long)d->batch * chw;
-  const long n_out = (long)d->batch * c.out_dim * c.image_size * c.image_size;
-  DMN_REQUIRE(d->scratch_bytes >= (size_t)(n_out + n + 2 * d->batch + 16) * sizeof(float), "loop scratch too small");
-  DMN_REQUIRE(d->state_elems == 0 || d->state_elems == n, "state_dev does not hold batch * channels * image_size^2 floats for this plan");
+  LoopWork w;
+  const size_t scratch_floats = loop_work_layout(c, *d, d->scratch_dev, &w);
+  DMN_REQUIRE(d->state_elems == 0 || d->state_elems == w.n, "state_dev does not hold batch * channels * image_size^2 floats for this plan");
   if (d->cfg_on) {
     DMN_REQUIRE(d->kind != DMN_LOOP_PC, "classifier-free guidance is built for the DDPM / learned / DDIM / DPM-Solver++ loops");
     DMN_REQUIRE(c.num_classes >= 0 && d->classes_dev, "classifier-free guidance needs a class-conditional U-Net and 2*batch labels");
     DMN_REQUIRE(2 * d->batch <= c.max_batch, "classifier-free guidance doubles the batch: plan max_batch too small");
-    DMN_REQUIRE(d->scratch_bytes >= (size_t)(3 * n_out + 3 * n + 2 * d->batch + 36) * sizeof(float), "loop scratch too small for guidance");
-    DMN_REQUIRE(n % 4 == 0 && n_out % 4 == 0, "guidance kernels need 16-byte multiples");
+    DMN_REQUIRE(w.n % 4 == 0 && w.n_out % 4 == 0, "guidance kernels need 16-byte multiples");
   }
-  if (d->kind == DMN_LOOP_DPMPP)
-    DMN_REQUIRE(d->scratch_bytes >= (dpmpp_ring_offset(d, n, n_out) + 3 * (size_t)n) * sizeof(float),
-                "loop scratch too small for the DPM-Solver++ history ring");
+  DMN_REQUIRE(d->scratch_bytes >= scratch_floats * sizeof(float), "loop scratch smaller than dmn_loop_scratch_bytes()");
   cudaStream_t st = (cudaStream_t)stream;
   int32_t* ctr = (int32_t*)(p->wsbase + p->counters.off);
-  float* xmean = d->scratch_dev + n_out;
   if ((rc = launch_set_counter(ctr, 0, d->rng, st))) return rc;
 
   if (d->noise_dev) {
     // parity mode: injected noise => per-step pointers differ, plain launches with the host step index
     const int draws = (d->kind == DMN_LOOP_PC) ? d->n_corr + 1 : (d->kind == DMN_LOOP_DPMPP ? 0 : 1);
     for (int s = 0; s < d->n_steps; ++s)
-      if ((rc = enqueue_step(p, d, ip, ctr, false, s, d->noise_dev + (long)s * draws * n, st))) return rc;
+      if ((rc = enqueue_step(p, d, w, ip, ctr, false, s, d->noise_dev + (long)s * draws * w.n, st))) return rc;
   } else if (!d->use_graph) {
     for (int s = 0; s < d->n_steps; ++s)
-      if ((rc = enqueue_step(p, d, ip, ctr, true, 0, nullptr, st))) return rc;
+      if ((rc = enqueue_step(p, d, w, ip, ctr, true, 0, nullptr, st))) return rc;
   } else {
     const dmn_inpaint_desc ip_key = ip ? *ip : dmn_inpaint_desc{};
     cudaGraphExec_t exec = nullptr;
     for (auto& g : p->graphs)
       if (same_graph_key(g.key, g.ip, *d, ip_key)) exec = g.exec;
     if (!exec) {
-      cudaStream_t cs;
-      DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-      cudaGraph_t graph = nullptr;
-      cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-      if (e != cudaSuccess) {
-        cudaStreamDestroy(cs);
-        return fail(DMN_ECUDA, std::string("begin capture: ") + cudaGetErrorString(e));
-      }
-      rc = enqueue_step(p, d, ip, ctr, true, 0, nullptr, cs);
-      e = cudaStreamEndCapture(cs, &graph);
-      cudaStreamDestroy(cs);
-      if (rc) {
-        if (graph) cudaGraphDestroy(graph);
+      if ((rc = capture_graph("sample loop graph", [&](cudaStream_t cs) { return enqueue_step(p, d, w, ip, ctr, true, 0, nullptr, cs); },
+                              &exec)))
         return rc;
-      }
-      if (e != cudaSuccess) return fail(DMN_ECUDA, std::string("end capture: ") + cudaGetErrorString(e));
-      e = cudaGraphInstantiate(&exec, graph, 0);
-      cudaGraphDestroy(graph);
-      if (e != cudaSuccess) return fail(DMN_ECUDA, std::string("graph instantiate: ") + cudaGetErrorString(e));
       if (p->graphs.size() >= 8) {
         cudaGraphExecDestroy(p->graphs.front().exec);
         p->graphs.erase(p->graphs.begin());
@@ -1332,16 +1346,20 @@ static int run_loop(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc*
       p->graphs.push_back(ge);
     }
     for (int s = 0; s < d->n_steps; ++s) DMN_CUDA_CHECK(cudaGraphLaunch(exec, st));
-    count_launch((int)((long)d->n_steps * (dmn_loop_launches_per_step(p, d) + (ip ? 1 : 0))));
   }
   if (d->kind == DMN_LOOP_PC && d->aux_dev)
-    DMN_CUDA_CHECK(cudaMemcpyAsync(d->aux_dev, xmean, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    DMN_CUDA_CHECK(cudaMemcpyAsync(d->aux_dev, w.xmean, w.n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return 0;
 }
 
 extern "C" {
 
 int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream) { return run_loop(p, d, nullptr, stream); }
+
+size_t dmn_loop_scratch_bytes(const dmn_plan* p, const dmn_loop_desc* d) {
+  if (!p || !d || d->kind < DMN_LOOP_DDPM || d->kind > DMN_LOOP_DPMPP || d->batch < 1) return 0;
+  return loop_work_layout(p->cfg, *d, nullptr, nullptr) * sizeof(float);
+}
 
 int dmn_sample_loop_inpaint(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc* ip, void* stream) {
   if (!d || !ip) return fail(DMN_EINVAL, "null descriptor");
@@ -1352,8 +1370,9 @@ int dmn_sample_loop_inpaint(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpai
   int rc = run_loop(p, d, ip, stream);
   if (rc) return rc;
   // final composite: row n_steps = {1, 0, 1, 0} puts the known pixels back exactly and draws nothing
-  const long n = (long)d->batch * p->cfg.channels * p->cfg.image_size * p->cfg.image_size;
-  return launch_inpaint_prepare(d->state_dev, ip->known_dev, ip->mask_dev, d->state_dev, n, ip->prep_coef_dev, nullptr, d->n_steps,
+  LoopWork w;
+  loop_work_layout(p->cfg, *d, d->scratch_dev, &w);
+  return launch_inpaint_prepare(d->state_dev, ip->known_dev, ip->mask_dev, d->state_dev, w.n, ip->prep_coef_dev, nullptr, d->n_steps,
                                 d->rng, nullptr, (cudaStream_t)stream);
 }
 
@@ -1414,62 +1433,40 @@ static bool same_ode_key(const dmn_ode_desc& a, const dmn_ode_desc& b) {
          a.result_dev == b.result_dev;
 }
 
+// init phase on the captured stream, then a WHILE node whose body (one attempt) is captured on a second stream, then the finish
 static int build_ode_graph(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w, const OdeParams& P, cudaGraphExec_t* out) {
-  cudaStream_t cs, bs;
-  DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-  if (cudaStreamCreateWithFlags(&bs, cudaStreamNonBlocking) != cudaSuccess) {
-    cudaStreamDestroy(cs);
-    return fail(DMN_ECUDA, "ode graph: stream create");
-  }
-  int rc = 0;
-  const char* where = "begin capture";
-  cudaGraph_t graph = nullptr;
-  cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-  bool capturing = e == cudaSuccess;
-  cudaGraphConditionalHandle hnd = 0;
-  if (capturing) {
+  cudaStream_t bs;
+  DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&bs, cudaStreamNonBlocking));
+  auto enqueue = [&](cudaStream_t cs) -> int {
     cudaStreamCaptureStatus cst;
+    cudaGraph_t graph = nullptr;
     const cudaGraphNode_t* deps = nullptr;
     size_t ndeps = 0;
-    where = "capture info";
-    e = cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps);
-    if (e == cudaSuccess) { where = "conditional handle"; e = cudaGraphConditionalHandleCreate(&hnd, graph, 0, cudaGraphCondAssignDefault); }
-    if (e == cudaSuccess) rc = enqueue_ode_init(p, d, w, P, hnd, 1, cs);
-    cudaGraph_t body = nullptr;
-    if (e == cudaSuccess && !rc) {
-      where = "while node";
-      e = cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps);
-      cudaGraphNodeParams np = {};
-      np.type = cudaGraphNodeTypeConditional;
-      np.conditional.handle = hnd;
-      np.conditional.type = cudaGraphCondTypeWhile;
-      np.conditional.size = 1;
-      cudaGraphNode_t node = nullptr;
-      if (e == cudaSuccess) e = cudaGraphAddNode(&node, graph, deps, ndeps, &np);
-      if (e == cudaSuccess) e = cudaStreamUpdateCaptureDependencies(cs, &node, 1, cudaStreamSetCaptureDependencies);
-      body = np.conditional.phGraph_out ? np.conditional.phGraph_out[0] : nullptr;
-      if (e == cudaSuccess) { where = "body capture"; e = cudaStreamBeginCaptureToGraph(bs, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal); }
-      if (e == cudaSuccess) {
-        rc = enqueue_ode_attempt(p, d, w, P, hnd, 1, bs);
-        cudaGraph_t bg = nullptr;
-        const cudaError_t e2 = cudaStreamEndCapture(bs, &bg);
-        if (!rc && e2 != cudaSuccess) { where = "body end capture"; e = e2; }
-      }
-    }
-    if (e == cudaSuccess && !rc) rc = launch_ode_finish(w, d->state_dev, cs);
-    cudaGraph_t g2 = nullptr;
-    const cudaError_t e3 = cudaStreamEndCapture(cs, &g2);
-    graph = g2;
-    if (e == cudaSuccess && !rc && e3 != cudaSuccess) { where = "end capture"; e = e3; }
-  }
+    cudaGraphConditionalHandle hnd = 0;
+    DMN_CUDA_CHECK(cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps));
+    DMN_CUDA_CHECK(cudaGraphConditionalHandleCreate(&hnd, graph, 0, cudaGraphCondAssignDefault));
+    int rc = enqueue_ode_init(p, d, w, P, hnd, 1, cs);
+    if (rc) return rc;
+    DMN_CUDA_CHECK(cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps));
+    cudaGraphNodeParams np = {};
+    np.type = cudaGraphNodeTypeConditional;
+    np.conditional.handle = hnd;
+    np.conditional.type = cudaGraphCondTypeWhile;
+    np.conditional.size = 1;
+    cudaGraphNode_t node = nullptr;
+    DMN_CUDA_CHECK(cudaGraphAddNode(&node, graph, deps, ndeps, &np));
+    DMN_CUDA_CHECK(cudaStreamUpdateCaptureDependencies(cs, &node, 1, cudaStreamSetCaptureDependencies));
+    cudaGraph_t body = np.conditional.phGraph_out[0];
+    DMN_CUDA_CHECK(cudaStreamBeginCaptureToGraph(bs, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
+    rc = enqueue_ode_attempt(p, d, w, P, hnd, 1, bs);
+    const cudaError_t e = cudaStreamEndCapture(bs, &body);
+    if (rc) return rc;
+    if (e != cudaSuccess) return fail(DMN_ECUDA, std::string("ode graph (body end capture): ") + cudaGetErrorString(e));
+    return launch_ode_finish(w, d->state_dev, cs);
+  };
+  const int rc = capture_graph("ode graph", enqueue, out);
   cudaStreamDestroy(bs);
-  cudaStreamDestroy(cs);
-  if (!rc && e == cudaSuccess) { where = "instantiate"; e = cudaGraphInstantiate(out, graph, 0); }
-  if (graph) cudaGraphDestroy(graph);
-  cudaGetLastError();
-  if (rc) return rc;
-  if (e != cudaSuccess) return fail(DMN_ECUDA, std::string("ode graph (") + where + "): " + cudaGetErrorString(e));
-  return 0;
+  return rc;
 }
 
 extern "C" {

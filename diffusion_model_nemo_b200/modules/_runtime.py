@@ -62,6 +62,16 @@ def coef_rows(cols: Sequence[torch.Tensor], device) -> torch.Tensor:
     return tab.to(device)
 
 
+def stable_copy(bufs: dict, name: str, src: torch.Tensor, like: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Copy `src` into bufs[name], a buffer whose address a cached CUDA graph bakes in.  The buffer takes the shape, dtype and
+    device of `like` (default: `src`) and is reallocated only when that shape changes."""
+    like = src if like is None else like
+    buf = bufs.get(name)
+    if buf is None or buf.shape != like.shape:
+        buf = bufs[name] = torch.empty_like(like)
+    return buf.copy_(src)
+
+
 class LoopResult:
     def __init__(self, final, aux, traj):
         self.final, self.aux, self.traj = final, aux, traj
@@ -100,6 +110,11 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
     plan = unet.plan(h, 2 * b if guided else b, device, time_rows=int(times.shape[0]))
     n = b * c * h * w
     draws = (n_corr + 1) if kind == L.LOOP_PC else (0 if kind == L.LOOP_DPMPP else 1)
+    d = L.LoopDesc()
+    d.kind, d.n_steps, d.batch, d.n_corr = kind, n_steps, b, n_corr
+    d.snr, d.denoise, d.use_graph, d.corr_kind = float(snr), int(denoise), int(use_graph), corr_kind
+    d.cfg_scale = float(cfg_scale) if guided else 0.0
+    d.cfg_on = 1 if guided else 0
     with torch.cuda.device(device):
         st = L.stream_ptr(device)
         tkey = (times.data_ptr(), int(times.shape[0]), tuple(times[:: max(1, int(times.shape[0]) // 7)].tolist()))
@@ -108,16 +123,13 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
             plan.time_rows_key = tkey
         rng = L.Rng(seed if seed is not None else draw_seed(), rank_stream_id())
         # loop buffers live with the plan so their addresses (baked into the cached CUDA graph) stay stable
-        n_out = b * unet.out_dim * h * w
         n_traj = (n_steps // traj_every) if traj_every > 0 else 0
         bkey = (kind, b, n_steps if (n_traj or kind == L.LOOP_BPD) else 0, n_traj, bool(denoise), guided)
         bufs = plan.__dict__.setdefault("_loop_bufs", {})
         if bkey not in bufs:
             bufs[bkey] = {
                 "state": torch.empty((b, c, h, w), dtype=torch.float32, device=device),
-                # + the DPM-Solver++ history ring (3 states) behind the common layout
-                "scratch": torch.empty((3 if guided else 1) * (n_out + n) + 2 * b + 64 + (3 * n if kind == L.LOOP_DPMPP else 0),
-                                       dtype=torch.float32, device=device),
+                "scratch": torch.empty(lib.dmn_loop_scratch_bytes(plan.h, C.byref(d)) // 4, dtype=torch.float32, device=device),
                 "aux": (torch.empty((b, c, h, w), dtype=torch.float32, device=device) if (kind == L.LOOP_PC and denoise) else
                         torch.zeros((b, n_steps), dtype=torch.float32, device=device) if kind == L.LOOP_BPD else None),
                 "traj": torch.empty((n_traj, b, c, h, w), dtype=torch.float32, device=device) if n_traj > 0 else None,
@@ -143,16 +155,7 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
             classes = classes.to(device, torch.int64).reshape(-1)
             if guided:     # doubled batch: [labels ; null class] (the padding row of class_embed, reference unet.py:118-120)
                 classes = torch.cat([classes, torch.full_like(classes, unet.num_classes)])
-            # persistent buffer: the cached CUDA graph bakes the pointer in
-            cb = bufs[bkey].get("classes")
-            if cb is None or cb.shape != classes.shape:
-                cb = torch.empty_like(classes)
-                bufs[bkey]["classes"] = cb
-            cb.copy_(classes)
-            classes = cb
-        d = L.LoopDesc()
-        d.kind, d.n_steps, d.batch, d.n_corr = kind, n_steps, b, n_corr
-        d.snr, d.denoise, d.use_graph, d.corr_kind = float(snr), int(denoise), int(use_graph), corr_kind
+            classes = stable_copy(bufs[bkey], "classes", classes)
         d.coef_dev = coef.data_ptr()
         d.coef2_dev = coef2.data_ptr() if coef2 is not None else None
         d.classes_dev = classes.data_ptr() if classes is not None else None
@@ -164,8 +167,6 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
         d.scratch_bytes = scratch.numel() * 4
         d.traj_dev = traj.data_ptr() if traj is not None else None
         d.traj_every = traj_every if traj is not None else 0
-        d.cfg_scale = float(cfg_scale) if guided else 0.0
-        d.cfg_on = 1 if guided else 0
         d.state_elems = state.numel()
         if inpaint is None:
             L.check(lib.dmn_sample_loop(plan.h, C.byref(d), st), "dmn_sample_loop")
@@ -173,12 +174,8 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
         else:
             assert noise_dev is None, "inpainting draws its noise in-kernel"
             known, mask, prep_coef = inpaint
-            # persistent expanded fp32 copies: the cached CUDA graph bakes the pointers in
-            for name, src in (("known", known), ("mask", mask)):
-                if name not in bufs[bkey]:
-                    bufs[bkey][name] = torch.empty_like(state)
-                bufs[bkey][name].copy_(src)
-            kb, mb = bufs[bkey]["known"], bufs[bkey]["mask"]
+            kb = stable_copy(bufs[bkey], "known", known, like=state)
+            mb = stable_copy(bufs[bkey], "mask", mask, like=state)      # broadcast to the state's shape
             ip = L.InpaintDesc()
             ip.known_dev, ip.mask_dev, ip.prep_coef_dev = kb.data_ptr(), mb.data_ptr(), prep_coef.data_ptr()
             L.check(lib.dmn_sample_loop_inpaint(plan.h, C.byref(d), C.byref(ip), st), "dmn_sample_loop_inpaint")

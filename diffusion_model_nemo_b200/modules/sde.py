@@ -562,12 +562,7 @@ class ProbabilityFlowSampler(torch.nn.Module):
             state, work, result = buf["state"], buf["work"], buf["result"]
             state.copy_(x.to(device, torch.float32))
             if classes is not None:
-                classes = classes.to(device, torch.int64).reshape(-1)
-                cb = buf.get("classes")
-                if cb is None or cb.shape != classes.shape:
-                    cb = buf["classes"] = torch.empty_like(classes)
-                cb.copy_(classes)
-                classes = cb
+                classes = R.stable_copy(buf, "classes", classes.to(device, torch.int64).reshape(-1))
             wp = (work.data_ptr() + 255) // 256 * 256
             d = L.OdeDesc()
             if isinstance(sde, VPSDE):

@@ -213,7 +213,7 @@ int dmn_axpby(const float* x, const float* y, float a, float b, float* out, int6
                                  coef_dev / coef2_dev rows as documented at dmn_bpd_term; noise_dev injects the q_sample draws */
 #define DMN_LOOP_DPMPP    5   /* DPM-Solver++ multistep: per step U-Net (or the guidance path) -> dmn_dpmpp_step; rows as documented
                                  there, one per (t_i, t_{i+1}) pair.  out_dim = C or 2C.  Draws nothing: noise_dev, if given, only
-                                 selects plain launches with the host step index.  The history ring lives in scratch_dev (below). */
+                                 selects plain launches with the host step index.  The history ring lives in scratch_dev. */
 
 typedef struct dmn_loop_desc {
   int32_t kind;            /* DMN_LOOP_* */
@@ -231,10 +231,8 @@ typedef struct dmn_loop_desc {
   dmn_rng        rng;            /* throughput mode */
   float*         state_dev;      /* in: x_T (fp32 NCHW); out: final state in [-1,1] space */
   float*         aux_dev;        /* PC: x_mean of the last step when denoise */
-  float*         scratch_dev;    /* >= 2*out_dim*S*S*batch floats + 64 bytes: model output, x_mean, counters.
-                                    DMN_LOOP_DPMPP appends its history ring of 3*C*S*S*batch floats at float offset
-                                    R = round_up(base, 4), base = out_dim*S*S*batch + C*S*S*batch + 2*batch + 16 (guidance:
-                                    3*out_dim*S*S*batch + 3*C*S*S*batch + 2*batch + 36), so it needs R + 3*C*S*S*batch floats */
+  float*         scratch_dev;    /* at least dmn_loop_scratch_bytes() bytes: model output, x_mean, the guidance buffers and
+                                    the DPM-Solver++ history ring */
   size_t         scratch_bytes;
   float*         traj_dev;       /* optional [n_traj][batch*C*H*W] trajectory capture, every traj_every steps */
   int32_t        traj_every;
@@ -242,8 +240,8 @@ typedef struct dmn_loop_desc {
                                     Classifier-free guidance (not in the reference: SURVEY.md section 8 config 5a).  Every step
                                     evaluates the U-Net on the doubled batch [x ; x] with classes_dev[0..batch) = labels and
                                     classes_dev[batch..2*batch) = num_classes (the null / padding row, unet.py:118-120) and uses
-                                    eps = eps_u + cfg_scale * (eps_c - eps_u).  Needs max_batch >= 2*batch and scratch for
-                                    3*out_dim*S*S*batch + 3*C*S*S*batch + 2*batch + 16 floats.  DDPM / learned / DDIM /
+                                    eps = eps_u + cfg_scale * (eps_c - eps_u).  Needs max_batch >= 2*batch and the larger
+                                    scratch dmn_loop_scratch_bytes() reports with cfg_on set.  DDPM / learned / DDIM /
                                     DPM-Solver++ loops only.
                                     With a learned-variance U-Net only the eps half is guided; the variance channels are the
                                     conditional branch's. */
@@ -254,6 +252,9 @@ typedef struct dmn_loop_desc {
 /* Runs the whole loop on `stream`; returns after enqueueing (no host sync unless use_graph needs capture,
  * which happens on first use of a given (plan, kind, batch) and is cached in the plan). */
 int dmn_sample_loop(dmn_plan* p, const dmn_loop_desc* d, void* stream);
+/* bytes of scratch_dev the descriptor needs on this plan; reads kind, batch and cfg_on only.  0 for a NULL argument, an unknown
+ * kind or batch < 1. */
+size_t dmn_loop_scratch_bytes(const dmn_plan* p, const dmn_loop_desc* d);
 /* kernels launched per loop step for the given descriptor (bench.py's gpu_launches). */
 int dmn_loop_launches_per_step(const dmn_plan* p, const dmn_loop_desc* d);
 

@@ -297,10 +297,12 @@ def test_loop_descriptor_checks_with_a_bound_plan():
         u = M.Unet(None, dim=32, dim_mults=[1, 2], channels=c, out_dim=out_dim, use_convnext=False, compute_dtype="fp32",
                    conv_engine="simt").to(DEV)
         plan = u.plan(hw, b, DEV, time_rows=4)
-        n_out = b * out_dim * hw * hw
-        ring_at = (n_out + n + 2 * b + 16 + 3) // 4 * 4
+        one = torch.zeros(1, device=DEV)
+        need = lib.dmn_loop_scratch_bytes(plan.h, C.byref(_desc(L.LOOP_DPMPP, one, state, coef, b))) // 4
+        no_ring = lib.dmn_loop_scratch_bytes(plan.h, C.byref(_desc(L.LOOP_DDIM, one, state, coef, b))) // 4
+        assert no_ring + 3 * n <= need
         st = L.stream_ptr(DEV)
-        for floats, fits in ((ring_at + 3 * n, True), (ring_at + 3 * n - 4, False), (n_out + n + 2 * b + 16, False)):
+        for floats, fits in ((need, True), (need - 4, False), (no_ring, False)):
             scratch = torch.zeros(floats, device=DEV)
             d = _desc(L.LOOP_DPMPP, scratch, state, coef, b)
             if ok and fits:
