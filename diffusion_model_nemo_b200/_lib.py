@@ -82,6 +82,34 @@ class AttnBlockArgs(C.Structure):
     ]
 
 
+class InitConvArgs(C.Structure):
+    _fields_ = [
+        ("batch", C.c_int32), ("cin", C.c_int32), ("size", C.c_int32), ("cout", C.c_int32), ("act", C.c_int32),
+        ("engine", C.c_int32), ("pad_class", C.c_int32),
+        ("x", C.c_void_p), ("w", C.c_void_p), ("bias", C.c_void_p), ("cls_w", C.c_void_p), ("classes", C.c_void_p),
+        ("y", C.c_void_p), ("scratch_dev", C.c_void_p), ("scratch_bytes", C.c_size_t),
+    ]
+
+
+class GnFinalizeArgs(C.Structure):
+    _fields_ = [
+        ("batch", C.c_int32), ("channels", C.c_int32), ("hw", C.c_int32), ("groups", C.c_int32), ("ogroups", C.c_int32),
+        ("silu", C.c_int32), ("act", C.c_int32),
+        ("raw", C.c_void_p), ("res", C.c_void_p), ("stats", C.c_void_p), ("gamma", C.c_void_p), ("beta", C.c_void_p),
+        ("y", C.c_void_p), ("out_stats", C.c_void_p), ("scratch_dev", C.c_void_p), ("scratch_bytes", C.c_size_t),
+    ]
+
+
+class FinalProjArgs(C.Structure):
+    _fields_ = [
+        ("batch", C.c_int32), ("channels", C.c_int32), ("hw", C.c_int32), ("cout", C.c_int32), ("groups", C.c_int32),
+        ("plain", C.c_int32), ("act", C.c_int32),
+        ("y", C.c_void_p), ("stats", C.c_void_p), ("gamma", C.c_void_p), ("beta", C.c_void_p), ("w", C.c_void_p),
+        ("bias", C.c_void_p), ("eps", C.c_void_p), ("x", C.c_void_p), ("coef", C.c_void_p), ("z", C.c_void_p),
+        ("step", C.c_int32), ("rng", Rng), ("x_out", C.c_void_p), ("scratch_dev", C.c_void_p), ("scratch_bytes", C.c_size_t),
+    ]
+
+
 # every symbol include/dmn_b200.h declares: (restype, argtypes)
 _P, _I, _L, _F = C.c_void_p, C.c_int, C.c_int64, C.c_float
 SYMBOLS = {
@@ -134,6 +162,12 @@ SYMBOLS = {
     "dmn_selftest_tma_sw128_gemm": (_I, [_P, _P, _P, _I, _I, _I, _P]),
     "dmn_linear_attention_block": (_I, [C.POINTER(AttnBlockArgs), _P]),
     "dmn_linear_attention_block_scratch_bytes": (C.c_size_t, [C.POINTER(AttnBlockArgs)]),
+    "dmn_init_conv_forward": (_I, [C.POINTER(InitConvArgs), _P]),
+    "dmn_init_conv_scratch_bytes": (C.c_size_t, [C.POINTER(InitConvArgs)]),
+    "dmn_gn_finalize_forward": (_I, [C.POINTER(GnFinalizeArgs), _P]),
+    "dmn_gn_finalize_scratch_bytes": (C.c_size_t, [C.POINTER(GnFinalizeArgs)]),
+    "dmn_final_proj_forward": (_I, [C.POINTER(FinalProjArgs), _P]),
+    "dmn_final_proj_scratch_bytes": (C.c_size_t, [C.POINTER(FinalProjArgs)]),
 }
 
 _lib = None

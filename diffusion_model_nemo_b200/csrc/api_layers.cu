@@ -300,4 +300,118 @@ int dmn_linear_attention_block(const dmn_attn_block_args* a, void* stream) {
   return nhwc_to_nchw(base + L.y, a->y, a->batch, C_, a->n_tokens, ACT_BF16, st);
 }
 
+// ---- 7x7 stem: run_forward's OP_INIT with the weights packed by dmn_plan_load_param's PK_INIT packers ----
+static bool init_tc(const dmn_init_conv_args* a) {
+  return a->engine == DMN_CONV_TCGEN05 && init_conv_tcgen05_supported(a->cin, a->size, a->cout, a->batch);
+}
+static size_t init_out_esz(const dmn_init_conv_args* a) { return init_tc(a) || a->act == DMN_ACT_BF16 ? 2 : 4; }
+size_t dmn_init_conv_scratch_bytes(const dmn_init_conv_args* a) {
+  if (!a) return 0;
+  const size_t w = init_tc(a) ? init_conv_tcgen05_weight_bytes(a->cout) : (size_t)49 * a->cin * a->cout * 4;
+  return al((size_t)a->batch * a->size * a->size * a->cout * init_out_esz(a)) + al(w);
+}
+
+int dmn_init_conv_forward(const dmn_init_conv_args* a, void* stream) {
+  if (!a) return fail(DMN_EINVAL, "null args");
+  DMN_REQUIRE(a->x && a->w && a->y && a->scratch_dev, "null tensor");
+  DMN_REQUIRE(a->batch > 0 && a->cin > 0 && a->size > 0 && a->cout > 0, "shape");
+  DMN_REQUIRE(a->act == DMN_ACT_F32 || a->act == DMN_ACT_BF16, "act");
+  DMN_REQUIRE(a->engine == DMN_CONV_SIMT || a->act == DMN_ACT_BF16, "tcgen05 engine needs bf16 activations");
+  DMN_REQUIRE(a->scratch_bytes >= dmn_init_conv_scratch_bytes(a), "scratch too small (dmn_init_conv_scratch_bytes)");
+  cudaStream_t st = (cudaStream_t)stream;
+  char* base = (char*)a->scratch_dev;
+  const bool tc = init_tc(a);
+  const size_t y_bytes = al((size_t)a->batch * a->size * a->size * a->cout * init_out_esz(a));
+  const size_t nw = (size_t)49 * a->cin * a->cout;
+  std::vector<float> hw(nw);
+  DMN_CUDA_CHECK(cudaMemcpyAsync(hw.data(), a->w, nw * 4, cudaMemcpyDeviceToHost, st));
+  DMN_CUDA_CHECK(cudaStreamSynchronize(st));
+  InitConvP q;
+  q.x = a->x; q.bias = a->bias;
+  q.cls_w = a->cls_w; q.classes = a->cls_w ? a->classes : nullptr; q.pad_class = a->pad_class;
+  q.out = base;
+  q.B = a->batch; q.Cin = a->cin; q.S = a->size; q.Cout = a->cout;
+  int rc;
+  if (tc) {
+    std::vector<char> img(init_conv_tcgen05_weight_bytes(a->cout));
+    init_conv_tcgen05_pack_weights(a->cin, a->cout, hw.data(), img.data());
+    DMN_CUDA_CHECK(cudaMemcpyAsync(base + y_bytes, img.data(), img.size(), cudaMemcpyHostToDevice, st));
+    DMN_CUDA_CHECK(cudaStreamSynchronize(st));
+    q.w = (const float*)(base + y_bytes);
+    if ((rc = init_conv_tcgen05(q, st))) return rc;
+  } else {
+    std::vector<float> pw(nw);
+    init_conv_pack_weights(a->cin, a->cout, hw.data(), pw.data());
+    DMN_CUDA_CHECK(cudaMemcpyAsync(base + y_bytes, pw.data(), nw * 4, cudaMemcpyHostToDevice, st));
+    DMN_CUDA_CHECK(cudaStreamSynchronize(st));
+    q.w = (const float*)(base + y_bytes);
+    if ((rc = init_conv(q, a->act, st))) return rc;
+  }
+  return nhwc_to_nchw(base, a->y, a->batch, a->cout, a->size * a->size, tc ? ACT_BF16 : a->act, st);
+}
+
+// ---- GroupNorm finalize: run_forward's OP_FINALIZE on caller-given fixed-point statistics ----
+size_t dmn_gn_finalize_scratch_bytes(const dmn_gn_finalize_args* a) {
+  if (!a) return 0;
+  return 3 * al((size_t)a->batch * a->hw * a->channels * (a->act == DMN_ACT_F32 ? 4 : 2));
+}
+
+int dmn_gn_finalize_forward(const dmn_gn_finalize_args* a, void* stream) {
+  if (!a) return fail(DMN_EINVAL, "null args");
+  DMN_REQUIRE(a->raw && a->stats && a->gamma && a->beta && a->y && a->scratch_dev, "null tensor");
+  DMN_REQUIRE(a->batch > 0 && a->hw > 0 && a->channels > 0 && a->groups > 0, "shape");
+  DMN_REQUIRE(a->act == DMN_ACT_F32 || a->act == DMN_ACT_BF16, "act");
+  DMN_REQUIRE(a->ogroups == 0 || a->out_stats, "out_stats is null");
+  DMN_REQUIRE(a->scratch_bytes >= dmn_gn_finalize_scratch_bytes(a), "scratch too small (dmn_gn_finalize_scratch_bytes)");
+  cudaStream_t st = (cudaStream_t)stream;
+  char* base = (char*)a->scratch_dev;
+  const size_t act_bytes = al((size_t)a->batch * a->hw * a->channels * (a->act == DMN_ACT_F32 ? 4 : 2));
+  int rc;
+  if ((rc = nchw_to_nhwc(a->raw, base, a->batch, a->channels, a->hw, a->act, st))) return rc;
+  if (a->res && (rc = nchw_to_nhwc(a->res, base + act_bytes, a->batch, a->channels, a->hw, a->act, st))) return rc;
+  FinalizeP q;
+  q.raw = base; q.stats = (const stat_t*)a->stats; q.groups = a->groups;
+  q.gamma = a->gamma; q.beta = a->beta; q.silu = a->silu;
+  q.res = a->res ? base + act_bytes : nullptr;
+  q.out = base + 2 * act_bytes;
+  q.B = a->batch; q.HW = a->hw; q.C = a->channels;
+  if (a->ogroups > 0) {
+    DMN_CUDA_CHECK(cudaMemsetAsync(a->out_stats, 0, (size_t)a->batch * a->ogroups * 2 * sizeof(stat_t), st));
+    q.ostats = (stat_t*)a->out_stats; q.ogroups = a->ogroups;
+  }
+  if ((rc = gn_finalize(q, a->act, st))) return rc;
+  return nhwc_to_nchw(base + 2 * act_bytes, a->y, a->batch, a->channels, a->hw, a->act, st);
+}
+
+// ---- final_conv tail: run_forward's OP_FINALPROJ, plain (final_proj) or fused with the DDPM update (launch_final_proj_ddpm) ----
+size_t dmn_final_proj_scratch_bytes(const dmn_final_proj_args* a) {
+  if (!a) return 0;
+  return al((size_t)a->batch * a->hw * a->channels * (a->act == DMN_ACT_F32 ? 4 : 2));
+}
+
+int dmn_final_proj_forward(const dmn_final_proj_args* a, void* stream) {
+  if (!a) return fail(DMN_EINVAL, "null args");
+  DMN_REQUIRE(a->y && a->w && a->scratch_dev, "null tensor");
+  DMN_REQUIRE(a->plain || (a->stats && a->gamma && a->beta && a->groups > 0), "null tensor (GroupNorm statistics / gamma / beta)");
+  DMN_REQUIRE(a->batch > 0 && a->hw > 0 && a->channels > 0 && a->cout > 0, "shape");
+  DMN_REQUIRE(a->act == DMN_ACT_F32 || a->act == DMN_ACT_BF16, "act");
+  DMN_REQUIRE(a->x ? (a->coef && a->x_out) : a->eps != nullptr, "null tensor (eps, or x / coef / x_out of the fused tail)");
+  DMN_REQUIRE(a->scratch_bytes >= dmn_final_proj_scratch_bytes(a), "scratch too small (dmn_final_proj_scratch_bytes)");
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc;
+  if ((rc = nchw_to_nhwc(a->y, a->scratch_dev, a->batch, a->channels, a->hw, a->act, st))) return rc;
+  FinalProjP q;
+  q.y = a->scratch_dev;
+  q.plain = a->plain ? 1 : 0;
+  q.stats = q.plain ? nullptr : (const stat_t*)a->stats;
+  q.groups = q.plain ? 0 : a->groups;
+  q.gamma = q.plain ? nullptr : a->gamma; q.beta = q.plain ? nullptr : a->beta;
+  q.w = a->w; q.bias = a->bias;
+  q.out = a->x ? nullptr : a->eps;
+  q.B = a->batch; q.HW = a->hw; q.C = a->channels; q.Cout = a->cout;
+  if (!a->x) return final_proj(q, a->act, st);
+  if (!fused_tail_supported(q, a->act)) return fail(DMN_ENOTSUP, "fused DDPM tail: shape not supported (the plan runs final_proj + dmn_ddpm_step)");
+  return launch_final_proj_ddpm(q, a->x, a->z, a->x_out, a->coef, nullptr, a->step, a->rng, nullptr, nullptr, st);
+}
+
 }  // extern "C"

@@ -243,6 +243,12 @@ __global__ void init_conv_kernel(const InitConvP p) {
   }
 }
 
+void init_conv_pack_weights(int cin, int cout, const float* w, float* dst) {
+  for (int co = 0; co < cout; ++co)
+    for (int ci = 0; ci < cin; ++ci)
+      for (int t = 0; t < 49; ++t) dst[((long)t * cin + ci) * cout + co] = w[((long)co * cin + ci) * 49 + t];
+}
+
 int init_conv(const InitConvP& p, int act, cudaStream_t st) {
   const size_t smem = (size_t)7 * (p.S + 6) * p.Cin * sizeof(float);
   DMN_REQUIRE(smem <= 48 * 1024, "init_conv: input row patch does not fit in shared memory");

@@ -70,6 +70,8 @@ struct InitConvP {
   int B = 0, Cin = 0, S = 0, Cout = 0;
 };
 int init_conv(const InitConvP& p, int act, cudaStream_t s);
+// SIMT packer: torch layout [Cout][Cin][7][7] -> [49*Cin][Cout] fp32
+void init_conv_pack_weights(int cin, int cout, const float* w_torch, float* dst_host);
 // tensor-core stem (bf16 activations): w = blocked bf16 image from init_conv_tcgen05_pack_weights
 int init_conv_tcgen05(const InitConvP& p, cudaStream_t s);
 bool init_conv_tcgen05_supported(int Cin, int S, int Cout, int B);
@@ -106,6 +108,10 @@ struct FinalProjP {
   int plain = 0;                   // 1: eps = conv1x1(y) only ('conv_bn_act' tail, unet.py:115-116); stats / gamma / beta unused
 };
 int final_proj(const FinalProjP& p, int act, cudaStream_t s);
+// the same projection fused with the DDPM posterior update and (advance != null) the loop's step counter (sampler.cu)
+bool fused_tail_supported(const FinalProjP& p, int act);
+int launch_final_proj_ddpm(const FinalProjP& p, const float* x, const float* z, float* out, const float* coef, const int32_t* step_dev,
+                           int step, dmn_rng rng, const dmn_rng* rng_dev, int32_t* advance, cudaStream_t st);
 
 int linattn_core(const void* qkv, void* out, int B, int heads, int dh, int N, int act, cudaStream_t s);
 int attn_core(const void* qkv, void* out, int B, int heads, int dh, int N, int act, cudaStream_t s);

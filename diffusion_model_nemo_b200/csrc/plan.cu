@@ -58,9 +58,6 @@ int launch_dpmpp(const float* x, const float* mo, float* hist, float* out, int b
                  const int32_t* step_dev, int step, cudaStream_t st);
 int launch_inpaint_prepare(const float* x, const float* known, const float* mask, float* out, long n, const float* coef,
                            const int32_t* step_dev, int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
-bool fused_tail_supported(const FinalProjP& p, int act);
-int launch_final_proj_ddpm(const FinalProjP& p, const float* x, const float* z, float* out, const float* coef, const int32_t* step_dev,
-                           int step, dmn_rng rng, const dmn_rng* rng_dev, int32_t* advance, cudaStream_t st);
 int launch_traj(const float* x, float* traj, long n, const int32_t* step_dev, int every, int n_steps, cudaStream_t st);
 int launch_bpd_qsample(const float* x0, const float* z, float* xt, long n, const float* coef, const int32_t* step_dev, int step, dmn_rng rng,
                        const dmn_rng* rng_dev, cudaStream_t st);
@@ -886,9 +883,7 @@ int dmn_plan_load_param(dmn_plan* p, const char* name, const float* host, int64_
     case PK_INIT: {
       const int dim = (int)q.shape[0], ch = (int)q.shape[1];
       tmp.resize(numel);
-      for (int co = 0; co < dim; ++co)
-        for (int ci = 0; ci < ch; ++ci)
-          for (int t = 0; t < 49; ++t) tmp[((long)t * ch + ci) * dim + co] = host[((long)co * ch + ci) * 49 + t];
+      init_conv_pack_weights(ch, dim, host, tmp.data());
       DMN_CUDA_CHECK(cudaMemcpyAsync(p->wbase + q.off, tmp.data(), numel * sizeof(float), cudaMemcpyHostToDevice, st));
       if (q.has_tc) {
         std::vector<char> img(init_conv_tcgen05_weight_bytes(dim));

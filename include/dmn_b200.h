@@ -396,6 +396,65 @@ typedef struct dmn_attn_block_args {
 int dmn_linear_attention_block(const dmn_attn_block_args* a, void* stream);
 size_t dmn_linear_attention_block_scratch_bytes(const dmn_attn_block_args* a);
 
+/* Unet.init_conv (unet.py:41, 7x7 pad 3) with the class embedding of unet.py:133-137 added in its epilogue:
+ *   y[b] = conv7x7(x[b]) + bias + cls_w[classes ? classes[b] : pad_class]       (cls_w NULL: no class term)
+ * x fp32 NCHW [batch][cin][size][size] (the sampler state), w [cout][cin][7][7], bias [cout], cls_w [rows][cout], classes int64
+ * [batch]; y fp32 NCHW [batch][cout][size][size] holding the act-typed values the engine stores.  Dispatch as the plan's:
+ * engine DMN_CONV_TCGEN05 and a shape the tensor-core stem supports -> tensor-core stem (bf16 out), otherwise the CUDA-core stem
+ * in `act`.  scratch_dev >= dmn_init_conv_scratch_bytes().  Validation path (host repack, sync copies). */
+typedef struct dmn_init_conv_args {
+  int32_t batch, cin, size, cout;
+  int32_t act, engine;
+  int32_t pad_class;
+  const float* x; const float* w; const float* bias;
+  const float* cls_w; const int64_t* classes;
+  float* y;
+  void* scratch_dev; size_t scratch_bytes;
+} dmn_init_conv_args;
+int dmn_init_conv_forward(const dmn_init_conv_args* a, void* stream);
+size_t dmn_init_conv_scratch_bytes(const dmn_init_conv_args* a);
+
+/* The ResnetBlock / attention-block epilogue (parts/convnext.py:35-45,86; utils.py:68-93):
+ *   y = act(GroupNorm(groups)(raw) * gamma + beta) + res        act = SiLU if silu, else identity; res optional (NULL)
+ * raw / res / y fp32 NCHW [batch][channels][hw] (y holds the act-typed values the engine stores).  The input statistics are the
+ * engine's fixed-point sums stats[batch][groups][2] = {round(sum * 2^24), round(sum of squares * 2^20)} (int64, device); with
+ * ogroups > 0 the call also returns the engine's fixed-point sums of y over ogroups groups in out_stats[batch][ogroups][2]
+ * (zeroed by the call, then accumulated by the kernel).  scratch_dev >= dmn_gn_finalize_scratch_bytes(). */
+typedef struct dmn_gn_finalize_args {
+  int32_t batch, channels, hw, groups, ogroups, silu, act;
+  const float* raw; const float* res;
+  const int64_t* stats;
+  const float* gamma; const float* beta;
+  float* y;
+  int64_t* out_stats;
+  void* scratch_dev; size_t scratch_bytes;
+} dmn_gn_finalize_args;
+int dmn_gn_finalize_forward(const dmn_gn_finalize_args* a, void* stream);
+size_t dmn_gn_finalize_scratch_bytes(const dmn_gn_finalize_args* a);
+
+/* The final_conv tail (unet.py:109-116): eps = conv1x1(SiLU(GroupNorm(groups)(y) * gamma + beta)) + bias, or with `plain`
+ * ('conv_bn_act' tail) eps = conv1x1(y) + bias (stats / gamma / beta unused).  y fp32 NCHW [batch][channels][hw], stats as for
+ * dmn_gn_finalize_forward, w [cout][channels], bias [cout]; eps fp32 NCHW [batch][cout][hw].
+ * With x != NULL the call runs the DDPM sampling loop's fused tail instead: the same projection followed by dmn_ddpm_step's update
+ * with coef row `step`, injected noise z (or, z NULL, the Philox draws of `rng` at loop step `step`), x_out = x_{t-1}
+ * [batch][cout][hw]; eps is then not written.  DMN_ENOTSUP where the plan would not fuse the tail.
+ * scratch_dev >= dmn_final_proj_scratch_bytes(). */
+typedef struct dmn_final_proj_args {
+  int32_t batch, channels, hw, cout, groups, plain, act;
+  const float* y;
+  const int64_t* stats;
+  const float* gamma; const float* beta;
+  const float* w; const float* bias;
+  float* eps;
+  const float* x; const float* coef; const float* z;
+  int32_t step;
+  dmn_rng rng;
+  float* x_out;
+  void* scratch_dev; size_t scratch_bytes;
+} dmn_final_proj_args;
+int dmn_final_proj_forward(const dmn_final_proj_args* a, void* stream);
+size_t dmn_final_proj_scratch_bytes(const dmn_final_proj_args* a);
+
 #ifdef __cplusplus
 }
 #endif

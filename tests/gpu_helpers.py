@@ -126,3 +126,96 @@ def linear_attention_block(x, sd, prefix, softmax=False):
         L.check(lib.dmn_linear_attention_block(C.byref(a), L.stream_ptr(dev)), "dmn_linear_attention_block")
     torch.cuda.synchronize(dev)
     return y
+
+
+def _scratch(nbytes, dev):
+    buf = torch.empty(nbytes + 256, dtype=torch.uint8, device=dev)
+    return buf, (buf.data_ptr() + 255) // 256 * 256
+
+
+def init_conv_forward(x, w, bias, *, cls_w=None, classes=None, pad_class=0, act=L.ACT_BF16, engine=L.CONV_TCGEN05):
+    """The 7x7 stem through dmn_init_conv_forward: x fp32 NCHW cuda state, w [Cout][Cin][7][7]; cls_w [rows][Cout] with int64 classes
+    (or None: every sample takes pad_class).  Returns y NCHW fp32 (holding the stored activation values)."""
+    lib = L.lib()
+    dev = x.device
+    b, cin, s, _ = x.shape
+    a = L.InitConvArgs()
+    a.batch, a.cin, a.size, a.cout, a.act, a.engine, a.pad_class = b, cin, s, w.shape[0], act, engine, pad_class
+    keep = [x.float().contiguous(), w.float().contiguous(), bias.float().contiguous()]
+    a.x, a.w, a.bias = (t.data_ptr() for t in keep)
+    if cls_w is not None:
+        keep.append(cls_w.float().contiguous())
+        a.cls_w = keep[-1].data_ptr()
+    if classes is not None:
+        keep.append(classes.to(torch.int64).contiguous())
+        a.classes = keep[-1].data_ptr()
+    y = torch.empty(b, w.shape[0], s, s, device=dev, dtype=torch.float32)
+    a.y = y.data_ptr()
+    buf, a.scratch_dev = _scratch(lib.dmn_init_conv_scratch_bytes(C.byref(a)), dev)
+    a.scratch_bytes = buf.numel() - 256
+    with torch.cuda.device(dev):
+        L.check(lib.dmn_init_conv_forward(C.byref(a), L.stream_ptr(dev)), "dmn_init_conv_forward")
+    torch.cuda.synchronize(dev)
+    return y
+
+
+def gn_finalize_forward(raw, stats, gamma, beta, *, res=None, silu=True, ogroups=0, act=L.ACT_BF16):
+    """gn_finalize through dmn_gn_finalize_forward: raw / res fp32 [B][C][HW] cuda, stats int64 [B][G][2] fixed-point sums.
+    Returns (y [B][C][HW] fp32, the kernel's int64 output sums [B][ogroups][2] or None)."""
+    lib = L.lib()
+    dev = raw.device
+    b, c, hw = raw.shape
+    a = L.GnFinalizeArgs()
+    a.batch, a.channels, a.hw, a.groups, a.ogroups, a.silu, a.act = b, c, hw, stats.shape[1], ogroups, int(silu), act
+    keep = [raw.float().contiguous(), stats.to(torch.int64).contiguous(), gamma.float().contiguous(), beta.float().contiguous()]
+    a.raw, a.stats, a.gamma, a.beta = (t.data_ptr() for t in keep)
+    if res is not None:
+        keep.append(res.float().contiguous())
+        a.res = keep[-1].data_ptr()
+    y = torch.empty(b, c, hw, device=dev, dtype=torch.float32)
+    a.y = y.data_ptr()
+    ost = None
+    if ogroups:
+        ost = torch.empty(b, ogroups, 2, device=dev, dtype=torch.int64)
+        a.out_stats = ost.data_ptr()
+    buf, a.scratch_dev = _scratch(lib.dmn_gn_finalize_scratch_bytes(C.byref(a)), dev)
+    a.scratch_bytes = buf.numel() - 256
+    with torch.cuda.device(dev):
+        L.check(lib.dmn_gn_finalize_forward(C.byref(a), L.stream_ptr(dev)), "dmn_gn_finalize_forward")
+    torch.cuda.synchronize(dev)
+    return y, ost
+
+
+def final_proj_forward(y, w, bias, *, stats=None, gamma=None, beta=None, plain=False, act=L.ACT_BF16, x=None, coef=None, step=0,
+                       z=None, rng=(0, 0)):
+    """final_conv tail through dmn_final_proj_forward: y fp32 [B][C][HW] cuda, w [Cout][C].  Without x: eps [B][Cout][HW]; with x
+    (and the coefficient table coef, noise z or Philox (seed, stream) rng at loop step `step`): the fused DDPM update x_{t-1}."""
+    lib = L.lib()
+    dev = y.device
+    b, c, hw = y.shape
+    a = L.FinalProjArgs()
+    a.batch, a.channels, a.hw, a.cout, a.plain, a.act = b, c, hw, w.shape[0], int(plain), act
+    keep = [y.float().contiguous(), w.float().reshape(w.shape[0], c).contiguous(), bias.float().contiguous()]
+    a.y, a.w, a.bias = (t.data_ptr() for t in keep)
+    if not plain:
+        a.groups = stats.shape[1]
+        keep += [stats.to(torch.int64).contiguous(), gamma.float().contiguous(), beta.float().contiguous()]
+        a.stats, a.gamma, a.beta = (t.data_ptr() for t in keep[-3:])
+    out = torch.empty(b, w.shape[0], hw, device=dev, dtype=torch.float32)
+    if x is None:
+        a.eps = out.data_ptr()
+    else:
+        keep += [x.float().contiguous(), coef.float().contiguous()]
+        a.x, a.coef = keep[-2].data_ptr(), keep[-1].data_ptr()
+        if z is not None:
+            keep.append(z.float().contiguous())
+            a.z = keep[-1].data_ptr()
+        a.step = step
+        a.rng = L.Rng(*rng)
+        a.x_out = out.data_ptr()
+    buf, a.scratch_dev = _scratch(lib.dmn_final_proj_scratch_bytes(C.byref(a)), dev)
+    a.scratch_bytes = buf.numel() - 256
+    with torch.cuda.device(dev):
+        L.check(lib.dmn_final_proj_forward(C.byref(a), L.stream_ptr(dev)), "dmn_final_proj_forward")
+    torch.cuda.synchronize(dev)
+    return out

@@ -13,6 +13,11 @@ that end in a partial 128-row tile.  Per case (tests/conv_ref.py):
   * GroupNorm output statistics against their derived bound, where the production conv has them;
   * the launch log (dmn_debug_conv_log) shows the tiling regime the case claims: (mt, mixed 256 / 128-row tiling, tiles > CTAs).
 
+The 7x7 stem (GEO_INIT: the fp32 NCHW sampler state rounded to bf16 by the producer, kx packed into 32 virtual channels, 3 shared
+zero rows between stacked images, the bias and class-embedding epilogue) runs through dmn_init_conv_forward with the same checks
+(tests/tail_ref.py): probes bit-equal for every (input channel, ky, kx) tap, corner taps included, with a class row per sample that
+differs from every other sample's; random weights within the element bound (K = 49 Cin); the tiling regime from the launch log.
+
 The reference runs on the GPU in float64.  Production defaults: no DMN_CONV_* switch is set.
 """
 import math
@@ -22,9 +27,10 @@ import torch
 
 from diffusion_model_nemo_b200 import _lib as L
 from conftest import make_unet
-from gpu_helpers import conv_forward, conv_log
+from gpu_helpers import conv_forward, conv_log, init_conv_forward
 from oracle import ref_port as O
 import conv_ref as R
+import tail_ref as T
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -139,8 +145,19 @@ CASES = [
     ("rag_u1_up_b255", 2, 4, 256, 0, 256, 8, 255, 0, 0, 0, (2, True, True)),
 ]
 CASE_BY_NAME = {c[0]: c for c in CASES}
-# the 7x7 stem (GEO_INIT, init_conv_tcgen05) has no layer entry point; it stays outside this coverage (class-embedding epilogue)
-EXCLUDED_GEO = {3: "7x7 stem (GEO_INIT)"}
+# the 7x7 stem: (name, Cin, S, Cout, B, class rows, claimed (mt, mixed, tiles > CTAs) or None where the plan runs the CUDA-core stem).
+# Class rows: "labels" = a random label per sample, "cfg" = labels for the first half and the pad row for the second (the
+# guidance-doubled batch), "pad" = no labels (every sample the pad row), None = no class table.
+STEM_CASES = [
+    ("stem_cfg1_b256", 3, 32, 128, 256, "labels", (2, False, True)),
+    ("stem_cfg1_b512", 3, 32, 128, 512, "cfg", (2, True, True)),
+    ("stem_cfg2_b128", 3, 64, 128, 128, None, (2, True, True)),
+    ("stem_cfg0_28x28_b256", 1, 28, 32, 256, None, (2, False, True)),
+    ("stem_rag_b37", 3, 32, 128, 37, "labels", (2, True, True)),
+    ("stem_rag_b255", 3, 32, 128, 255, "pad", (2, False, True)),
+]
+STEM_BY_NAME = {c[0]: c for c in STEM_CASES}
+NUM_CLASSES = 10
 CASE_KEYS = {}      # case name -> set of launch keys it produced
 SLACK = {}          # case name -> measured slack (printed by the coverage test)
 
@@ -266,6 +283,91 @@ def test_conv_tile_case(name):
     SLACK[name] = slack
 
 
+def _stem_inputs(case, seed):
+    name, cin, s, cout, b, cls_kind, _ = case
+    g = _g(seed)
+    x = torch.randn(b, cin, s, s, device=DEV, generator=g)        # fp32 state: the producer's bf16 rounding is part of the check
+    bias = torch.randn(cout, device=DEV, generator=g) * 0.1
+    cls_w = labels = rows = None
+    if cls_kind:
+        cls_w = torch.randn(NUM_CLASSES + 1, cout, device=DEV, generator=g)
+        if cls_kind == "labels":
+            labels = torch.randint(0, NUM_CLASSES, (b,), device=DEV, generator=g)
+        elif cls_kind == "cfg":
+            labels = torch.cat([torch.randint(0, NUM_CLASSES, (b // 2,), device=DEV, generator=g),
+                                torch.full((b - b // 2,), NUM_CLASSES, device=DEV)])
+        rows = cls_w[labels] if labels is not None else cls_w[NUM_CLASSES].expand(b, -1)
+    return x, bias, cls_w, labels, rows
+
+
+def _stem(case, x, w, bias, cls_w, labels):
+    conv_log()
+    y = init_conv_forward(x, w, bias, cls_w=cls_w, classes=labels, pad_class=NUM_CLASSES)
+    recs = conv_log()
+    assert len(recs) <= 1, recs
+    return y, (recs[0] if recs else None)
+
+
+def _check_stem_regime(case, rec):
+    name, cin, s, cout, b, cls_kind, claim = case
+    if rec is None:
+        assert claim is None, f"{name}: the tensor-core stem did not run"
+        return
+    assert claim is not None, f"{name}: the tensor-core stem ran where the case claims the CUDA-core stem"
+    assert (rec["geo"], rec["C1"], rec["Cout"], rec["H"], rec["B"]) == (3, cin, cout, s, b), rec
+    assert (rec["mt"], rec["mixed"], rec["multi"]) == claim, (name, rec)
+
+
+def run_stem_case(case, seed=0):
+    name, cin, s, cout, b, cls_kind, claim = case
+    x, bias, cls_w, labels, rows = _stem_inputs(case, seed)
+    keys, slack = set(), {}
+    # ---- probes: every (input channel, ky, kx) tap -- corners included -- with each sample's own class row ----
+    for j in range(R.probe_count(cin, cout, 0, 7)):
+        w = R.probe_weights(cin, cout, 0, 7, j).to(DEV)
+        y, rec = _stem(case, x, w, bias, cls_w, labels)
+        _check_stem_regime(case, rec)
+        tc = rec is not None
+        if tc:
+            keys.add(_key(rec))
+        xo, _ = T.stem_operands(x, w, tc)
+        r0, _ = R.probe_ref(xo, cin, cout, 0, 7, j)
+        nbad, where = R.check_probe(y, T.stem_epilogue(r0, bias, rows, tc))
+        assert nbad == 0, f"{name} probe {j}: {nbad} elements differ, first at (b, o, y, x) {where}"
+    # ---- random weights ----
+    w = torch.randn(cout, cin, 7, 7, device=DEV, generator=_g(seed + 1)) / math.sqrt(49 * cin)
+    y, rec = _stem(case, x, w, bias, cls_w, labels)
+    _check_stem_regime(case, rec)
+    tc = rec is not None
+    r, rabs = T.stem_ref(x, w, bias, rows, tc)
+    nv, ratio, frac = R.check_bound(y, r, T.stem_bound(r, rabs, cin))
+    assert nv == 0, f"{name} random: {nv} elements over the bound (max err / bound {ratio:.3g})"
+    assert frac <= FRAC_GATE, f"{name} random: {frac:.4f} of the elements differ from bf16_RN(fp64)"
+    # the price of the bf16 operand: distance of the result from the convolution of the fp32 state (same bf16 weights)
+    r32 = R.conv_ref(x.double(), R.bf16(w).double() if tc else w.double(), bias, 0, 7)
+    if rows is not None:
+        r32 = r32 + rows.double()[:, :, None, None]
+    slack.update(rand=ratio, frac=frac, bf16_state_rel_l2=float((y.double() - r32).norm() / r32.norm()))
+    return keys, slack
+
+
+@pytest.mark.parametrize("name", [c[0] for c in STEM_CASES])
+def test_stem_case(name):
+    keys, slack = run_stem_case(STEM_BY_NAME[name])
+    CASE_KEYS[name] = keys
+    SLACK[name] = slack
+
+
+def test_stem_case_runs_the_stem_the_plan_runs():
+    """The configs[0] shape (1 x 28 x 28, dim 32) is pinned on whichever stem its plan dispatches to."""
+    cfg = dict(dim=32, dim_mults=[1, 2, 4], channels=1, groups=8)
+    u = make_unet(cfg, O.random_state_dict(cfg, seed=0), dtype="bf16", engine="tcgen05", device=DEV)
+    init = [o for o in u.plan(28, 256, DEV).op_table() if o[0] == "init_conv"]
+    assert len(init) == 1
+    claim = STEM_BY_NAME["stem_cfg0_28x28_b256"][6]
+    assert init[0][2] == (0 if claim is None else 1), f"the plan's stem engine is {init[0][2]}, the case claims {claim}"
+
+
 def _plan_keys(cfg, size, batch):
     sd = O.random_state_dict(cfg, seed=0)
     u = make_unet(cfg, sd, dtype="bf16", engine="tcgen05", device=DEV)
@@ -289,21 +391,20 @@ def test_cases_cover_every_production_instantiation():
              "configs[2] B=128": (dict(c1, learned_variance=True), 64, 128), "configs[3] B=256": (dict(c1, groups=4), 32, 256)}
     need = {}
     for pname, (cfg, size, batch) in plans.items():
-        for rec in _plan_keys(cfg, size, batch):
-            if rec["geo"] in EXCLUDED_GEO:
-                need.setdefault(("excluded", EXCLUDED_GEO[rec["geo"]]), set()).add(pname)
-                continue
+        recs = _plan_keys(cfg, size, batch)
+        assert sum(r["geo"] == 3 for r in recs) == 1, f"{pname}: the tensor-core stem is not launched once per forward"
+        for rec in recs:
             need.setdefault(_key(rec), set()).add(pname)
     have = {}
-    for case in CASES:
+    for case, runner in [(c, run_case) for c in CASES] + [(c, run_stem_case) for c in STEM_CASES]:
         if case[0] not in CASE_KEYS:
-            CASE_KEYS[case[0]], SLACK[case[0]] = run_case(case)
+            CASE_KEYS[case[0]], SLACK[case[0]] = runner(case)
         for kk in CASE_KEYS[case[0]]:
             have.setdefault(kk, case[0])
     print(f"\n{nsm} SMs; production keys (kernel, mt, mixed, tiles > CTAs) -> covering case:")
     missing = []
     for kk, pl in sorted(need.items(), key=str):
-        cov = "EXCLUDED" if kk[0] == "excluded" else have.get(kk)
+        cov = have.get(kk)
         print(f"  {kk} [{', '.join(sorted(pl))}] -> {cov}")
         if cov is None:
             missing.append(kk)
