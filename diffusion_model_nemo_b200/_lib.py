@@ -128,6 +128,9 @@ SYMBOLS = {
     "dmn_plan_ready": (_I, [_P]),
     "dmn_plan_film_layout": (_I, [_P, _P, _I]),
     "dmn_time_table": (_I, [_P, _P, _I, _I, _P]),
+    "dmn_plan_time_table_info": (_I, [_P, C.POINTER(C.c_size_t), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
+    "dmn_plan_param_time_col": (_I, [_P, _I]),
+    "dmn_plan_film_col": (_I, [_P, _I]),
     "dmn_unet_forward": (_I, [_P, _P, _P, _P, _P, _I, _P]),
     "dmn_plan_launches_per_forward": (_I, [_P]),
     "dmn_plan_num_ops": (_I, [_P]),

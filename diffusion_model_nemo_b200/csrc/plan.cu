@@ -154,7 +154,7 @@ struct dmn_plan {
   size_t off_freqs = 0, off_wct = 0, off_bc = 0;
   bool freqs_loaded = false;
   // FiLM (WaveGradUNet): channels of every evaluated FiLM layer, in table-column order
-  std::vector<int> film_channels;
+  std::vector<int> film_channels, film_cols;   // film_cols: first table column of each FiLM layer
   Buf time_tmp, time_table;
   // statistics arena
   size_t stats_off = 0, stats_bytes = 0;
@@ -331,6 +331,7 @@ struct Builder {
     const int col = P.sumC;
     P.sumC += C;
     P.film_channels.push_back(C);
+    P.film_cols.push_back(col);
     conv(p + ".signal_conv.0", CONV_SAME, 3, x, C, Buf(), 0, C, H, tmp, true, 0);
     conv(p + ".scale_conv", CONV_SAME, 3, tmp, C, Buf(), 0, C, H, scale, true, 0, PRO_LRELU | PRO_TEMB, 0, Buf(), -1, -1, col);
     conv(p + ".shift_conv", CONV_SAME, 3, tmp, C, Buf(), 0, C, H, shift, true, 0, PRO_LRELU | PRO_TEMB, 0, Buf(), -1, -1, col);
@@ -1010,6 +1011,8 @@ int dmn_plan_film_layout(const dmn_plan* p, int32_t* channels_out, int cap) {
 }
 
 int dmn_time_table(dmn_plan* p, const float* times_dev, int row0, int rows, void* stream) {
+  // rows_linear_kernel puts the rows on grid.y; refuse a count it cannot launch before anything is enqueued
+  DMN_REQUIRE(rows <= 65535, "dmn_time_table takes at most 65535 rows per call");
   int rc = check_ready(p);
   if (rc) return rc;
   DMN_REQUIRE(times_dev && row0 >= 0 && rows > 0 && row0 + rows <= p->cfg.max_time_rows, "time table rows out of range");
@@ -1033,6 +1036,26 @@ int dmn_time_table(dmn_plan* p, const float* times_dev, int row0, int rows, void
   t.table = (float*)(p->wsbase + p->time_table.off) + (size_t)row0 * p->sumC;
   t.rows = rows; t.dim = dim; t.sumC = p->sumC;
   return time_table(t, (cudaStream_t)stream);
+}
+
+int dmn_plan_time_table_info(const dmn_plan* p, size_t* ws_offset, int32_t* sum_c, int32_t* max_rows) {
+  if (!p) return fail(DMN_EINVAL, "null plan");
+  DMN_REQUIRE(p->time_table.valid(), "plan has neither a time embedding nor FiLM: no time table");
+  if (ws_offset) *ws_offset = p->time_table.off;
+  if (sum_c) *sum_c = p->sumC;
+  if (max_rows) *max_rows = p->cfg.max_time_rows;
+  return 0;
+}
+
+int dmn_plan_param_time_col(const dmn_plan* p, int i) {
+  if (!p || i < 0 || i >= (int)p->params.size()) return -1;
+  const Param& q = p->params[i];
+  return (q.kind == PK_BLOCK_MLP_W || q.kind == PK_BLOCK_MLP_B) ? q.col : -1;
+}
+
+int dmn_plan_film_col(const dmn_plan* p, int layer) {
+  if (!p || layer < 0 || layer >= (int)p->film_cols.size()) return -1;
+  return p->film_cols[layer];
 }
 
 int dmn_unet_forward(dmn_plan* p, const float* x_dev, const int32_t* row_dev, const int64_t* classes_dev, float* out_dev,

@@ -96,8 +96,17 @@ int dmn_plan_ready(const dmn_plan* p);                 /* 1 when every parameter
 int dmn_plan_film_layout(const dmn_plan* p, int32_t* channels_out, int cap);
 
 /* time_mlp + the 16 per-block `mlp` projections for `rows` time values -> table rows [row0, row0+rows).
- * Replaces Unet.time_mlp (unet.py:61-66) and ResnetBlock.mlp (convnext.py:68-72,81-83). */
+ * Replaces Unet.time_mlp (unet.py:61-66) and ResnetBlock.mlp (convnext.py:68-72,81-83).  At most 65535 rows per call
+ * (DMN_EINVAL otherwise, before anything is enqueued). */
 int dmn_time_table(dmn_plan* p, const float* times_dev, int row0, int rows, void* stream);
+/* Read-only view of the table (validation aid): row r, column c is the fp32 at workspace + *ws_offset + (r * *sum_c + c) * 4 for
+ * r < *max_rows.  DMN_EINVAL for a plan with neither time embedding nor FiLM.  Any output pointer may be NULL. */
+int dmn_plan_time_table_info(const dmn_plan* p, size_t* ws_offset, int32_t* sum_c, int32_t* max_rows);
+/* First table column of parameter i: a ResnetBlock's `mlp.1.weight` / `mlp.1.bias` fill columns [col, col + Cout); -1 for any
+ * other parameter or a bad index. */
+int dmn_plan_param_time_col(const dmn_plan* p, int i);
+/* film plans: first table column of FiLM layer `layer` (dmn_plan_film_layout order; it fills [col, col + channels)); -1 otherwise. */
+int dmn_plan_film_col(const dmn_plan* p, int layer);
 /* film plans: `times_dev` holds continuous noise levels and the table rows are the FiLM positional encodings
  * sin | cos (5000 * level * exponents) of every FiLM layer (parts/film.py:17-26); dmn_unet_forward then evaluates
  * WaveGradUNet.forward(x, noise_level) (unet.py:212-266).  Plans with neither time embedding nor FiLM ignore the call. */

@@ -128,6 +128,29 @@ def linear_attention_block(x, sd, prefix, softmax=False):
     return y
 
 
+def time_layout(h):
+    """(workspace byte offset, sumC, max_time_rows, {block prefix or 'films.<i>': first table column}) of plan h's time table, read
+    through the C ABI (no device access)."""
+    lib = L.lib()
+    off, sum_c, rows = C.c_size_t(), C.c_int32(), C.c_int32()
+    L.check(lib.dmn_plan_time_table_info(h, C.byref(off), C.byref(sum_c), C.byref(rows)), "dmn_plan_time_table_info")
+    cols = {}
+    for i in range(lib.dmn_plan_num_params(h)):
+        name = lib.dmn_plan_param_name(h, i).decode()
+        if name.endswith(".mlp.1.weight"):
+            cols[name[:-len(".mlp.1.weight")]] = lib.dmn_plan_param_time_col(h, i)
+    for j in range(lib.dmn_plan_film_layout(h, None, 0)):
+        cols[f"films.{j}"] = lib.dmn_plan_film_col(h, j)
+    return off.value, sum_c.value, rows.value, cols
+
+
+def time_table_view(plan):
+    """The fp32 [max_time_rows][sumC] time table of an engine.UnetPlan as a view into its workspace tensor."""
+    off, sum_c, rows, _ = time_layout(plan.h)
+    base = (plan.workspace.data_ptr() + 255) // 256 * 256 - plan.workspace.data_ptr() + off
+    return plan.workspace[base:base + rows * sum_c * 4].view(torch.float32).view(rows, sum_c)
+
+
 def _scratch(nbytes, dev):
     buf = torch.empty(nbytes + 256, dtype=torch.uint8, device=dev)
     return buf, (buf.data_ptr() + 255) // 256 * 256
