@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdmn_b200.so")
-SOURCES = ["plan.cu", "kernels_simt.cu", "conv_tcgen05.cu", "linattn_mma.cu", "attn_fused.cu", "sampler.cu", "api_layers.cu", "ode.cu"]
+SOURCES = ["plan.cu", "kernels_simt.cu", "conv_tcgen05.cu", "linattn_mma.cu", "attn_fused.cu", "sampler.cu", "api_layers.cu", "ode.cu", "jvp.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xptxas", "-v",

@@ -62,6 +62,19 @@ class OdeDesc(C.Structure):
     ]
 
 
+HUTCH_RADEMACHER, HUTCH_GAUSSIAN = 0, 1
+
+
+class OdeLikelihoodDesc(C.Structure):
+    _fields_ = [
+        ("sde_kind", C.c_int32), ("N", C.c_int32), ("beta_0", C.c_double), ("beta_1", C.c_double), ("sigma_min", C.c_double),
+        ("sigma_max", C.c_double), ("t0", C.c_double), ("t1", C.c_double), ("rtol", C.c_double), ("atol", C.c_double),
+        ("max_nfe", C.c_int32), ("batch", C.c_int32), ("use_graph", C.c_int32), ("hutchinson", C.c_int32), ("rng", Rng),
+        ("noise_dev", C.c_void_p), ("classes_dev", C.c_void_p), ("state_dev", C.c_void_p), ("state_elems", C.c_int64),
+        ("work_dev", C.c_void_p), ("work_bytes", C.c_size_t), ("result_dev", C.c_void_p),
+    ]
+
+
 class ConvArgs(C.Structure):
     _fields_ = [
         ("mode", C.c_int32), ("ksize", C.c_int32), ("batch", C.c_int32), ("cin", C.c_int32), ("cout", C.c_int32),
@@ -132,6 +145,8 @@ SYMBOLS = {
     "dmn_plan_param_time_col": (_I, [_P, _I]),
     "dmn_plan_film_col": (_I, [_P, _I]),
     "dmn_unet_forward": (_I, [_P, _P, _P, _P, _P, _I, _P]),
+    "dmn_unet_jvp": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _I, _P]),
+    "dmn_unet_jvp_work_bytes": (C.c_size_t, [_P, _I]),
     "dmn_plan_launches_per_forward": (_I, [_P]),
     "dmn_plan_num_ops": (_I, [_P]),
     "dmn_plan_op_info": (_I, [_P, _I, C.c_char_p, _I, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_double),
@@ -156,6 +171,8 @@ SYMBOLS = {
     "dmn_sample_loop_inpaint": (_I, [_P, C.POINTER(LoopDesc), C.POINTER(InpaintDesc), _P]),
     "dmn_ode_sample": (_I, [_P, C.POINTER(OdeDesc), _P]),
     "dmn_ode_work_bytes": (C.c_size_t, [_P, _I]),
+    "dmn_ode_likelihood": (_I, [_P, C.POINTER(OdeLikelihoodDesc), _P]),
+    "dmn_ode_likelihood_work_bytes": (C.c_size_t, [_P, _I]),
     "dmn_conv_forward": (_I, [C.POINTER(ConvArgs), _P]),
     "dmn_conv_scratch_bytes": (C.c_size_t, [C.POINTER(ConvArgs)]),
     "dmn_conv_forward_cat": (_I, [C.POINTER(ConvArgs), _P, C.c_int32, _P]),

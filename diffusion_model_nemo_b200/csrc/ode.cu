@@ -153,12 +153,12 @@ __global__ void __launch_bounds__(kThreads) ode_init_elem_kernel(OdeWork w, OdeP
   double a = 0.0, b = 0.0;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
     if (mode == 0) {
-      y[i] = (double)state[i];
-      w.x32[i] = state[i];
+      y[i] = i < w.nx ? (double)state[i] : 0.0;
+      if (i < w.nx) w.x32[i] = state[i];
     } else if (mode == 2) {
-      w.x32[i] = __double2float_rn(y[i] + hd * (double)K0[i]);
+      if (i < w.nx) w.x32[i] = __double2float_rn(y[i] + hd * (double)K0[i]);
     } else {
-      const float f = drift(P.sde_kind, w.x32[i], w.mo[i], fx, sc, g2);
+      const float f = i < w.nx ? drift(P.sde_kind, w.x32[i], w.mo[i], fx, sc, g2) : w.mo[i];
       const double s = P.atol + fabs(y[i]) * P.rtol;
       if (mode == 1) {
         K0[i] = f;
@@ -229,21 +229,21 @@ __global__ void __launch_bounds__(kThreads) ode_stage_kernel(OdeWork w, OdeParam
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
     float k = 0.f;
     if (S >= 1) {
-      k = drift(P.sde_kind, w.x32[i], w.mo[i], fx, sc, g2);
+      k = i < w.nx ? drift(P.sde_kind, w.x32[i], w.mo[i], fx, sc, g2) : w.mo[i];
       Ks[i] = k;
     }
     if (S <= 4) {
       double acc = 0.0;
 #pragma unroll
       for (int j = 0; j <= S; ++j) acc = __dadd_rn(acc, __dmul_rn((double)(S >= 1 && j == S ? k : Kj[j][i]), kA[S + 1][j]));
-      w.x32[i] = __double2float_rn(__dadd_rn(y[i], __dmul_rn(acc, h)));
+      if (i < w.nx) w.x32[i] = __double2float_rn(__dadd_rn(y[i], __dmul_rn(acc, h)));
     } else if (S == 5) {
       double acc = 0.0;
 #pragma unroll
       for (int j = 0; j <= 5; ++j) acc = __dadd_rn(acc, __dmul_rn((double)(j == 5 ? k : Kj[j][i]), kB[j]));
       const double v = __dadd_rn(y[i], __dmul_rn(h, acc));
       yn[i] = v;
-      w.x32[i] = __double2float_rn(v);
+      if (i < w.nx) w.x32[i] = __double2float_rn(v);
     } else {
       double acc = 0.0;
 #pragma unroll
@@ -294,6 +294,34 @@ __global__ void __launch_bounds__(kThreads) ode_control_kernel(OdeWork w, OdePar
   publish(r, w.result);
 }
 
+// ---- likelihood (augmented state [x ; delta_logp]) ----------------------------------------------------------------------------
+// Hutchinson divergence of the drift at the evaluation of stage row `row`: mo[nx + b] = sum_i eps_i * drift(eps_i, dmo_i) over
+// sample b, where dmo is the U-Net JVP in direction eps (drift is linear in (x, model output), so drift(eps, dmo) is its tangent).
+// One block per sample, fp64 per-thread sums in a fixed order, then a fixed-order block reduction.
+__global__ void __launch_bounds__(kThreads) ode_div_kernel(OdeWork w, OdeParams P, int row, long chw) {
+  __shared__ double red[kThreads];
+  const OdeRec& r = *w.rec;
+  const float fx = r.fx[row], sc = r.sc[row], g2 = r.g2[row];
+  const long base = (long)blockIdx.x * chw;
+  double a = 0.0;
+  for (long i = threadIdx.x; i < chw; i += kThreads) {
+    const float e = w.eps[base + i];
+    a += (double)e * (double)drift(P.sde_kind, e, w.dmo[base + i], fx, sc, g2);
+  }
+  red[threadIdx.x] = a;
+  __syncthreads();
+  for (int s = kThreads / 2; s > 0; s >>= 1) {
+    if ((int)threadIdx.x < s) red[threadIdx.x] += red[threadIdx.x + s];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) w.mo[w.nx + blockIdx.x] = __double2float_rn(red[0]);
+}
+
+// Rademacher noise from a Gaussian draw: +1 where the draw is >= 0, -1 elsewhere
+__global__ void __launch_bounds__(kThreads) ode_rademacher_kernel(float* __restrict__ e, long n) {
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) e[i] = e[i] >= 0.f ? 1.f : -1.f;
+}
+
 // solution.y[:, -1] cast to fp32 (the last accepted state)
 __global__ void __launch_bounds__(kThreads) ode_finish_kernel(OdeWork w, float* __restrict__ state) {
   const double* y = w.y + (long)w.rec->cur * w.n;
@@ -320,6 +348,7 @@ size_t ode_work_layout(long n, char* base, OdeWork* w) {
   const size_t o_p = off;    off += up((size_t)2 * ode_grid(n) * sizeof(double));
   if (w) {
     w->n = n;
+    w->nx = n;
     w->rec = (OdeRec*)(base + o_rec);
     w->rows = (int32_t*)(base + o_rec + sizeof(OdeRec));
     w->y = (double*)(base + o_y);
@@ -368,6 +397,18 @@ int launch_ode_control(const OdeWork& w, const OdeParams& P, cudaGraphConditiona
   ode_control_kernel<<<1, kThreads, 0, st>>>(w, P, ode_grid(w.n), hnd, use_cond);
   count_launch();
   DMN_LAUNCH_CHECK("ode_control");
+  return 0;
+}
+int launch_ode_div(const OdeWork& w, const OdeParams& P, int row, int batch, cudaStream_t st) {
+  ode_div_kernel<<<batch, kThreads, 0, st>>>(w, P, row, w.nx / batch);
+  count_launch();
+  DMN_LAUNCH_CHECK("ode_div");
+  return 0;
+}
+int launch_ode_rademacher(float* e, long n, cudaStream_t st) {
+  ode_rademacher_kernel<<<ode_grid(n), kThreads, 0, st>>>(e, n);
+  count_launch();
+  DMN_LAUNCH_CHECK("ode_rademacher");
   return 0;
 }
 int launch_ode_finish(const OdeWork& w, float* state, cudaStream_t st) {

@@ -142,6 +142,25 @@ int attn_softmax_fused(const LinAttnFusedP& p, cudaStream_t s);
 // plumbing self-test of the TMA tensor copies + 128-byte-swizzle UMMA descriptors: D[M][N] = A[M][K] . B[N][K]^T (row-major bf16 in, fp32 out)
 int selftest_tma_sw128_gemm(const void* a_bf16, const void* b_bf16, float* d, int M, int N, int K, cudaStream_t s);
 
+// ---- forward-mode JVP tangents (jvp.cu, fp32 NHWC) ----
+// out = act'(a) * gamma * rstd * (dh - mean_g(dh) - hn * mean_g(hn * dh)) [+ dres]: the tangent of act(GroupNorm(h)) [+ res]
+// from the primal statistics of h (act = SiLU when silu, identity otherwise)
+struct GnTangentP {
+  const float* h = nullptr;        // primal input of the norm
+  const float* dh = nullptr;       // its tangent
+  const stat_t* stats = nullptr;   // primal statistics of h [B][groups][2]
+  int groups = 0;
+  const float* gamma = nullptr;
+  const float* beta = nullptr;
+  int silu = 0;
+  const float* dres = nullptr;     // optional residual tangent
+  float* out = nullptr;
+  int B = 0, HW = 0, C = 0;
+};
+int gn_tangent(const GnTangentP& p, cudaStream_t s);
+int linattn_jvp(const void* qkv, const void* dqkv, void* dout, int B, int heads, int dh, int N, cudaStream_t s);
+int attn_jvp(const void* qkv, const void* dqkv, void* dout, int B, int heads, int dh, int N, cudaStream_t s);
+
 // time path
 struct TimeP {
   const float* times = nullptr;    // [rows]
@@ -191,7 +210,8 @@ struct OdeRec {
 };
 // views into the caller's work buffer
 struct OdeWork {
-  long n = 0;                            // batch * C * H * W
+  long n = 0;                            // state elements: batch * C * H * W, + batch log-density rows for the likelihood
+  long nx = 0;                           // image elements (the U-Net's input); elements [nx, n) take their drift from mo[i]
   OdeRec* rec = nullptr;
   int32_t* rows = nullptr;               // {0..5}: time-table row of each stage (row_dev of the U-Net forwards)
   double* y = nullptr;                   // [2][n]
@@ -200,6 +220,8 @@ struct OdeWork {
   float* mo = nullptr;                   // [n] U-Net output
   double* partials = nullptr;            // [ode_grid(n)][2]
   dmn_ode_result* result = nullptr;
+  const float* eps = nullptr;            // likelihood: [nx] Hutchinson noise
+  float* dmo = nullptr;                  // likelihood: [nx] U-Net JVP in direction eps
 };
 size_t ode_work_layout(long n, char* base, OdeWork* w);    // bytes; fills w when given
 int ode_grid(long n);
@@ -209,5 +231,7 @@ int launch_ode_init_step(const OdeWork& w, const OdeParams& P, int mode, cudaGra
 int launch_ode_stage(const OdeWork& w, const OdeParams& P, int s, cudaStream_t st);
 int launch_ode_control(const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd, int use_cond, cudaStream_t st);
 int launch_ode_finish(const OdeWork& w, float* state, cudaStream_t st);
+int launch_ode_div(const OdeWork& w, const OdeParams& P, int row, int batch, cudaStream_t st);
+int launch_ode_rademacher(float* e, long n, cudaStream_t st);
 
 }  // namespace dmn

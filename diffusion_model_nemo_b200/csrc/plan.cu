@@ -169,11 +169,13 @@ struct dmn_plan {
     dmn_inpaint_desc ip{};   // all null for a plain sampling loop
   };
   std::vector<GraphEntry> graphs;
+  template <class Desc>
   struct OdeGraphEntry {
     cudaGraphExec_t exec = nullptr;
-    dmn_ode_desc key;
+    Desc key;
   };
-  std::vector<OdeGraphEntry> ode_graphs;
+  std::vector<OdeGraphEntry<dmn_ode_desc>> ode_graphs;
+  std::vector<OdeGraphEntry<dmn_ode_likelihood_desc>> lik_graphs;
   void drop_graphs() {
     for (auto& g : graphs)
       if (g.exec) cudaGraphExecDestroy(g.exec);
@@ -181,6 +183,9 @@ struct dmn_plan {
     for (auto& g : ode_graphs)
       if (g.exec) cudaGraphExecDestroy(g.exec);
     ode_graphs.clear();
+    for (auto& g : lik_graphs)
+      if (g.exec) cudaGraphExecDestroy(g.exec);
+    lik_graphs.clear();
   }
   ~dmn_plan() { drop_graphs(); }
 };
@@ -654,110 +659,117 @@ __global__ void stamp_kernel(unsigned long long* t) {
   *t = v;
 }
 
-static int run_forward(dmn_plan* P, const float* x_dev, const int32_t* row_dev, const int64_t* classes_dev, float* out_dev,
-                       int batch, cudaStream_t st, std::vector<cudaEvent_t>* evs = nullptr, const TailFuse* tail = nullptr,
-                       unsigned long long* stamps = nullptr) {
+// one op of the forward program
+static int enqueue_op(dmn_plan* P, const Op& o, const float* x_dev, const int32_t* row_dev, const int64_t* classes_dev, float* out_dev,
+                      int batch, cudaStream_t st, const TailFuse* tail) {
   const dmn_unet_cfg& c = P->cfg;
   auto W = [&](int pi) -> const float* { return pi < 0 ? nullptr : (const float*)(P->wbase + P->params[pi].off); };
   auto B = [&](const Buf& b) -> void* { return b.valid() ? (void*)(P->wsbase + b.off) : nullptr; };
+  int rc = 0;
+  switch (o.kind) {
+    case OP_MEMSET: {
+      DMN_CUDA_CHECK(cudaMemsetAsync(P->wsbase + P->stats_off, 0, P->stats_bytes, st));
+      count_launch();
+      break;
+    }
+    case OP_INIT: {
+      InitConvP q;
+      q.x = x_dev;
+      q.w = W(P->pidx["init_conv.weight"]);
+      q.bias = W(P->pidx["init_conv.bias"]);
+      if (c.num_classes >= 0 && !c.film) {
+        q.cls_w = W(P->pidx["class_embed.weight"]);
+        q.classes = classes_dev;
+        q.pad_class = c.num_classes;
+      }
+      q.out = B(o.out);
+      q.B = batch; q.Cin = c.channels; q.S = c.image_size; q.Cout = c.dim;
+      if (P->init_tc) {
+        q.w = (const float*)(P->wbase + P->params[P->pidx["init_conv.weight"]].off2);
+        rc = init_conv_tcgen05(q, st);
+      } else {
+        rc = init_conv(q, P->act, st);
+      }
+      break;
+    }
+    case OP_CONV: {
+      ConvP q;
+      q.src1 = B(o.src1); q.src2 = B(o.src2); q.C1 = o.C1; q.C2 = o.C2;
+      q.B = batch; q.Hin = q.Win = o.Hin; q.Hout = q.Wout = o.Hout; q.Cout = o.Cout;
+      q.mode = o.mode; q.ksize = o.ksize;
+      const Param& wp = P->params[o.w];
+      q.w = o.tc ? (const void*)(P->wbase + wp.off2) : (const void*)(P->wbase + wp.off);
+      q.bias = W(o.bias);
+      q.pro = o.pro; q.pstats = (const stat_t*)B(o.pstats); q.pgroups = o.pgroups;
+      q.pgamma = W(o.pgamma); q.pbeta = W(o.pbeta);
+      if (o.pro & PRO_TEMB) {
+        q.temb = (const float*)B(P->time_table) + o.temb_col;
+        if (row_dev) { q.d_row = row_dev; q.temb_rstride = P->sumC; q.temb_bstride = 0; }
+        else { q.d_row = nullptr; q.temb_rstride = 0; q.temb_bstride = P->sumC; }
+      }
+      if (o.fold) {
+        q.pro = PRO_NONE;
+        q.pgroups = 1;
+        q.fold_s1 = (const float*)(P->wbase + o.fold_off);
+        q.fold_s2 = q.fold_s1 + o.Cout;
+      }
+      q.out = B(o.out); q.res = B(o.res);
+      q.ostats = (stat_t*)B(o.ostats); q.ogroups = o.ogroups;
+      rc = o.tc ? conv_tcgen05(q, st) : conv_simt(q, P->act, st);
+      break;
+    }
+    case OP_FINALIZE: {
+      FinalizeP q;
+      q.raw = B(o.raw); q.stats = (const stat_t*)B(o.stats); q.groups = o.groups;
+      q.gamma = W(o.gamma); q.beta = W(o.beta); q.silu = o.silu;
+      q.res = B(o.res); q.out = B(o.out); q.ostats = (stat_t*)B(o.ostats); q.ogroups = o.ogroups;
+      q.B = batch; q.HW = o.HW; q.C = o.C;
+      rc = gn_finalize(q, P->act, st);
+      break;
+    }
+    case OP_LINATTN:
+      rc = linattn_core(B(o.src1), B(o.out), batch, o.heads, o.dh, o.N, P->act, st);
+      break;
+    case OP_ATTN:
+      rc = attn_core(B(o.src1), B(o.out), batch, o.heads, o.dh, o.N, P->act, st);
+      break;
+    case OP_ATTN_FUSED: {
+      LinAttnFusedP q;
+      q.x = B(o.src1); q.out = B(o.out); q.pstats = (const stat_t*)B(o.pstats);
+      q.wqkv = P->wbase + P->params[o.w].off;
+      q.wo = P->wbase + P->params[o.wo].off;
+      q.s1 = (const float*)(P->wbase + o.fold_off);
+      q.s2 = q.s1 + 384;
+      q.bo = W(o.bo); q.go = W(o.gamma); q.beo = W(o.beta);
+      q.B = batch; q.N = o.N; q.C = o.C;
+      rc = o.softmax ? attn_softmax_fused(q, st) : linattn_fused(q, st);
+      break;
+    }
+    case OP_CLASSADD:
+      rc = class_embed_add(B(o.src1), W(P->pidx["class_embed.weight"]), classes_dev, c.num_classes, batch, o.HW, o.C, P->act, st);
+      break;
+    case OP_MODULATE:
+      rc = film_modulate(B(o.src1), B(o.src2), B(o.res), B(o.out), (long)batch * o.HW * o.C, P->act, st);
+      break;
+    case OP_FINALPROJ: {
+      const FinalProjP q = final_proj_params(P, o, out_dev, batch);
+      if (tail) rc = launch_final_proj_ddpm(q, tail->x, tail->z, tail->out, tail->coef, tail->step_dev, tail->step, tail->rng, tail->rng_dev, tail->advance, st);
+      else rc = final_proj(q, P->act, st);
+      break;
+    }
+  }
+  return rc;
+}
+
+static int run_forward(dmn_plan* P, const float* x_dev, const int32_t* row_dev, const int64_t* classes_dev, float* out_dev,
+                       int batch, cudaStream_t st, std::vector<cudaEvent_t>* evs = nullptr, const TailFuse* tail = nullptr,
+                       unsigned long long* stamps = nullptr) {
   const long launches0 = g_launches;
   size_t op_i = 0;
   if (evs) cudaEventRecord((*evs)[0], st);
   if (stamps) stamp_kernel<<<1, 1, 0, st>>>(stamps);
   for (const Op& o : P->ops) {
-    int rc = 0;
-    switch (o.kind) {
-      case OP_MEMSET: {
-        DMN_CUDA_CHECK(cudaMemsetAsync(P->wsbase + P->stats_off, 0, P->stats_bytes, st));
-        count_launch();
-        break;
-      }
-      case OP_INIT: {
-        InitConvP q;
-        q.x = x_dev;
-        q.w = W(P->pidx["init_conv.weight"]);
-        q.bias = W(P->pidx["init_conv.bias"]);
-        if (c.num_classes >= 0 && !c.film) {
-          q.cls_w = W(P->pidx["class_embed.weight"]);
-          q.classes = classes_dev;
-          q.pad_class = c.num_classes;
-        }
-        q.out = B(o.out);
-        q.B = batch; q.Cin = c.channels; q.S = c.image_size; q.Cout = c.dim;
-        if (P->init_tc) {
-          q.w = (const float*)(P->wbase + P->params[P->pidx["init_conv.weight"]].off2);
-          rc = init_conv_tcgen05(q, st);
-        } else {
-          rc = init_conv(q, P->act, st);
-        }
-        break;
-      }
-      case OP_CONV: {
-        ConvP q;
-        q.src1 = B(o.src1); q.src2 = B(o.src2); q.C1 = o.C1; q.C2 = o.C2;
-        q.B = batch; q.Hin = q.Win = o.Hin; q.Hout = q.Wout = o.Hout; q.Cout = o.Cout;
-        q.mode = o.mode; q.ksize = o.ksize;
-        const Param& wp = P->params[o.w];
-        q.w = o.tc ? (const void*)(P->wbase + wp.off2) : (const void*)(P->wbase + wp.off);
-        q.bias = W(o.bias);
-        q.pro = o.pro; q.pstats = (const stat_t*)B(o.pstats); q.pgroups = o.pgroups;
-        q.pgamma = W(o.pgamma); q.pbeta = W(o.pbeta);
-        if (o.pro & PRO_TEMB) {
-          q.temb = (const float*)B(P->time_table) + o.temb_col;
-          if (row_dev) { q.d_row = row_dev; q.temb_rstride = P->sumC; q.temb_bstride = 0; }
-          else { q.d_row = nullptr; q.temb_rstride = 0; q.temb_bstride = P->sumC; }
-        }
-        if (o.fold) {
-          q.pro = PRO_NONE;
-          q.pgroups = 1;
-          q.fold_s1 = (const float*)(P->wbase + o.fold_off);
-          q.fold_s2 = q.fold_s1 + o.Cout;
-        }
-        q.out = B(o.out); q.res = B(o.res);
-        q.ostats = (stat_t*)B(o.ostats); q.ogroups = o.ogroups;
-        rc = o.tc ? conv_tcgen05(q, st) : conv_simt(q, P->act, st);
-        break;
-      }
-      case OP_FINALIZE: {
-        FinalizeP q;
-        q.raw = B(o.raw); q.stats = (const stat_t*)B(o.stats); q.groups = o.groups;
-        q.gamma = W(o.gamma); q.beta = W(o.beta); q.silu = o.silu;
-        q.res = B(o.res); q.out = B(o.out); q.ostats = (stat_t*)B(o.ostats); q.ogroups = o.ogroups;
-        q.B = batch; q.HW = o.HW; q.C = o.C;
-        rc = gn_finalize(q, P->act, st);
-        break;
-      }
-      case OP_LINATTN:
-        rc = linattn_core(B(o.src1), B(o.out), batch, o.heads, o.dh, o.N, P->act, st);
-        break;
-      case OP_ATTN:
-        rc = attn_core(B(o.src1), B(o.out), batch, o.heads, o.dh, o.N, P->act, st);
-        break;
-      case OP_ATTN_FUSED: {
-        LinAttnFusedP q;
-        q.x = B(o.src1); q.out = B(o.out); q.pstats = (const stat_t*)B(o.pstats);
-        q.wqkv = P->wbase + P->params[o.w].off;
-        q.wo = P->wbase + P->params[o.wo].off;
-        q.s1 = (const float*)(P->wbase + o.fold_off);
-        q.s2 = q.s1 + 384;
-        q.bo = W(o.bo); q.go = W(o.gamma); q.beo = W(o.beta);
-        q.B = batch; q.N = o.N; q.C = o.C;
-        rc = o.softmax ? attn_softmax_fused(q, st) : linattn_fused(q, st);
-        break;
-      }
-      case OP_CLASSADD:
-        rc = class_embed_add(B(o.src1), W(P->pidx["class_embed.weight"]), classes_dev, c.num_classes, batch, o.HW, o.C, P->act, st);
-        break;
-      case OP_MODULATE:
-        rc = film_modulate(B(o.src1), B(o.src2), B(o.res), B(o.out), (long)batch * o.HW * o.C, P->act, st);
-        break;
-      case OP_FINALPROJ: {
-        const FinalProjP q = final_proj_params(P, o, out_dev, batch);
-        if (tail) rc = launch_final_proj_ddpm(q, tail->x, tail->z, tail->out, tail->coef, tail->step_dev, tail->step, tail->rng, tail->rng_dev, tail->advance, st);
-        else rc = final_proj(q, P->act, st);
-        break;
-      }
-    }
+    const int rc = enqueue_op(P, o, x_dev, row_dev, classes_dev, out_dev, batch, st, tail);
     if (rc) {
       set_error(o.name + ": " + g_err);
       return rc;
@@ -768,6 +780,106 @@ static int run_forward(dmn_plan* P, const float* x_dev, const int32_t* row_dev, 
   }
   if (stamps) stamp_kernel<<<1, 1, 0, st>>>(stamps + op_i + 1);      // two stamps back to back: the cost of a stamp itself
   P->launches_per_forward = (int)(g_launches - launches0);
+  return 0;
+}
+
+// ---- forward-mode JVP (fp32 SIMT plans) ----
+// The tangent of workspace buffer b lives at work + b.off (same layout as the workspace); behind that arena, a scratch of
+// batch * jvp_scratch_per_sample floats holds the materialised operand of a tangent convolution whose primal has a
+// GroupNorm(+SiLU) prologue (jvp.cu: gn_tangent).
+static size_t jvp_scratch_per_sample(const dmn_plan* P) {
+  size_t m = 0;
+  for (const Op& o : P->ops) {
+    if (o.kind == OP_CONV && (o.pro & PRO_GN)) m = std::max(m, (size_t)o.Hin * o.Hin * o.C1);
+    if (o.kind == OP_FINALPROJ && o.groups > 0) m = std::max(m, (size_t)o.HW * o.C);
+  }
+  return m;
+}
+
+static size_t jvp_work_bytes(const dmn_plan* P, int batch) {
+  return align_up(P->ws_bytes, 256) + (size_t)batch * jvp_scratch_per_sample(P) * sizeof(float);
+}
+
+// the tangent of op o (run right after o itself, while o's primal inputs and outputs are live): v = input tangent (NCHW),
+// tan_out = output tangent (NCHW)
+static int enqueue_tangent_op(dmn_plan* P, const Op& o, const float* v_dev, float* tan_out, char* work, int batch, cudaStream_t st) {
+  auto W = [&](int pi) -> const float* { return pi < 0 ? nullptr : (const float*)(P->wbase + P->params[pi].off); };
+  auto B = [&](const Buf& b) -> float* { return b.valid() ? (float*)(P->wsbase + b.off) : nullptr; };
+  auto T = [&](const Buf& b) -> float* { return b.valid() ? (float*)(work + b.off) : nullptr; };
+  float* du = (float*)(work + align_up(P->ws_bytes, 256));
+  auto gn_tan = [&](const float* h, const float* dh, const Buf& stats, int groups, int gamma, int beta, int silu, const float* dres,
+                    float* out, int HW, int C) {
+    GnTangentP g;
+    g.h = h; g.dh = dh; g.stats = (const stat_t*)B(stats); g.groups = groups; g.gamma = W(gamma); g.beta = W(beta); g.silu = silu;
+    g.dres = dres; g.out = out; g.B = batch; g.HW = HW; g.C = C;
+    return gn_tangent(g, st);
+  };
+  int rc = 0;
+  switch (o.kind) {
+    case OP_MEMSET:
+      break;
+    case OP_INIT: {       // class embedding and bias do not depend on x
+      InitConvP q;
+      q.x = v_dev;
+      q.w = W(P->pidx["init_conv.weight"]);
+      q.out = T(o.out);
+      q.B = batch; q.Cin = P->cfg.channels; q.S = P->cfg.image_size; q.Cout = P->cfg.dim;
+      rc = init_conv(q, ACT_F32, st);
+      break;
+    }
+    case OP_CONV: {
+      ConvP q;
+      q.src1 = T(o.src1); q.src2 = T(o.src2); q.C1 = o.C1; q.C2 = o.C2;
+      q.B = batch; q.Hin = q.Win = o.Hin; q.Hout = q.Wout = o.Hout; q.Cout = o.Cout;
+      q.mode = o.mode; q.ksize = o.ksize;
+      q.w = P->wbase + P->params[o.w].off;
+      if (o.pro & PRO_GN) {    // the time-embedding add of the prologue is constant in x
+        if ((rc = gn_tan(B(o.src1), T(o.src1), o.pstats, o.pgroups, o.pgamma, o.pbeta, (o.pro & PRO_SILU) ? 1 : 0, nullptr, du,
+                         o.Hin * o.Hin, o.C1)))
+          return rc;
+        q.src1 = du;
+      }
+      q.out = T(o.out); q.res = T(o.res);
+      rc = conv_simt(q, ACT_F32, st);
+      break;
+    }
+    case OP_FINALIZE:
+      rc = gn_tan(B(o.raw), T(o.raw), o.stats, o.groups, o.gamma, o.beta, o.silu, T(o.res), T(o.out), o.HW, o.C);
+      break;
+    case OP_LINATTN:
+      rc = linattn_jvp(B(o.src1), T(o.src1), T(o.out), batch, o.heads, o.dh, o.N, st);
+      break;
+    case OP_ATTN:
+      rc = attn_jvp(B(o.src1), T(o.src1), T(o.out), batch, o.heads, o.dh, o.N, st);
+      break;
+    case OP_FINALPROJ: {
+      FinalProjP q = final_proj_params(P, o, tan_out, batch);
+      if (o.groups > 0) {
+        if ((rc = gn_tan(B(o.src1), T(o.src1), o.stats, o.groups, o.gamma, o.beta, 1, nullptr, du, o.HW, o.C))) return rc;
+        q.y = du;
+      } else {
+        q.y = T(o.src1);
+      }
+      q.plain = 1; q.stats = nullptr; q.gamma = q.beta = nullptr; q.bias = nullptr;
+      rc = final_proj(q, ACT_F32, st);
+      break;
+    }
+    default:
+      return fail(DMN_ENOTSUP, "no tangent for this op (FiLM / fused tensor-core ops)");
+  }
+  return rc;
+}
+
+static int run_jvp(dmn_plan* P, const float* x_dev, const float* v_dev, const int32_t* row_dev, const int64_t* classes_dev, float* out_dev,
+                   float* tan_out, char* work, int batch, cudaStream_t st) {
+  for (const Op& o : P->ops) {
+    int rc = enqueue_op(P, o, x_dev, row_dev, classes_dev, out_dev, batch, st, nullptr);
+    if (!rc) rc = enqueue_tangent_op(P, o, v_dev, tan_out, work, batch, st);
+    if (rc) {
+      set_error(o.name + ": " + g_err);
+      return rc;
+    }
+  }
   return 0;
 }
 
@@ -1065,6 +1177,26 @@ int dmn_unet_forward(dmn_plan* p, const float* x_dev, const int32_t* row_dev, co
   DMN_REQUIRE(x_dev && out_dev, "null tensor");
   DMN_REQUIRE(batch >= 1 && batch <= p->cfg.max_batch, "batch exceeds the plan's max_batch");
   return run_forward(p, x_dev, row_dev, classes_dev, out_dev, batch, (cudaStream_t)stream);
+}
+
+size_t dmn_unet_jvp_work_bytes(const dmn_plan* p, int batch) {
+  if (!p || batch < 1) return 0;
+  return jvp_work_bytes(p, batch);
+}
+
+int dmn_unet_jvp(dmn_plan* p, const float* x_dev, const float* v_dev, const int32_t* row_dev, const int64_t* classes_dev, float* out_dev,
+                 float* out_tangent_dev, void* work_dev, size_t work_bytes, int batch, void* stream) {
+  if (!p) return fail(DMN_EINVAL, "null plan");
+  if (p->act != DMN_ACT_F32 || p->engine != DMN_CONV_SIMT)
+    return fail(DMN_ENOTSUP, "dmn_unet_jvp: the JVP is built for fp32 plans on the SIMT engine only (bf16 / tcgen05 have no tangent kernels)");
+  if (p->cfg.film) return fail(DMN_ENOTSUP, "dmn_unet_jvp: FiLM plans (WaveGradUNet) have no tangent program");
+  DMN_REQUIRE(x_dev && v_dev && out_dev && out_tangent_dev && work_dev, "null tensor");
+  DMN_REQUIRE(batch >= 1 && batch <= p->cfg.max_batch, "batch exceeds the plan's max_batch");
+  DMN_REQUIRE(((uintptr_t)work_dev % 256) == 0, "work buffer must be 256-byte aligned");
+  int rc = check_ready(p);
+  if (rc) return rc;
+  DMN_REQUIRE(work_bytes >= jvp_work_bytes(p, batch), "work buffer smaller than dmn_unet_jvp_work_bytes()");
+  return run_jvp(p, x_dev, v_dev, row_dev, classes_dev, out_dev, out_tangent_dev, (char*)work_dev, batch, (cudaStream_t)stream);
 }
 
 int dmn_plan_launches_per_forward(const dmn_plan* p) { return p ? p->launches_per_forward : 0; }
@@ -1413,29 +1545,33 @@ int dmn_loop_launches_per_step(const dmn_plan* p, const dmn_loop_desc* d) {
 // ---------------------------------------------------------------------------------------------------------
 // probability-flow ODE driver (kernels: ode.cu)
 // ---------------------------------------------------------------------------------------------------------
-// One RK45 attempt: the input of stage 1, the 6 stage rows of the time table, then per stage the U-Net and the stage kernel,
-// then the controller (accept / reject, next step, WHILE condition).
-static int enqueue_ode_attempt(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd,
-                               int use_cond, cudaStream_t st) {
+// One RK45 attempt: the input of stage 1, the 6 stage rows of the time table, then per stage the model evaluation and the stage
+// kernel, then the controller (accept / reject, next step, WHILE condition).  eval(row, stream) evaluates the model at U-Net input
+// w.x32 with time-table row w.rows[row] and writes what the stage kernels read (w.mo: the model output, plus the drift of the
+// log-density rows for the likelihood).
+template <class Eval>
+static int enqueue_ode_attempt(dmn_plan* p, const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd, int use_cond,
+                               cudaStream_t st, Eval& eval) {
   int rc;
   if ((rc = launch_ode_stage(w, P, 0, st))) return rc;
   if ((rc = dmn_time_table(p, w.rec->labels, 0, 6, st))) return rc;
   for (int s = 1; s <= 6; ++s) {
-    if ((rc = run_forward(p, w.x32, w.rows + (s - 1), d->classes_dev, w.mo, d->batch, st))) return rc;
+    if ((rc = eval(s - 1, st))) return rc;
     if ((rc = launch_ode_stage(w, P, s, st))) return rc;
   }
   return launch_ode_control(w, P, hnd, use_cond, st);
 }
 
 // init phase: y0, f0 = f(t0, y0), select_initial_step (one more evaluation), first attempt's stage rows
-static int enqueue_ode_init(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd,
-                            int use_cond, cudaStream_t st) {
+template <class Eval>
+static int enqueue_ode_init(dmn_plan* p, const float* state, const OdeWork& w, const OdeParams& P, cudaGraphConditionalHandle hnd,
+                            int use_cond, cudaStream_t st, Eval& eval) {
   int rc;
   if ((rc = launch_ode_init(w, P, st))) return rc;
-  if ((rc = launch_ode_init_elem(w, P, d->state_dev, 0, st))) return rc;
+  if ((rc = launch_ode_init_elem(w, P, state, 0, st))) return rc;
   for (int k = 0; k < 2; ++k) {
     if ((rc = dmn_time_table(p, w.rec->labels, 0, 6, st))) return rc;
-    if ((rc = run_forward(p, w.x32, w.rows, d->classes_dev, w.mo, d->batch, st))) return rc;
+    if ((rc = eval(0, st))) return rc;
     if ((rc = launch_ode_init_elem(w, P, nullptr, k == 0 ? 1 : 3, st))) return rc;
     if ((rc = launch_ode_init_step(w, P, k, hnd, use_cond && k == 1, st))) return rc;
     if (k == 0 && (rc = launch_ode_init_elem(w, P, nullptr, 2, st))) return rc;
@@ -1444,7 +1580,10 @@ static int enqueue_ode_init(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w
 }
 
 // the graph bakes in every pointer and scalar of the descriptor
-static bool same_ode_key(const dmn_ode_desc& a, const dmn_ode_desc& b) {
+static bool same_ode_inputs(const dmn_ode_desc&, const dmn_ode_desc&) { return true; }
+static bool same_ode_inputs(const dmn_ode_likelihood_desc& a, const dmn_ode_likelihood_desc& b) { return a.noise_dev == b.noise_dev; }
+template <class Desc>
+static bool same_ode_key(const Desc& a, const Desc& b) {
   return a.sde_kind == b.sde_kind && a.N == b.N && a.beta_0 == b.beta_0 && a.beta_1 == b.beta_1 && a.sigma_min == b.sigma_min &&
          a.sigma_max == b.sigma_max && a.t0 == b.t0 && a.t1 == b.t1 && a.rtol == b.rtol && a.atol == b.atol && a.max_nfe == b.max_nfe &&
          a.batch == b.batch && a.classes_dev == b.classes_dev && a.state_dev == b.state_dev && a.work_dev == b.work_dev &&
@@ -1452,7 +1591,8 @@ static bool same_ode_key(const dmn_ode_desc& a, const dmn_ode_desc& b) {
 }
 
 // init phase on the captured stream, then a WHILE node whose body (one attempt) is captured on a second stream, then the finish
-static int build_ode_graph(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w, const OdeParams& P, cudaGraphExec_t* out) {
+template <class Eval>
+static int build_ode_graph(dmn_plan* p, float* state, const OdeWork& w, const OdeParams& P, Eval& eval, cudaGraphExec_t* out) {
   cudaStream_t bs;
   DMN_CUDA_CHECK(cudaStreamCreateWithFlags(&bs, cudaStreamNonBlocking));
   auto enqueue = [&](cudaStream_t cs) -> int {
@@ -1463,7 +1603,7 @@ static int build_ode_graph(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w,
     cudaGraphConditionalHandle hnd = 0;
     DMN_CUDA_CHECK(cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps));
     DMN_CUDA_CHECK(cudaGraphConditionalHandleCreate(&hnd, graph, 0, cudaGraphCondAssignDefault));
-    int rc = enqueue_ode_init(p, d, w, P, hnd, 1, cs);
+    int rc = enqueue_ode_init(p, state, w, P, hnd, 1, cs, eval);
     if (rc) return rc;
     DMN_CUDA_CHECK(cudaStreamGetCaptureInfo(cs, &cst, nullptr, &graph, &deps, &ndeps));
     cudaGraphNodeParams np = {};
@@ -1476,15 +1616,96 @@ static int build_ode_graph(dmn_plan* p, const dmn_ode_desc* d, const OdeWork& w,
     DMN_CUDA_CHECK(cudaStreamUpdateCaptureDependencies(cs, &node, 1, cudaStreamSetCaptureDependencies));
     cudaGraph_t body = np.conditional.phGraph_out[0];
     DMN_CUDA_CHECK(cudaStreamBeginCaptureToGraph(bs, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
-    rc = enqueue_ode_attempt(p, d, w, P, hnd, 1, bs);
+    rc = enqueue_ode_attempt(p, w, P, hnd, 1, bs, eval);
     const cudaError_t e = cudaStreamEndCapture(bs, &body);
     if (rc) return rc;
     if (e != cudaSuccess) return fail(DMN_ECUDA, std::string("ode graph (body end capture): ") + cudaGetErrorString(e));
-    return launch_ode_finish(w, d->state_dev, cs);
+    return launch_ode_finish(w, state, cs);
   };
   const int rc = capture_graph("ode graph", enqueue, out);
   cudaStreamDestroy(bs);
   return rc;
+}
+
+// plain launches: the init phase, then one attempt at a time with a host read of the status in between
+template <class Eval>
+static int run_ode_plain(dmn_plan* p, float* state, const OdeWork& w, const OdeParams& P, Eval& eval, cudaStream_t st) {
+  int rc;
+  if ((rc = enqueue_ode_init(p, state, w, P, 0, 0, st, eval))) return rc;
+  dmn_ode_result r;
+  for (long it = 0;; ++it) {
+    DMN_CUDA_CHECK(cudaMemcpyAsync(&r, w.result, sizeof(r), cudaMemcpyDeviceToHost, st));
+    DMN_CUDA_CHECK(cudaStreamSynchronize(st));
+    if (r.status != DMN_ODE_RUNNING) break;
+    if (it > (long)P.max_nfe) return fail(DMN_ESTATE, "ODE controller did not stop within max_nfe");
+    if ((rc = enqueue_ode_attempt(p, w, P, 0, 0, st, eval))) return rc;
+  }
+  return launch_ode_finish(w, state, st);
+}
+
+// descriptor checks and solver constants shared by the sampler and the likelihood (their descriptors share these fields)
+template <class Desc>
+static int check_ode_desc(const dmn_plan* p, const Desc* d) {
+  const dmn_unet_cfg& c = p->cfg;
+  DMN_REQUIRE(d->sde_kind == DMN_SDE_VP || d->sde_kind == DMN_SDE_VE, "unknown SDE kind");
+  if (d->sde_kind == DMN_SDE_VP) DMN_REQUIRE(d->N >= 1 && std::isfinite(d->beta_0) && std::isfinite(d->beta_1), "VP-SDE needs N >= 1 and finite betas");
+  else DMN_REQUIRE(d->sigma_min > 0 && d->sigma_max > 0 && std::isfinite(d->sigma_min) && std::isfinite(d->sigma_max), "VE-SDE needs positive sigmas");
+  DMN_REQUIRE(std::isfinite(d->t0) && std::isfinite(d->t1) && d->t0 != d->t1, "t0 and t1 must be finite and different");
+  DMN_REQUIRE(std::isfinite(d->rtol) && d->rtol > 0 && std::isfinite(d->atol) && d->atol >= 0, "tolerances: rtol > 0, atol >= 0, finite");
+  DMN_REQUIRE(d->max_nfe >= 2, "max_nfe must be >= 2 (the initial step selection evaluates twice)");
+  DMN_REQUIRE(d->batch >= 1 && d->batch <= c.max_batch, "batch exceeds the plan's max_batch");
+  DMN_REQUIRE(d->state_dev && d->work_dev && d->result_dev, "null device pointer in ODE descriptor");
+  DMN_REQUIRE(((uintptr_t)d->work_dev % 256) == 0, "work buffer must be 256-byte aligned");
+  return 0;
+}
+
+template <class Desc>
+static OdeParams ode_params(const Desc* d) {
+  OdeParams P;
+  P.sde_kind = d->sde_kind; P.N = d->N; P.max_nfe = d->max_nfe;
+  P.beta_0 = d->beta_0; P.beta_1 = d->beta_1; P.sigma_min = d->sigma_min; P.sigma_max = d->sigma_max;
+  P.t0 = d->t0; P.t1 = d->t1; P.atol = d->atol;
+  P.rtol = d->rtol < 100 * DBL_EPSILON ? 100 * DBL_EPSILON : d->rtol;     // scipy validate_tol
+  return P;
+}
+
+// the cached graph of descriptor d (built with build() on a miss; at most 4 per plan and kind), launched on st
+template <class Desc, class Build>
+static int launch_ode_graph(std::vector<dmn_plan::OdeGraphEntry<Desc>>& cache, const Desc* d, Build&& build, cudaStream_t st) {
+  cudaGraphExec_t exec = nullptr;
+  for (auto& g : cache)
+    if (same_ode_key(g.key, *d) && same_ode_inputs(g.key, *d)) exec = g.exec;
+  if (!exec) {
+    int rc = build(&exec);
+    if (rc) return rc;
+    if (cache.size() >= 4) {
+      cudaGraphExecDestroy(cache.front().exec);
+      cache.erase(cache.begin());
+    }
+    dmn_plan::OdeGraphEntry<Desc> ge;
+    ge.exec = exec;
+    ge.key = *d;
+    cache.push_back(ge);
+  }
+  DMN_CUDA_CHECK(cudaGraphLaunch(exec, st));
+  return 0;
+}
+
+// likelihood work: the RK45 work of the augmented state, then the Hutchinson noise, the JVP output and the JVP work
+static size_t lik_work_layout(const dmn_plan* p, int batch, char* base, OdeWork* w, char** jvp_work) {
+  const dmn_unet_cfg& c = p->cfg;
+  const long nx = (long)batch * c.channels * c.image_size * c.image_size;
+  size_t off = align_up(ode_work_layout(nx + batch, base, w), 256);
+  const size_t o_eps = off;  off += align_up((size_t)nx * sizeof(float), 256);
+  const size_t o_dmo = off;  off += align_up((size_t)nx * sizeof(float), 256);
+  const size_t o_jvp = off;  off += jvp_work_bytes(p, batch);
+  if (w) {
+    w->nx = nx;
+    w->eps = (const float*)(base + o_eps);
+    w->dmo = (float*)(base + o_dmo);
+    *jvp_work = base + o_jvp;
+  }
+  return off;
 }
 
 extern "C" {
@@ -1499,59 +1720,68 @@ int dmn_ode_sample(dmn_plan* p, const dmn_ode_desc* d, void* stream) {
   if (!p) return fail(DMN_EINVAL, "null plan");
   if (!d) return fail(DMN_EINVAL, "null descriptor");
   const dmn_unet_cfg& c = p->cfg;
-  DMN_REQUIRE(d->sde_kind == DMN_SDE_VP || d->sde_kind == DMN_SDE_VE, "unknown SDE kind");
-  if (d->sde_kind == DMN_SDE_VP) DMN_REQUIRE(d->N >= 1 && std::isfinite(d->beta_0) && std::isfinite(d->beta_1), "VP-SDE needs N >= 1 and finite betas");
-  else DMN_REQUIRE(d->sigma_min > 0 && d->sigma_max > 0 && std::isfinite(d->sigma_min) && std::isfinite(d->sigma_max), "VE-SDE needs positive sigmas");
-  DMN_REQUIRE(std::isfinite(d->t0) && std::isfinite(d->t1) && d->t0 != d->t1, "t0 and t1 must be finite and different");
-  DMN_REQUIRE(std::isfinite(d->rtol) && d->rtol > 0 && std::isfinite(d->atol) && d->atol >= 0, "tolerances: rtol > 0, atol >= 0, finite");
-  DMN_REQUIRE(d->max_nfe >= 2, "max_nfe must be >= 2 (the initial step selection evaluates twice)");
-  DMN_REQUIRE(d->batch >= 1 && d->batch <= c.max_batch, "batch exceeds the plan's max_batch");
-  DMN_REQUIRE(d->state_dev && d->work_dev && d->result_dev, "null device pointer in ODE descriptor");
-  DMN_REQUIRE(((uintptr_t)d->work_dev % 256) == 0, "work buffer must be 256-byte aligned");
+  int rc = check_ode_desc(p, d);
+  if (rc) return rc;
   const long n = (long)d->batch * c.channels * c.image_size * c.image_size;
   DMN_REQUIRE(d->state_elems == n, "state_dev does not hold batch * channels * image_size^2 floats for this plan");
   DMN_REQUIRE(d->work_bytes >= dmn_ode_work_bytes(p, d->batch), "work buffer smaller than dmn_ode_work_bytes()");
   DMN_REQUIRE(c.out_dim == c.channels && !c.film, "the ODE drift needs a U-Net with out_dim == channels (no FiLM)");
   DMN_REQUIRE(c.max_time_rows >= 6, "the plan's time table needs >= 6 rows (one per stage of an attempt)");
-  int rc = check_ready(p);
-  if (rc) return rc;
+  if ((rc = check_ready(p))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  OdeParams P;
-  P.sde_kind = d->sde_kind; P.N = d->N; P.max_nfe = d->max_nfe;
-  P.beta_0 = d->beta_0; P.beta_1 = d->beta_1; P.sigma_min = d->sigma_min; P.sigma_max = d->sigma_max;
-  P.t0 = d->t0; P.t1 = d->t1; P.atol = d->atol;
-  P.rtol = d->rtol < 100 * DBL_EPSILON ? 100 * DBL_EPSILON : d->rtol;     // scipy validate_tol
+  const OdeParams P = ode_params(d);
   OdeWork w;
   ode_work_layout(n, (char*)d->work_dev, &w);
   w.result = d->result_dev;
-  if (!d->use_graph) {
-    if ((rc = enqueue_ode_init(p, d, w, P, 0, 0, st))) return rc;
-    dmn_ode_result r;
-    for (long it = 0;; ++it) {
-      DMN_CUDA_CHECK(cudaMemcpyAsync(&r, d->result_dev, sizeof(r), cudaMemcpyDeviceToHost, st));
-      DMN_CUDA_CHECK(cudaStreamSynchronize(st));
-      if (r.status != DMN_ODE_RUNNING) break;
-      if (it > (long)d->max_nfe) return fail(DMN_ESTATE, "ODE controller did not stop within max_nfe");
-      if ((rc = enqueue_ode_attempt(p, d, w, P, 0, 0, st))) return rc;
-    }
-    return launch_ode_finish(w, d->state_dev, st);
-  }
-  cudaGraphExec_t exec = nullptr;
-  for (auto& g : p->ode_graphs)
-    if (same_ode_key(g.key, *d)) exec = g.exec;
-  if (!exec) {
-    if ((rc = build_ode_graph(p, d, w, P, &exec))) return rc;
-    if (p->ode_graphs.size() >= 4) {
-      cudaGraphExecDestroy(p->ode_graphs.front().exec);
-      p->ode_graphs.erase(p->ode_graphs.begin());
-    }
-    dmn_plan::OdeGraphEntry ge;
-    ge.exec = exec;
-    ge.key = *d;
-    p->ode_graphs.push_back(ge);
-  }
-  DMN_CUDA_CHECK(cudaGraphLaunch(exec, st));
-  return 0;
+  auto eval = [&](int row, cudaStream_t s) { return run_forward(p, w.x32, w.rows + row, d->classes_dev, w.mo, d->batch, s); };
+  if (!d->use_graph) return run_ode_plain(p, d->state_dev, w, P, eval, st);
+  return launch_ode_graph(p->ode_graphs, d, [&](cudaGraphExec_t* e) { return build_ode_graph(p, d->state_dev, w, P, eval, e); }, st);
+}
+
+size_t dmn_ode_likelihood_work_bytes(const dmn_plan* p, int batch) {
+  if (!p || batch < 1) return 0;
+  return lik_work_layout(p, batch, nullptr, nullptr, nullptr);
+}
+
+int dmn_ode_likelihood(dmn_plan* p, const dmn_ode_likelihood_desc* d, void* stream) {
+  if (!p) return fail(DMN_EINVAL, "null plan");
+  if (!d) return fail(DMN_EINVAL, "null descriptor");
+  const dmn_unet_cfg& c = p->cfg;
+  if (p->act != DMN_ACT_F32 || p->engine != DMN_CONV_SIMT)
+    return fail(DMN_ENOTSUP, "dmn_ode_likelihood: the U-Net JVP is built for fp32 plans on the SIMT engine only");
+  int rc = check_ode_desc(p, d);
+  if (rc) return rc;
+  DMN_REQUIRE(d->hutchinson == DMN_HUTCH_RADEMACHER || d->hutchinson == DMN_HUTCH_GAUSSIAN, "unknown Hutchinson noise type");
+  const long nx = (long)d->batch * c.channels * c.image_size * c.image_size;
+  DMN_REQUIRE(d->state_elems == nx + d->batch, "state_dev does not hold batch * (channels * image_size^2 + 1) floats for this plan");
+  DMN_REQUIRE(d->noise_dev || nx % 4 == 0, "in-kernel Hutchinson noise needs batch * channels * image_size^2 % 4 == 0");
+  DMN_REQUIRE(d->work_bytes >= dmn_ode_likelihood_work_bytes(p, d->batch), "work buffer smaller than dmn_ode_likelihood_work_bytes()");
+  DMN_REQUIRE(c.out_dim == c.channels && !c.film, "the ODE drift needs a U-Net with out_dim == channels (no FiLM)");
+  DMN_REQUIRE(c.max_time_rows >= 6, "the plan's time table needs >= 6 rows (one per stage of an attempt)");
+  if ((rc = check_ready(p))) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const OdeParams P = ode_params(d);
+  OdeWork w;
+  char* jvp_work = nullptr;
+  lik_work_layout(p, d->batch, (char*)d->work_dev, &w, &jvp_work);
+  w.result = d->result_dev;
+  float* eps_buf = const_cast<float*>(w.eps);
+  if (d->noise_dev) w.eps = d->noise_dev;
+  // one JVP pass in direction eps: the model output for the x rows, then the divergence rows
+  auto eval = [&](int row, cudaStream_t s) {
+    const int r = run_jvp(p, w.x32, w.eps, w.rows + row, d->classes_dev, w.mo, w.dmo, jvp_work, d->batch, s);
+    return r ? r : launch_ode_div(w, P, row, d->batch, s);
+  };
+  // the Hutchinson draw, once per solve on the stream ahead of the solve (the graph reads it from the work buffer)
+  auto draw = [&](cudaStream_t s) -> int {
+    if (d->noise_dev) return 0;
+    int r = dmn_randn(eps_buf, nx, d->rng, 0, s);
+    if (!r && d->hutchinson == DMN_HUTCH_RADEMACHER) r = launch_ode_rademacher(eps_buf, nx, s);
+    return r;
+  };
+  if ((rc = draw(st))) return rc;
+  if (!d->use_graph) return run_ode_plain(p, d->state_dev, w, P, eval, st);
+  return launch_ode_graph(p->lik_graphs, d, [&](cudaGraphExec_t* e) { return build_ode_graph(p, d->state_dev, w, P, eval, e); }, st);
 }
 
 }  // extern "C"

@@ -122,6 +122,29 @@ class UnetPlan:
                     "dmn_unet_forward")
         return out
 
+    def jvp(self, x: torch.Tensor, time: torch.Tensor, v: torch.Tensor, classes: Optional[torch.Tensor] = None):
+        """(u(x, time), du/dx . v) in one pass of the forward program with its tangent program (fp32 SIMT plans only)."""
+        b = x.shape[0]
+        shape = (b, self.out_dim, self.image_size, self.image_size)
+        out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        tangent = torch.empty(shape, dtype=torch.float32, device=self.device)
+        self.time_table(time.reshape(-1).float(), 0)
+        if classes is not None:
+            classes = classes.to(self.device, torch.int64).contiguous()
+        work = self.jvp_work(b)
+        with torch.cuda.device(self.device):
+            L.check(self.lib.dmn_unet_jvp(self.h, L.ptr(x), L.ptr(v), None, L.ptr(classes), L.ptr(out), L.ptr(tangent),
+                                          self._aligned(work), work.numel() - 256, b, L.stream_ptr(self.device)), "dmn_unet_jvp")
+        return out, tangent
+
+    def jvp_work(self, batch: int) -> torch.Tensor:
+        """Device buffer of dmn_unet_jvp for `batch` samples (kept with the plan, grown on demand; 256 bytes of alignment slack)."""
+        nbytes = int(self.lib.dmn_unet_jvp_work_bytes(self.h, batch)) + 256
+        w = getattr(self, "_jvp_work", None)
+        if w is None or w.numel() < nbytes:
+            w = self._jvp_work = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        return w
+
     def op_table(self):
         """[(name, kind, engine, flops_per_sample, bytes_per_sample)] of the forward program."""
         out = []

@@ -15,7 +15,7 @@ _API = {
     "dpm_solver_diffusion": ("DPMSolverDiffusion",),
     "wavegrad_diffusion": ("WaveGradDiffusion",),
     "sde": (
-        "SDE", "VPSDE", "VESDE", "PredictorCorrectorSampler", "ProbabilityFlowSampler", "resolve_score_function",
+        "SDE", "VPSDE", "VESDE", "PredictorCorrectorSampler", "ProbabilityFlowSampler", "LikelihoodEstimate", "resolve_score_function",
         "Predictor", "NonePredictor", "EulerMaruyamaPredictor", "AncestralSamplingPredictor", "ReverseDiffusionPredictor",
         "register_predictor", "get_predictor",
         "Corrector", "NoneCorrector", "LangevinCorrector", "AnnealedLangevinDynamics", "register_corrector", "get_corrector",

@@ -9,6 +9,8 @@ computed with the reference's torch CPU ops, and the device runs ONE fused kerne
 
 ProbabilityFlowSampler (modules/sde_samplers/probability_flow_sampler.py) solves the probability-flow ODE with scipy's RK45
 rules on the device (dmn_ode_sample): the step control runs in device code, so the adaptive solve is one CUDA graph.
+LikelihoodEstimate (score_sde's get_likelihood_fn) runs the same solver over [x ; delta_logp] with a forward-mode JVP of the fp32
+Unet per evaluation for the Hutchinson divergence (dmn_ode_likelihood).
 """
 import abc
 import ctypes as C
@@ -599,3 +601,121 @@ class ProbabilityFlowSampler(torch.nn.Module):
         if device is None:
             device = next(model.parameters()).device
         return self.forward(model=model, shape=shape, device=device, return_nfe=return_nfe, noise=noise)
+
+
+class LikelihoodEstimate(torch.nn.Module):
+    """Exact log-likelihood of a score-SDE model under its probability-flow ODE, in bits/dim (score_sde's get_likelihood_fn; the
+    reference's modules/sde_lib/likelihood.py): the augmented state [x ; delta_logp] is integrated from eps to sde.T with scipy's
+    RK45 rules, where d delta_logp / dt is the Hutchinson estimate eps^T (d drift / dx) eps of the drift's divergence.  Everything
+    runs on the GPU: one forward-mode JVP pass of this package's fp32 Unet per evaluation gives both the model output and the
+    directional derivative, and with `use_cuda_graph` (default) the whole adaptive solve is one CUDA graph replay.
+
+    likelihood(model, data, noise=None) -> (bpd [B], z [B, C, H, W], nfe).  data is in the model's [-1, 1] space, already
+    dequantised; bpd = -(prior_logp(z) + delta_logp) / ln 2 / D + 7 (score_sde's offset 7 - inverse_scaler(-1) for centred
+    data).  `noise` injects the Hutchinson noise; otherwise it is drawn once per call by the in-kernel Philox generator keyed by
+    (`seed` or a draw from torch's CPU generator, data-parallel rank).  Needs this package's Unet in fp32 (compute_dtype='fp32')."""
+
+    def __init__(self, hutchinson_type: str = "Rademacher", rtol: float = 1e-5, atol: float = 1e-5, method: str = "RK45",
+                 eps: float = 1e-5, max_nfe: int = 100_000):
+        super().__init__()
+        if hutchinson_type not in ("Rademacher", "Gaussian"):
+            raise NotImplementedError(f"Hutchinson type {hutchinson_type} unknown.")
+        if method != "RK45":
+            raise NotImplementedError(f"method={method!r}: only the RK45 solver is built")
+        for name, v in (("rtol", rtol), ("atol", atol), ("eps", eps)):
+            if isinstance(v, bool) or not isinstance(v, (int, float, np.floating, np.integer)):
+                raise ValueError(f"{name} must be a scalar number, got {type(v).__name__}")
+            if not np.isfinite(v) or v < 0 or (name != "atol" and v == 0):
+                raise ValueError(f"{name} must be finite and {'>= 0' if name == 'atol' else '> 0'}, got {v}")
+        if isinstance(max_nfe, bool) or not isinstance(max_nfe, (int, np.integer)) or max_nfe < 2:
+            raise ValueError(f"max_nfe must be an integer >= 2, got {max_nfe!r}")
+        self.hutchinson_type, self.rtol, self.atol, self.method = hutchinson_type, float(rtol), float(atol), method
+        self.eps, self.max_nfe = float(eps), int(max_nfe)
+        self.sde: Optional[SDE] = None
+        self.seed: Optional[int] = None
+        self.use_cuda_graph = True
+        self.last_stats: Optional[dict] = None
+
+    def update_sde(self, sde: SDE):
+        self.sde = sde
+
+    def likelihood(self, model, data: torch.Tensor, noise: Optional[torch.Tensor] = None):
+        if self.sde is None:
+            raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling likelihood()")
+        sde = self.sde
+        if not isinstance(sde, (VPSDE, VESDE)):
+            raise NotImplementedError(f"SDE class {sde.__class__.__name__} not yet supported.")
+        unet, classes = R.resolve_model(model)
+        if unet is None or unet._film:
+            raise NotImplementedError("LikelihoodEstimate runs this package's Unet natively (its forward-mode JVP); other model "
+                                      "callables have no host path")
+        if unet.compute_dtype not in ("fp32", "float32"):
+            raise ValueError("LikelihoodEstimate needs the Unet in fp32 (compute_dtype='fp32'): likelihoods are an fp32 metric")
+        if data.dim() != 4:
+            raise ValueError(f"data must be [B, C, H, W], got shape {tuple(data.shape)}")
+        b, c, h, w = (int(v) for v in data.shape)
+        if c != unet.channels or h != w:
+            raise ValueError(f"data shape {tuple(data.shape)} does not fit the U-Net ({unet.channels} channels, square images)")
+        if unet.out_dim != unet.channels:
+            raise ValueError("the probability-flow drift needs a U-Net whose output has as many channels as its input")
+        if noise is not None and tuple(noise.shape) != tuple(data.shape):
+            raise ValueError(f"noise has shape {tuple(noise.shape)}; expected {tuple(data.shape)}")
+        device = data.device
+        R.require_cuda(device)
+        lib = L.lib()
+        plan = unet.plan(h, b, device, time_rows=6)
+        n = b * c * h * w
+        with torch.cuda.device(device):
+            st = L.stream_ptr(device)
+            # buffers live with the plan so the addresses baked into the cached graph stay valid
+            bufs = plan.__dict__.setdefault("_lik_bufs", {})
+            if b not in bufs:
+                nbytes = int(lib.dmn_ode_likelihood_work_bytes(plan.h, b))
+                bufs[b] = {"state": torch.empty(n + b, dtype=torch.float32, device=device),
+                           "work": torch.empty(nbytes + 256, dtype=torch.uint8, device=device),
+                           "result": torch.zeros(3, dtype=torch.float64, device=device)}
+            buf = bufs[b]
+            state, work, result = buf["state"], buf["work"], buf["result"]
+            state[:n].copy_(data.reshape(-1).to(torch.float32))
+            state[n:].zero_()
+            if classes is not None:
+                classes = R.stable_copy(buf, "classes", classes.to(device, torch.int64).reshape(-1))
+            if noise is not None:
+                noise = R.stable_copy(buf, "noise", noise.to(device, torch.float32).reshape(-1))
+            wp = (work.data_ptr() + 255) // 256 * 256
+            d = L.OdeLikelihoodDesc()
+            if isinstance(sde, VPSDE):
+                d.sde_kind, d.N, d.beta_0, d.beta_1 = L.SDE_VP, int(sde.N), float(sde.beta_0), float(sde.beta_1)
+            else:
+                d.sde_kind, d.N, d.sigma_min, d.sigma_max = L.SDE_VE, int(sde.N), float(sde.sigma_min), float(sde.sigma_max)
+            d.t0, d.t1, d.rtol, d.atol = self.eps, float(sde.T), self.rtol, self.atol
+            d.max_nfe, d.batch, d.use_graph = self.max_nfe, b, int(bool(self.use_cuda_graph))
+            d.hutchinson = L.HUTCH_RADEMACHER if self.hutchinson_type == "Rademacher" else L.HUTCH_GAUSSIAN
+            d.rng = L.Rng(self.seed if self.seed is not None else R.draw_seed(), R.rank_stream_id())
+            d.noise_dev = noise.data_ptr() if noise is not None else None
+            d.classes_dev = classes.data_ptr() if classes is not None else None
+            d.state_dev, d.state_elems = state.data_ptr(), state.numel()
+            d.work_dev, d.work_bytes = wp, work.numel() - (wp - work.data_ptr())
+            d.result_dev = result.data_ptr()
+            L.check(lib.dmn_ode_likelihood(plan.h, C.byref(d), st), "dmn_ode_likelihood")
+            plan.time_rows_key = None            # the solve rewrote rows 0..5 of the time table
+            raw = result.cpu().numpy().tobytes()
+            z = state[:n].reshape(b, c, h, w).clone()
+            delta_logp = state[n:].clone()
+        res = L.OdeResult.from_buffer_copy(raw)
+        self.last_stats = {"status": int(res.status), "nfev": int(res.nfev), "n_accepted": int(res.n_accepted),
+                           "n_rejected": int(res.n_rejected), "t_final": float(res.t_final)}
+        if res.status == L.ODE_LIMIT:
+            raise RuntimeError(f"likelihood ODE: stopped at {res.nfev} model evaluations (max_nfe={self.max_nfe}) at "
+                               f"t={res.t_final:.6g}, before reaching T={float(sde.T):g}")
+        if res.status == L.ODE_TOO_SMALL_STEP:
+            warnings.warn(f"likelihood ODE: required step size became too small at t={res.t_final:.6g} (scipy status -1); "
+                          "returning the last accepted state, as solve_ivp does")
+        bpd = likelihood_bpd(sde, z, delta_logp)
+        return bpd, z, int(res.nfev)
+
+
+def likelihood_bpd(sde: SDE, z: torch.Tensor, delta_logp: torch.Tensor) -> torch.Tensor:
+    """score_sde likelihood_fn's tail: bpd = -(prior_logp(z) + delta_logp) / ln 2 / D + (7 - inverse_scaler(-1)) for centred data."""
+    bpd = -(sde.prior_logp(z) + delta_logp) / np.log(2)
+    return bpd / np.prod(z.shape[1:]) + 7.0

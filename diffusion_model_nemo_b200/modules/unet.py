@@ -186,6 +186,23 @@ class Unet(nn.Module):
         p = self.plan(x.shape[-1], x.shape[0], x.device)
         return p.forward(x.float().contiguous(), time, classes)
 
+    def jvp(self, x, time, v, classes=None):
+        """Forward-mode Jacobian-vector product: (forward(x, time, classes), d forward / dx . v) in one native pass.
+
+        fp32 only (compute_dtype='fp32'); the output equals forward() bit for bit.  time and classes enter through embeddings
+        that do not depend on x, so their tangents are zero."""
+        if _DTYPES[self.compute_dtype] != L.ACT_F32:
+            raise ValueError("Unet.jvp runs in fp32 only: set compute_dtype='fp32' (set_precision('fp32'))")
+        if x.device.type != "cuda":
+            raise L.DmnError("diffusion_model_nemo_b200.Unet runs on CUDA only: there is no CPU fallback")
+        assert x.dim() == 4 and x.shape[1] == self.channels and x.shape[2] == x.shape[3], f"bad input shape {tuple(x.shape)}"
+        if tuple(v.shape) != tuple(x.shape):
+            raise ValueError(f"tangent direction v has shape {tuple(v.shape)}; expected {tuple(x.shape)}")
+        time = time.reshape(-1)
+        assert time.shape[0] == x.shape[0], "time must have one entry per sample"
+        p = self.plan(x.shape[-1], x.shape[0], x.device)
+        return p.jvp(x.float().contiguous(), time, v.to(x.device, torch.float32).contiguous(), classes)
+
 
 def _film(c):
     # reference parts/film.py:29-54 (signal conv3x3 + LeakyReLU, scale / shift conv3x3)
@@ -243,3 +260,6 @@ class WaveGradUNet(Unet):
         assert level.shape[0] == x.shape[0], "noise_level must have one entry per sample"
         p = self.plan(x.shape[-1], x.shape[0], x.device)
         return p.forward(x.float().contiguous(), level, classes)
+
+    def jvp(self, x, noise_level, v, classes=None):
+        raise NotImplementedError("WaveGradUNet has no tangent program: the JVP is built for Unet only")

@@ -121,6 +121,15 @@ int dmn_unet_forward(dmn_plan* p, const float* x_dev, const int32_t* row_dev, co
 /* number of kernel launches one dmn_unet_forward enqueues (for bench.py's gpu_launches). */
 int dmn_plan_launches_per_forward(const dmn_plan* p);
 
+/* Forward-mode JVP: out = u(x, t) and out_tangent = (du/dx) . v, for fp32 plans on the SIMT engine (DMN_ENOTSUP for bf16 /
+ * tcgen05 plans and for FiLM plans).  x_dev, v_dev, out_dev, out_tangent_dev and the time / class arguments as in
+ * dmn_unet_forward; out_dev is bit-identical to what dmn_unet_forward writes.  The time and class embeddings do not depend on x.
+ * work_dev: caller-owned, 256-byte aligned, >= dmn_unet_jvp_work_bytes(p, batch) bytes (the tangents of the workspace buffers
+ * and the operand of the tangent convolutions).  No device allocation; graph-capturable. */
+int dmn_unet_jvp(dmn_plan* p, const float* x_dev, const float* v_dev, const int32_t* row_dev, const int64_t* classes_dev,
+                 float* out_dev, float* out_tangent_dev, void* work_dev, size_t work_bytes, int batch, void* stream);
+size_t dmn_unet_jvp_work_bytes(const dmn_plan* p, int batch);
+
 /* Measurement aids for bench.py's roofline (no reference counterpart).
  * dmn_plan_num_ops / dmn_plan_op_info: static description of launch i of the forward program -- name, kind
  *   (0 memset, 1 init_conv, 2 conv, 3 gn_finalize, 4 linattn, 5 attn, 6 final_proj, 7 film_modulate, 8 class_embed_add), engine (0 CUDA cores, 1 tcgen05),
@@ -339,6 +348,41 @@ typedef struct dmn_ode_desc {
 
 int    dmn_ode_sample(dmn_plan* p, const dmn_ode_desc* d, void* stream);
 size_t dmn_ode_work_bytes(const dmn_plan* p, int batch);
+
+/* Probability-flow ODE log-likelihood (score_sde's get_likelihood_fn; reference modules/sde_lib/likelihood.py): the same device
+ * RK45 over the augmented state [x ; delta_logp] (batch * channels * image_size^2 + batch elements) from t0 = eps to t1 = sde.T.
+ * The drift of x is the probability-flow drift above; the drift of delta_logp[b] is the Hutchinson divergence
+ * sum_i eps_i * (d drift / dx . eps)_i over sample b, from one dmn_unet_jvp pass in direction eps per evaluation (which also
+ * gives the model output).  The error norm runs over all elements, as scipy's does over the concatenated vector.  eps is
+ * noise_dev (injected, fp32 [batch, C, S, S]) or, when NULL, drawn once per solve with Philox4x32-10 keyed rng
+ * (Rademacher: the sign of the Gaussian draw).  Needs an fp32 SIMT plan (DMN_ENOTSUP otherwise) with the dmn_ode_sample
+ * requirements.  use_graph as in dmn_ode_sample (one cached graph per plan and descriptor). */
+#define DMN_HUTCH_RADEMACHER 0
+#define DMN_HUTCH_GAUSSIAN   1
+
+typedef struct dmn_ode_likelihood_desc {
+  int32_t sde_kind;        /* DMN_SDE_VP / DMN_SDE_VE */
+  int32_t N;               /* VP: label = t * (N - 1) */
+  double  beta_0, beta_1;  /* VP */
+  double  sigma_min, sigma_max;   /* VE */
+  double  t0, t1;          /* integration interval (eps -> sde.T); t0 != t1 */
+  double  rtol, atol;      /* as in dmn_ode_desc */
+  int32_t max_nfe;         /* evaluation budget, >= 2 */
+  int32_t batch;
+  int32_t use_graph;
+  int32_t hutchinson;      /* DMN_HUTCH_RADEMACHER / DMN_HUTCH_GAUSSIAN (ignored when noise_dev is given) */
+  dmn_rng rng;             /* Philox key of the Hutchinson draw when noise_dev == NULL */
+  const float* noise_dev;  /* injected Hutchinson noise [batch * channels * image_size^2] or NULL */
+  const int64_t* classes_dev;     /* optional class labels [batch] */
+  float*   state_dev;      /* in: data in the first batch * channels * image_size^2 floats; out: z, then delta_logp[batch] */
+  int64_t  state_elems;    /* floats behind state_dev: batch * (channels * image_size^2 + 1) */
+  void*    work_dev;       /* caller-owned, 256-byte aligned, >= dmn_ode_likelihood_work_bytes(plan, batch) */
+  size_t   work_bytes;
+  dmn_ode_result* result_dev;     /* device record, valid once the stream has run the solve */
+} dmn_ode_likelihood_desc;
+
+int    dmn_ode_likelihood(dmn_plan* p, const dmn_ode_likelihood_desc* d, void* stream);
+size_t dmn_ode_likelihood_work_bytes(const dmn_plan* p, int batch);
 
 /* ------------------------------------------------------------------------------------------------------
  * Layer-level entry points (unit tests and INTEGRATION.md's per-module swap).  Activations are fp32 NCHW at
