@@ -157,6 +157,7 @@ SYMBOLS = {
     "dmn_learned_step": (_I, [_P, _P, _P, _P, _I, _L, _P, _P, _I, Rng, _P]),
     "dmn_ddim_step": (_I, [_P, _P, _P, _P, _L, _P, _P, _I, Rng, _P]),
     "dmn_dpmpp_step": (_I, [_P, _P, _P, _P, _I, _L, _L, _P, _P, _I, _P]),
+    "dmn_dpmpp_sde_step": (_I, [_P, _P, _P, _P, _P, _I, _L, _L, _P, _P, _P, _I, Rng, _P]),
     "dmn_affine_noise_step": (_I, [_P, _P, _P, _P, _P, _L, _P, _P, _I, Rng, _P]),
     "dmn_langevin_step": (_I, [_P, _P, _P, _P, _P, _I, _L, _F, _P, _P, _I, _P, Rng, _P]),
     "dmn_bpd_qsample": (_I, [_P, _P, _P, _L, _P, _P, _I, Rng, _P]),

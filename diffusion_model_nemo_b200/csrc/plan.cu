@@ -55,7 +55,7 @@ int launch_learned(const float* x, const float* mo, const float* z, float* out, 
 int launch_ddim(const float* x, const float* eps, const float* z, float* out, long n, const float* coef, const int32_t* step_dev,
                 int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
 int launch_dpmpp(const float* x, const float* mo, float* hist, float* out, int batch, long chw, long mo_chw, const float* coef,
-                 const int32_t* step_dev, int step, cudaStream_t st);
+                 const float* coef2, const float* z, const int32_t* step_dev, int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
 int launch_inpaint_prepare(const float* x, const float* known, const float* mask, float* out, long n, const float* coef,
                            const int32_t* step_dev, int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st);
 int launch_traj(const float* x, float* traj, long n, const int32_t* step_dev, int every, int n_steps, cudaStream_t st);
@@ -1417,7 +1417,8 @@ static int enqueue_step(dmn_plan* p, const dmn_loop_desc* d, const LoopWork& w, 
     else if (d->kind == DMN_LOOP_DDIM)
       rc = launch_ddim(d->state_dev, w.mo, z0, d->state_dev, w.n, d->coef_dev, step_dev, s, d->rng, rng_dev, st);
     else
-      rc = launch_dpmpp(d->state_dev, w.mo, w.ring, d->state_dev, d->batch, w.chw, w.n_out / d->batch, d->coef_dev, step_dev, s, st);
+      rc = launch_dpmpp(d->state_dev, w.mo, w.ring, d->state_dev, d->batch, w.chw, w.n_out / d->batch, d->coef_dev, d->coef2_dev, z0,
+                        step_dev, s, d->rng, rng_dev, st);
     if (rc) return rc;
   }
   if (d->traj_dev && d->traj_every > 0)
@@ -1470,7 +1471,7 @@ static int run_loop(dmn_plan* p, const dmn_loop_desc* d, const dmn_inpaint_desc*
 
   if (d->noise_dev) {
     // parity mode: injected noise => per-step pointers differ, plain launches with the host step index
-    const int draws = (d->kind == DMN_LOOP_PC) ? d->n_corr + 1 : (d->kind == DMN_LOOP_DPMPP ? 0 : 1);
+    const int draws = (d->kind == DMN_LOOP_PC) ? d->n_corr + 1 : (d->kind == DMN_LOOP_DPMPP && !d->coef2_dev ? 0 : 1);
     for (int s = 0; s < d->n_steps; ++s)
       if ((rc = enqueue_step(p, d, w, ip, ctr, false, s, d->noise_dev + (long)s * draws * w.n, st))) return rc;
   } else if (!d->use_graph) {

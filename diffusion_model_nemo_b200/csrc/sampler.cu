@@ -135,17 +135,30 @@ __global__ void __launch_bounds__(256) ddim_step_kernel(const float* __restrict_
   }
 }
 
-// DPM-Solver++ multistep (Lu et al. 2022): the update is affine in (x, m_i, m_{i-1}, m_{i-2}), m = clamped data prediction.
-// row: {c_x, c_0, c_1, c_2, k_x, k_m, slot, pred_x0}.  hist is a 3-slot ring [3][n]: slot = i mod 3 receives m_i, (slot+2)%3 holds
-// m_{i-1} and (slot+1)%3 holds m_{i-2}.  A slot whose coefficient is 0 is never read (the ring starts as uninitialised scratch).
-// The model output has `mo_chw4` float4 per sample (C or 2C channels); only the first chw4 of them are used.
+// DPM-Solver++ multistep (Lu et al. 2022): the update is affine in (x, m_i, m_{i-1}, m_{i-2}), m = data prediction.
+// row: {c_x, c_0, c_1, c_2, k_x, k_m, slot, mode}.  mode (column 7): 0 = m = clamp(k_x x - k_m mo), 2 = the same without the clamp
+// (score-SDE models), any other value = m = clamp(mo) (the output is the data prediction).  hist is a 3-slot ring [3][n]: slot = i mod 3
+// receives m_i, (slot+2)%3 holds m_{i-1} and (slot+1)%3 holds m_{i-2}.  A slot whose coefficient is 0 is never read (the ring starts as
+// uninitialised scratch).  The model output has `mo_chw4` float4 per sample (C or 2C channels); only the first chw4 of them are used.
+// NOISE (SDE-DPM-Solver++): + g z with g = coef2 row[0], z injected or Philox draw 0 of the step word (the x_T draw uses word 0).
+template <bool NOISE>
 __global__ void __launch_bounds__(256) dpmpp_step_kernel(const float* x, const float* __restrict__ mo, float* __restrict__ hist,
                                                          float* out, long chw4, long mo_chw4, long n4, const float* __restrict__ coef,
-                                                         const int32_t* step_dev, int step) {
+                                                         const float* __restrict__ coef2, const float* __restrict__ z,
+                                                         const int32_t* step_dev, int step, dmn_rng rng_v, const dmn_rng* rng_dev) {
   const float* c = coef_row(coef, step_dev, step);
   const float cx = c[0], c0 = c[1], c1 = c[2], c2 = c[3], kx = c[4], km = c[5];
   const int slot = (int)c[6];
-  const bool pred_x0 = c[7] != 0.f;
+  const bool pred_x0 = c[7] != 0.f && c[7] != 2.f;
+  const bool clamp = c[7] != 2.f;
+  float g = 0.f;
+  uint32_t sw = 0;
+  dmn_rng rng{};
+  if (NOISE) {
+    g = coef_row(coef2, step_dev, step)[0];
+    sw = step_word(step_dev, step, 0);
+    rng = pick_rng(rng_v, rng_dev);
+  }
   float4* h_cur = reinterpret_cast<float4*>(hist) + (long)slot * n4;
   const float4* h_m1 = reinterpret_cast<const float4*>(hist) + (long)((slot + 2) % 3) * n4;
   const float4* h_m2 = reinterpret_cast<const float4*>(hist) + (long)((slot + 1) % 3) * n4;
@@ -154,7 +167,12 @@ __global__ void __launch_bounds__(256) dpmpp_step_kernel(const float* x, const f
     const float4 xv = reinterpret_cast<const float4*>(x)[i];
     const float4 ev = reinterpret_cast<const float4*>(mo)[mi];
     float4 m, o;
-#define DMN_DPM_M(f) m.f = clamp1(pred_x0 ? ev.f : (kx * xv.f - km * ev.f)); o.f = cx * xv.f + c0 * m.f;
+#define DMN_DPM_M(f)                                         \
+  {                                                          \
+    const float raw = pred_x0 ? ev.f : (kx * xv.f - km * ev.f); \
+    m.f = clamp ? clamp1(raw) : raw;                         \
+    o.f = cx * xv.f + c0 * m.f;                              \
+  }
     DMN_DPM_M(x) DMN_DPM_M(y) DMN_DPM_M(z) DMN_DPM_M(w)
 #undef DMN_DPM_M
     if (c1 != 0.f) {
@@ -164,6 +182,10 @@ __global__ void __launch_bounds__(256) dpmpp_step_kernel(const float* x, const f
     if (c2 != 0.f) {
       const float4 h = h_m2[i];
       o.x += c2 * h.x; o.y += c2 * h.y; o.z += c2 * h.z; o.w += c2 * h.w;
+    }
+    if (NOISE) {
+      const float4 zv = z ? reinterpret_cast<const float4*>(z)[i] : Philox::normal4(rng.seed, rng.stream_id, sw, (uint64_t)i);
+      o.x += g * zv.x; o.y += g * zv.y; o.z += g * zv.z; o.w += g * zv.w;
     }
     h_cur[i] = m;
     reinterpret_cast<float4*>(out)[i] = o;
@@ -663,12 +685,17 @@ int launch_ddim(const float* x, const float* eps, const float* z, float* out, lo
   return 0;
 }
 int launch_dpmpp(const float* x, const float* mo, float* hist, float* out, int batch, long chw, long mo_chw, const float* coef,
-                 const int32_t* step_dev, int step, cudaStream_t st) {
+                 const float* coef2, const float* z, const int32_t* step_dev, int step, dmn_rng rng, const dmn_rng* rng_dev, cudaStream_t st) {
   DMN_REQUIRE(batch > 0 && chw > 0 && chw % 4 == 0 && mo_chw >= chw && mo_chw % 4 == 0,
               "dpmpp_step: C*H*W must be a positive multiple of 4 and the model output at least C*H*W per sample");
   DMN_REQUIRE(x && mo && hist && out && coef, "dpmpp_step: null pointer");
   const long n4 = (long)batch * chw / 4;
-  dpmpp_step_kernel<<<grid_for(n4), 256, 0, st>>>(x, mo, hist, out, chw / 4, mo_chw / 4, n4, coef, step_dev, step);
+  if (coef2)
+    dpmpp_step_kernel<true><<<grid_for(n4), 256, 0, st>>>(x, mo, hist, out, chw / 4, mo_chw / 4, n4, coef, coef2, z, step_dev, step, rng,
+                                                          rng_dev);
+  else
+    dpmpp_step_kernel<false><<<grid_for(n4), 256, 0, st>>>(x, mo, hist, out, chw / 4, mo_chw / 4, n4, coef, nullptr, nullptr, step_dev,
+                                                           step, rng, nullptr);
   count_launch();
   DMN_LAUNCH_CHECK("dpmpp_step");
   return 0;
@@ -706,7 +733,16 @@ int dmn_ddim_step(const float* x, const float* eps, const float* z_dev, float* x
 
 int dmn_dpmpp_step(const float* x, const float* model_out, float* hist, float* x_out, int batch, int64_t chw, int64_t mo_chw,
                    const float* coef_dev, const int32_t* step_dev, int step, void* stream) {
-  return launch_dpmpp(x, model_out, hist, x_out, batch, chw, mo_chw, coef_dev, step_dev, step, (cudaStream_t)stream);
+  return launch_dpmpp(x, model_out, hist, x_out, batch, chw, mo_chw, coef_dev, nullptr, nullptr, step_dev, step, dmn_rng{}, nullptr,
+                      (cudaStream_t)stream);
+}
+
+int dmn_dpmpp_sde_step(const float* x, const float* model_out, const float* z_dev, float* hist, float* x_out, int batch, int64_t chw,
+                       int64_t mo_chw, const float* coef_dev, const float* coef2_dev, const int32_t* step_dev, int step, dmn_rng rng,
+                       void* stream) {
+  DMN_REQUIRE(coef2_dev, "dpmpp_sde_step: null noise-weight table");
+  return launch_dpmpp(x, model_out, hist, x_out, batch, chw, mo_chw, coef_dev, coef2_dev, z_dev, step_dev, step, rng, nullptr,
+                      (cudaStream_t)stream);
 }
 
 int dmn_inpaint_prepare(const float* x, const float* known, const float* mask, float* x_out, int64_t n, const float* coef_dev,

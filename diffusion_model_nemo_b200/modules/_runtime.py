@@ -85,7 +85,8 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
                     init_scale: float = 1.0, n_steps: Optional[int] = None, cfg_scale: Optional[float] = None,
                     inpaint: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None) -> LoopResult:
     """Run n_steps of (U-Net + update) natively.  noise: [1 + n_steps*draws, B, C, H, W] injected N(0,1) tensors in
-    the reference's draw order (element 0 = x_T), or None for in-kernel Philox; LOOP_DPMPP draws nothing and uses only noise[0].
+    the reference's draw order (element 0 = x_T), or None for in-kernel Philox; LOOP_DPMPP draws nothing and uses only noise[0],
+    unless coef2 holds the noise weights of SDE-DPM-Solver++ (one draw per step).
     cfg_scale: classifier-free guidance weight (None = off; 0.0 is a valid weight and gives the unconditional prediction).
     inpaint: (known [B, C, H, W], mask broadcasting to it, prep_coef [n_steps + 1][8] device rows) runs the loop through
     dmn_sample_loop_inpaint (in-kernel noise only)."""
@@ -109,7 +110,7 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
             raise NotImplementedError("classifier-free guidance is built for the DDPM / learned-variance / DDIM / DPM-Solver++ loops")
     plan = unet.plan(h, 2 * b if guided else b, device, time_rows=int(times.shape[0]))
     n = b * c * h * w
-    draws = (n_corr + 1) if kind == L.LOOP_PC else (0 if kind == L.LOOP_DPMPP else 1)
+    draws = (n_corr + 1) if kind == L.LOOP_PC else (0 if kind == L.LOOP_DPMPP and coef2 is None else 1)
     d = L.LoopDesc()
     d.kind, d.n_steps, d.batch, d.n_corr = kind, n_steps, b, n_corr
     d.snr, d.denoise, d.use_graph, d.corr_kind = float(snr), int(denoise), int(use_graph), corr_kind

@@ -5,7 +5,7 @@ Not in the reference: an extension, like classifier-free guidance.  It reuses th
 DDIM grid, so a config swaps `_target_` from GeneralizedGaussianDiffusion to this class and keeps the U-Net's time labels.  Each step
 is one U-Net evaluation and one elementwise update kernel (`dmn_dpmpp_step`) that keeps the last three data predictions in a device
 ring; with this package's Unet the whole loop is one replayed CUDA graph (`DMN_LOOP_DPMPP`).  The solver is deterministic: only x_T
-is random.
+is random.  `multistep_coefs` is the multistep algebra this sampler shares with sde.DPMSolverSampler (score-SDE models).
 """
 import math
 from typing import List, Optional
@@ -16,6 +16,39 @@ from .. import _lib as L
 from . import _runtime as R
 from .gaussian_diffusion import GaussianDiffusion
 from .generalized_gaussian_diffusion import strided_pairs
+
+
+def multistep_coefs(alpha, sigma, lam, orders):
+    """DPM-Solver++ multistep coefficients (c_x, c_0, c_1, c_2) of every step, in fp64, for the grid points 0..steps with their
+    alpha, sigma and lambda = log(alpha / sigma) and the per-step orders.  Step i goes from point i to point i + 1 and reads the data
+    predictions m_i, m_{i-1}, m_{i-2}:  x' = c_x x + c_0 m_i + c_1 m_{i-1} + c_2 m_{i-2}.  A step into sigma = 0 returns m_i."""
+    rows = []
+    for i, order in enumerate(orders):
+        if sigma[i + 1] == 0.0:             # sigma' = 0, lambda' = inf: x' = m_i
+            rows.append((0.0, 1.0, 0.0, 0.0))
+            continue
+        a_n, s_n, s_t = alpha[i + 1], sigma[i + 1], sigma[i]
+        h = lam[i + 1] - lam[i]
+        em = math.expm1(-h)
+        A = -a_n * em
+        cx, c0, c1, c2 = s_n / s_t, A, 0.0, 0.0
+        if order >= 2:
+            r0 = (lam[i] - lam[i - 1]) / h
+        if order == 2:                       # x' = cx x + A m0 + A/2 (m0 - m1)/r0
+            c0 += A / (2.0 * r0)
+            c1 = -A / (2.0 * r0)
+        elif order == 3:                     # x' = cx x + A m0 + B1 D1 + B2 D2
+            r1 = (lam[i - 1] - lam[i - 2]) / h
+            b1 = a_n * (em / h + 1.0)
+            b2 = -a_n * ((em + h) / (h * h) - 0.5)
+            q = r0 / (r0 + r1)
+            a0 = b1 * (1.0 + q) + b2 / (r0 + r1)      # coefficient of D1_0 = (m0 - m1)/r0
+            a1 = -b1 * q - b2 / (r0 + r1)             # coefficient of D1_1 = (m1 - m2)/r1
+            c0 += a0 / r0
+            c1 = -a0 / r0 + a1 / r1
+            c2 = -a1 / r1
+        rows.append((cx, c0, c1, c2))
+    return rows
 
 
 class DPMSolverDiffusion(GaussianDiffusion):
@@ -55,44 +88,15 @@ class DPMSolverDiffusion(GaussianDiffusion):
         alphas_cumprod table and rounded to fp32 once."""
         pairs = self.timestep_pairs()
         ac = self.alphas_cumprod.double()
-
-        def abar(t):
-            return 1.0 if t < 0 else float(ac[t])
-
-        def lam(t):
-            a = abar(t)
-            return 0.5 * (math.log(a) - math.log1p(-a))
-
+        abar = [float(ac[t]) for t, _ in pairs] + [1.0 if pairs[-1][1] < 0 else float(ac[pairs[-1][1]])]
+        alpha = [math.sqrt(a) for a in abar]
+        sigma = [math.sqrt(1.0 - a) for a in abar]
+        lam = [math.inf if a == 1.0 else 0.5 * (math.log(a) - math.log1p(-a)) for a in abar]
+        flag = 1.0 if self.objective == "pred_x0" else 0.0
         rows = []
-        ts = [p[0] for p in pairs]
-        for i, (order, (t, tn)) in enumerate(zip(self.step_orders(), pairs)):
+        for i, (coefs, (t, _)) in enumerate(zip(multistep_coefs(alpha, sigma, lam, self.step_orders()), pairs)):
             kx, km = float(self.sqrt_recip_alphas_cumprod[t]), float(self.sqrt_recipm1_alphas_cumprod[t])
-            flag = 1.0 if self.objective == "pred_x0" else 0.0
-            slot = float(i % 3)
-            if tn < 0:                       # sigma' = 0, lambda' = inf: x' = m_i
-                rows.append([0.0, 1.0, 0.0, 0.0, kx, km, slot, flag])
-                continue
-            a_n, s_n, s_t = math.sqrt(abar(tn)), math.sqrt(1.0 - abar(tn)), math.sqrt(1.0 - abar(t))
-            h = lam(tn) - lam(t)
-            em = math.expm1(-h)
-            A = -a_n * em
-            cx, c0, c1, c2 = s_n / s_t, A, 0.0, 0.0
-            if order >= 2:
-                r0 = (lam(t) - lam(ts[i - 1])) / h
-            if order == 2:                   # x' = cx x + A m0 + A/2 (m0 - m1)/r0
-                c0 += A / (2.0 * r0)
-                c1 = -A / (2.0 * r0)
-            elif order == 3:                 # x' = cx x + A m0 + B1 D1 + B2 D2
-                r1 = (lam(ts[i - 1]) - lam(ts[i - 2])) / h
-                b1 = a_n * (em / h + 1.0)
-                b2 = -a_n * ((em + h) / (h * h) - 0.5)
-                q = r0 / (r0 + r1)
-                a0 = b1 * (1.0 + q) + b2 / (r0 + r1)      # coefficient of D1_0 = (m0 - m1)/r0
-                a1 = -b1 * q - b2 / (r0 + r1)             # coefficient of D1_1 = (m1 - m2)/r1
-                c0 += a0 / r0
-                c1 = -a0 / r0 + a1 / r1
-                c2 = -a1 / r1
-            rows.append([cx, c0, c1, c2, kx, km, slot, flag])
+            rows.append(list(coefs) + [kx, km, float(i % 3), flag])
         return torch.tensor(rows, dtype=torch.float64).to(torch.float32)
 
     def _loop_tables(self, ts, device):

@@ -11,9 +11,12 @@ ProbabilityFlowSampler (modules/sde_samplers/probability_flow_sampler.py) solves
 rules on the device (dmn_ode_sample): the step control runs in device code, so the adaptive solve is one CUDA graph.
 LikelihoodEstimate (score_sde's get_likelihood_fn) runs the same solver over [x ; delta_logp] with a forward-mode JVP of the fp32
 Unet per evaluation for the Hutchinson divergence (dmn_ode_likelihood).
+DPMSolverSampler (not in the reference) is few-step DPM-Solver++ / SDE-DPM-Solver++ sampling of VP and VE score models on the
+DPM-Solver++ loop of DPMSolverDiffusion (dmn_dpmpp_step / dmn_dpmpp_sde_step, DMN_LOOP_DPMPP).
 """
 import abc
 import ctypes as C
+import math
 import warnings
 from typing import List, Optional
 
@@ -22,6 +25,7 @@ import torch
 
 from .. import _lib as L
 from . import _runtime as R
+from .dpm_solver_diffusion import multistep_coefs
 
 # ------------------------------------------------------------------------------------------------------
 # SDEs (tables are CPU fp32, reference op order => bit-exact)
@@ -719,3 +723,214 @@ def likelihood_bpd(sde: SDE, z: torch.Tensor, delta_logp: torch.Tensor) -> torch
     """score_sde likelihood_fn's tail: bpd = -(prior_logp(z) + delta_logp) / ln 2 / D + (7 - inverse_scaler(-1)) for centred data."""
     bpd = -(sde.prior_logp(z) + delta_logp) / np.log(2)
     return bpd / np.prod(z.shape[1:]) + 7.0
+
+
+# ------------------------------------------------------------------------------------------------------
+# few-step DPM-Solver++ / SDE-DPM-Solver++ (Lu et al. 2022) for VP and VE score models; not in the reference
+# ------------------------------------------------------------------------------------------------------
+
+
+def score_sde_schedule(sde, t: float):
+    """(alpha_t, sigma_t, lambda_t) of a VP or VE SDE at time t, in fp64.  VP: log alpha = -t^2 (b1 - b0) / 4 - t b0 / 2 and
+    sigma = sqrt(1 - alpha^2) (ScoreFunction.scale's std); VE: alpha = 1, sigma = sigma_min (sigma_max / sigma_min)^t."""
+    if isinstance(sde, VPSDE):
+        la = -0.25 * t * t * (sde.beta_1 - sde.beta_0) - 0.5 * t * sde.beta_0
+        sigma = math.sqrt(-math.expm1(2.0 * la))
+        return math.exp(la), sigma, la - math.log(sigma)
+    ls = math.log(sde.sigma_min) + t * math.log(sde.sigma_max / sde.sigma_min)
+    return 1.0, math.exp(ls), -ls
+
+
+def score_sde_inverse_lambda(sde, lam: float) -> float:
+    """The time t whose lambda_t is `lam` (score_sde_schedule's inverse)."""
+    if isinstance(sde, VPSDE):
+        L_ = 0.5 * np.logaddexp(0.0, -2.0 * lam)          # -log alpha
+        b0, db = sde.beta_0, sde.beta_1 - sde.beta_0
+        return float(2.0 * L_ / (0.5 * b0 + math.sqrt(0.25 * b0 * b0 + db * L_)))
+    return math.log(math.exp(-lam) / sde.sigma_min) / math.log(sde.sigma_max / sde.sigma_min)
+
+
+def score_sde_grid(sde, steps: int, eps: float, skip_type: str) -> List[float]:
+    """steps + 1 fp64 times from sde.T down to eps (both exact): uniform in t ("time_uniform") or in lambda ("logSNR")."""
+    T = float(sde.T)
+    if skip_type == "time_uniform":
+        ts = np.linspace(T, eps, steps + 1).tolist()
+    else:
+        lams = np.linspace(score_sde_schedule(sde, T)[2], score_sde_schedule(sde, eps)[2], steps + 1)
+        ts = [score_sde_inverse_lambda(sde, float(v)) for v in lams]
+    ts[0], ts[-1] = T, float(eps)
+    return ts
+
+
+def sde_dpmpp_coefs(alpha, sigma, lam, orders):
+    """SDE-DPM-Solver++ coefficients (c_x, c_0, c_1, g) of every step (data-prediction SDE form, 2M as the midpoint variant):
+    x' = c_x x + c_0 m_i + c_1 m_{i-1} + g z, with h = lambda' - lambda, c_x = sigma'/sigma e^-h, k = alpha' (1 - e^-2h),
+    order 1: c_0 = k; order 2: c_0 = k (1 + 1 / (2 r0)), c_1 = -k / (2 r0); g = sigma' sqrt(1 - e^-2h)."""
+    rows = []
+    for i, order in enumerate(orders):
+        h = lam[i + 1] - lam[i]
+        e2 = -math.expm1(-2.0 * h)
+        k = alpha[i + 1] * e2
+        cx, c0, c1 = sigma[i + 1] / sigma[i] * math.exp(-h), k, 0.0
+        if order == 2:
+            r0 = (lam[i] - lam[i - 1]) / h
+            c0 = k * (1.0 + 1.0 / (2.0 * r0))
+            c1 = -k / (2.0 * r0)
+        rows.append((cx, c0, c1, sigma[i + 1] * math.sqrt(e2)))
+    return rows
+
+
+class DPMSolverSampler(torch.nn.Module):
+    """Few-step sampler of a VP or VE score-SDE model: DPM-Solver++ multistep ("dpmsolver++", deterministic, orders 1-3) or
+    SDE-DPM-Solver++ ("sde-dpmsolver++", orders 1-2) on a grid of `steps` + 1 times from sde.T to eps, uniform in logSNR or in t.
+    One model evaluation per step (nfe = steps) and one update kernel (dmn_dpmpp_step / dmn_dpmpp_sde_step) with the earlier data
+    predictions in a device ring; with this package's Unet the loop is one replayed CUDA graph (DMN_LOOP_DPMPP), and
+    `guidance_scale` runs classifier-free guidance on a class-conditional Unet.  The data prediction is not clamped, like the
+    PC and ODE samplers; the sampler returns the state at t = eps with no denoising step.
+
+    `noise`: noise[0] is x_T (times sigma_max for VE); for "sde-dpmsolver++" noise[1 + s] is the z of step s.  Without it every
+    draw is in-kernel Philox keyed (`seed` or a draw from torch's CPU generator, data-parallel rank); x_T is the draw the PC
+    sampler makes for the same seed."""
+
+    def __init__(self, steps: int = 20, order: int = 2, skip_type: str = "logSNR", algorithm_type: str = "dpmsolver++",
+                 eps: float = None):
+        super().__init__()
+        if isinstance(steps, bool) or not isinstance(steps, (int, np.integer)) or steps < 1:
+            raise ValueError(f"`steps` must be an integer >= 1, got {steps!r}")
+        if algorithm_type not in ("dpmsolver++", "sde-dpmsolver++"):
+            raise ValueError(f"`algorithm_type` must be 'dpmsolver++' or 'sde-dpmsolver++', got {algorithm_type!r}")
+        max_order = 3 if algorithm_type == "dpmsolver++" else 2
+        if isinstance(order, bool) or order not in range(1, max_order + 1):
+            raise ValueError(f"`order` must be in 1..{max_order} for {algorithm_type}, got {order!r}")
+        if skip_type not in ("logSNR", "time_uniform"):
+            raise ValueError(f"`skip_type` must be 'logSNR' or 'time_uniform', got {skip_type!r}")
+        if eps is not None and (isinstance(eps, bool) or not isinstance(eps, (int, float, np.floating, np.integer))
+                                or not 0 < eps < 1):
+            raise ValueError(f"`eps` must be a number in (0, 1), got {eps!r}")
+        self.steps, self.order, self.skip_type, self.algorithm_type = int(steps), int(order), skip_type, algorithm_type
+        self.eps = None if eps is None else float(eps)
+        self.sde: Optional[SDE] = None
+        self.seed: Optional[int] = None
+        self.guidance_scale: Optional[float] = None
+        self.trajectory_every = 0
+        self.use_cuda_graph = True
+        self._cache = {}
+
+    def update_sde(self, sde: SDE):
+        self.sde = sde
+        self._cache = {}
+
+    def _check_sde(self):
+        if self.sde is None:
+            raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling forward()")
+        if not isinstance(self.sde, (VPSDE, VESDE)):
+            raise NotImplementedError(f"SDE class {self.sde.__class__.__name__} not yet supported.")
+        return self.sde
+
+    def timesteps(self) -> List[float]:
+        """The fp64 grid: steps + 1 times from sde.T to eps."""
+        sde = self._check_sde()
+        return score_sde_grid(sde, self.steps, sde.sampling_epsilon if self.eps is None else self.eps, self.skip_type)
+
+    def step_orders(self) -> List[int]:
+        """min(order, i + 1) at step i (warm-up); with fewer than 15 steps also at most steps - i, so the last step is first order."""
+        k = self.steps
+        return [min(self.order, i + 1, k - i) if k < 15 else min(self.order, i + 1) for i in range(k)]
+
+    def rows(self):
+        """(coef [steps][8], coef2 [steps][8] or None, labels [steps]) as CPU fp32: the kernel rows of dmn_dpmpp_step (mode 2:
+        unclamped data prediction) / dmn_dpmpp_sde_step expanded in fp64 and rounded once, and the U-Net labels
+        ScoreFunction.labels of the fp32 grid."""
+        sde = self._check_sde()
+        ts = self.timesteps()
+        alpha, sigma, lam = zip(*(score_sde_schedule(sde, t) for t in ts))
+        orders = self.step_orders()
+        vp = isinstance(sde, VPSDE)
+        coef2 = None
+        if self.algorithm_type == "dpmsolver++":
+            coefs = multistep_coefs(alpha, sigma, lam, orders)
+        else:
+            sde_coefs = sde_dpmpp_coefs(alpha, sigma, lam, orders)
+            coefs = [(cx, c0, c1, 0.0) for cx, c0, c1, _ in sde_coefs]
+            coef2 = torch.zeros(self.steps, L.COEF_STRIDE, dtype=torch.float64)
+            coef2[:, 0] = torch.tensor([r[3] for r in sde_coefs], dtype=torch.float64)
+            coef2 = coef2.to(torch.float32)
+        rows = []
+        for i, c in enumerate(coefs):
+            # m = k_x x - k_m out: VP (eps-like output, score = -out / sigma): x / alpha - sigma / alpha out; VE (the output is the
+            # score): x + sigma^2 out
+            kx, km = (1.0 / alpha[i], sigma[i] / alpha[i]) if vp else (1.0, -sigma[i] * sigma[i])
+            rows.append(list(c) + [kx, km, float(i % 3), 2.0])
+        labels = ScoreFunction(None, sde).labels(torch.tensor(ts[:-1], dtype=torch.float64).to(torch.float32))
+        return torch.tensor(rows, dtype=torch.float64).to(torch.float32), coef2, labels.to(torch.float32)
+
+    def forward(self, model, shape: List[int], device, return_nfe: bool = True, use_tqdm: bool = True, noise=None):
+        sde = self._check_sde()
+        R.require_cuda(device)
+        device = torch.device(device)
+        if len(shape) != 4:
+            raise ValueError(f"shape must be [B, C, H, W], got {list(shape)}")
+        b, c, h, w = (int(v) for v in shape)
+        stochastic = self.algorithm_type == "sde-dpmsolver++"
+        if noise is not None:
+            need = 1 + (self.steps if stochastic else 0)
+            if noise.dim() != 5 or tuple(noise.shape[1:]) != (b, c, h, w) or noise.shape[0] < need:
+                raise ValueError(f"noise has shape {tuple(noise.shape)}; expected [n >= {need}, {b}, {c}, {h}, {w}]")
+        key = str(device)
+        hit = self._cache.get(key)
+        if hit is None:
+            coef, coef2, labels = self.rows()
+            hit = (coef.to(device), None if coef2 is None else coef2.to(device), labels.to(device))
+            self._cache[key] = hit
+        coef, coef2, labels = hit
+        init_scale = float(sde.sigma_max) if isinstance(sde, VESDE) else 1.0
+        unet, classes = R.resolve_model(model)
+        if unet is not None:
+            if c != unet.channels or h != w:
+                raise ValueError(f"shape {list(shape)} does not fit the U-Net ({unet.channels} channels, square images)")
+            if unet.out_dim != unet.channels:
+                raise ValueError("the score-SDE data prediction needs a U-Net whose output has as many channels as its input")
+            guided = self.guidance_scale is not None and classes is not None
+            res = R.run_native_loop(unet, kind=L.LOOP_DPMPP, shape=shape, device=device, times=labels, coef=coef, coef2=coef2,
+                                    noise=noise, classes=classes, seed=self.seed, traj_every=self.trajectory_every,
+                                    use_graph=self.use_cuda_graph, init_scale=init_scale,
+                                    cfg_scale=float(self.guidance_scale) if guided else None)
+            imgs = R.to_image_list(res.final, res.traj)
+        else:
+            # foreign model: call it per step, the update is the native kernel with a local history ring
+            if self.guidance_scale is not None:
+                raise NotImplementedError("guidance_scale needs this package's class-conditional Unet (doubled-batch native loop)")
+            lib = L.lib()
+            with torch.cuda.device(device):
+                st = L.stream_ptr(device)
+                rng = L.Rng(self.seed if self.seed is not None else R.draw_seed(), R.rank_stream_id())
+                x = torch.empty((b, c, h, w), dtype=torch.float32, device=device)
+                if noise is not None:
+                    x.copy_(noise[0])
+                else:
+                    L.check(lib.dmn_randn(L.ptr(x), x.numel(), rng, -1, st), "dmn_randn")
+                if init_scale != 1.0:
+                    x.mul_(init_scale)
+                ring = torch.empty((3, b, c, h, w), dtype=torch.float32, device=device)
+                chw = x[0].numel()
+                keep = []
+                for s in range(self.steps):
+                    mo = model(x, labels[s].repeat(b)).float().contiguous()
+                    if tuple(mo.shape) != (b, c, h, w):
+                        raise ValueError(f"model output has shape {tuple(mo.shape)}; expected {(b, c, h, w)}")
+                    if stochastic:
+                        z = None if noise is None else noise[1 + s].to(device, torch.float32).contiguous()
+                        L.check(lib.dmn_dpmpp_sde_step(L.ptr(x), L.ptr(mo), L.ptr(z), L.ptr(ring), L.ptr(x), b, chw, chw, L.ptr(coef),
+                                                       L.ptr(coef2), None, s, rng, st), "dmn_dpmpp_sde_step")
+                    else:
+                        L.check(lib.dmn_dpmpp_step(L.ptr(x), L.ptr(mo), L.ptr(ring), L.ptr(x), b, chw, chw, L.ptr(coef), None, s, st),
+                                "dmn_dpmpp_step")
+                    if self.trajectory_every and (s + 1) % self.trajectory_every == 0:
+                        keep.append(x.clone())
+                traj = torch.stack(keep) if keep else None
+            imgs = R.to_image_list(x, traj)
+        return (imgs, self.steps) if return_nfe else imgs
+
+    def sample(self, model, shape: List[int], device=None, return_nfe: bool = False, noise=None):
+        device = R.default_device(model, device)
+        return self.forward(model=model, shape=shape, device=device, return_nfe=return_nfe, noise=noise)

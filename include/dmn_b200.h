@@ -170,15 +170,25 @@ int dmn_learned_step(const float* x, const float* model_out, const float* z_dev,
 int dmn_ddim_step(const float* x, const float* eps, const float* z_dev, float* x_out, int64_t n,
                   const float* coef_dev, const int32_t* step_dev, int step, dmn_rng rng, void* stream);
 /* DPM-Solver++ multistep update, orders 1-3 (Lu et al. 2022, "DPM-Solver++", Algorithm 2 and its third-order extension; not in
- * the reference: modules/dpm_solver_diffusion.py in the package builds the rows).  Deterministic: draws no noise.
- *   m  = clamp(pred_x0 ? model_out : k_x * x - k_m * model_out, -1, 1)      (data prediction; first C channels of each sample)
+ * the reference: modules/dpm_solver_diffusion.py and DPMSolverSampler in modules/sde.py build the rows).  Deterministic: draws no noise.
+ *   m  = k_x * x - k_m * model_out, clamped to [-1, 1] unless mode == 2     (data prediction; first C channels of each sample)
+ *        model_out itself, clamped, for any other nonzero mode (the output is the data prediction)
  *   x' = c_x * x + c_0 * m + c_1 * hist[(slot+2)%3] + c_2 * hist[(slot+1)%3] ;  hist[slot] = m
- * coef row: {c_x, c_0, c_1, c_2, k_x, k_m, slot, pred_x0 ? 1 : 0}.  hist_dev is a ring of 3 slots [3][batch*chw] fp32 holding the
- * previous steps' m (slot = step mod 3); a slot whose coefficient is 0 is not read, so the ring needs no initialisation.
- * model_out is [batch, mo_chw] with mo_chw = C*H*W or 2*C*H*W (learned variance: the variance channels are ignored).
- * x_out may alias x. */
+ * coef row: {c_x, c_0, c_1, c_2, k_x, k_m, slot, mode} with mode 0 = eps-like output (DDPM), 1 = data-prediction output (DDPM),
+ * 2 = unclamped k_x * x - k_m * model_out (score-SDE models, whose samplers never clamp).  hist_dev is a ring of 3 slots
+ * [3][batch*chw] fp32 holding the previous steps' m (slot = step mod 3); a slot whose coefficient is 0 is not read, so the ring needs
+ * no initialisation.  model_out is [batch, mo_chw] with mo_chw = C*H*W or 2*C*H*W (learned variance: the variance channels are
+ * ignored).  x_out may alias x. */
 int dmn_dpmpp_step(const float* x, const float* model_out, float* hist_dev, float* x_out, int batch, int64_t chw, int64_t mo_chw,
                    const float* coef_dev, const int32_t* step_dev, int step, void* stream);
+/* SDE-DPM-Solver++ (Lu et al. 2022, the data-prediction SDE solver; 2M in its midpoint form): dmn_dpmpp_step's update plus noise,
+ *   x' = c_x * x + c_0 * m + c_1 * hist[(slot+2)%3] + c_2 * hist[(slot+1)%3] + g * z
+ * with g = coef2_dev[row][0] (a [rows][DMN_COEF_STRIDE] table; the row is selected like the coef row, coef2_dev must not be NULL).
+ * z_dev is this step's injected N(0,1) tensor or NULL for the in-kernel Philox draw 0 of the step (counter word (step + 1) * 8,
+ * so every step's draw is independent of the others' and of dmn_randn's x_T draw with step -1). */
+int dmn_dpmpp_sde_step(const float* x, const float* model_out, const float* z_dev, float* hist_dev, float* x_out, int batch, int64_t chw,
+                       int64_t mo_chw, const float* coef_dev, const float* coef2_dev, const int32_t* step_dev, int step, dmn_rng rng,
+                       void* stream);
 /* ReverseDiffusionPredictor / EulerMaruyamaPredictor with the score wrapper folded in
  * (reverse_diffusion_predictor.py:11-16, euler_maruyama_predictor.py:11-17, sde_lib.py:91-105,
  *  score_function_loss.py:47-91):  x_mean = a*x + b*model_out ; x = x_mean + g*z.  coef row: {a, b, g} */
@@ -230,8 +240,10 @@ int dmn_axpby(const float* x, const float* y, float a, float b, float* out, int6
                                  state_dev = x_0 (read only), aux_dev = terms [batch][n_steps] (column = coef2 row[1]),
                                  coef_dev / coef2_dev rows as documented at dmn_bpd_term; noise_dev injects the q_sample draws */
 #define DMN_LOOP_DPMPP    5   /* DPM-Solver++ multistep: per step U-Net (or the guidance path) -> dmn_dpmpp_step; rows as documented
-                                 there, one per (t_i, t_{i+1}) pair.  out_dim = C or 2C.  Draws nothing: noise_dev, if given, only
-                                 selects plain launches with the host step index.  The history ring lives in scratch_dev. */
+                                 there, one per (t_i, t_{i+1}) pair.  out_dim = C or 2C.  coef2_dev == NULL: draws nothing, and
+                                 noise_dev, if given, only selects plain launches with the host step index.  coef2_dev != NULL: the
+                                 stochastic form of dmn_dpmpp_sde_step with g in coef2 row[0], one draw per step (noise_dev holds
+                                 n_steps blocks).  The history ring lives in scratch_dev. */
 
 typedef struct dmn_loop_desc {
   int32_t kind;            /* DMN_LOOP_* */
@@ -243,7 +255,7 @@ typedef struct dmn_loop_desc {
   int32_t use_graph;       /* 1 = CUDA graph replay, 0 = plain launches (debug) */
   int32_t corr_kind;       /* PC corrector: 0 = Langevin (batch-mean norms), 1 = affine-noise rows {a,b,g} in coef2 (ALD) */
   const float*   coef_dev;       /* [n_steps][DMN_COEF_STRIDE]  update coefficients (predictor for PC) */
-  const float*   coef2_dev;      /* PC: [n_steps][DMN_COEF_STRIDE] corrector coefficients */
+  const float*   coef2_dev;      /* PC: [n_steps][DMN_COEF_STRIDE] corrector coefficients; DPM-Solver++: noise weights {g} or NULL */
   const int64_t* classes_dev;    /* optional class labels */
   const float*   noise_dev;      /* parity mode: [n_steps * draws_per_step][batch*C*H*W] in draw order, else NULL */
   dmn_rng        rng;            /* throughput mode */
