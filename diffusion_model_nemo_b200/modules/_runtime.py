@@ -1,8 +1,9 @@
-"""Shared host logic of the native sampling loops: model resolution, coefficient rows, loop launch, outputs."""
+"""Shared host logic of the sampling loops: model resolution, coefficient rows, the native loop and the per-step host loop of
+other model callables, outputs."""
 import ctypes as C
 import functools
 import os
-from typing import List, Optional, Sequence, Tuple
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import torch
 
@@ -77,6 +78,36 @@ class LoopResult:
         self.final, self.aux, self.traj = final, aux, traj
 
 
+def loop_draws(kind: int, n_corr: int = 0, coef2: Optional[torch.Tensor] = None) -> int:
+    """N(0,1) draws a loop of `kind` makes per step (the PC corrector's, then the predictor's; none for deterministic
+    DPM-Solver++, which has no noise-weight table coef2)."""
+    if kind == L.LOOP_PC:
+        return n_corr + 1
+    return 0 if kind == L.LOOP_DPMPP and coef2 is None else 1
+
+
+def launch_step(kind: int, x, model_out, z, out, coef, step: int, rng, st, coef2=None, ring=None):
+    """One standalone update of loop `kind` at `step`: the kernel the native loop enqueues for that kind.  The DPM-Solver++
+    kinds keep their data predictions in `ring` ([3, *x.shape])."""
+    lib = L.lib()
+    x_, mo, z_, out_, c = L.ptr(x), L.ptr(model_out), L.ptr(z), L.ptr(out), L.ptr(coef)
+    n, b = x.numel(), x.shape[0]
+    if kind == L.LOOP_DDPM:
+        name, rc = "dmn_ddpm_step", lib.dmn_ddpm_step(x_, mo, z_, out_, n, c, None, step, rng, st)
+    elif kind == L.LOOP_LEARNED:
+        name, rc = "dmn_learned_step", lib.dmn_learned_step(x_, mo, z_, out_, b, n // b, c, None, step, rng, st)
+    elif kind == L.LOOP_DDIM:
+        name, rc = "dmn_ddim_step", lib.dmn_ddim_step(x_, mo, z_, out_, n, c, None, step, rng, st)
+    elif kind == L.LOOP_DPMPP and coef2 is None:
+        name, rc = "dmn_dpmpp_step", lib.dmn_dpmpp_step(x_, mo, L.ptr(ring), out_, b, n // b, model_out[0].numel(), c, None, step, st)
+    elif kind == L.LOOP_DPMPP:
+        name, rc = "dmn_dpmpp_sde_step", lib.dmn_dpmpp_sde_step(x_, mo, z_, L.ptr(ring), out_, b, n // b, model_out[0].numel(), c,
+                                                                L.ptr(coef2), None, step, rng, st)
+    else:
+        raise ValueError(f"loop kind {kind} has no standalone update kernel")
+    L.check(rc, name)
+
+
 def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, times: torch.Tensor, coef: torch.Tensor,
                     coef2: Optional[torch.Tensor] = None, x_init: Optional[torch.Tensor] = None,
                     noise: Optional[torch.Tensor] = None, classes: Optional[torch.Tensor] = None,
@@ -110,7 +141,7 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
             raise NotImplementedError("classifier-free guidance is built for the DDPM / learned-variance / DDIM / DPM-Solver++ loops")
     plan = unet.plan(h, 2 * b if guided else b, device, time_rows=int(times.shape[0]))
     n = b * c * h * w
-    draws = (n_corr + 1) if kind == L.LOOP_PC else (0 if kind == L.LOOP_DPMPP and coef2 is None else 1)
+    draws = loop_draws(kind, n_corr, coef2)
     d = L.LoopDesc()
     d.kind, d.n_steps, d.batch, d.n_corr = kind, n_steps, b, n_corr
     d.snr, d.denoise, d.use_graph, d.corr_kind = float(snr), int(denoise), int(use_graph), corr_kind
@@ -185,6 +216,69 @@ def run_native_loop(unet: Unet, *, kind: int, shape: Sequence[int], device, time
         # keep every buffer alive until the stream has consumed it
         torch.cuda.current_stream(device).synchronize()
     return LoopResult(state.clone(), None if aux is None else aux.clone(), traj)
+
+
+def run_loop(model, *, kind: int, shape: Sequence[int], device, times: torch.Tensor, coef: torch.Tensor,
+             model_arg: Callable[[int], torch.Tensor], coef2: Optional[torch.Tensor] = None, x_init: Optional[torch.Tensor] = None,
+             noise: Optional[torch.Tensor] = None, seed: Optional[int] = None, traj_every: int = 0, use_graph: bool = True,
+             init_scale: float = 1.0, guidance_scale: Optional[float] = None, out_widths: Sequence[int] = (1,),
+             inpaint: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None) -> List[torch.Tensor]:
+    """Sample with the loop of `kind` and return `to_image_list` of the result.  This package's Unet (or a partial of it with
+    `classes`) runs the native loop (`run_native_loop`, same arguments); any other callable is called per step as
+    model(x, model_arg(s)) and only the update is native: the same kernels, rows, step words, x_T and noise as the native loop.
+    out_widths: the model output channel counts accepted from such a callable, in multiples of the image's channels.
+    guidance_scale applies when the Unet has `classes`, and needs this package's Unet."""
+    unet, classes = resolve_model(model)
+    if unet is not None:
+        guided = guidance_scale is not None and classes is not None
+        res = run_native_loop(unet, kind=kind, shape=shape, device=device, times=times, coef=coef, coef2=coef2, x_init=x_init,
+                              noise=noise, classes=classes, seed=seed, traj_every=traj_every, use_graph=use_graph,
+                              init_scale=init_scale, cfg_scale=float(guidance_scale) if guided else None, inpaint=inpaint)
+        return to_image_list(res.final, res.traj)
+    if guidance_scale is not None:
+        raise NotImplementedError("guidance_scale needs this package's class-conditional Unet (doubled-batch native loop)")
+    lib = L.lib()
+    b, c, h, w = (int(s) for s in shape)
+    outs = [(b, k * c, h, w) for k in out_widths]
+    draws = loop_draws(kind, 0, coef2)
+    first = 0 if x_init is not None else 1          # noise[0] is x_T unless x_init is given
+    rng = L.Rng(seed if seed is not None else draw_seed(), rank_stream_id())
+    with torch.cuda.device(device):
+        st = L.stream_ptr(device)
+        x = torch.empty((b, c, h, w), dtype=torch.float32, device=device)
+        if x_init is not None:
+            x.copy_(x_init)
+        else:
+            if noise is not None:
+                x.copy_(noise[0])
+            else:
+                L.check(lib.dmn_randn(L.ptr(x), x.numel(), rng, -1, st), "dmn_randn")
+            if init_scale != 1.0:
+                x.mul_(init_scale)
+        ring = torch.empty((3, b, c, h, w), dtype=torch.float32, device=device) if kind == L.LOOP_DPMPP else None
+        if inpaint is not None:
+            known, mask, prep = inpaint
+            known = known.to(device, torch.float32).contiguous()
+            mask = torch.empty_like(known).copy_(mask)
+
+            def merge(e):
+                L.check(lib.dmn_inpaint_prepare(L.ptr(x), L.ptr(known), L.ptr(mask), L.ptr(x), x.numel(), L.ptr(prep), None, e, rng,
+                                                st), "dmn_inpaint_prepare")
+        keep = []
+        for s in range(int(times.shape[0])):
+            if inpaint is not None:
+                merge(s)
+            mo = model(x, model_arg(s)).float().contiguous()
+            if tuple(mo.shape) not in outs:
+                raise ValueError(f"model output has shape {tuple(mo.shape)}; expected one of {outs}")
+            z = None if noise is None or not draws else noise[first + s * draws].to(device, torch.float32).contiguous()
+            launch_step(kind, x, mo, z, x, coef, s, rng, st, coef2=coef2, ring=ring)
+            if traj_every and (s + 1) % traj_every == 0:
+                keep.append(x.clone())
+        if inpaint is not None:
+            merge(int(times.shape[0]))          # the final composite
+        traj = torch.stack(keep) if keep else None
+    return to_image_list(x, traj)
 
 
 def to_image_list(final: torch.Tensor, traj: Optional[torch.Tensor]) -> List[torch.Tensor]:

@@ -53,6 +53,7 @@ def multistep_coefs(alpha, sigma, lam, orders):
 
 class DPMSolverDiffusion(GaussianDiffusion):
     _loop_kind = L.LOOP_DPMPP
+    _out_widths = (1, 2)        # a learned-variance model's variance channels are not read
 
     def __init__(self, timesteps: int, schedule_name: str, schedule_cfg=None, objective: str = "pred_noise",
                  class_conditional: bool = False, steps: int = 20, order: int = 2):
@@ -126,45 +127,7 @@ class DPMSolverDiffusion(GaussianDiffusion):
     def p_sample_loop(self, model, shape, device=None, use_tqdm=True, noise=None, img=None):
         """Solve from x_T (img, else noise[0], else a Philox draw with self.seed -- the draw DDIM makes for that seed) to the data
         prediction at t = 0.  Returns the reference's list of CPU images in [0, 1], the last being the final sample."""
-        device = R.default_device(model, device)
-        R.require_cuda(device)
-        ts = self._visit_order()
-        coef, times = self._loop_tables(ts, device)
-        unet, classes = R.resolve_model(model)
-        if unet is not None:
-            res = R.run_native_loop(unet, kind=L.LOOP_DPMPP, shape=shape, device=device, times=times, coef=coef,
-                                    x_init=img, noise=noise, classes=classes, seed=self.seed,
-                                    traj_every=self.trajectory_every, use_graph=self.use_cuda_graph,
-                                    cfg_scale=float(self.guidance_scale) if (self.guidance_scale is not None and classes is not None) else None)
-            return R.to_image_list(res.final, res.traj)
-        # foreign model: call it per step, the update is the native kernel with a local history ring
-        if self.guidance_scale is not None:
-            raise NotImplementedError("guidance_scale needs this package's class-conditional Unet (doubled-batch native loop)")
-        b = shape[0]
-        lib = L.lib()
-        with torch.cuda.device(device):
-            st = L.stream_ptr(device)
-            x = torch.empty(tuple(shape), dtype=torch.float32, device=device)
-            if img is not None:
-                x.copy_(img)
-            elif noise is not None:
-                x.copy_(noise[0])
-            else:
-                rng = L.Rng(self.seed if self.seed is not None else R.draw_seed(), R.rank_stream_id())
-                L.check(lib.dmn_randn(L.ptr(x), x.numel(), rng, -1, st), "dmn_randn")
-            ring = torch.empty((3,) + tuple(shape), dtype=torch.float32, device=device)
-            chw = x[0].numel()
-            keep = []
-            for s, ti in enumerate(ts.tolist()):
-                mo = model(x, self._model_arg(ti, b, device)).float().contiguous()
-                if mo.shape[0] != b or mo[0].numel() not in (chw, 2 * chw):
-                    raise ValueError(f"model output has shape {tuple(mo.shape)}; expected {b} samples of C or 2C channels")
-                L.check(lib.dmn_dpmpp_step(L.ptr(x), L.ptr(mo), L.ptr(ring), L.ptr(x), b, chw, mo[0].numel(), L.ptr(coef), None, s, st),
-                        "dmn_dpmpp_step")
-                if self.trajectory_every and (s + 1) % self.trajectory_every == 0:
-                    keep.append(x.clone())
-            traj = torch.stack(keep) if keep else None
-        return R.to_image_list(x, traj)
+        return super().p_sample_loop(model, shape, device=device, use_tqdm=use_tqdm, noise=noise, img=img)
 
     @torch.no_grad()
     def sample(self, model, shape, device=None, noise=None):

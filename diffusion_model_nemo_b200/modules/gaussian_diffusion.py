@@ -86,6 +86,7 @@ class GaussianDiffusion(AbstractDiffusionProcess):
                 self.posterior_mean_coef2[ts], sigma, flag]
 
     _loop_kind = L.LOOP_DDPM
+    _out_widths = (1,)          # model output channels, in multiples of the image's, that the update reads
 
     def _loop_tables(self, ts: torch.Tensor, device):
         key = (str(device), tuple(ts[:: max(1, len(ts) // 5)].tolist()), len(ts), self.objective)
@@ -143,13 +144,9 @@ class GaussianDiffusion(AbstractDiffusionProcess):
         model_out = model_out.float().contiguous()
         rng = L.Rng(seed if seed is not None else R.draw_seed(), R.rank_stream_id())
         with torch.cuda.device(x.device):
-            self._launch_step(lib, x, model_out, None if noise is None else noise.float().contiguous(), out, coef, 0, rng,
-                              L.stream_ptr(x.device))
+            R.launch_step(self._loop_kind, x, model_out, None if noise is None else noise.float().contiguous(), out, coef, 0, rng,
+                          L.stream_ptr(x.device))
         return out
-
-    def _launch_step(self, lib, x, model_out, z, out, coef, step, rng, st):
-        L.check(lib.dmn_ddpm_step(L.ptr(x), L.ptr(model_out), L.ptr(z), L.ptr(out), x.numel(), L.ptr(coef), None, step, rng, st),
-                "dmn_ddpm_step")
 
     @torch.no_grad()
     def p_sample(self, model, x, t, noise=None):
@@ -169,42 +166,11 @@ class GaussianDiffusion(AbstractDiffusionProcess):
         device = R.default_device(model, device)
         R.require_cuda(device)
         ts = self._visit_order(start)
-        unet, classes = R.resolve_model(model)
-        if unet is not None:
-            coef, times = self._loop_tables(ts, device)
-            res = R.run_native_loop(unet, kind=self._loop_kind, shape=shape, device=device, times=times, coef=coef,
-                                    x_init=img, noise=noise, classes=classes, seed=self.seed,
-                                    traj_every=self.trajectory_every, use_graph=self.use_cuda_graph,
-                                    cfg_scale=float(self.guidance_scale) if (self.guidance_scale is not None and classes is not None) else None)
-            return R.to_image_list(res.final, res.traj)
-        # foreign model: call it per step, fuse only the update
-        if self.guidance_scale is not None:
-            raise NotImplementedError("guidance_scale needs this package's class-conditional Unet (doubled-batch native loop)")
-        b = shape[0]
-        seed = self.seed if self.seed is not None else R.draw_seed()
-        lib = L.lib()
-        coef, _ = self._loop_tables(ts, device)
-        with torch.cuda.device(device):
-            st = L.stream_ptr(device)
-            x = torch.empty(tuple(shape), dtype=torch.float32, device=device)
-            rng = L.Rng(seed, R.rank_stream_id())
-            k = 0
-            if img is not None:
-                x.copy_(img)
-            elif noise is not None:
-                x.copy_(noise[0])
-                k = 1
-            else:
-                L.check(lib.dmn_randn(L.ptr(x), x.numel(), rng, -1, st), "dmn_randn")
-            keep = []
-            for s, ti in enumerate(ts.tolist()):
-                mo = model(x, self._model_arg(ti, b, device)).float().contiguous()
-                z = None if noise is None else noise[k + s].to(device, torch.float32).contiguous()
-                self._launch_step(lib, x, mo, z, x, coef, s, rng, st)
-                if self.trajectory_every and (s + 1) % self.trajectory_every == 0:
-                    keep.append(x.clone())
-            traj = torch.stack(keep) if keep else None
-        return R.to_image_list(x, traj)
+        coef, times = self._loop_tables(ts, device)
+        return R.run_loop(model, kind=self._loop_kind, shape=shape, device=device, times=times, coef=coef, x_init=img, noise=noise,
+                          seed=self.seed, traj_every=self.trajectory_every, use_graph=self.use_cuda_graph,
+                          guidance_scale=self.guidance_scale, out_widths=self._out_widths,
+                          model_arg=lambda s: self._model_arg(int(ts[s]), shape[0], device))
 
     # ---- bits-per-dimension evaluation (SURVEY 8f rank 3) ------------------------------------------------------------
     @torch.no_grad()
@@ -330,43 +296,10 @@ class GaussianDiffusion(AbstractDiffusionProcess):
         if noise is not None and tuple(noise.shape[1:]) != tuple(shape):
             raise ValueError(f"noise has shape {tuple(noise.shape)}; expected [n, {', '.join(map(str, shape))}]")
         coef, times, prep, labels = self._inpaint_tables(jump_length, jump_n_sample, device)
-        unet, classes = R.resolve_model(model)
-        if unet is not None:
-            res = R.run_native_loop(unet, kind=self._loop_kind, shape=shape, device=device, times=times, coef=coef,
-                                    x_init=None if noise is None else noise[0], classes=classes, seed=self.seed,
-                                    traj_every=self.trajectory_every, use_graph=self.use_cuda_graph,
-                                    cfg_scale=float(self.guidance_scale) if (self.guidance_scale is not None and classes is not None) else None,
-                                    inpaint=(x_known, mask, prep))
-            return R.to_image_list(res.final, res.traj)
-        # foreign model: call it per event; the same kernels, rows and step words as the graph
-        if self.guidance_scale is not None:
-            raise NotImplementedError("guidance_scale needs this package's class-conditional Unet (doubled-batch native loop)")
-        b = shape[0]
-        seed = self.seed if self.seed is not None else R.draw_seed()
-        lib = L.lib()
-        with torch.cuda.device(device):
-            st = L.stream_ptr(device)
-            known = x_known.to(device, torch.float32).contiguous()
-            m = torch.empty_like(known)
-            m.copy_(mask)
-            x = torch.empty(tuple(shape), dtype=torch.float32, device=device)
-            rng = L.Rng(seed, R.rank_stream_id())
-            if noise is not None:
-                x.copy_(noise[0])
-            else:
-                L.check(lib.dmn_randn(L.ptr(x), x.numel(), rng, -1, st), "dmn_randn")
-            keep = []
-            for e, ti in enumerate(labels):
-                L.check(lib.dmn_inpaint_prepare(L.ptr(x), L.ptr(known), L.ptr(m), L.ptr(x), x.numel(), L.ptr(prep), None, e, rng, st),
-                        "dmn_inpaint_prepare")
-                mo = model(x, self._model_arg(ti, b, device)).float().contiguous()
-                self._launch_step(lib, x, mo, None, x, coef, e, rng, st)
-                if self.trajectory_every and (e + 1) % self.trajectory_every == 0:
-                    keep.append(x.clone())
-            L.check(lib.dmn_inpaint_prepare(L.ptr(x), L.ptr(known), L.ptr(m), L.ptr(x), x.numel(), L.ptr(prep), None, len(labels), rng,
-                                            st), "dmn_inpaint_prepare(final)")
-            traj = torch.stack(keep) if keep else None
-        return R.to_image_list(x, traj)
+        return R.run_loop(model, kind=self._loop_kind, shape=shape, device=device, times=times, coef=coef,
+                          x_init=None if noise is None else noise[0], seed=self.seed, traj_every=self.trajectory_every,
+                          use_graph=self.use_cuda_graph, guidance_scale=self.guidance_scale, out_widths=self._out_widths,
+                          inpaint=(x_known, mask, prep), model_arg=lambda e: self._model_arg(labels[e], shape[0], device))
 
     @torch.no_grad()
     def sample(self, model, shape, device=None, noise=None):

@@ -46,10 +46,6 @@ class GeneralizedGaussianDiffusion(GaussianDiffusion):
         flag = torch.full_like(at, 1.0 if self.objective == "pred_x0" else 0.0)
         return [(1.0 - at).sqrt(), at.sqrt(), an.sqrt(), c1, c2, flag]
 
-    def _launch_step(self, lib, x, model_out, z, out, coef, step, rng, st):
-        L.check(lib.dmn_ddim_step(L.ptr(x), L.ptr(model_out), L.ptr(z), L.ptr(out), x.numel(), L.ptr(coef), None, step, rng, st),
-                "dmn_ddim_step")
-
     def generalized_predict_start_from_noise(self, x_t, t, noise):
         assert x_t.shape == noise.shape, f"{x_t.shape} != {noise.shape}"
         a = self.extract(self.alphas_extended_cumprod, t + 1, x_t.shape)
@@ -71,8 +67,8 @@ class GeneralizedGaussianDiffusion(GaussianDiffusion):
         coef = R.coef_rows(self._pair_rows(torch.tensor([ti]), torch.tensor([tn])), x.device)
         out = torch.empty_like(x, dtype=torch.float32)
         with torch.cuda.device(x.device):
-            self._launch_step(L.lib(), x.float().contiguous(), mo, None if noise is None else noise.float().contiguous(), out, coef, 0,
-                              L.Rng(R.draw_seed(), R.rank_stream_id()), L.stream_ptr(x.device))
+            R.launch_step(L.LOOP_DDIM, x.float().contiguous(), mo, None if noise is None else noise.float().contiguous(), out, coef, 0,
+                          L.Rng(R.draw_seed(), R.rank_stream_id()), L.stream_ptr(x.device))
         x0 = self.generalized_predict_start_from_noise(x, t, mo).clamp(-1.0, 1.0) if self.objective == "pred_noise" else mo.clamp(-1, 1)
         return out, x0
 

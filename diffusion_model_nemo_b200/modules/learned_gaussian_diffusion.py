@@ -10,6 +10,7 @@ class LearnedGaussianDiffusion(GaussianDiffusion):
     posterior log-variance, per pixel (reference learned_gaussian_diffusion.py:36-43)."""
 
     _loop_kind = L.LOOP_LEARNED
+    _out_widths = (2,)
 
     def __init__(self, timesteps: int, schedule_name: str, schedule_cfg=None, objective: str = "pred_noise"):
         super().__init__(timesteps=timesteps, schedule_name=schedule_name, schedule_cfg=schedule_cfg, objective=objective)
@@ -18,11 +19,6 @@ class LearnedGaussianDiffusion(GaussianDiffusion):
         mask = 1 - (ts == 0).float()
         return [self.sqrt_recip_alphas_cumprod[ts], self.sqrt_recipm1_alphas_cumprod[ts], self.posterior_mean_coef1[ts],
                 self.posterior_mean_coef2[ts], mask, self.posterior_log_variance_clipped[ts], torch.log(self.betas)[ts]]
-
-    def _launch_step(self, lib, x, model_out, z, out, coef, step, rng, st):
-        b = x.shape[0]
-        L.check(lib.dmn_learned_step(L.ptr(x), L.ptr(model_out), L.ptr(z), L.ptr(out), b, x.numel() // b, L.ptr(coef), None, step,
-                                     rng, st), "dmn_learned_step")
 
     def p_mean_variance(self, model, x, t, model_output=None, return_pred_x_start: bool = False):
         model_output = _default(model_output, lambda: model(x, t))

@@ -89,8 +89,8 @@ class VPSDE(SDE):
         return -0.5 * beta_t[:, None, None, None] * x, torch.sqrt(beta_t)
 
     def marginal_prob(self, x, t):
-        lmc = -0.25 * t ** 2 * (self.beta_1 - self.beta_0) - 0.5 * t * self.beta_0
-        return torch.exp(lmc[:, None, None, None]) * x, torch.sqrt(1.0 - torch.exp(2.0 * lmc))
+        lmc, std = _vp_log_mean_std(self, t)
+        return torch.exp(lmc[:, None, None, None]) * x, std
 
     def prior_sampling(self, shape):
         return torch.randn(*shape)
@@ -104,6 +104,13 @@ class VPSDE(SDE):
         beta = self.betas.to(x.device)[ts]
         alpha = self.alphas.to(x.device)[ts]
         return torch.sqrt(alpha)[:, None, None, None] * x - x, torch.sqrt(beta)
+
+
+def _vp_log_mean_std(sde: VPSDE, t):
+    """(log mean coefficient, std) of the VP marginal p(x_t | x_0) at the times t, in the reference's op order (vp_sde.py
+    marginal_prob), so that every table built from it is bit-identical to the reference's."""
+    lmc = -0.25 * t ** 2 * (sde.beta_1 - sde.beta_0) - 0.5 * t * sde.beta_0
+    return lmc, torch.sqrt(1.0 - torch.exp(2.0 * lmc))
 
 
 class VESDE(SDE):
@@ -140,6 +147,20 @@ class VESDE(SDE):
         return torch.zeros_like(x), torch.sqrt(sig ** 2 - adj ** 2)
 
 
+def init_scale(sde: SDE) -> float:
+    """Factor from an N(0, I) draw to x_T: the prior of a VE SDE has std sigma_max, a VP prior is N(0, I)."""
+    return float(sde.sigma_max) if isinstance(sde, VESDE) else 1.0
+
+
+def _checked_sde(sde: Optional[SDE], call: str = "forward()") -> SDE:
+    """The SDE a sampler was given with update_sde; the native samplers are built for VP and VE."""
+    if sde is None:
+        raise ValueError(f"Must explicitly set `update_sde(sde)` for this module prior to calling {call}")
+    if not isinstance(sde, (VPSDE, VESDE)):
+        raise NotImplementedError(f"SDE class {sde.__class__.__name__} not yet supported.")
+    return sde
+
+
 # ------------------------------------------------------------------------------------------------------
 # score wrapper (reference loss/sde_loss/score_function_loss.py:47-91, continuous=True)
 # ------------------------------------------------------------------------------------------------------
@@ -162,8 +183,7 @@ class ScoreFunction:
 
     def scale(self, t):
         if isinstance(self.sde, VPSDE):
-            lmc = -0.25 * t ** 2 * (self.sde.beta_1 - self.sde.beta_0) - 0.5 * t * self.sde.beta_0
-            return -1.0 / torch.sqrt(1.0 - torch.exp(2.0 * lmc))
+            return -1.0 / _vp_log_mean_std(self.sde, t)[1]
         return torch.ones_like(t)
 
     def raw(self, x, t):
@@ -235,8 +255,7 @@ def corrector_rows(name: Optional[str], sde, sf: ScoreFunction, t: torch.Tensor,
     if name == "langevin":                  # langevin_corrector.py:15-35 (step size needs the batch-mean norms: on device)
         return 0, [scale, alpha]
     if name == "ald":                       # annealed_langevin_dynamics_corrector.py:21-41
-        std = sde.marginal_prob(None, t)[1] if isinstance(sde, VESDE) else torch.sqrt(
-            1.0 - torch.exp(2.0 * (-0.25 * t ** 2 * (sde.beta_1 - sde.beta_0) - 0.5 * t * sde.beta_0)))
+        std = sde.marginal_prob(None, t)[1] if isinstance(sde, VESDE) else _vp_log_mean_std(sde, t)[1]
         step = (snr * std) ** 2 * 2 * alpha
         return 1, [torch.ones_like(t), step * scale, torch.sqrt(step * 2)]
     raise NotImplementedError(f"corrector `{name}` has no native update (built: langevin, ald, none)")
@@ -439,15 +458,13 @@ class PredictorCorrectorSampler(torch.nn.Module):
         return builtin_p and builtin_c and isinstance(self.sde, (VPSDE, VESDE))
 
     def forward(self, model, shape: List[int], device, return_nfe: bool = True, use_tqdm: bool = True, noise=None):
-        if self.sde is None:
-            raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling forward()")
+        sde = _checked_sde(self.sde)
         R.require_cuda(device)
-        sde = self.sde
         ts = self.timesteps()
         sf = ScoreFunction(model, sde, self.continuous)
         unet, classes = R.resolve_model(model)
         n_corr = self.n_steps if _NATIVE_CORRECTORS.get(self.corrector) else 0
-        init_scale = float(sde.sigma_max) if isinstance(sde, VESDE) else 1.0
+        scale = init_scale(sde)
         if unet is not None and self._native_ok():
             key = (str(device), self.predictor, self.corrector, float(self.snr), sde.N, self.eps, bool(self.probability_flow))
             hit = self._cache.get(key)
@@ -463,7 +480,7 @@ class PredictorCorrectorSampler(torch.nn.Module):
             res = R.run_native_loop(unet, kind=L.LOOP_PC, shape=shape, device=device, times=labels, coef=coef, coef2=coef2,
                                     noise=noise, classes=classes, n_corr=n_corr, corr_kind=kind, snr=float(self.snr),
                                     denoise=self.denoise, seed=self.seed, traj_every=self.trajectory_every,
-                                    use_graph=self.use_cuda_graph, init_scale=init_scale)
+                                    use_graph=self.use_cuda_graph, init_scale=scale)
             final = res.aux if self.denoise else res.final
             imgs = R.to_image_list(final, res.traj)
         else:
@@ -472,7 +489,7 @@ class PredictorCorrectorSampler(torch.nn.Module):
             corr = (get_corrector(self.corrector) if self.corrector else NoneCorrector)(sde, sf, self.snr, self.n_steps)
             k = 0
             if noise is not None:
-                x = noise[0].to(device, torch.float32) * init_scale
+                x = noise[0].to(device, torch.float32) * scale
                 k = 1
             else:
                 x = sde.prior_sampling(shape).to(device)
@@ -499,6 +516,91 @@ class PredictorCorrectorSampler(torch.nn.Module):
 # ------------------------------------------------------------------------------------------------------
 
 
+def _check_solver_args(method, max_nfe, **scalars):
+    """Constructor arguments of the RK45 solvers: every scalar (rtol, atol, eps) finite, > 0 except atol (>= 0)."""
+    if method != "RK45":
+        raise NotImplementedError(f"method={method!r}: only the RK45 solver is built")
+    for name, v in scalars.items():
+        if isinstance(v, bool) or not isinstance(v, (int, float, np.floating, np.integer)):
+            raise ValueError(f"{name} must be a scalar number (per-component values are not supported), got {type(v).__name__}")
+        if not np.isfinite(v) or v < 0 or (name != "atol" and v == 0):
+            raise ValueError(f"{name} must be finite and {'>= 0' if name == 'atol' else '> 0'}, got {v}")
+    if isinstance(max_nfe, bool) or not isinstance(max_nfe, (int, np.integer)) or max_nfe < 2:
+        raise ValueError(f"max_nfe must be an integer >= 2, got {max_nfe!r}")
+
+
+def _check_ode_unet(unet, shape):
+    b, c, h, w = (int(v) for v in shape)
+    if c != unet.channels or h != w:
+        raise ValueError(f"shape {list(shape)} does not fit the U-Net ({unet.channels} channels, square images)")
+    if unet.out_dim != unet.channels:
+        raise ValueError("the probability-flow drift needs a U-Net whose output has as many channels as its input")
+
+
+# per solve: descriptor, work-size query, entry point, plan attribute of its buffers (one set per solve: each has its own graph
+# cache), how its errors name it and its end time
+_ODE_SOLVES = {
+    "sample": (L.OdeDesc, "dmn_ode_work_bytes", "dmn_ode_sample", "_ode_bufs", "probability-flow", "eps"),
+    "likelihood": (L.OdeLikelihoodDesc, "dmn_ode_likelihood_work_bytes", "dmn_ode_likelihood", "_lik_bufs", "likelihood", "T"),
+}
+
+
+def _ode_solve(solver, kind: str, unet, classes, x: torch.Tensor, t0: float, t1: float, noise: Optional[torch.Tensor] = None,
+               **fields) -> torch.Tensor:
+    """One adaptive RK45 solve of solver.sde's probability-flow ODE from t0 to t1 with this package's Unet, on x's device: the
+    "sample" solve integrates x, the "likelihood" solve [x ; delta_logp] from delta_logp = 0 with `noise` (optional, x's shape)
+    as its Hutchinson noise.  `fields` sets the remaining descriptor fields.  Records solver.last_stats and returns the final
+    state (flat, a copy); a solve stopped by max_nfe raises RuntimeError."""
+    desc_t, work_bytes, entry, bufs_name, what, end = _ODE_SOLVES[kind]
+    sde, lib, device = solver.sde, L.lib(), x.device
+    b, h, n = x.shape[0], x.shape[2], x.numel()
+    plan = unet.plan(h, b, device, time_rows=6)
+    with torch.cuda.device(device):
+        st = L.stream_ptr(device)
+        # buffers live with the plan so the addresses baked into the cached graph stay valid
+        bufs = plan.__dict__.setdefault(bufs_name, {})
+        if b not in bufs:
+            nbytes = int(getattr(lib, work_bytes)(plan.h, b))
+            bufs[b] = {"state": torch.empty(n + (b if kind == "likelihood" else 0), dtype=torch.float32, device=device),
+                       "work": torch.empty(nbytes + 256, dtype=torch.uint8, device=device),
+                       "result": torch.zeros(3, dtype=torch.float64, device=device)}
+        buf = bufs[b]
+        state, work, result = buf["state"], buf["work"], buf["result"]
+        state[:n].copy_(x.reshape(-1))
+        state[n:].zero_()
+        d = desc_t()
+        if classes is not None:
+            d.classes_dev = R.stable_copy(buf, "classes", classes.to(device, torch.int64).reshape(-1)).data_ptr()
+        if noise is not None:
+            d.noise_dev = R.stable_copy(buf, "noise", noise.to(device, torch.float32).reshape(-1)).data_ptr()
+        wp = (work.data_ptr() + 255) // 256 * 256
+        if isinstance(sde, VPSDE):
+            d.sde_kind, d.N, d.beta_0, d.beta_1 = L.SDE_VP, int(sde.N), float(sde.beta_0), float(sde.beta_1)
+        else:
+            d.sde_kind, d.N, d.sigma_min, d.sigma_max = L.SDE_VE, int(sde.N), float(sde.sigma_min), float(sde.sigma_max)
+        d.t0, d.t1, d.rtol, d.atol = t0, t1, solver.rtol, solver.atol
+        d.max_nfe, d.batch, d.use_graph = solver.max_nfe, b, int(bool(solver.use_cuda_graph))
+        for k, v in fields.items():
+            setattr(d, k, v)
+        d.state_dev, d.state_elems = state.data_ptr(), state.numel()
+        d.work_dev, d.work_bytes = wp, work.numel() - (wp - work.data_ptr())
+        d.result_dev = result.data_ptr()
+        L.check(getattr(lib, entry)(plan.h, C.byref(d), st), entry)
+        plan.time_rows_key = None            # the solve rewrote rows 0..5 of the time table
+        raw = result.cpu().numpy().tobytes()
+        out = state.clone()
+    res = L.OdeResult.from_buffer_copy(raw)
+    solver.last_stats = {"status": int(res.status), "nfev": int(res.nfev), "n_accepted": int(res.n_accepted),
+                         "n_rejected": int(res.n_rejected), "t_final": float(res.t_final)}
+    if res.status == L.ODE_LIMIT:
+        raise RuntimeError(f"{what} ODE: stopped at {res.nfev} model evaluations (max_nfe={solver.max_nfe}) at "
+                           f"t={res.t_final:.6g}, before reaching {end}={t1:g}")
+    if res.status == L.ODE_TOO_SMALL_STEP:
+        warnings.warn(f"{what} ODE: required step size became too small at t={res.t_final:.6g} (scipy status -1); "
+                      "returning the last accepted state, as solve_ivp does")
+    return out
+
+
 class ProbabilityFlowSampler(torch.nn.Module):
     """Deterministic sampler of a score-SDE model: integrates the probability-flow ODE dx/dt = f(x,t) - 0.5 g(t)^2 score(x,t) from
     sde.T down to eps with scipy's adaptive RK45 rules (solve_ivp(..., method='RK45')), entirely on the GPU: every model
@@ -513,15 +615,7 @@ class ProbabilityFlowSampler(torch.nn.Module):
     def __init__(self, denoise: bool = False, rtol: float = 1e-5, atol: float = 1e-5, method: str = "RK45", eps: float = None,
                  max_nfe: int = 100_000):
         super().__init__()
-        if method != "RK45":
-            raise NotImplementedError(f"method={method!r}: only the RK45 solver is built")
-        for name, v in (("rtol", rtol), ("atol", atol)):
-            if isinstance(v, bool) or not isinstance(v, (int, float, np.floating, np.integer)):
-                raise ValueError(f"{name} must be a scalar number (per-component tolerances are not supported), got {type(v).__name__}")
-            if not np.isfinite(v) or v < 0 or (name == "rtol" and v == 0):
-                raise ValueError(f"{name} must be finite and {'> 0' if name == 'rtol' else '>= 0'}, got {v}")
-        if isinstance(max_nfe, bool) or not isinstance(max_nfe, (int, np.integer)) or max_nfe < 2:
-            raise ValueError(f"max_nfe must be an integer >= 2, got {max_nfe!r}")
+        _check_solver_args(method, max_nfe, rtol=rtol, atol=atol)
         self.denoise, self.rtol, self.atol, self.method, self.eps = denoise, float(rtol), float(atol), method, eps
         self.max_nfe = int(max_nfe)
         self.sde: Optional[SDE] = None
@@ -532,11 +626,7 @@ class ProbabilityFlowSampler(torch.nn.Module):
         self.sde = sde
 
     def forward(self, model, shape: List[int], device, return_nfe: bool = True, use_tqdm: bool = True, noise=None):
-        if self.sde is None:
-            raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling forward()")
-        sde = self.sde
-        if not isinstance(sde, (VPSDE, VESDE)):
-            raise NotImplementedError(f"SDE class {sde.__class__.__name__} not yet supported.")
+        sde = _checked_sde(self.sde)
         R.require_cuda(device)
         device = torch.device(device)
         unet, classes = R.resolve_model(model)
@@ -544,62 +634,18 @@ class ProbabilityFlowSampler(torch.nn.Module):
             raise NotImplementedError("ProbabilityFlowSampler runs this package's Unet natively; other model callables have no "
                                       "host solver path")
         b, c, h, w = (int(v) for v in shape)
-        if c != unet.channels or h != w:
-            raise ValueError(f"shape {list(shape)} does not fit the U-Net ({unet.channels} channels, square images)")
-        if unet.out_dim != unet.channels:
-            raise ValueError("the probability-flow drift needs a U-Net whose output has as many channels as its input")
+        _check_ode_unet(unet, shape)
         eps = sde.sampling_epsilon if self.eps is None else float(self.eps)
-        init_scale = float(sde.sigma_max) if isinstance(sde, VESDE) else 1.0
-        x = noise[0] * init_scale if noise is not None else sde.prior_sampling(shape)
+        x = noise[0] * init_scale(sde) if noise is not None else sde.prior_sampling(shape)
         if tuple(x.shape) != (b, c, h, w):
             raise ValueError(f"x_T has shape {tuple(x.shape)}; expected {(b, c, h, w)}")
-        lib = L.lib()
-        plan = unet.plan(h, b, device, time_rows=6)
-        with torch.cuda.device(device):
-            st = L.stream_ptr(device)
-            # buffers live with the plan so the addresses baked into the cached graph stay valid
-            bufs = plan.__dict__.setdefault("_ode_bufs", {})
-            if b not in bufs:
-                nbytes = int(lib.dmn_ode_work_bytes(plan.h, b))
-                bufs[b] = {"state": torch.empty((b, c, h, w), dtype=torch.float32, device=device),
-                           "work": torch.empty(nbytes + 256, dtype=torch.uint8, device=device),
-                           "result": torch.zeros(3, dtype=torch.float64, device=device)}
-            buf = bufs[b]
-            state, work, result = buf["state"], buf["work"], buf["result"]
-            state.copy_(x.to(device, torch.float32))
-            if classes is not None:
-                classes = R.stable_copy(buf, "classes", classes.to(device, torch.int64).reshape(-1))
-            wp = (work.data_ptr() + 255) // 256 * 256
-            d = L.OdeDesc()
-            if isinstance(sde, VPSDE):
-                d.sde_kind, d.N, d.beta_0, d.beta_1 = L.SDE_VP, int(sde.N), float(sde.beta_0), float(sde.beta_1)
-            else:
-                d.sde_kind, d.N, d.sigma_min, d.sigma_max = L.SDE_VE, int(sde.N), float(sde.sigma_min), float(sde.sigma_max)
-            d.t0, d.t1, d.rtol, d.atol = float(sde.T), eps, self.rtol, self.atol
-            d.max_nfe, d.batch, d.use_graph = self.max_nfe, b, int(bool(self.use_cuda_graph))
-            d.classes_dev = classes.data_ptr() if classes is not None else None
-            d.state_dev, d.state_elems = state.data_ptr(), state.numel()
-            d.work_dev, d.work_bytes = wp, work.numel() - (wp - work.data_ptr())
-            d.result_dev = result.data_ptr()
-            L.check(lib.dmn_ode_sample(plan.h, C.byref(d), st), "dmn_ode_sample")
-            plan.time_rows_key = None            # the solve rewrote rows 0..5 of the time table
-            raw = result.cpu().numpy().tobytes()
-            x = state.clone()
-        res = L.OdeResult.from_buffer_copy(raw)
-        self.last_stats = {"status": int(res.status), "nfev": int(res.nfev), "n_accepted": int(res.n_accepted),
-                           "n_rejected": int(res.n_rejected), "t_final": float(res.t_final)}
-        if res.status == L.ODE_LIMIT:
-            raise RuntimeError(f"probability-flow ODE: stopped at {res.nfev} model evaluations (max_nfe={self.max_nfe}) at "
-                               f"t={res.t_final:.6g}, before reaching eps={eps:g}")
-        if res.status == L.ODE_TOO_SMALL_STEP:
-            warnings.warn(f"probability-flow ODE: required step size became too small at t={res.t_final:.6g} (scipy status -1); "
-                          "returning the last accepted state, as solve_ivp does")
+        x = _ode_solve(self, "sample", unet, classes, x.to(device, torch.float32), float(sde.T), eps).view(b, c, h, w)
         if self.denoise:      # one reverse-diffusion predictor step at eps, probability_flow=False, keeping x_mean
             vec_eps = torch.ones(b, device=device) * eps
             pred = ReverseDiffusionPredictor(sde, ScoreFunction(model, sde), probability_flow=False)
             _, x = pred.update_fn(x, vec_eps)
         imgs = R.to_image_list(x.float().contiguous(), None)
-        return (imgs, int(res.nfev)) if return_nfe else imgs
+        return (imgs, self.last_stats["nfev"]) if return_nfe else imgs
 
     def sample(self, model, shape: List[int], device=None, return_nfe: bool = False, noise=None):
         if device is None:
@@ -624,15 +670,7 @@ class LikelihoodEstimate(torch.nn.Module):
         super().__init__()
         if hutchinson_type not in ("Rademacher", "Gaussian"):
             raise NotImplementedError(f"Hutchinson type {hutchinson_type} unknown.")
-        if method != "RK45":
-            raise NotImplementedError(f"method={method!r}: only the RK45 solver is built")
-        for name, v in (("rtol", rtol), ("atol", atol), ("eps", eps)):
-            if isinstance(v, bool) or not isinstance(v, (int, float, np.floating, np.integer)):
-                raise ValueError(f"{name} must be a scalar number, got {type(v).__name__}")
-            if not np.isfinite(v) or v < 0 or (name != "atol" and v == 0):
-                raise ValueError(f"{name} must be finite and {'>= 0' if name == 'atol' else '> 0'}, got {v}")
-        if isinstance(max_nfe, bool) or not isinstance(max_nfe, (int, np.integer)) or max_nfe < 2:
-            raise ValueError(f"max_nfe must be an integer >= 2, got {max_nfe!r}")
+        _check_solver_args(method, max_nfe, rtol=rtol, atol=atol, eps=eps)
         self.hutchinson_type, self.rtol, self.atol, self.method = hutchinson_type, float(rtol), float(atol), method
         self.eps, self.max_nfe = float(eps), int(max_nfe)
         self.sde: Optional[SDE] = None
@@ -644,11 +682,7 @@ class LikelihoodEstimate(torch.nn.Module):
         self.sde = sde
 
     def likelihood(self, model, data: torch.Tensor, noise: Optional[torch.Tensor] = None):
-        if self.sde is None:
-            raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling likelihood()")
-        sde = self.sde
-        if not isinstance(sde, (VPSDE, VESDE)):
-            raise NotImplementedError(f"SDE class {sde.__class__.__name__} not yet supported.")
+        sde = _checked_sde(self.sde, "likelihood()")
         unet, classes = R.resolve_model(model)
         if unet is None or unet._film:
             raise NotImplementedError("LikelihoodEstimate runs this package's Unet natively (its forward-mode JVP); other model "
@@ -658,65 +692,18 @@ class LikelihoodEstimate(torch.nn.Module):
         if data.dim() != 4:
             raise ValueError(f"data must be [B, C, H, W], got shape {tuple(data.shape)}")
         b, c, h, w = (int(v) for v in data.shape)
-        if c != unet.channels or h != w:
-            raise ValueError(f"data shape {tuple(data.shape)} does not fit the U-Net ({unet.channels} channels, square images)")
-        if unet.out_dim != unet.channels:
-            raise ValueError("the probability-flow drift needs a U-Net whose output has as many channels as its input")
+        _check_ode_unet(unet, data.shape)
         if noise is not None and tuple(noise.shape) != tuple(data.shape):
             raise ValueError(f"noise has shape {tuple(noise.shape)}; expected {tuple(data.shape)}")
-        device = data.device
-        R.require_cuda(device)
-        lib = L.lib()
-        plan = unet.plan(h, b, device, time_rows=6)
+        R.require_cuda(data.device)
+        # the state is [x ; delta_logp]: delta_logp starts at 0
+        state = _ode_solve(self, "likelihood", unet, classes, data.to(torch.float32), self.eps, float(sde.T), noise=noise,
+                           hutchinson=L.HUTCH_RADEMACHER if self.hutchinson_type == "Rademacher" else L.HUTCH_GAUSSIAN,
+                           rng=L.Rng(self.seed if self.seed is not None else R.draw_seed(), R.rank_stream_id()))
         n = b * c * h * w
-        with torch.cuda.device(device):
-            st = L.stream_ptr(device)
-            # buffers live with the plan so the addresses baked into the cached graph stay valid
-            bufs = plan.__dict__.setdefault("_lik_bufs", {})
-            if b not in bufs:
-                nbytes = int(lib.dmn_ode_likelihood_work_bytes(plan.h, b))
-                bufs[b] = {"state": torch.empty(n + b, dtype=torch.float32, device=device),
-                           "work": torch.empty(nbytes + 256, dtype=torch.uint8, device=device),
-                           "result": torch.zeros(3, dtype=torch.float64, device=device)}
-            buf = bufs[b]
-            state, work, result = buf["state"], buf["work"], buf["result"]
-            state[:n].copy_(data.reshape(-1).to(torch.float32))
-            state[n:].zero_()
-            if classes is not None:
-                classes = R.stable_copy(buf, "classes", classes.to(device, torch.int64).reshape(-1))
-            if noise is not None:
-                noise = R.stable_copy(buf, "noise", noise.to(device, torch.float32).reshape(-1))
-            wp = (work.data_ptr() + 255) // 256 * 256
-            d = L.OdeLikelihoodDesc()
-            if isinstance(sde, VPSDE):
-                d.sde_kind, d.N, d.beta_0, d.beta_1 = L.SDE_VP, int(sde.N), float(sde.beta_0), float(sde.beta_1)
-            else:
-                d.sde_kind, d.N, d.sigma_min, d.sigma_max = L.SDE_VE, int(sde.N), float(sde.sigma_min), float(sde.sigma_max)
-            d.t0, d.t1, d.rtol, d.atol = self.eps, float(sde.T), self.rtol, self.atol
-            d.max_nfe, d.batch, d.use_graph = self.max_nfe, b, int(bool(self.use_cuda_graph))
-            d.hutchinson = L.HUTCH_RADEMACHER if self.hutchinson_type == "Rademacher" else L.HUTCH_GAUSSIAN
-            d.rng = L.Rng(self.seed if self.seed is not None else R.draw_seed(), R.rank_stream_id())
-            d.noise_dev = noise.data_ptr() if noise is not None else None
-            d.classes_dev = classes.data_ptr() if classes is not None else None
-            d.state_dev, d.state_elems = state.data_ptr(), state.numel()
-            d.work_dev, d.work_bytes = wp, work.numel() - (wp - work.data_ptr())
-            d.result_dev = result.data_ptr()
-            L.check(lib.dmn_ode_likelihood(plan.h, C.byref(d), st), "dmn_ode_likelihood")
-            plan.time_rows_key = None            # the solve rewrote rows 0..5 of the time table
-            raw = result.cpu().numpy().tobytes()
-            z = state[:n].reshape(b, c, h, w).clone()
-            delta_logp = state[n:].clone()
-        res = L.OdeResult.from_buffer_copy(raw)
-        self.last_stats = {"status": int(res.status), "nfev": int(res.nfev), "n_accepted": int(res.n_accepted),
-                           "n_rejected": int(res.n_rejected), "t_final": float(res.t_final)}
-        if res.status == L.ODE_LIMIT:
-            raise RuntimeError(f"likelihood ODE: stopped at {res.nfev} model evaluations (max_nfe={self.max_nfe}) at "
-                               f"t={res.t_final:.6g}, before reaching T={float(sde.T):g}")
-        if res.status == L.ODE_TOO_SMALL_STEP:
-            warnings.warn(f"likelihood ODE: required step size became too small at t={res.t_final:.6g} (scipy status -1); "
-                          "returning the last accepted state, as solve_ivp does")
+        z, delta_logp = state[:n].view(b, c, h, w), state[n:]
         bpd = likelihood_bpd(sde, z, delta_logp)
-        return bpd, z, int(res.nfev)
+        return bpd, z, self.last_stats["nfev"]
 
 
 def likelihood_bpd(sde: SDE, z: torch.Tensor, delta_logp: torch.Tensor) -> torch.Tensor:
@@ -820,16 +807,9 @@ class DPMSolverSampler(torch.nn.Module):
         self.sde = sde
         self._cache = {}
 
-    def _check_sde(self):
-        if self.sde is None:
-            raise ValueError("Must explicitly set `update_sde(sde)` for this module prior to calling forward()")
-        if not isinstance(self.sde, (VPSDE, VESDE)):
-            raise NotImplementedError(f"SDE class {self.sde.__class__.__name__} not yet supported.")
-        return self.sde
-
     def timesteps(self) -> List[float]:
         """The fp64 grid: steps + 1 times from sde.T to eps."""
-        sde = self._check_sde()
+        sde = _checked_sde(self.sde)
         return score_sde_grid(sde, self.steps, sde.sampling_epsilon if self.eps is None else self.eps, self.skip_type)
 
     def step_orders(self) -> List[int]:
@@ -841,7 +821,7 @@ class DPMSolverSampler(torch.nn.Module):
         """(coef [steps][8], coef2 [steps][8] or None, labels [steps]) as CPU fp32: the kernel rows of dmn_dpmpp_step (mode 2:
         unclamped data prediction) / dmn_dpmpp_sde_step expanded in fp64 and rounded once, and the U-Net labels
         ScoreFunction.labels of the fp32 grid."""
-        sde = self._check_sde()
+        sde = _checked_sde(self.sde)
         ts = self.timesteps()
         alpha, sigma, lam = zip(*(score_sde_schedule(sde, t) for t in ts))
         orders = self.step_orders()
@@ -865,15 +845,14 @@ class DPMSolverSampler(torch.nn.Module):
         return torch.tensor(rows, dtype=torch.float64).to(torch.float32), coef2, labels.to(torch.float32)
 
     def forward(self, model, shape: List[int], device, return_nfe: bool = True, use_tqdm: bool = True, noise=None):
-        sde = self._check_sde()
+        sde = _checked_sde(self.sde)
         R.require_cuda(device)
         device = torch.device(device)
         if len(shape) != 4:
             raise ValueError(f"shape must be [B, C, H, W], got {list(shape)}")
         b, c, h, w = (int(v) for v in shape)
-        stochastic = self.algorithm_type == "sde-dpmsolver++"
         if noise is not None:
-            need = 1 + (self.steps if stochastic else 0)
+            need = 1 + (self.steps if self.algorithm_type == "sde-dpmsolver++" else 0)
             if noise.dim() != 5 or tuple(noise.shape[1:]) != (b, c, h, w) or noise.shape[0] < need:
                 raise ValueError(f"noise has shape {tuple(noise.shape)}; expected [n >= {need}, {b}, {c}, {h}, {w}]")
         key = str(device)
@@ -883,52 +862,15 @@ class DPMSolverSampler(torch.nn.Module):
             hit = (coef.to(device), None if coef2 is None else coef2.to(device), labels.to(device))
             self._cache[key] = hit
         coef, coef2, labels = hit
-        init_scale = float(sde.sigma_max) if isinstance(sde, VESDE) else 1.0
-        unet, classes = R.resolve_model(model)
+        unet, _ = R.resolve_model(model)
         if unet is not None:
             if c != unet.channels or h != w:
                 raise ValueError(f"shape {list(shape)} does not fit the U-Net ({unet.channels} channels, square images)")
             if unet.out_dim != unet.channels:
                 raise ValueError("the score-SDE data prediction needs a U-Net whose output has as many channels as its input")
-            guided = self.guidance_scale is not None and classes is not None
-            res = R.run_native_loop(unet, kind=L.LOOP_DPMPP, shape=shape, device=device, times=labels, coef=coef, coef2=coef2,
-                                    noise=noise, classes=classes, seed=self.seed, traj_every=self.trajectory_every,
-                                    use_graph=self.use_cuda_graph, init_scale=init_scale,
-                                    cfg_scale=float(self.guidance_scale) if guided else None)
-            imgs = R.to_image_list(res.final, res.traj)
-        else:
-            # foreign model: call it per step, the update is the native kernel with a local history ring
-            if self.guidance_scale is not None:
-                raise NotImplementedError("guidance_scale needs this package's class-conditional Unet (doubled-batch native loop)")
-            lib = L.lib()
-            with torch.cuda.device(device):
-                st = L.stream_ptr(device)
-                rng = L.Rng(self.seed if self.seed is not None else R.draw_seed(), R.rank_stream_id())
-                x = torch.empty((b, c, h, w), dtype=torch.float32, device=device)
-                if noise is not None:
-                    x.copy_(noise[0])
-                else:
-                    L.check(lib.dmn_randn(L.ptr(x), x.numel(), rng, -1, st), "dmn_randn")
-                if init_scale != 1.0:
-                    x.mul_(init_scale)
-                ring = torch.empty((3, b, c, h, w), dtype=torch.float32, device=device)
-                chw = x[0].numel()
-                keep = []
-                for s in range(self.steps):
-                    mo = model(x, labels[s].repeat(b)).float().contiguous()
-                    if tuple(mo.shape) != (b, c, h, w):
-                        raise ValueError(f"model output has shape {tuple(mo.shape)}; expected {(b, c, h, w)}")
-                    if stochastic:
-                        z = None if noise is None else noise[1 + s].to(device, torch.float32).contiguous()
-                        L.check(lib.dmn_dpmpp_sde_step(L.ptr(x), L.ptr(mo), L.ptr(z), L.ptr(ring), L.ptr(x), b, chw, chw, L.ptr(coef),
-                                                       L.ptr(coef2), None, s, rng, st), "dmn_dpmpp_sde_step")
-                    else:
-                        L.check(lib.dmn_dpmpp_step(L.ptr(x), L.ptr(mo), L.ptr(ring), L.ptr(x), b, chw, chw, L.ptr(coef), None, s, st),
-                                "dmn_dpmpp_step")
-                    if self.trajectory_every and (s + 1) % self.trajectory_every == 0:
-                        keep.append(x.clone())
-                traj = torch.stack(keep) if keep else None
-            imgs = R.to_image_list(x, traj)
+        imgs = R.run_loop(model, kind=L.LOOP_DPMPP, shape=shape, device=device, times=labels, coef=coef, coef2=coef2, noise=noise,
+                          seed=self.seed, traj_every=self.trajectory_every, use_graph=self.use_cuda_graph, init_scale=init_scale(sde),
+                          guidance_scale=self.guidance_scale, model_arg=lambda s: labels[s].repeat(b))
         return (imgs, self.steps) if return_nfe else imgs
 
     def sample(self, model, shape: List[int], device=None, return_nfe: bool = False, noise=None):
