@@ -1041,6 +1041,233 @@ __global__ void __launch_bounds__(kThreads, 1) attn_softmax_fused_kernel(const _
 
 constexpr size_t kSmemSoftmax = 1024 + (size_t)(kXS + kWS) * kSlab + 3 * (size_t)kOpBytes + (128 + 256) * 4 + (S_COUNT + 2) * 8 + 64;
 
+// =====================================================================================================================
+// softmax Attention core for bottlenecks of more than 64 tokens (16x16 maps at 128x128 images): flash attention on the tensor cores
+//   o[b][i][(h,e)] = sum_j softmax_j(scale * q_i . k_j) v_j[e]      (reference parts/mha.py:18-29, between to_qkv and to_out)
+// qkv bf16 [B][N][384] (channel = which * 128 + head * 32 + d, as to_qkv writes it), o bf16 [B][N][128].
+// One CTA per work item (image, 128-query tile, head); work items of an image are adjacent, so its k / v tiles are read from L2.
+// The rank-3 tensor map [B][N][384] gives each image its own bounds: rows past N arrive as zeros and never come from the next
+// image.  Per 128-key tile j (ring of kFlStages tiles brought by TMA, 128 rows x 32 channels, SWIZZLE_64B):
+//   MMA       S = q k_j^T                       M128 x N128 x K32 (two k16 steps), fp32 in TMEM columns [0, 128)
+//   epilogue  lane = query row: running max m and sum l in the log2 domain; padded key columns (j*128 + c >= N) get zero weight;
+//             when m moves, the O accumulator row is rescaled in TMEM; P = bf16(ex2(s * scale * log2 e - m)) -> shared memory
+//             (UMMA K-major no-swizzle layout), l sums the ROUNDED P so numerator and denominator agree; v_j is transposed into
+//             the K-major B operand v^T [32 e][128 keys]
+//   MMA       O += P v_j                        M128 x N32 x K128 (eight k16 steps), fp32 in TMEM columns [128, 160)
+// Finally o = O / l, stored as bf16 for the tile's real query rows only.
+// Warp roles (192 threads): warps 0-3 epilogue (warp w reads TMEM lanes [32w, 32w + 32)), warp 4 TMA, warp 5 TMEM + MMA issuer.
+// 256 TMEM columns and ~98 KB of shared memory per CTA: two CTAs per SM overlap one's softmax with the other's products.
+// =====================================================================================================================
+constexpr int kFlThreads = 192, kFlTmaWarp = 4, kFlMmaWarp = 5, kFlStages = 3;
+constexpr uint32_t kFlTile = 128u * 64u;                 // 128 tokens x 32 channels bf16 (64-byte rows, SWIZZLE_64B)
+constexpr uint32_t kFlVtLbo = 32u * 16u;                 // v^T operand [16 k-chunks][32 rows][16 B]: k-chunk stride
+enum { F_FULLQ = 0, F_FULL, F_EMPTY = F_FULL + kFlStages, F_S = F_EMPTY + kFlStages, F_P, F_O, F_COUNT };
+
+struct FlashP {
+  CUtensorMap m;                 // qkv as [B][N][384], box 32 channels x 128 tokens x 1 image
+  bf16* o;
+  int N, QT;                     // tokens per image, 128-token tiles per image
+};
+
+// rank-3 bf16 map [d2][d1][d0], box = 32 x 128 x 1, 64-byte swizzle; out-of-range rows read as zero
+static int make_map3_sw64(CUtensorMap* m, const void* base, uint64_t d0, uint64_t d1, uint64_t d2) {
+  EncodeTiledFn fn = encode_fn();
+  if (!fn) return fail(-3, "cuTensorMapEncodeTiled is not available from this driver");
+  cuuint64_t dims[3] = {d0, d1, d2};
+  cuuint64_t strides[2] = {d0 * 2, d0 * d1 * 2};
+  cuuint32_t box[3] = {32, 128, 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  const CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(-3, "cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
+  return 0;
+}
+__device__ __forceinline__ void tma_load3(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, uint32_t bar) {
+  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+               ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
+               : "memory");
+}
+// K-major SWIZZLE_64B descriptor: rows of 64 B, 8-row groups 512 B apart (SBO), LBO unused (1), layout type 4 (as the conv engine)
+__device__ __forceinline__ uint64_t make_desc_sw64(uint32_t saddr) {
+  return (uint64_t)((saddr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(512u >> 4) << 32) | (1ull << 46) | (4ull << 61);
+}
+
+__global__ void __launch_bounds__(kFlThreads, 2) attn_flash_kernel(const __grid_constant__ FlashP p) {
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  const uint32_t base0 = smem_u32(smem_raw);
+  uint8_t* smem = smem_raw + ((1024u - (base0 & 1023u)) & 1023u);
+  uint8_t* s_q = smem;                                   // q tile
+  uint8_t* s_k = s_q + kFlTile;                          // kFlStages k tiles
+  uint8_t* s_v = s_k + kFlStages * kFlTile;              // kFlStages v tiles (token-major, as TMA brings them)
+  uint8_t* s_vt = s_v + kFlStages * kFlTile;             // v^T: B operand of the P v product
+  uint8_t* s_p = s_vt + kFlTile;                         // P: A operand of the P v product (kOpBytes)
+  uint64_t* bars = reinterpret_cast<uint64_t*>(s_p + kOpBytes);
+  uint32_t* tslot = reinterpret_cast<uint32_t*>(bars + F_COUNT);
+
+  pdl_trigger();
+  pdl_wait();
+  const int tid = threadIdx.x;
+  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0), lane = tid & 31;
+  const int N = p.N, T = p.QT;
+  const int h = blockIdx.x & 3, qt = (blockIdx.x >> 2) % T, b = (blockIdx.x >> 2) / T;
+  const int q0 = qt * 128;
+  auto bar = [&](int i) { return smem_u32(&bars[i]); };
+
+  if (warp == kFlTmaWarp) {
+    if (lane < F_COUNT) mbar_init(bar(lane), lane == F_P ? 128u : 1u);
+    fence_barrier_init();
+  }
+  if (warp == kFlMmaWarp) tmem_alloc(smem_u32(tslot), 256);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *tslot;
+  const uint32_t tS = tmem, tO = tmem + 128;
+
+  if (warp == kFlTmaWarp) {
+    // =============================================== TMA ===============================================
+    const bool leader = elect_one();
+    if (leader) {
+      mbar_arrive_expect_tx(bar(F_FULLQ), kFlTile);
+      tma_load3(smem_u32(s_q), &p.m, h * 32, q0, b, bar(F_FULLQ));
+    }
+    __syncwarp();
+    for (int j = 0; j < T; ++j) {
+      const int st = j % kFlStages;
+      mbar_wait_relaxed(bar(F_EMPTY + st), ((j / kFlStages) & 1) ^ 1);
+      if (leader) {
+        mbar_arrive_expect_tx(bar(F_FULL + st), 2 * kFlTile);
+        tma_load3(smem_u32(s_k) + st * kFlTile, &p.m, 128 + h * 32, j * 128, b, bar(F_FULL + st));
+        tma_load3(smem_u32(s_v) + st * kFlTile, &p.m, 256 + h * 32, j * 128, b, bar(F_FULL + st));
+      }
+      __syncwarp();
+    }
+  } else if (warp == kFlMmaWarp) {
+    // =============================================== MMA issuer ===============================================
+    const bool leader = elect_one();
+    const uint32_t idescS = make_idesc(128, 128), idescO = make_idesc(128, 32);
+    const uint32_t sq = smem_u32(s_q), sp = smem_u32(s_p), svt = smem_u32(s_vt);
+    mbar_wait(bar(F_FULLQ), 0);
+    for (int j = 0; j < T; ++j) {
+      const int st = j % kFlStages;
+      mbar_wait(bar(F_FULL + st), (j / kFlStages) & 1);   // (S of the previous tile was read out before its F_P arrival)
+      tc_fence_after();
+      const uint32_t sk = smem_u32(s_k) + st * kFlTile;
+      if (leader) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) umma_bf16(tS, make_desc_sw64(sq + k * 32), make_desc_sw64(sk + k * 32), idescS, k ? 1u : 0u);
+        umma_commit(bar(F_S));
+      }
+      __syncwarp();
+      mbar_wait(bar(F_P), j & 1);
+      tc_fence_after();
+      if (leader) {
+#pragma unroll
+        for (int k = 0; k < 8; ++k)
+          umma_bf16(tO, make_desc(sp + k * kOpK16, kOpLbo, kOpSbo), make_desc(svt + k * 2 * kFlVtLbo, kFlVtLbo, kOpSbo), idescO,
+                    (j | k) ? 1u : 0u);
+        umma_commit(bar(F_O));                 // P, v^T and the accumulator are free again once these retire
+        umma_commit(bar(F_EMPTY + st));
+      }
+      __syncwarp();
+    }
+  } else {
+    // =============================================== epilogue: online softmax ===============================================
+    const int row = warp * 32 + lane;                      // query row of the tile = TMEM lane
+    const uint32_t lane_base = (uint32_t)(warp * 32) << 16;
+    const float c2 = rsqrtf(32.f) * kLog2e;                // scale, in the log2 domain
+    const uint32_t sp = smem_u32(s_p), svt = smem_u32(s_vt);
+    float m_run = -INFINITY, l_run = 0.f;
+    uint32_t r[32];
+    for (int j = 0; j < T; ++j) {
+      const int nvalid = N - j * 128;                      // key columns >= nvalid are padding
+      mbar_wait_relaxed(bar(F_S), j & 1);
+      tc_fence_after();
+      float tmax = -INFINITY;
+#pragma unroll
+      for (int c0 = 0; c0 < 128; c0 += 32) {
+        tmem_ld32(tS + lane_base + c0, r);
+#pragma unroll
+        for (int i = 0; i < 32; ++i)
+          if (c0 + i < nvalid) tmax = fmaxf(tmax, __uint_as_float(r[i]));
+      }
+      const float m_new = fmaxf(m_run, tmax * c2);
+      const float corr = ex2(m_run - m_new);              // 0 on the first tile (m_run = -inf)
+      if (j > 0) {                                         // the previous P v product has retired: P, v^T and O may be touched
+        mbar_wait_relaxed(bar(F_O), (j - 1) & 1);
+        tc_fence_after();
+        if (__any_sync(0xffffffffu, corr != 1.f)) {
+          tmem_ld32(tO + lane_base, r);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) r[i] = __float_as_uint(__uint_as_float(r[i]) * corr);
+          tmem_st32(tO + lane_base, r);
+          tmem_st_wait();
+        }
+      }
+      float psum = 0.f;
+#pragma unroll
+      for (int c0 = 0; c0 < 128; c0 += 32) {
+        tmem_ld32(tS + lane_base + c0, r);
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+          uint32_t w[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const int i0 = g * 8 + 2 * e;
+            const bf16 p0 = __float2bfloat16_rn(c0 + i0 < nvalid ? ex2(fmaf(__uint_as_float(r[i0]), c2, -m_new)) : 0.f);
+            const bf16 p1 = __float2bfloat16_rn(c0 + i0 + 1 < nvalid ? ex2(fmaf(__uint_as_float(r[i0 + 1]), c2, -m_new)) : 0.f);
+            psum += __bfloat162float(p0) + __bfloat162float(p1);
+            w[e] = (uint32_t)(*reinterpret_cast<const unsigned short*>(&p0)) | ((uint32_t)(*reinterpret_cast<const unsigned short*>(&p1)) << 16);
+          }
+          sts128(sp + (uint32_t)((((c0 >> 3) + g) * 128 + row) * 16), make_uint4(w[0], w[1], w[2], w[3]));
+        }
+      }
+      l_run = l_run * corr + psum;
+      m_run = m_new;
+      // v^T: this thread's key row (SWIZZLE_64B: logical 16-byte chunk c of row t sits at chunk c ^ ((t >> 1) & 3))
+      const int st = j % kFlStages;
+      mbar_wait_relaxed(bar(F_FULL + st), (j / kFlStages) & 1);
+      const uint32_t vrow = smem_u32(s_v) + st * kFlTile + (uint32_t)row * 64u;
+      const uint32_t vdst = svt + (uint32_t)(row >> 3) * kFlVtLbo + (uint32_t)(row & 7) * 2u;
+#pragma unroll
+      for (int c = 0; c < 4; ++c) {
+        const uint4 v = lds128(vrow + (uint32_t)((c ^ ((row >> 1) & 3)) * 16));
+        const uint32_t u[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          sts16(vdst + (uint32_t)(c * 8 + 2 * e) * 16u, (unsigned short)(u[e] & 0xffffu));
+          sts16(vdst + (uint32_t)(c * 8 + 2 * e + 1) * 16u, (unsigned short)(u[e] >> 16));
+        }
+      }
+      fence_proxy_async();
+      tc_fence_before();
+      mbar_arrive(bar(F_P));
+    }
+    mbar_wait_relaxed(bar(F_O), (T - 1) & 1);
+    tc_fence_after();
+    tmem_ld32(tO + lane_base, r);
+    if (q0 + row < N) {
+      const float inv = 1.f / l_run;
+      bf16* dst = p.o + ((long)b * N + q0 + row) * 128 + h * 32;
+#pragma unroll
+      for (int g = 0; g < 4; ++g) {
+        float y[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) y[e] = __uint_as_float(r[g * 8 + e]) * inv;
+        *reinterpret_cast<uint4*>(dst + g * 8) = pack8(y);
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == kFlMmaWarp) {
+    tc_fence_after();
+    tmem_dealloc(tmem, 256);
+  }
+}
+
+constexpr size_t kSmemFlash = 1024 + (size_t)(2 + 2 * kFlStages) * kFlTile + kOpBytes + (F_COUNT + 2) * 8 + 64;
+
 }  // namespace fa
 
 bool linattn_fused_supported(int B, int N, int C) {
@@ -1102,6 +1329,26 @@ int attn_softmax_fused(const LinAttnFusedP& q, cudaStream_t st) {
   DMN_CUDA_CHECK(launch_pdl(fa::attn_softmax_fused_kernel, dim3(grid), dim3(fa::kThreads), fa::kSmemSoftmax, st, p));
   count_launch();
   DMN_LAUNCH_CHECK("attn_softmax_fused");
+  return 0;
+}
+
+int attn_flash(const void* qkv, void* out, int B, int heads, int N, cudaStream_t st) {
+  DMN_REQUIRE(heads == 4, "attn_flash: heads must be 4 (384 qkv channels)");
+  DMN_REQUIRE(B >= 1 && N > 64, "attn_flash: needs more than 64 tokens");
+  fa::FlashP p;
+  memset(&p, 0, sizeof(p));
+  int rc;
+  if ((rc = fa::make_map3_sw64(&p.m, qkv, 384, (uint64_t)N, (uint64_t)B))) return rc;
+  p.o = (bf16*)out;
+  p.N = N;
+  p.QT = (N + 127) / 128;
+  const long grid = (long)B * p.QT * 4;
+  DMN_REQUIRE(grid < (1L << 31), "attn_flash: too many work items");
+  static DeviceOnce attr;
+  if (attr.first()) DMN_CUDA_CHECK(cudaFuncSetAttribute(fa::attn_flash_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fa::kSmemFlash));
+  DMN_CUDA_CHECK(launch_pdl(fa::attn_flash_kernel, dim3((unsigned)grid), dim3(fa::kFlThreads), fa::kSmemFlash, st, p));
+  count_launch();
+  DMN_LAUNCH_CHECK("attn_flash");
   return 0;
 }
 

@@ -685,58 +685,73 @@ int linattn_core(const void* qkv, void* out, int B, int heads, int dh, int N, in
 
 // =====================================================================================================
 // softmax Attention core (parts/mha.py:16-29), dim_head = 32.  One block per (sample, head), thread per query.
+// k / v stream through shared memory in chunks of at most kAttnChunk tokens; each query still visits the keys in order j = 0..N-1
+// with the same fmaf / __expf chain, so up to kAttnChunk tokens (one chunk) the result is that of the all-resident kernel.
 // =====================================================================================================
+constexpr int kAttnChunk = 192;   // 2 x 192 x 32 fp32 = 48 KB
 template <typename T>
-__global__ void attn_kernel(const T* __restrict__ qkv, T* __restrict__ out, int heads, int N) {
+__global__ void attn_kernel(const T* __restrict__ qkv, T* __restrict__ out, int heads, int N, int chunk) {
   pdl_trigger();
   pdl_wait();
   constexpr int D = 32;
-  extern __shared__ float kv[];   // k[N][D], v[N][D]
+  extern __shared__ float kv[];   // k[chunk][D], v[chunk][D]
   float* ks = kv;
-  float* vs = kv + (long)N * D;
+  float* vs = kv + (long)chunk * D;
   const int b = blockIdx.x / heads, h = blockIdx.x % heads;
   const int C3 = 3 * heads * D;
   const T* base = qkv + (long)b * N * C3;
   const int qo = h * D, ko = heads * D + h * D, vo = 2 * heads * D + h * D;
-  for (int i = threadIdx.x; i < N * D; i += blockDim.x) {
-    const int n = i / D, d = i % D;
-    ks[i] = to_f<T>(base[(long)n * C3 + ko + d]);
-    vs[i] = to_f<T>(base[(long)n * C3 + vo + d]);
-  }
-  __syncthreads();
   const float scale = rsqrtf((float)D);
-  for (int i = threadIdx.x; i < N; i += blockDim.x) {
+  for (int i0 = 0; i0 < N; i0 += blockDim.x) {      // block-uniform: every thread takes part in the chunk loads
+    const int i = i0 + threadIdx.x;
+    const bool live = i < N;
     float q[D], o[D];
 #pragma unroll
-    for (int d = 0; d < D; ++d) { q[d] = to_f<T>(base[(long)i * C3 + qo + d]) * scale; o[d] = 0.f; }
+    for (int d = 0; d < D; ++d) { q[d] = live ? to_f<T>(base[(long)i * C3 + qo + d]) * scale : 0.f; o[d] = 0.f; }
     float mx = -INFINITY, sum = 0.f;
-    for (int j = 0; j < N; ++j) {
-      float s = 0.f;
+    for (int j0 = 0; j0 < N; j0 += chunk) {
+      const int nj = min(chunk, N - j0);
+      __syncthreads();                               // the previous chunk has been consumed
+      for (int e = threadIdx.x; e < nj * D; e += blockDim.x) {
+        const int n = j0 + e / D, d = e % D;
+        ks[e] = to_f<T>(base[(long)n * C3 + ko + d]);
+        vs[e] = to_f<T>(base[(long)n * C3 + vo + d]);
+      }
+      __syncthreads();
+      if (live) {
+        for (int j = 0; j < nj; ++j) {
+          float s = 0.f;
 #pragma unroll
-      for (int d = 0; d < D; ++d) s = fmaf(q[d], ks[j * D + d], s);
-      const float nm = fmaxf(mx, s);
-      const float corr = __expf(mx - nm);
-      const float pj = __expf(s - nm);
-      sum = sum * corr + pj;
+          for (int d = 0; d < D; ++d) s = fmaf(q[d], ks[j * D + d], s);
+          const float nm = fmaxf(mx, s);
+          const float corr = __expf(mx - nm);
+          const float pj = __expf(s - nm);
+          sum = sum * corr + pj;
 #pragma unroll
-      for (int d = 0; d < D; ++d) o[d] = fmaf(pj, vs[j * D + d], o[d] * corr);
-      mx = nm;
+          for (int d = 0; d < D; ++d) o[d] = fmaf(pj, vs[j * D + d], o[d] * corr);
+          mx = nm;
+        }
+      }
     }
-    const float inv = 1.f / sum;
-    T* op = out + ((long)b * N + i) * (heads * D) + h * D;
+    if (live) {
+      const float inv = 1.f / sum;
+      T* op = out + ((long)b * N + i) * (heads * D) + h * D;
 #pragma unroll
-    for (int d = 0; d < D; ++d) op[d] = from_f<T>(o[d] * inv);
+      for (int d = 0; d < D; ++d) op[d] = from_f<T>(o[d] * inv);
+    }
   }
 }
 
+// bf16 above 64 tokens: the tcgen05 flash-attention kernel (attn_fused.cu); bf16 up to 64 tokens and fp32 at any N: attn_kernel
 int attn_core(const void* qkv, void* out, int B, int heads, int dh, int N, int act, cudaStream_t st) {
   DMN_REQUIRE(dh == 32, "attn_core: dim_head must be 32");
-  const size_t smem = (size_t)2 * N * 32 * sizeof(float);
-  DMN_REQUIRE(smem <= 48 * 1024, "attn_core: too many tokens for the bottleneck attention kernel");
+  if (act == ACT_BF16 && N > 64) return attn_flash(qkv, out, B, heads, N, st);
+  const int chunk = N < kAttnChunk ? N : kAttnChunk;
+  const size_t smem = (size_t)2 * chunk * 32 * sizeof(float);
   int threads = ((N + 31) / 32) * 32;
   if (threads > 256) threads = 256;
-  if (act == ACT_F32) DMN_CUDA_CHECK(launch_pdl(attn_kernel<float>, dim3(B * heads), dim3(threads), smem, st, (const float*)qkv, (float*)out, heads, N));
-  else DMN_CUDA_CHECK(launch_pdl(attn_kernel<bf16>, dim3(B * heads), dim3(threads), smem, st, (const bf16*)qkv, (bf16*)out, heads, N));
+  if (act == ACT_F32) DMN_CUDA_CHECK(launch_pdl(attn_kernel<float>, dim3(B * heads), dim3(threads), smem, st, (const float*)qkv, (float*)out, heads, N, chunk));
+  else DMN_CUDA_CHECK(launch_pdl(attn_kernel<bf16>, dim3(B * heads), dim3(threads), smem, st, (const bf16*)qkv, (bf16*)out, heads, N, chunk));
   count_launch();
   DMN_LAUNCH_CHECK("attn_core");
   return 0;

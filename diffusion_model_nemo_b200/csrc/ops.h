@@ -115,6 +115,8 @@ int launch_final_proj_ddpm(const FinalProjP& p, const float* x, const float* z, 
 
 int linattn_core(const void* qkv, void* out, int B, int heads, int dh, int N, int act, cudaStream_t s);
 int attn_core(const void* qkv, void* out, int B, int heads, int dh, int N, int act, cudaStream_t s);
+// bf16 tcgen05 flash-attention core (heads = 4, dim_head = 32, N > 64; attn_fused.cu); attn_core dispatches to it for ACT_BF16
+int attn_flash(const void* qkv, void* out, int B, int heads, int N, cudaStream_t s);
 // bf16 tensor-core LinearAttention core (heads = 4, dim_head = 32); linattn_core dispatches to it for ACT_BF16
 int linattn_core_bf16_mma(const void* qkv, void* out, int B, int N, cudaStream_t s);
 

@@ -1240,7 +1240,9 @@ int dmn_plan_op_info(const dmn_plan* p, int i, char* name_out, int name_cap, int
     name_out[name_cap - 1] = 0;
   }
   if (kind) *kind = o.kind;
-  if (engine) *engine = ((o.kind == OP_CONV && o.tc) || (o.kind == OP_INIT && p->init_tc) || o.kind == OP_ATTN_FUSED) ? 1 : 0;
+  // OP_ATTN in bf16 above 64 tokens runs attn_flash_kernel (tcgen05)
+  const bool flash = o.kind == OP_ATTN && p->act == ACT_BF16 && o.N > 64;
+  if (engine) *engine = ((o.kind == OP_CONV && o.tc) || (o.kind == OP_INIT && p->init_tc) || o.kind == OP_ATTN_FUSED || flash) ? 1 : 0;
   if (flops_per_sample) *flops_per_sample = fl;
   if (bytes_per_sample) *bytes_per_sample = by;
   return 0;

@@ -426,7 +426,10 @@ size_t dmn_conv_scratch_bytes(const dmn_conv_args* a);
 int dmn_conv_forward_cat(const dmn_conv_args* a, const float* x2, int32_t cin2, void* stream);
 
 /* LinearAttention core (mha.py:44-58, between to_qkv and to_out) / Attention core (mha.py:16-29).
- * qkv fp32 NCHW [batch, 3*heads*dim_head, H, W] -> out fp32 NCHW [batch, heads*dim_head, H, W]. */
+ * qkv fp32 NCHW [batch, 3*heads*dim_head, H, W] -> out fp32 NCHW [batch, heads*dim_head, H, W].
+ * Attention core kernels: act = DMN_ACT_BF16 with n_tokens > 64 runs attn_flash_kernel (tcgen05 flash attention; heads must be 4);
+ * DMN_ACT_BF16 with n_tokens <= 64 and DMN_ACT_F32 at any n_tokens run the CUDA-core attn_kernel (k / v streamed through shared
+ * memory in chunks of 192 tokens). */
 int dmn_linear_attention_core(const float* qkv, float* out, int batch, int heads, int dim_head, int n_tokens,
                               int act, void* scratch_dev, size_t scratch_bytes, void* stream);
 int dmn_attention_core(const float* qkv, float* out, int batch, int heads, int dim_head, int n_tokens,
